@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json metric: aligned reads/sec (error profile + T>C pileup) on synthetic PAR-CLIP reads.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path over one batch of synthetic coordinate-sorted reads: the profile kernel (which also
@@ -16,6 +16,9 @@ head partial of shard s).  One NCCL all-reduce of the profile count vector and o
 rank and step; the e2e leg adds one small all-gather of the boundary-cluster pieces.
 --impl reference times the CPU restatement of the Java loops (oracle/; plus the jar itself on a sample when `java` is on PATH) on the host cores, on
 the whole batch.
+--dump-outputs DIR writes what the last timed step of each leg handed back -- the profile arrays, the pileup counters and
+records -- as DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output: the workload is
+generated from fixed seeds and is the same in every run with the same arguments.
 """
 import argparse
 import json
@@ -310,6 +313,48 @@ def merge_boundary(res, next_head, n_own_reads):
     return m["open_cluster"], m["open_sites"]
 
 
+DUMP_ROWS = 1 << 17     # record rows per table and rank in --dump-outputs: two legs stay below 64 MB in all
+DUMP_SEED = 0x5EED0003
+
+
+def dump_outputs(out_dir, prefix, profile, pileup, max_rows):
+    """Writes one step's results as <out_dir>/<prefix><name>.npy in float64 (every field is an integer below 2^53, so
+    the values are exact): profile_<array> for the profile result, pileup_counters in the order of ps_pileup_counters,
+    pileup_<table>_<field> for the cluster / site records and the boundary clusters of the shard.  A table longer than
+    max_rows is sampled at row indices drawn with a fixed seed, written as pileup_<table>_rows.  What the step did not
+    produce writes no file: an empty table, a boundary cluster the shard does not have (a head partial exists only
+    behind a shard cut inside a cluster), its sites or coverage when it has none."""
+    from parasuite_b200 import abi
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, a):
+        a = np.asarray(a)
+        if a.dtype.kind in "iu" and a.size and int(np.abs(a).max()) >= 1 << 53:
+            raise ValueError(f"{name}: values beyond 2^53 have no exact float64")
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a.astype(np.float64))
+
+    for name, a in profile.items():
+        save("profile_" + name, a)
+    save("pileup_counters", [pileup["counters"][f] for f, _ in abi.ps_pileup_counters._fields_])
+    tables = {"clusters": pileup["clusters"], "sites": pileup["sites"]}
+    for one, sites, cov in (("open_cluster", "open_sites", "open_cov"), ("head_partial", "head_sites", "head_cov")):
+        if pileup.get(one) is not None:
+            tables[one], tables[sites] = np.atleast_1d(pileup[one]), pileup[sites]
+            if cov in pileup and len(pileup[cov][1]):
+                save(f"pileup_{cov}_pos0", [pileup[cov][0]])
+                save(f"pileup_{cov}", pileup[cov][1])
+    for table, rows in tables.items():
+        if not len(rows):
+            continue
+        idx = np.arange(len(rows))
+        if len(rows) > max_rows:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(len(rows), max_rows, replace=False))
+            save(f"pileup_{table}_rows", idx)
+        for f in rows.dtype.names:
+            if f != "reserved":
+                save(f"pileup_{table}_{f}", rows[f][idx])
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -317,10 +362,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--small", action="store_true", help="CI-sized workload (not a bench value)")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the host-buffer leg (default min(steps, 10))")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the host-buffer leg (default: --steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle comparison (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step of both legs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and not args.small:
         args.warmup = 3
     if args.impl == "reference":
@@ -374,10 +423,11 @@ def main():
     side = torch.cuda.Stream(device=dev) if world > 1 else None
     red = torch.cuda.Stream(device=dev) if world > 1 else None
 
-    def step_resident(keep=False):
+    def step_resident(keep=False, hold=False):
         # the whole hot path on a batch that is already in HBM: profile kernel (+ the tiny all-reduce), read-back of
         # the < 10 KB of counts, then the pileup kernels; cluster / site records stay in HBM behind the handle, their
-        # counters come back to the host
+        # counters come back to the host.  hold: the handle is left open in pile["held"], for a fetch of the records
+        # after the clock has stopped
         keys = None
         ctx.profile_begin(max_len, emit_t2c_masks=True)
         ctx.profile_batch_device(dbatch, stream.cuda_stream)
@@ -401,12 +451,18 @@ def main():
         carry_keys = (keys.data_ptr(), rank) if keys is not None else None
         # ps_pileup_submit_device: the call returns behind its launches, so the host takes back the profile (and does its
         # own bookkeeping) while the pileup kernels run; the wait for the pileup is the only one left at the end
-        with ctx.pileup_run(dbatch, first_running_id=1, carry_keys=carry_keys, stream=stream.cuda_stream, defer=True,
-                            masks=masks) as h:
+        h = ctx.pileup_run(dbatch, first_running_id=1, carry_keys=carry_keys, stream=stream.cuda_stream, defer=True,
+                           masks=masks)
+        try:
             res = ctx.profile_end()
             pile["counters"] = h.counters
             if keep:
                 pile["res_resident"] = h.fetch(boundary=True)
+        finally:
+            if hold:
+                pile["held"] = h
+            else:
+                h.close()
         return res
 
     # ---- warm-up ------------------------------------------------------------------------------------
@@ -422,12 +478,16 @@ def main():
     e0 = torch.cuda.Event(enable_timing=True)
     e1 = torch.cuda.Event(enable_timing=True)
     e0.record(stream)
-    for _ in range(args.steps):
-        res = step_resident()
+    for k in range(args.steps):
+        res = step_resident(hold=bool(args.dump_outputs) and k + 1 == args.steps)
         stage_ms.append(ctx.pileup_stage_ms())       # events of the step just finished (already synchronised)
     e1.record(stream)
     barrier()
     sampler.stop_flag = True
+    dumps = []
+    if args.dump_outputs:
+        with pile.pop("held") as h:
+            dumps.append(("resident_", res, h.fetch(boundary=True)))
     ms = e0.elapsed_time(e1)
     launches = ctx.kernel_launches() - launches0
     ktimes = ctx.kernel_times_ms()
@@ -444,7 +504,7 @@ def main():
 
     # ---- end-to-end leg: pinned HOST buffers through the C ABI, copies inside the timed region -------
     # one upload of the records serves both tools; every cluster and site record comes back to (pinned) host memory
-    e2e_steps = args.e2e_steps or min(args.steps, 10)
+    e2e_steps = args.e2e_steps or args.steps
     # the compact host form of the batch (ps_read_batch: one flag byte per read instead of the meta word, no cigar stream
     # -- every read of this workload is `36M` -- and qualities packed 6 bits each): 16 of 57 bytes per read less over the
     # host link, expanded on the device by the upload, inside the timed region
@@ -520,6 +580,10 @@ def main():
     e2e_value = total_reads * e2e_steps / (e2e_ms_max * 1e-3)
     pr = pile["res_e2e"]
     d2h = int(res_e2e["wide"].nbytes + 8 + pr["clusters"].nbytes + pr["sites"].nbytes)
+    if args.dump_outputs:
+        dumps.append(("e2e_", res_e2e, pr))
+        for prefix, prof, recs in dumps:
+            dump_outputs(args.dump_outputs, (f"rank{rank}_" if world > 1 else "") + prefix, prof, recs, DUMP_ROWS // world)
     h2d = pinned.h2d_bytes
 
     # ---- what the host link gives a plain pinned copy with every rank copying at once (the ceiling of the e2e leg) ----

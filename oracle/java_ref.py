@@ -2,14 +2,14 @@
 (Main.java:559-600) and `... clust ...` (Main.java:608-640) on a BAM + FASTA written by the test, and hand back the
 output files as text.  Test infrastructure only; nothing in the product imports this.
 
-The jar is looked for in $PARASUITE_JAR, then in /root/reference/bin/parasuite.jar (the build container; the GPU box has
-neither, and no JRE is in this image -- the tests that use this module skip with the reason spelled out)."""
+The jar is the one $PARASUITE_JAR names (a build of the reference's bin/parasuite.jar); without it, or without `java`
+on the PATH, the tests that use this module skip with the reason spelled out."""
 import os
 import shutil
 import subprocess
 import time
 
-JAR_CANDIDATES = (os.environ.get("PARASUITE_JAR", ""), "/root/reference/bin/parasuite.jar")
+JAR_CANDIDATES = (os.environ.get("PARASUITE_JAR", ""),)
 
 PROFILE_SUFFIXES = ("errorprofile", "errorprofile.vcf", "qualityPerMismatch", "indels", "indelprofile", "qualities")
 CLUST_FILES = {"pileup": "{out}", "ccr.fasta": "{out}.ccr.fasta", "ccr.tsv": "{out}.ccr.tsv", "report": "{out}.report",

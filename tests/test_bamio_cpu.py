@@ -146,18 +146,20 @@ def test_synthetic_batch_round_trip(tmp_path):
     assert np.array_equal(g.qual[:g.qual_bytes], batch.qual[:batch.qual_bytes])
 
 
-REF_FIXTURE = "/root/reference/examples/references/reference_chr1.fa"
+REF_FIXTURE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "config1", "reference_chr1.fa.gz")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_FIXTURE), reason="reference checkout not mounted (build container only)")
 def test_reference_fixture_fasta(tmp_path):
-    """The reference's own example genome (chr1, 483 300 bp, N runs, soft-masked): native pack == Python pack."""
-    raw = open(REF_FIXTURE, "rb").read().split(b"\n")
+    """The reference's own example genome (chr1, 483 300 bp, N runs, soft-masked; kept byte for byte, gzipped, in the
+    config-1 fixture): native pack == Python pack."""
+    import gzip
+    text = gzip.open(REF_FIXTURE, "rb").read()
+    raw = text.split(b"\n")
     name = raw[0][1:].split()[0].decode()
     seq = b"".join(raw[1:])
     fa = str(tmp_path / "chr1.fa")
     write_fasta(fa, [(name, seq)], line_width=len(raw[1]))
-    assert open(fa, "rb").read().rstrip(b"\n") == open(REF_FIXTURE, "rb").read().rstrip(b"\n")   # same bytes as the fixture
+    assert open(fa, "rb").read().rstrip(b"\n") == text.rstrip(b"\n")   # same bytes as the fixture
     pf = PackedFasta(fa)
     got, exp = pf.reference(), PackedReference.from_contigs([(name, seq)])
     assert got.lengths == [483300]
