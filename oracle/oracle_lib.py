@@ -67,6 +67,8 @@ def load() -> C.CDLL:
         lib.or_pileup_open.restype = C.c_int64
         lib.or_pileup_open.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
         lib.or_pileup_free.argtypes = [C.c_void_p]
+        lib.or_read_t2c_masks.restype = C.c_int
+        lib.or_read_t2c_masks.argtypes = [C.POINTER(abi.ps_reference), C.POINTER(abi.ps_read_batch), C.c_void_p]
         lib.or_pileup_head.restype = C.c_int64
         lib.or_pileup_head.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
         lib.or_pileup_boundary_cov.restype = C.c_int64
@@ -147,6 +149,19 @@ def pileup_count(ref, batch) -> int:
         return int(ctr.n_clusters)
     finally:
         lib.or_pileup_free(h)
+
+
+def read_t2c_masks(ref, batch) -> np.ndarray:
+    """uint64 per read: bit i = T>C at index i of the strand-oriented read (PileupClusters.java:637-661, no 51 limit,
+    bits 0..61); 0 for records the pileup loop skips or would die on."""
+    lib = load()
+    rs = ref.as_struct()
+    bs = batch.as_struct()
+    out = np.zeros(batch.n_reads, dtype=np.uint64)
+    st = lib.or_read_t2c_masks(C.byref(rs), C.byref(bs), out.ctypes.data)
+    if st != 0:
+        raise RuntimeError(f"oracle status {st}")
+    return out
 
 
 def pileup(ref, batch, first_running_id: int = 1, carry=None) -> dict:

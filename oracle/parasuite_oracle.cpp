@@ -292,6 +292,46 @@ void profile_range(const ps_reference* ref, const ps_read_batch* b, uint64_t lo,
   }
 }
 
+// calculateClusterInformation :585-613 up to the count loop: the read and reference bases of the alignment blocks
+// (SAMUtils.getAlignmentBlocks), strand-oriented.  Returns 0, or the PS_THROW code of the JVM's death on this record.
+int32_t cluster_read_bases(const ps_reference* ref, const ReadView& v, int64_t contig, int64_t start,
+                           std::vector<uint8_t>& readBases, std::vector<uint8_t>& readSequence,
+                           std::vector<uint8_t>& refSequenceForRead) {
+  read_ascii(v, readBases);
+  readSequence.clear();
+  refSequenceForRead.clear();
+  int64_t rd = 0;        // 0-based read cursor  (block.getReadStart()-1)
+  int64_t rf = start;    // 1-based reference cursor
+  for (uint32_t e = 0; e < v.ncig; ++e) {
+    uint32_t op = v.cigar[e] & 15;
+    int64_t n = v.cigar[e] >> 4;
+    if (op == 5 || op == 6) continue;                  // H, P
+    if (op == 4 || op == 1) rd += n;                   // S, I
+    else if (op == 2 || op == 3) rf += n;              // D, N
+    else if (op == 0 || op == 7 || op == 8) {          // M, =, X
+      if (rd + n > (int64_t)v.L) return PS_THROW_BLOCK_RANGE;
+      // FASTA fetch [rf, rf+n-1] on this contig
+      bool bad = (v.flags & PS_RF_REF_RANGE) != 0;
+      uint64_t g0 = 0;
+      if (!bad) {
+        g0 = ref->contig_off[contig] + (uint64_t)(rf - 1);
+        if (g0 + n > ref->contig_off[contig + 1]) bad = true;
+      }
+      if (bad) return PS_THROW_REF_RANGE;
+      readSequence.insert(readSequence.end(), readBases.begin() + rd, readBases.begin() + rd + n);
+      size_t at = refSequenceForRead.size();
+      refSequenceForRead.resize(at + n);
+      ref_ascii(ref, g0, n, refSequenceForRead, at);
+      rd += n; rf += n;
+    }
+  }
+  if (v.flags & PS_RF_REVERSE) {                       // :606-613
+    reverse_complement(readSequence);
+    reverse_complement(refSequenceForRead);
+  }
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -461,42 +501,11 @@ or_pileup_result* or_pileup_run(const ps_reference* ref, const ps_read_batch* b,
       numReadsPerCluster++;                                               // :488
     }
     // calculateClusterInformation :585-673
-    read_ascii(v, readBases);
-    readSequence.clear();
-    refSequenceForRead.clear();
-    {
-      int64_t rd = 0;        // 0-based read cursor  (block.getReadStart()-1)
-      int64_t rf = start;    // 1-based reference cursor
-      for (uint32_t e = 0; e < v.ncig; ++e) {   // SAMUtils.getAlignmentBlocks
-        uint32_t op = v.cigar[e] & 15;
-        int64_t n = v.cigar[e] >> 4;
-        if (op == 5 || op == 6) continue;                  // H, P
-        if (op == 4 || op == 1) rd += n;                   // S, I
-        else if (op == 2 || op == 3) rf += n;              // D, N
-        else if (op == 0 || op == 7 || op == 8) {          // M, =, X
-          if (rd + n > (int64_t)v.L) { R->fault.code = PS_THROW_BLOCK_RANGE; R->fault.read_ordinal = ord; return R; }
-          // FASTA fetch [rf, rf+n-1] on this contig
-          bool bad = (v.flags & PS_RF_REF_RANGE) != 0;
-          uint64_t g0 = 0;
-          if (!bad) {
-            g0 = ref->contig_off[contig] + (uint64_t)(rf - 1);
-            if (g0 + n > ref->contig_off[contig + 1]) bad = true;
-          }
-          if (bad) { R->fault.code = PS_THROW_REF_RANGE; R->fault.read_ordinal = ord; return R; }
-          readSequence.insert(readSequence.end(), readBases.begin() + rd, readBases.begin() + rd + n);
-          size_t at = refSequenceForRead.size();
-          refSequenceForRead.resize(at + n);
-          ref_ascii(ref, g0, n, refSequenceForRead, at);
-          rd += n; rf += n;
-        }
-      }
+    if (int32_t code = cluster_read_bases(ref, v, contig, start, readBases, readSequence, refSequenceForRead)) {
+      R->fault.code = code; R->fault.read_ordinal = ord; return R;
     }
     bool neg = (v.flags & PS_RF_REVERSE) != 0;
-    if (neg) {                                                            // :606-613
-      reverse_complement(readSequence);
-      reverse_complement(refSequenceForRead);
-      isReverse = 1;
-    }
+    if (neg) isReverse = 1;                                               // :606-613
     for (size_t i = 0; i < readSequence.size(); ++i) {                    // :637
       int32_t checkPosition = (int32_t)(neg ? end - (int64_t)i : start + (int64_t)i);
       if (array_pos(refSequenceForRead[i]) == 3 && array_pos(readSequence[i]) == 1) {  // :651
@@ -530,6 +539,33 @@ or_pileup_result* or_pileup_run(const ps_reference* ref, const ps_read_batch* b,
   R->counters.n_clusters = R->clusters.size();
   R->counters.n_sites = R->sites.size();
   return R;
+}
+
+// Per read, what the pileup loop's mutationMapInRead would hold (PileupClusters.java:637-661) without the 51-entry
+// array: bit i = T>C at index i of the strand-oriented read, for i < 62 (the layout of the profile kernel's mask words,
+// whose bits 62 and 63 are flags).  0 for a record the loop skips (unmapped, I/D with N) or would die on.
+int or_read_t2c_masks(const ps_reference* ref, const ps_read_batch* b, uint64_t* out) {
+  BatchCursor cur(b);
+  if (b->n_reads) cur.enter_tile(0);
+  ReadView v;
+  std::vector<uint8_t> readBases, readSequence, refSequenceForRead;
+  for (uint64_t r = 0; r < b->n_reads; ++r, cur.advance()) {
+    cur.get(v);
+    out[r] = 0;
+    if (v.flags & (PS_RF_UNMAPPED | PS_RF_POS_ZERO)) continue;          // :146; POS 0 kills the JVM
+    bool hasID = false, hasN = false;
+    for (uint32_t e = 0; e < v.ncig; ++e) {
+      uint32_t op = v.cigar[e] & 15;
+      hasID |= op == 1 || op == 2; hasN |= op == 3;
+    }
+    if (hasID && hasN) continue;                                          // :152-157
+    const int64_t contig = contig_of(ref, v.ref_start);
+    const int64_t start = (int64_t)(v.ref_start - ref->contig_off[contig]) + 1;
+    if (cluster_read_bases(ref, v, contig, start, readBases, readSequence, refSequenceForRead)) continue;
+    for (size_t i = 0; i < readSequence.size() && i < 62; ++i)
+      if (array_pos(refSequenceForRead[i]) == 3 && array_pos(readSequence[i]) == 1) out[r] |= 1ull << i;
+  }
+  return PS_OK;
 }
 
 int or_pileup_counters(const or_pileup_result* r, ps_pileup_counters* out) { *out = r->counters; return PS_OK; }

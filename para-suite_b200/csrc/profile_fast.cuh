@@ -775,7 +775,13 @@ cudaError_t launch_fast(ps_ctx* ctx, const ProfileParams& P, uint32_t n_wt, cuda
   const uint32_t need = (n_wt + FAST_WARPS - 1) / FAST_WARPS;
   if (grid > need) grid = need;
   // keep every block under FAST_MAX_READS_PER_BLOCK by splitting very large batches into several launches
-  const uint64_t per_launch = (uint64_t)grid * FAST_MAX_READS_PER_BLOCK / WT_READS;
+  uint64_t per_block = FAST_MAX_READS_PER_BLOCK;
+  if (const char* ev = getenv("PARASUITE_B200_FAST_READS_PER_BLOCK")) {   // tests: split batches of test size too
+    // whole tiles only, so that every launch starts on a tile of the exception table
+    const long v = atol(ev);
+    if (v >= PS_TILE_READS && v <= (long)FAST_MAX_READS_PER_BLOCK && v % PS_TILE_READS == 0) per_block = (uint64_t)v;
+  }
+  const uint64_t per_launch = (uint64_t)grid * per_block / WT_READS;
   for (uint64_t first = 0; first < n_wt; first += per_launch) {
     ProfileParams Q = P;
     const uint64_t cnt = std::min<uint64_t>(per_launch, n_wt - first);

@@ -204,3 +204,69 @@ def test_pileup_cpp_vs_python_random(oracle, seed, kinds):
     assert res["counters"]["skipped_due_indel"] == st.skipped_due_indel
     assert res["counters"]["num_reads_processed"] == st.num_reads_processed
     assert int(res["open_cluster"]["start"]) == st.open_cluster.start
+
+
+def full_range_records(seed, n, kinds, Lrange):
+    """Random records with quality bytes over the whole range 0..254: Java reads them as signed bytes (values 128..254
+    are negative, ErrorProfiling.java:301); 0xFF is left out, as the first byte it would mean "no qualities"."""
+    from parasuite_b200 import Record
+    rng = random.Random(seed)
+    contigs = random_genome(rng, n_contigs=2, length=700)
+    recs = random_records(rng, contigs, n, kinds=kinds, Lrange=Lrange, flags_special=0.05)
+    recs = [Record(r.flag, r.rname, r.pos, r.cigar, r.seq, bytes(rng.randint(0, 254) for _ in r.seq)) for r in recs]
+    assert any(q >= 128 for r in recs for q in r.qual)
+    return contigs, recs
+
+
+@pytest.mark.parametrize("infer_q", [False, True])
+@pytest.mark.parametrize("seed,kinds", [(21, ("M",)), (22, ("M", "clip", "indel", "wild"))])
+def test_profile_cpp_vs_python_full_range_qualities(oracle, seed, kinds, infer_q):
+    """The signed-byte rule, and the -q histogram (C++: by byte value 0..255, Python: by the signed Java byte)."""
+    contigs, recs = full_range_records(seed, 400, kinds, (1, 60))
+    g = po.Genome(dict(contigs))
+    ref = PackedReference.from_contigs(contigs)
+    max_len = 64
+    keep = []
+    for r in recs:
+        try:
+            po.profile(to_py([r]), g, max_len, infer_q)
+            keep.append(r)
+        except po.ReferenceWouldThrow:
+            with pytest.raises(oracle.OracleFault):
+                oracle.profile(ref, ReadBatch.from_records([r], ref), max_len, infer_q)
+    assert len(keep) > 300
+    st = po.profile(to_py(keep), g, max_len, infer_q)
+    got = oracle.profile(ref, ReadBatch.from_records(keep, ref), max_len, infer_q)
+    assert_profile_equal(got, py_profile_dict(st), f"seed {seed} -q {infer_q}")
+    assert (got["quality_per_mismatch"] < 0).any()         # the bytes above 127 do go in as negative numbers
+    if infer_q:
+        hist = np.zeros((max_len, 256), dtype=np.int64)
+        for i, d in enumerate(st.qual_hist):
+            for q, c in d.items():
+                hist[i, q & 0xFF] += c
+        assert np.array_equal(got["quality_hist"], hist)
+        assert hist[:, 128:].sum() > 0
+
+
+@pytest.mark.parametrize("seed,kinds", [(31, ("M",)), (32, ("M", "clip", "indel", "wild", "splice"))])
+def test_read_t2c_masks_cpp_vs_python(oracle, seed, kinds):
+    """oracle.read_t2c_masks (the per-read T>C masks the profile kernel hands the pileup) against the Python pileup's
+    per-read mutation map (calculateClusterInformation, PileupClusters.java:637-661) with room for 64 indices."""
+    contigs, recs = full_range_records(seed, 500, kinds, (1, 60))
+    g = po.Genome(dict(contigs))
+    ref = PackedReference.from_contigs(contigs)
+    got = oracle.read_t2c_masks(ref, ReadBatch.from_records(recs, ref))
+    n_set = 0
+    for k, (r, p) in enumerate(zip(recs, to_py(recs))):
+        exp = 0
+        has_id = any(op in "ID" for op, _ in p.cigar)
+        if not p.unmapped and p.pos > 0 and not (has_id and any(op == "N" for op, _ in p.cigar)):
+            mask = po.JArray(64)
+            try:
+                po._cluster_information(k, p, g, [False], po.JHashMap(), po.JHashMap(), mask, 0)
+                exp = sum(1 << i for i, m in enumerate(mask.a) if m)
+            except po.ReferenceWouldThrow:
+                pass
+        assert int(got[k]) == exp, (k, r, hex(int(got[k])), hex(exp))
+        n_set += exp != 0
+    assert n_set > 50
