@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define PS_ABI_VERSION 2
+#define PS_ABI_VERSION 3
 
 /* ---- status codes ------------------------------------------------------------------------ */
 #define PS_OK 0
@@ -33,7 +33,8 @@ extern "C" {
 #define PS_ERR_OOM (-4)
 #define PS_ERR_IO (-5)
 #define PS_ERR_FORMAT (-6)             /* malformed BAM / FASTA / .fai */
-#define PS_ERR_UNSORTED (-7)           /* header SO != coordinate (ErrorProfiling.java:124-132) */
+#define PS_ERR_UNSORTED (-7)           /* header SO != coordinate (ErrorProfiling.java:124-132), or records whose contigs go
+                                          backwards against the contig order (ps_reference_set_contig_order) */
 #define PS_ERR_REFERENCE_WOULD_THROW (-8) /* input on which the JVM dies with an uncaught exception */
 #define PS_ERR_STATE (-9)              /* call order violated (e.g. batch before begin) */
 #define PS_ERR_UNSUPPORTED (-10)
@@ -237,6 +238,23 @@ int ps_reference_upload(ps_ctx* ctx, const ps_reference* host_ref);
 int ps_reference_load_fasta(ps_ctx* ctx, const char* fasta_path); /* needs <fasta>.fai */
 /* adopt device-resident arrays (no copy; caller keeps them alive) */
 int ps_reference_adopt_device(ps_ctx* ctx, const ps_reference* dev_ref, const uint64_t* host_contig_off);
+/* The order the input's records take through the contigs (a coordinate-sorted file follows the @SQ order of its own
+ * header, which need not be the FASTA's).  The Java tools fetch bases by contig NAME (getSubsequenceAt(chr, ..),
+ * ErrorProfiling.java:169-172, PileupClusters.java:598-601) and close a cluster whenever the contig CHANGES
+ * (PileupClusters.java:175-176), so they follow any order; the pileup keeps a running maximum over the records and needs
+ * to know it.  order[k] = FASTA index of the k-th contig; contigs not listed come after the listed ones, in FASTA order.
+ * order == NULL or n == 0: FASTA order, which is also the state after every reference upload, load or adopt.
+ *   - A kept record on a contig that comes earlier in this order than the record before it: PS_ERR_UNSORTED.
+ *   - ps_pileup_opts.carry_contig and the `contig` of ps_pileup_max_key stay FASTA indices; the device keys
+ *     (ps_pileup_max_key_device, carry_keys_device) are (position in this order + 1) << 32 | end, so keys of two contexts
+ *     compare only when both have the same order.
+ *   - The profile does not depend on the order.  The file tools (ps_pileup_bam, ps_clust_bam and their ps_multi_* forms)
+ *     take the order of the file's header for the call, on every context they drive, and leave the caller's order in
+ *     force afterwards.
+ * Waits for all work already queued on the context's device before it changes the table.  PS_ERR_INVALID_ARG: an
+ * index twice, an index >= n_contigs, n > n_contigs; PS_ERR_STATE: no reference yet, or a ps_pileup_submit_device call
+ * not waited for. */
+int ps_reference_set_contig_order(ps_ctx* ctx, const uint32_t* order, uint32_t n);
 
 /* ---- batches -----------------------------------------------------------------------------------
  * Copy a host batch (pinned or pageable) into device memory owned by the context, asynchronously on the context's
@@ -300,12 +318,15 @@ int ps_pileup_batch_device(ps_ctx* ctx, const ps_read_batch* dev_batch, const ps
 int ps_pileup_submit_device(ps_ctx* ctx, const ps_read_batch* dev_batch, const ps_pileup_opts* opts, void* stream,
                             ps_pileup** out);
 int ps_pileup_wait(ps_pileup* h);
-/* Region sharding: max over the batch's kept records of (contig, alignment end).  The exclusive prefix-max of these
- * over the shards (one pair per shard: an all-gather of 8 scalars) is shard s's carry-in, so all shards run at once. */
+/* Region sharding: max over the batch's kept records of (contig, alignment end), contigs compared by their position in
+ * the context's contig order (ps_reference_set_contig_order); *contig is the FASTA index.  The exclusive prefix-max of
+ * these over the shards (one pair per shard: an all-gather of 8 scalars) is shard s's carry-in, so all shards run at
+ * once. */
 int ps_pileup_max_key(ps_ctx* ctx, const ps_read_batch* dev_batch, void* stream, uint32_t* valid, uint32_t* contig,
                       int32_t* end);
 /* The same maximum left on the device, asynchronously on `stream`: *dev_key points to one uint64 owned by the context,
- * (contig + 1) << 32 | end, 0 if the batch holds no kept record; valid until the next call of this function. */
+ * (position of the contig in the context's contig order + 1) << 32 | end, 0 if the batch holds no kept record; valid
+ * until the next call of this function. */
 int ps_pileup_max_key_device(ps_ctx* ctx, const ps_read_batch* dev_batch, void* stream, uint64_t** dev_key);
 int ps_pileup_counters_get(const ps_pileup* h, ps_pileup_counters* out);
 /* copy up to `max_clusters` closed clusters starting at `first` (and their sites) into caller arrays;
@@ -323,8 +344,8 @@ int ps_pileup_head_partial(ps_pileup* h, ps_cluster* cluster, ps_site* sites, ui
 int64_t ps_pileup_boundary_coverage(ps_pileup* h, int which, int32_t* first_pos, uint32_t* cov, uint64_t max);
 int ps_pileup_fault(const ps_pileup* h, ps_fault* out);
 void ps_pileup_close(ps_pileup* h);
-/* The file is taken in windows of records (PARASUITE_B200_WINDOW_READS, default 2^23): every window's carry-in is the
- * maximum (contig, end) over the windows before it, the reads at its head that continue the cluster left open by the
+/* The file is taken in windows of records (PARASUITE_B200_WINDOW_READS, default 2^23), in the contig order of the file's
+ * header (ps_reference_set_contig_order): every window's carry-in is the maximum (contig, end) over the windows before it, the reads at its head that continue the cluster left open by the
  * window before are folded into that cluster on the host (halo merge).  The handle holds the merged records of the whole
  * file on the host; no limit on the number of records. */
 int ps_pileup_bam(ps_ctx* ctx, const char* bam_path, const ps_pileup_opts* opts, ps_pileup** out);
@@ -387,8 +408,21 @@ const char* ps_fasta_contig_name(const ps_packed_fasta* f, uint32_t i);
 const char* ps_fasta_error(const ps_packed_fasta* f);
 void ps_fasta_free(ps_packed_fasta* f);
 /* Opens a coordinate-sorted BAM (PS_ERR_UNSORTED otherwise: ErrorProfiling.java:124-132).  Contigs are matched to the
- * FASTA by name; max_batch_reads = 0 picks a default; threads <= 0 uses the host cores. */
+ * FASTA by name, as getSubsequenceAt(chr, ..) does (ErrorProfiling.java:169-172); records on a contig the FASTA lacks
+ * carry PS_RF_REF_RANGE.  max_batch_reads = 0 picks a default; threads <= 0 uses the host cores.
+ * ps_bam_open answers PS_ERR_UNSUPPORTED when the header lists the FASTA's contigs in another order than the FASTA index:
+ * its records would not follow the FASTA order a context keys the pileup in by default.  ps_bam_open_ex with
+ * PS_BAM_ANY_CONTIG_ORDER takes any header order, as the Java tools do; the caller then keys the pileup in the header's
+ * order (ps_bam_contig_order -> ps_reference_set_contig_order).  The file tools (ps_profile_bam, ps_pileup_bam,
+ * ps_clust_bam, ps_error_bam and the ps_multi_* forms) open their input this way and do that themselves. */
+#define PS_BAM_ANY_CONTIG_ORDER 1u
 int ps_bam_open(ps_bam** out, const char* bam_path, const ps_packed_fasta* ref, uint64_t max_batch_reads, int threads);
+int ps_bam_open_ex(ps_bam** out, const char* bam_path, const ps_packed_fasta* ref, uint64_t max_batch_reads, int threads,
+                   uint32_t flags);
+/* The file's contig order for ps_reference_set_contig_order: FASTA indices of the @SQ lines in header order, contigs the
+ * FASTA lacks left out.  Returns its length; order == NULL asks for the length only (PS_ERR_INVALID_ARG if it exceeds
+ * max). */
+int64_t ps_bam_contig_order(const ps_bam* b, uint32_t* order, uint64_t max);
 /* 1: *batch filled (host pointers, valid until the third-next call); 0: end of file; < 0: status */
 int ps_bam_next(ps_bam* b, ps_read_batch* batch);
 const char* ps_bam_error(const ps_bam* b);

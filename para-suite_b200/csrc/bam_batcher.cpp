@@ -255,6 +255,7 @@ struct ps_bam {
   bool sorted = false;
   std::vector<std::string> ref_names;
   std::vector<int64_t> ref_to_contig;   // BAM refID -> FASTA contig (-1: absent from the FASTA)
+  std::vector<uint32_t> contig_order;   // FASTA contigs in @SQ order, those the FASTA lacks left out (ps_bam_contig_order)
   const ps_packed_fasta* fa = nullptr;
   uint64_t max_batch = 0;
   int threads = 1;
@@ -468,7 +469,7 @@ static int bam_fill(ps_bam* B, size_t want) {
   return PS_OK;
 }
 
-static int bam_header(ps_bam* B) {
+static int bam_header(ps_bam* B, bool any_contig_order) {
   int st = bam_fill(B, 12);
   if (st) return st;
   auto avail = [&] { return B->buf.size() - B->head; };
@@ -503,18 +504,26 @@ static int bam_header(ps_bam* B) {
     o += 8 + (size_t)l_name;
   }
   B->head = o;
+  // contigs are matched by name (getSubsequenceAt(chr, ..), ErrorProfiling.java:169-172, PileupClusters.java:598-601):
+  // the header may list them in any order; the records follow the header's order, which the pileup keys take over
+  // (ps_bam_contig_order).  A caller that has not asked for that (PS_BAM_ANY_CONTIG_ORDER) keys the pileup in FASTA
+  // order and is told at once that the file does not follow it.
   std::unordered_map<std::string, int64_t> idx;
   for (size_t c = 0; c < B->fa->names.size(); ++c) idx.emplace(B->fa->names[c], (int64_t)c);
+  std::vector<char> listed(B->fa->names.size(), 0);
   int64_t last = -1;
   for (auto& nm : B->ref_names) {
     auto it = idx.find(nm);
     const int64_t c = it == idx.end() ? -1 : it->second;
     B->ref_to_contig.push_back(c);
-    if (c >= 0) {
-      if (c < last)
+    if (c >= 0 && !listed[(size_t)c]) {
+      if (!any_contig_order && c < last)
         return bam_fail(B, PS_ERR_UNSUPPORTED, "the BAM header lists contigs in a different order than the FASTA index: "
-                                               "coordinate order of the reads would not follow the packed reference");
+                                               "open it with PS_BAM_ANY_CONTIG_ORDER and key the pileup in the header's "
+                                               "order (ps_bam_contig_order, ps_reference_set_contig_order)");
       last = c;
+      listed[(size_t)c] = 1;
+      B->contig_order.push_back((uint32_t)c);
     }
   }
   B->header_done = true;
@@ -538,6 +547,11 @@ const char* ps_fasta_error(const ps_packed_fasta* f) { return f ? f->err.c_str()
 void ps_fasta_free(ps_packed_fasta* f) { delete f; }
 
 int ps_bam_open(ps_bam** out, const char* bam_path, const ps_packed_fasta* ref, uint64_t max_batch_reads, int threads) {
+  return ps_bam_open_ex(out, bam_path, ref, max_batch_reads, threads, 0);
+}
+
+int ps_bam_open_ex(ps_bam** out, const char* bam_path, const ps_packed_fasta* ref, uint64_t max_batch_reads, int threads,
+                   uint32_t flags) {
   if (!out || !bam_path || !ref) return PS_ERR_INVALID_ARG;
   ps_bam* B = new ps_bam();
   *out = B;      // returned even on failure so the caller can read ps_bam_error
@@ -554,7 +568,7 @@ int ps_bam_open(ps_bam** out, const char* bam_path, const ps_packed_fasta* ref, 
   if (B->mf.n >= 2 && B->mf.p[0] == 0x1f && B->mf.p[1] == 0x8b) st = bam_scan_blocks(B);      // BGZF: a BAM
   else { B->sam_text = true; st = sam_header(B); }                                             // anything else: SAM text
   if (st) return st;
-  st = bam_header(B);
+  st = bam_header(B, (flags & PS_BAM_ANY_CONTIG_ORDER) != 0);
   if (st) return st;
   // SamReader header check of both tools (ErrorProfiling.java:124-132, PileupClusters.java:85-92)
   if (!B->sorted) return bam_fail(B, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
@@ -562,6 +576,15 @@ int ps_bam_open(ps_bam** out, const char* bam_path, const ps_packed_fasta* ref, 
 }
 
 const char* ps_bam_error(const ps_bam* b) { return b ? b->err.c_str() : "no object"; }
+
+int64_t ps_bam_contig_order(const ps_bam* b, uint32_t* order, uint64_t max) {
+  if (!b || !b->header_done) return PS_ERR_INVALID_ARG;
+  const uint64_t n = b->contig_order.size();
+  if (!order) return (int64_t)n;
+  if (n > max) return PS_ERR_INVALID_ARG;
+  if (n) memcpy(order, b->contig_order.data(), n * 4);
+  return (int64_t)n;
+}
 
 void ps_bam_close(ps_bam* b) {
   if (!b) return;
@@ -884,7 +907,8 @@ int ps_reference_load_fasta(ps_ctx* ctx, const char* fasta_path) {
 
 int open_for_ctx(ps_ctx* ctx, const char* bam_path, uint64_t max_batch, ps_bam** B) {
   if (!ctx->fasta) return set_error(ctx, PS_ERR_STATE, "ps_reference_load_fasta must come first (contig names are needed)");
-  int st = ps_bam_open(B, bam_path, ctx->fasta, max_batch, 0);
+  // the file tools follow the header's contig order (the pileup loop sets it on its contexts: tool_loops.cpp)
+  int st = ps_bam_open_ex(B, bam_path, ctx->fasta, max_batch, 0, PS_BAM_ANY_CONTIG_ORDER);
   if (st != PS_OK) {
     st = set_error(ctx, st, *B ? (*B)->err : "cannot open BAM");
     ps_bam_close(*B);

@@ -185,6 +185,57 @@ void timer_end(ps_ctx* ctx, cudaStream_t st) {
   ctx->ev_count++;
 }
 
+// ---- reference: contig table and contig order -----------------------------------------------------
+// Contig order of the pileup keys: by_rank[k] = FASTA index of the k-th contig (a permutation of 0 .. n_contigs-1).
+// The table is read by kernels queued on any stream of the device: everything queued before is waited for, so none of
+// them sees a half-written table.
+static int upload_contig_order(ps_ctx* ctx, std::vector<uint32_t>&& by_rank) {
+  const uint32_t n = (uint32_t)by_rank.size();
+  std::vector<uint32_t> rank(n);
+  for (uint32_t k = 0; k < n; ++k) rank[by_rank[k]] = k;
+  PS_CUDA(ctx, cudaDeviceSynchronize());
+  PS_CUDA(ctx, ctx->ref_rank.reserve((size_t)n * 4));
+  PS_CUDA(ctx, cudaMemcpy(ctx->ref_rank.p, rank.data(), (size_t)n * 4, cudaMemcpyHostToDevice));
+  ctx->ref.contig_rank = (const uint32_t*)ctx->ref_rank.p;
+  ctx->contig_rank.swap(rank);
+  ctx->contig_by_rank.swap(by_rank);
+  return PS_OK;
+}
+
+static int set_contigs(ps_ctx* ctx, const uint64_t* host_contig_off, uint32_t n_contigs, uint64_t n_bases) {
+  if (!host_contig_off || n_contigs == 0) return set_error(ctx, PS_ERR_INVALID_ARG, "reference without contigs");
+  if (n_bases >= (1ull << 32)) return set_error(ctx, PS_ERR_UNSUPPORTED, "reference >= 2^32 bases");
+  ctx->contig_off.assign(host_contig_off, host_contig_off + n_contigs + 1);
+  if (ctx->contig_off.back() != n_bases) return set_error(ctx, PS_ERR_INVALID_ARG, "contig table does not sum to n_bases");
+  PS_CUDA(ctx, ctx->ref_contig.reserve((n_contigs + 1) * 8));
+  PS_CUDA(ctx, cudaMemcpy(ctx->ref_contig.p, host_contig_off, (n_contigs + 1) * 8, cudaMemcpyHostToDevice));
+  ctx->ref.contig_off = (const uint64_t*)ctx->ref_contig.p;
+  ctx->ref.n_contigs = n_contigs;
+  ctx->ref.n_bases = n_bases;
+  std::vector<uint32_t> fasta_order(n_contigs);
+  for (uint32_t c = 0; c < n_contigs; ++c) fasta_order[c] = c;
+  return upload_contig_order(ctx, std::move(fasta_order));
+}
+
+int set_contig_order(ps_ctx* ctx, const uint32_t* order, uint32_t n) {
+  cudaSetDevice(ctx->device);
+  const uint32_t nc = ctx->ref.n_contigs;
+  if (n > nc) return set_error(ctx, PS_ERR_INVALID_ARG, "contig order lists more contigs than the reference has");
+  if (n && !order) return set_error(ctx, PS_ERR_INVALID_ARG, "NULL contig order");
+  std::vector<uint32_t> by_rank;
+  by_rank.reserve(nc);
+  std::vector<char> listed(nc, 0);
+  for (uint32_t k = 0; k < n; ++k) {
+    if (order[k] >= nc) return set_error(ctx, PS_ERR_INVALID_ARG, "contig order names a contig the reference lacks");
+    if (listed[order[k]]) return set_error(ctx, PS_ERR_INVALID_ARG, "contig order lists a contig twice");
+    listed[order[k]] = 1;
+    by_rank.push_back(order[k]);
+  }
+  for (uint32_t c = 0; c < nc; ++c)      // contigs not listed follow, in FASTA order
+    if (!listed[c]) by_rank.push_back(c);
+  return upload_contig_order(ctx, std::move(by_rank));
+}
+
 extern "C" {
 
 int ps_abi_version(void) { return PS_ABI_VERSION; }
@@ -266,7 +317,7 @@ void ps_destroy(ps_ctx* ctx) {
   if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
   if (ctx->stream_rb) cudaStreamDestroy(ctx->stream_rb);
   if (ctx->prof_done_ev) cudaEventDestroy(ctx->prof_done_ev);
-  ctx->ref_seq2.release(); ctx->ref_inv.release(); ctx->ref_contig.release();
+  ctx->ref_seq2.release(); ctx->ref_inv.release(); ctx->ref_contig.release(); ctx->ref_rank.release();
   ctx->acc.release(); ctx->fault.release(); ctx->deferred.release(); ctx->t2c_mask.release();
   ctx->rg_okmap.release(); ctx->rg_off.release(); ctx->rg_bases.release(); ctx->rg_qual.release(); ctx->rg_op0.release();
   for (auto& s : ctx->staged) {
@@ -281,19 +332,6 @@ void ps_destroy(ps_ctx* ctx) {
 const char* ps_last_error(const ps_ctx* ctx) { return ctx ? ctx->err.c_str() : "no context"; }
 
 // ---- reference ---------------------------------------------------------------------------------------
-static int set_contigs(ps_ctx* ctx, const uint64_t* host_contig_off, uint32_t n_contigs, uint64_t n_bases) {
-  if (!host_contig_off || n_contigs == 0) return set_error(ctx, PS_ERR_INVALID_ARG, "reference without contigs");
-  if (n_bases >= (1ull << 32)) return set_error(ctx, PS_ERR_UNSUPPORTED, "reference >= 2^32 bases");
-  ctx->contig_off.assign(host_contig_off, host_contig_off + n_contigs + 1);
-  if (ctx->contig_off.back() != n_bases) return set_error(ctx, PS_ERR_INVALID_ARG, "contig table does not sum to n_bases");
-  PS_CUDA(ctx, ctx->ref_contig.reserve((n_contigs + 1) * 8));
-  PS_CUDA(ctx, cudaMemcpy(ctx->ref_contig.p, host_contig_off, (n_contigs + 1) * 8, cudaMemcpyHostToDevice));
-  ctx->ref.contig_off = (const uint64_t*)ctx->ref_contig.p;
-  ctx->ref.n_contigs = n_contigs;
-  ctx->ref.n_bases = n_bases;
-  return PS_OK;
-}
-
 int ps_reference_upload(ps_ctx* ctx, const ps_reference* r) {
   if (!ctx || !r || !r->seq2 || !r->inv) return set_error(ctx, PS_ERR_INVALID_ARG, "bad reference");
   cudaSetDevice(ctx->device);
@@ -308,6 +346,14 @@ int ps_reference_upload(ps_ctx* ctx, const ps_reference* r) {
   ctx->ref.inv = (const uint32_t*)ctx->ref_inv.p;
   ctx->ref_loaded = true;
   return PS_OK;
+}
+
+int ps_reference_set_contig_order(ps_ctx* ctx, const uint32_t* order, uint32_t n) {
+  if (!ctx) return PS_ERR_INVALID_ARG;
+  if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
+  if (ctx->pl_pending) return set_error(ctx, PS_ERR_STATE, "a submitted pileup call of this context has not been waited for");
+  cudaSetDevice(ctx->device);
+  return set_contig_order(ctx, order, n);
 }
 
 int ps_reference_adopt_device(ps_ctx* ctx, const ps_reference* r, const uint64_t* host_contig_off) {

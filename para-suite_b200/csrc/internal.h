@@ -17,6 +17,7 @@ struct DeviceRef {
   const uint32_t* seq2 = nullptr;
   const uint32_t* inv = nullptr;
   const uint64_t* contig_off = nullptr;  // device copy
+  const uint32_t* contig_rank = nullptr; // [n_contigs] position of each contig in the input's sort order (pileup keys)
   uint64_t n_bases = 0;
   uint32_t n_contigs = 0;
 };
@@ -96,8 +97,11 @@ struct ps_ctx {
   std::string err;
   // reference
   DeviceRef ref;
-  DevBuf ref_seq2, ref_inv, ref_contig;
+  DevBuf ref_seq2, ref_inv, ref_contig, ref_rank;
   std::vector<uint64_t> contig_off;  // host copy
+  // sort order of the input's contigs (ps_reference_set_contig_order): rank[c] = position of FASTA contig c in it,
+  // by_rank = the inverse; identity after every reference upload.  ref.contig_rank is the device copy of `rank`.
+  std::vector<uint32_t> contig_rank, contig_by_rank;
   bool ref_loaded = false;
   ps_packed_fasta* fasta = nullptr;   // set by ps_reference_load_fasta: contig names for BAM headers
   bool fasta_shared = false;          // the packed FASTA belongs to a ps_multi (several contexts share one)
@@ -164,6 +168,21 @@ ps_pileup* pileup_host_handle(ps_ctx* ctx, std::vector<ps_cluster>&& clusters, s
 void pileup_set_fault(ps_pileup* h, const ps_fault& f);
 // wrap the int64 accumulator vector of a profile run into the caller's arrays (ctx.cu; Java int wrap-around, Q8)
 void profile_fill_result(const ProfileLayout& l, const int64_t* acc, ps_profile_result* out);
+
+// sets the pileup key order of a context with a reference (ctx.cu; ps_reference_set_contig_order without the state checks)
+int set_contig_order(ps_ctx* ctx, const uint32_t* order, uint32_t n);
+
+// ---- pileup keys: (rank of the contig + 1) << 32 | alignment end, 0 = no kept record ------------------------------
+// The running maximum of these keys is Java's (tempClusterChr, tempClusterEnd): a contig change is a larger key only when
+// contigs come in the order `rank` describes (ps_reference_set_contig_order).  rank: ps_ctx::contig_rank.
+inline uint64_t pileup_key(const std::vector<uint32_t>& rank, uint32_t contig, int32_t end) {
+  return ((uint64_t)(rank[contig] + 1) << 32) | (uint32_t)end;
+}
+// inverse of pileup_key (key != 0); by_rank: ps_ctx::contig_by_rank
+inline void pileup_key_decode(const std::vector<uint32_t>& by_rank, uint64_t key, uint32_t* contig, int32_t* end) {
+  *contig = by_rank[(uint32_t)(key >> 32) - 1];
+  *end = (int32_t)(uint32_t)key;
+}
 
 // ---- kernel launchers (defined in the .cu files) ----------------------------------------------------
 // t2c_mask (optional): n_reads words; *mask_written tells whether the batch took the fast kernel, which fills them

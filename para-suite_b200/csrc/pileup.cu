@@ -103,10 +103,12 @@ struct PlRead {              // what the pileup needs from one read
 struct ContigCache {         // contig bounds of the last read looked up by this thread
   uint64_t lo = 1, hi = 0;
   uint32_t idx = 0;
+  uint32_t rank = 0;         // position of contig idx in the input's sort order (the pileup keys)
 };
 struct ContigCache32 {       // same in 32 bits (the global coordinate space is < 2^32 bases: set_contigs in ctx.cu)
   uint32_t lo = 0, hi = 0;     // empty: hi - lo == 0, no offset passes the one-compare range test
   uint32_t idx = 0;
+  uint32_t rank = 0;
 };
 __device__ __forceinline__ bool contig_lookup(const DeviceRef& ref, uint32_t g0, ContigCache32& c) {
   if (g0 - c.lo < c.hi - c.lo) return true;       // lo <= g0 < hi in one unsigned compare
@@ -114,6 +116,7 @@ __device__ __forceinline__ bool contig_lookup(const DeviceRef& ref, uint32_t g0,
   c.idx = contig_of(ref, g0);
   c.lo = (uint32_t)__ldg(ref.contig_off + c.idx);
   c.hi = (uint32_t)__ldg(ref.contig_off + c.idx + 1);
+  c.rank = __ldg(ref.contig_rank + c.idx);
   return true;
 }
 __device__ __forceinline__ bool contig_lookup(const DeviceRef& ref, uint64_t g0, ContigCache& c) {
@@ -122,6 +125,7 @@ __device__ __forceinline__ bool contig_lookup(const DeviceRef& ref, uint64_t g0,
   c.idx = contig_of(ref, g0);
   c.lo = __ldg(ref.contig_off + c.idx);
   c.hi = __ldg(ref.contig_off + c.idx + 1);
+  c.rank = __ldg(ref.contig_rank + c.idx);
   return true;
 }
 
@@ -149,7 +153,9 @@ struct FlagParams {
   uint32_t scan_in_expand;        // no pl_flag_scan_kernel: the expand kernel sums the tile counts itself
 };
 
-// (contig+1) << 32 | end of a kept record, 0 otherwise (PileupClusters.java:146-158)
+// (rank of the contig + 1) << 32 | end of a kept record, 0 otherwise (PileupClusters.java:146-158).  The rank is the
+// contig's position in the input's sort order (DeviceRef::contig_rank), so that the running maximum of the keys follows
+// the records across a contig change whatever order the file lists its contigs in.
 template <bool COUNT = true>
 __device__ __forceinline__ unsigned long long pl_key(const FlagParams& P, uint64_t r, uint32_t meta, const uint32_t* cig,
                                                      uint32_t g0, ContigCache& cc, int32_t& start) {
@@ -172,7 +178,7 @@ __device__ __forceinline__ unsigned long long pl_key(const FlagParams& P, uint64
   if (!contig_lookup(P.ref, g0, cc)) return 0;    // likewise
   start = (int32_t)((uint64_t)g0 - cc.lo) + 1;
   const int32_t end = start + (int32_t)R - 1;
-  return ((unsigned long long)(cc.idx + 1) << 32) | (uint32_t)end;
+  return ((unsigned long long)(cc.rank + 1) << 32) | (uint32_t)end;
 }
 
 // same for a record with exactly one cigar op `cg` (a lone I or D next to no N is kept: :152-157 needs both)
@@ -187,11 +193,11 @@ __device__ __forceinline__ unsigned long long pl_key1(const FlagParams& P, uint3
   const uint32_t R = op_consumes_ref(cg & 15u) ? cg >> 4 : 0u;
   const int32_t s = (int32_t)(g0 - (uint32_t)cc.lo) + 1;      // offsets inside a contig fit 32 bits (the whole reference does)
   start = ok ? s : 0;
-  const unsigned long long key = ((unsigned long long)(cc.idx + 1) << 32) | (uint32_t)(s + (int32_t)R - 1);
+  const unsigned long long key = ((unsigned long long)(cc.rank + 1) << 32) | (uint32_t)(s + (int32_t)R - 1);
   return ok ? key : 0ull;
 }
 
-// max over the records of a batch of (contig, end): what a following shard needs as carry-in (region sharding: the
+// max over the records of a batch of (contig rank, end): what a following shard needs as carry-in (region sharding: the
 // exclusive prefix-max of these keys over the shards replaces Java's (tempClusterChr, tempClusterEnd) at the cut)
 __global__ void __launch_bounds__(PL_THREADS) pl_maxkey_kernel(const __grid_constant__ FlagParams P, unsigned long long* out) {
   ContigCache cc;
@@ -314,7 +320,7 @@ __global__ void __launch_bounds__(FLAG_THREADS, FLAG_BLOCKS_PER_SM) pl_flag_kern
           const uint32_t R = op_consumes_ref(cigs[j] & 15u) ? cigs[j] >> 4 : 0u;
           const int32_t st = (int32_t)(starts[j] - cc.lo) + 1;
           start[g + j] = ok ? st : 0;
-          key[g + j] = ok ? (((unsigned long long)(cc.idx + 1) << 32) | (uint32_t)(st + (int32_t)R - 1)) : 0ull;
+          key[g + j] = ok ? (((unsigned long long)(cc.rank + 1) << 32) | (uint32_t)(st + (int32_t)R - 1)) : 0ull;
         }
       } else {
 #pragma unroll
@@ -329,7 +335,7 @@ __global__ void __launch_bounds__(FLAG_THREADS, FLAG_BLOCKS_PER_SM) pl_flag_kern
     if (!in_range) start[0] = 0;
   }
 
-  // ---- look-back #1: running max of (contig, end) -----------------------------------------------------------
+  // ---- look-back #1: running max of (contig rank, end) -----------------------------------------------------------
   unsigned long long tmax = 0;
 #pragma unroll
   for (int j = 0; j < ITEMS; ++j) tmax = key[j] > tmax ? key[j] : tmax;
@@ -377,7 +383,8 @@ __global__ void __launch_bounds__(FLAG_THREADS, FLAG_BLOCKS_PER_SM) pl_flag_kern
     const uint32_t pc = (uint32_t)(E >> 32), mc = (uint32_t)(my >> 32);
     // tempClusterEnd = 0, tempClusterChr = "" (:118-120) | contig changed | (clusterEnd - start) < 5; predicated, no branches
     const bool f = kept & ((E == 0) | (pc != mc) | (((int64_t)(int32_t)(uint32_t)E - (int64_t)start[j]) < 5));
-    unsorted |= kept & (pc > mc);                       // contig order went backwards: not coordinate sorted
+    unsorted |= kept & (pc > mc);                       // contig order went backwards: not coordinate sorted (in the
+                                                        // order the keys follow: ps_reference_set_contig_order)
     E = my > E ? my : E;                                // my == 0 leaves E alone
     fl |= (uint32_t)f << j;
     nfl += (uint32_t)f;
@@ -1587,8 +1594,7 @@ static int pileup_launch(ps_ctx* ctx, ps_pileup* H) {
   if (err != cudaSuccess) return cuda_fail(ctx, err, "pileup scratch");
 
   unsigned long long carry_key = 0;
-  if (opts && opts->carry_valid)
-    carry_key = ((unsigned long long)(opts->carry_contig + 1) << 32) | (uint32_t)opts->carry_cluster_end;
+  if (opts && opts->carry_valid) carry_key = pileup_key(ctx->contig_rank, opts->carry_contig, opts->carry_cluster_end);
 
   const uint64_t cap_cl = std::min<uint64_t>(ctx->pl_cap_cl, n + 2), cap_sites = ctx->pl_cap_ev;
   H->cap_cl = cap_cl; H->cap_sites = cap_sites;
@@ -1728,6 +1734,8 @@ static int pileup_finish(ps_ctx* ctx, ps_pileup* H) {
 static int run_pileup(ps_ctx* ctx, const DeviceBatch& b, const ps_pileup_opts* opts, cudaStream_t st, ps_pileup** out,
                       bool wait = true) {
   if (ctx->pl_pending) return set_error(ctx, PS_ERR_STATE, "a submitted pileup call of this context has not been waited for");
+  if (opts && opts->carry_valid && opts->carry_contig >= ctx->ref.n_contigs)
+    return set_error(ctx, PS_ERR_INVALID_ARG, "carry_contig is not a contig of the reference");
   // A batch that sits in a staging slot of this context (ps_batch_upload / ps_pileup_batch): the pileup never reads
   // qualities, so it may start as soon as the other streams of the records have arrived (event staged_core), while the
   // quality bytes (more than half of the upload) are still on their way.  Asked to run on the context's own stream --
@@ -1942,7 +1950,7 @@ int ps_pileup_max_key(ps_ctx* ctx, const ps_read_batch* dev_batch, void* stream,
   PS_CUDA(ctx, cudaMemcpyAsync(hk ? hk : &tmp, d_key, 8, cudaMemcpyDeviceToHost, st));
   PS_CUDA(ctx, cudaStreamSynchronize(st));
   const unsigned long long k = hk ? *hk : tmp;
-  if (k) { *valid = 1; *contig = (uint32_t)(k >> 32) - 1; *end = (int32_t)(uint32_t)k; }
+  if (k) { *valid = 1; pileup_key_decode(ctx->contig_by_rank, k, contig, end); }
   return PS_OK;
 }
 

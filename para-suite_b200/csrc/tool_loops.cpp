@@ -49,8 +49,9 @@ static int multi_fail(ps_multi* m, int st, const std::string& msg) {
 
 namespace {
 
-// max over the kept records of a host batch of (contig + 1) << 32 | alignment end (what pl_maxkey_kernel computes)
-uint64_t host_max_key(const ps_read_batch& b, const std::vector<uint64_t>& contig_off) {
+// max over the kept records of a host batch of their pileup keys (what pl_maxkey_kernel computes); rank: the context's
+// contig order (ps_ctx::contig_rank)
+uint64_t host_max_key(const ps_read_batch& b, const std::vector<uint64_t>& contig_off, const std::vector<uint32_t>& rank) {
   uint64_t best = 0, coff = (!b.uniform_ncigar && b.tile_cigar_off) ? b.tile_cigar_off[0] : 0;
   size_t ci = 0;
   for (uint64_t r = 0; r < b.n_reads; ++r) {
@@ -71,8 +72,7 @@ uint64_t host_max_key(const ps_read_batch& b, const std::vector<uint64_t>& conti
     if (!(g >= contig_off[ci] && g < contig_off[ci + 1]))
       ci = (size_t)(std::upper_bound(contig_off.begin(), contig_off.end(), g) - contig_off.begin()) - 1;
     const uint64_t end = g - contig_off[ci] + R;          // start + R - 1 with start = g - off + 1
-    const uint64_t key = ((uint64_t)(ci + 1) << 32) | (uint32_t)end;
-    best = std::max(best, key);
+    best = std::max(best, pileup_key(rank, (uint32_t)ci, (int32_t)(uint32_t)end));
   }
   return best;
 }
@@ -149,18 +149,16 @@ struct InFlight {
 
 int sync_fail(ps_multi* m, ps_ctx* c, int st) { return multi_fail(m, st, ps_last_error(c)); }
 
-// The windowed pileup over a file.  counters / open: the run's totals and the cluster left open at the end.
-int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts, uint64_t window_reads, const WindowSink& sink,
-                   ps_pileup_counters* counters, OpenCluster* open_out, ps_fault* fault) {
-  if (m->ctx.empty()) return multi_fail(m, PS_ERR_STATE, "no context");
+// The windowed pileup over an open file, every context keyed in the file's contig order.  counters / open: the run's
+// totals and the cluster left open at the end.
+int pileup_windows_run(ps_multi* m, ps_bam* B, const ps_pileup_opts* opts, const WindowSink& sink, ps_pileup_counters* counters,
+                       OpenCluster* open_out, ps_fault* fault) {
   ps_ctx* c0 = m->ctx[0];
-  ps_bam* B = nullptr;
-  int st = open_for_ctx(c0, bam_path, window_reads, &B);
-  if (st) return sync_fail(m, c0, st);
+  int st = PS_OK;
   const std::vector<uint64_t>& contig_off = c0->contig_off;
   const uint32_t first_id = opts ? opts->first_running_id : 1u;
   uint64_t carry_key = 0;
-  if (opts && opts->carry_valid) carry_key = ((uint64_t)(opts->carry_contig + 1) << 32) | (uint32_t)opts->carry_cluster_end;
+  if (opts && opts->carry_valid) carry_key = pileup_key(c0->contig_rank, opts->carry_contig, opts->carry_cluster_end);
   memset(counters, 0, sizeof *counters);
   OpenCluster open;
   uint64_t created = 0, offset = 0, window = 0;
@@ -290,7 +288,7 @@ int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts
     // when the window completes (they are not known yet: those windows may still be running)
     ps_pileup_opts o{};
     o.first_running_id = first_id;
-    if (carry_key) { o.carry_valid = 1; o.carry_contig = (uint32_t)(carry_key >> 32) - 1; o.carry_cluster_end = (int32_t)(uint32_t)carry_key; }
+    if (carry_key) { o.carry_valid = 1; pileup_key_decode(c0->contig_by_rank, carry_key, &o.carry_contig, &o.carry_cluster_end); }
     f.ctx = c; f.host = hb; f.offset = offset;
     // upload without the quality bytes (the pileup never reads them: more than half of the records' bytes)
     StagedBatch* sb = nullptr;
@@ -305,7 +303,7 @@ int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts
     }
     if (st != PS_OK) { sync_fail(m, c, st); break; }
     f.live = true;
-    carry_key = std::max(carry_key, host_max_key(hb, contig_off));
+    carry_key = std::max(carry_key, host_max_key(hb, contig_off, c0->contig_rank));
     offset += hb.n_reads;
   }
   for (int i = 0; i < 2 && st == PS_OK; ++i) {
@@ -318,11 +316,42 @@ int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts
   }
   for (InFlight& f : fl)
     if (f.live) { ps_pileup_close(f.h); f.live = false; }
-  ps_bam_close(B);
   if (st != PS_OK) return st;
   counters->has_open_cluster = open.have ? 1 : 0;
   if (open_out) *open_out = std::move(open);
   return PS_OK;
+}
+
+// The windowed pileup over a file.  The records follow the contig order of the file's header, which need not be the
+// FASTA's: every context takes that order for the call (the window carry and the boundary keys follow it) and has the
+// caller's own order back afterwards, whatever the outcome.
+int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts, uint64_t window_reads, const WindowSink& sink,
+                   ps_pileup_counters* counters, OpenCluster* open_out, ps_fault* fault) {
+  if (m->ctx.empty()) return multi_fail(m, PS_ERR_STATE, "no context");
+  for (ps_ctx* c : m->ctx)
+    if (c->pl_pending) return multi_fail(m, PS_ERR_STATE, "a submitted pileup call of a context has not been waited for");
+  ps_ctx* c0 = m->ctx[0];
+  if (opts && opts->carry_valid && opts->carry_contig >= c0->ref.n_contigs)
+    return multi_fail(m, PS_ERR_INVALID_ARG, "carry_contig is not a contig of the reference");
+  ps_bam* B = nullptr;
+  int st = open_for_ctx(c0, bam_path, window_reads, &B);
+  if (st) return sync_fail(m, c0, st);
+  std::vector<uint32_t> file_order((size_t)std::max<int64_t>(ps_bam_contig_order(B, nullptr, 0), 0));
+  ps_bam_contig_order(B, file_order.data(), file_order.size());
+  std::vector<std::vector<uint32_t>> saved;
+  for (ps_ctx* c : m->ctx) {
+    if (!c->ref_loaded) { st = multi_fail(m, PS_ERR_STATE, "no reference loaded"); break; }
+    saved.push_back(c->contig_by_rank);
+    st = set_contig_order(c, file_order.data(), (uint32_t)file_order.size());
+    if (st != PS_OK) { sync_fail(m, c, st); break; }
+  }
+  if (st == PS_OK) st = pileup_windows_run(m, B, opts, sink, counters, open_out, fault);
+  ps_bam_close(B);
+  for (size_t i = 0; i < saved.size(); ++i) {
+    const int rc = set_contig_order(m->ctx[i], saved[i].data(), (uint32_t)saved[i].size());
+    if (rc != PS_OK && st == PS_OK) st = sync_fail(m, m->ctx[i], rc);
+  }
+  return st;
 }
 
 }  // namespace

@@ -15,7 +15,7 @@ CSRC_DIR = os.path.join(ROOT_DIR, "csrc")
 REPO_DIR = os.path.dirname(ROOT_DIR)
 INCLUDE_DIR = os.path.join(REPO_DIR, "include")
 
-PS_ABI_VERSION = 2
+PS_ABI_VERSION = 3
 PS_OK = 0
 PS_ERR_INVALID_ARG = -1
 PS_ERR_NO_DEVICE = -2
@@ -48,6 +48,8 @@ PS_RF_QUAL_MISSING = 0x10
 PS_RF_HAS_INVALID = 0x20
 PS_RF_REF_RANGE = 0x40
 PS_RF_CIGAR_OVERFLOW = 0x80
+
+PS_BAM_ANY_CONTIG_ORDER = 0x1
 
 PS_PC_NAMES = ["num_reads_processed", "unmapped", "duplicates", "start_zero", "indel_read", "skipped_reads",
                "longer_indels", "total_bases_checked"]
@@ -149,6 +151,7 @@ EXPORTS = {
     "ps_reference_upload": (C.c_int, [VP, C.POINTER(ps_reference)]),
     "ps_reference_load_fasta": (C.c_int, [VP, C.c_char_p]),
     "ps_reference_adopt_device": (C.c_int, [VP, C.POINTER(ps_reference), VP]),
+    "ps_reference_set_contig_order": (C.c_int, [VP, VP, C.c_uint32]),
     "ps_batch_upload": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_read_batch)]),
     "ps_profile_acc_len": (C.c_size_t, [C.c_uint32, C.c_uint32]),
     "ps_clust_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint32, C.POINTER(ps_pileup_counters),
@@ -208,8 +211,10 @@ EXPORTS = {
     "ps_fasta_error": (C.c_char_p, [VP]),
     "ps_fasta_free": (None, [VP]),
     "ps_bam_open": (C.c_int, [C.POINTER(VP), C.c_char_p, VP, C.c_uint64, C.c_int]),
+    "ps_bam_open_ex": (C.c_int, [C.POINTER(VP), C.c_char_p, VP, C.c_uint64, C.c_int, C.c_uint32]),
     "ps_bam_next": (C.c_int, [VP, C.POINTER(ps_read_batch)]),
     "ps_bam_error": (C.c_char_p, [VP]),
+    "ps_bam_contig_order": (C.c_int64, [VP, VP, C.c_uint64]),
     "ps_bam_close": (None, [VP]),
     "ps_flush_create": (C.c_int, [C.POINTER(VP), C.c_uint32, C.c_uint32, C.POINTER(C.c_char_p)]),
     "ps_flush_add_snp": (C.c_int, [VP, C.c_char_p, C.c_int32, C.c_char_p, C.c_char_p]),

@@ -233,18 +233,33 @@ class PackedFasta:
 
 
 class BamBatcher:
-    """ps_bam: iterate a coordinate-sorted BAM as SoA batches (numpy copies of the native slabs)."""
+    """ps_bam: iterate a coordinate-sorted BAM as SoA batches (numpy copies of the native slabs).
+    any_contig_order=True: take a header that lists the contigs in another order than the FASTA (contig_order gives it,
+    Context.set_contig_order keys the pileup in it); otherwise such a file raises PS_ERR_UNSUPPORTED."""
 
-    def __init__(self, path: str, fasta: PackedFasta, max_batch_reads: int = 0, threads: int = 0):
+    def __init__(self, path: str, fasta: PackedFasta, max_batch_reads: int = 0, threads: int = 0,
+                 any_contig_order: bool = False):
         self.lib = abi.load_library()
         self._fasta = fasta
         h = C.c_void_p()
-        st = self.lib.ps_bam_open(C.byref(h), path.encode(), fasta.h, max_batch_reads, threads)
+        flags = abi.PS_BAM_ANY_CONTIG_ORDER if any_contig_order else 0
+        st = self.lib.ps_bam_open_ex(C.byref(h), path.encode(), fasta.h, max_batch_reads, threads, flags)
         self.h = h
         if st != abi.PS_OK:
             msg = self.lib.ps_bam_error(h).decode() if h else self.lib.ps_strerror(st).decode()
             self.close()
             raise abi.PsError(st, msg)
+
+    @property
+    def contig_order(self) -> List[int]:
+        """FASTA indices of the header's @SQ contigs in header order, contigs the FASTA lacks left out: the order the
+        records of a coordinate-sorted file follow (Context.set_contig_order)."""
+        n = int(self.lib.ps_bam_contig_order(self.h, None, 0))
+        if n < 0:
+            raise abi.PsError(n, self.lib.ps_strerror(n).decode())
+        a = np.zeros(max(n, 1), dtype=np.uint32)
+        self.lib.ps_bam_contig_order(self.h, a.ctypes.data, n)
+        return [int(x) for x in a[:n]]
 
     def __iter__(self):
         return self

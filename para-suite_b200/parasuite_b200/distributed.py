@@ -21,12 +21,24 @@ from .sharding import merge_pileup_shards
 Key = Optional[Tuple[int, int]]
 
 
-def exclusive_prefix_max(keys: Sequence[Key]) -> list:
-    """keys[r] = (contig, end) maximum of shard r or None -> carry-in of every shard (None for shard 0 / empty prefix)."""
+def _rank_key(order: Optional[Sequence[int]]) -> Callable:
+    """(contig, end) -> what orders it: (position of the contig in `order`, end).  Contigs `order` does not list come
+    after the listed ones in FASTA order (Context.set_contig_order); order=None: FASTA order."""
+    if order is None:
+        return lambda k: k
+    rank = {int(c): i for i, c in enumerate(order)}
+    return lambda k: (rank.get(k[0], len(rank) + k[0]), k[1])
+
+
+def exclusive_prefix_max(keys: Sequence[Key], order: Optional[Sequence[int]] = None) -> list:
+    """keys[r] = (contig, end) maximum of shard r or None -> carry-in of every shard (None for shard 0 / empty prefix).
+    Contigs are FASTA indices, compared by their position in `order` (the records' contig order, e.g.
+    BamBatcher.contig_order; None: FASTA order)."""
+    rk = _rank_key(order)
     out, best = [], None
     for k in keys:
         out.append(best)
-        if k is not None and (best is None or k > best):
+        if k is not None and (best is None or rk(k) > rk(best)):
             best = k
     return out
 
@@ -34,10 +46,11 @@ def exclusive_prefix_max(keys: Sequence[Key]) -> list:
 class _KeyGather:
     """In-flight all-gather of one (valid, contig, end) triple per rank."""
 
-    def __init__(self, local: Key, group=None, device=None):
+    def __init__(self, local: Key, group=None, device=None, order=None):
         import torch
         import torch.distributed as dist
         self.group = group
+        self.order = order
         world = dist.get_world_size(group)
         self.t = torch.tensor([1 if local is not None else 0, local[0] if local else 0, local[1] if local else 0],
                               dtype=torch.int64, device=device)
@@ -51,12 +64,13 @@ class _KeyGather:
 
     def carry(self) -> Key:
         import torch.distributed as dist
-        return exclusive_prefix_max(self.keys())[dist.get_rank(self.group)]
+        return exclusive_prefix_max(self.keys(), self.order)[dist.get_rank(self.group)]
 
 
-def all_gather_keys_async(local: Key, group=None, device=None) -> _KeyGather:
-    """Start the exchange; call .carry() when the carry-in is needed (other work can be queued in between)."""
-    return _KeyGather(local, group, device)
+def all_gather_keys_async(local: Key, group=None, device=None, order=None) -> _KeyGather:
+    """Start the exchange; call .carry() when the carry-in is needed (other work can be queued in between).  order: the
+    records' contig order (exclusive_prefix_max)."""
+    return _KeyGather(local, group, device, order)
 
 
 def all_gather_keys(local: Key, group=None, device=None) -> list:
@@ -74,19 +88,22 @@ def gather_keys_device(key_tensor, group=None):
     return out
 
 
-def sharded_pileup_carry(local_key: Key, group=None, device=None) -> Key:
-    """The carry-in of this rank's region: one all-gather of 3 scalars per rank + a prefix-max on the host."""
+def sharded_pileup_carry(local_key: Key, group=None, device=None, order=None) -> Key:
+    """The carry-in of this rank's region: one all-gather of 3 scalars per rank + a prefix-max on the host (contigs
+    compared in the records' contig order `order`, FASTA order when None)."""
     import torch.distributed as dist
     keys = all_gather_keys(local_key, group, device)
-    return exclusive_prefix_max(keys)[dist.get_rank(group)]
+    return exclusive_prefix_max(keys, order)[dist.get_rank(group)]
 
 
 def sharded_pileup(local_batch, max_key_fn: Callable, pileup_fn: Callable, read_offset: int, group=None, device=None,
-                   gather_to: Optional[int] = 0):
+                   gather_to: Optional[int] = 0, order=None):
     """Region-sharded T>C pileup.  max_key_fn(batch) -> Key; pileup_fn(batch, carry) -> result dict (Context.pileup).
+    order: the records' contig order when it is not the FASTA's (BamBatcher.contig_order; the contexts behind
+    max_key_fn / pileup_fn need the same order, Context.set_contig_order).
     Returns (local result, merged whole-stream result on rank `gather_to` else None)."""
     import torch.distributed as dist
-    carry = sharded_pileup_carry(max_key_fn(local_batch), group, device)
+    carry = sharded_pileup_carry(max_key_fn(local_batch), group, device, order)
     res = pileup_fn(local_batch, carry)
     merged = None
     if gather_to is not None:

@@ -176,6 +176,14 @@ class Context:
         _check(self.lib, self.h, self.lib.ps_reference_load_fasta(self.h, path.encode()))
         self.ref = None
 
+    def set_contig_order(self, order=None):
+        """The contig order the records of the following pileup calls take: order[k] = FASTA index of the k-th contig
+        (BamBatcher.contig_order gives a file's), contigs not listed after the listed ones in FASTA order; None or []:
+        FASTA order, the state after every reference upload.  Records whose contig goes backwards against it raise
+        PS_ERR_UNSORTED.  Carry tuples and pileup_max_key keep FASTA indices; the device keys follow the order."""
+        a = np.ascontiguousarray(order if order is not None else [], dtype=np.uint32)
+        _check(self.lib, self.h, self.lib.ps_reference_set_contig_order(self.h, a.ctypes.data if a.size else None, a.size))
+
     # ---- whole-tool loops from files ------------------------------------------------------------------
     def profile_bam(self, bam_path: str, max_read_length: int, infer_qualities: bool = False) -> dict:
         """The record loop of the `error` tool (ErrorProfiling.java:104-409) on a coordinate-sorted BAM."""
@@ -370,15 +378,18 @@ class Context:
         return res
 
     def pileup_max_key(self, dbatch, stream: int = 0):
-        """(contig, end) maximum over the kept records of a device-resident batch, or None (region sharding carry)."""
+        """(contig, end) maximum over the kept records of a device-resident batch, or None (region sharding carry).  Contigs
+        compare by their position in the context's contig order (set_contig_order); the contig returned is a FASTA index."""
         v, c, e = C.c_uint32(), C.c_uint32(), C.c_int32()
         _check(self.lib, self.h, self.lib.ps_pileup_max_key(self.h, C.byref(dbatch.struct), stream or None, C.byref(v),
                                                              C.byref(c), C.byref(e)))
         return (int(c.value), int(e.value)) if v.value else None
 
     def pileup_max_key_tensor(self, dbatch, stream: int = 0):
-        """The same maximum as a 1-element int64 CUDA tensor aliasing library memory ((contig + 1) << 32 | end, 0 = none),
-        computed asynchronously on `stream`: feed it to an all-gather and hand the gathered keys to pileup_run(carry_keys=)."""
+        """The same maximum as a 1-element int64 CUDA tensor aliasing library memory, computed asynchronously on `stream`:
+        (position of the contig in the context's contig order + 1) << 32 | end, 0 = none -- the position is the FASTA index
+        unless set_contig_order changed the order, and keys of two contexts compare only under the same order.  Feed it
+        to an all-gather and hand the gathered keys to pileup_run(carry_keys=)."""
         import torch
         p = C.c_void_p()
         _check(self.lib, self.h, self.lib.ps_pileup_max_key_device(self.h, C.byref(dbatch.struct), stream or None, C.byref(p)))
