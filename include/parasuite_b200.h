@@ -6,6 +6,8 @@
  *   error profile : src/src/utils/errorprofile/ErrorProfiling.java:146-409   (tool `error`, `map --refine`)
  *   T>C pileup    : src/src/utils/pileupclusters/PileupClusters.java:137-500 (tool `clust`)
  *
+ * and adds one tool the Java toolkit does not have: the per-position T>C conversion and coverage track (tool `track`).
+ *
  * The reference has no FFI of its own (pure Java).  This header is the boundary a thin JNI shim
  * binds (jni/parasuite_jni.c, INTEGRATION.md): plain C types, caller-owned output arrays, negative
  * PS_ERR_* status codes, no exception or CUDA error ever crosses it.  There is NO CPU fallback:
@@ -23,7 +25,7 @@
 extern "C" {
 #endif
 
-#define PS_ABI_VERSION 3
+#define PS_ABI_VERSION 4
 
 /* ---- status codes ------------------------------------------------------------------------ */
 #define PS_OK 0
@@ -358,6 +360,61 @@ int ps_clust_bam(ps_ctx* ctx, const char* bam_path, const char* out_path, const 
  * output files next to the BAM (ps_profile_write_files).  counters_out: [PS_PC_COUNT] or NULL. */
 int ps_error_bam(ps_ctx* ctx, const char* bam_path, const ps_profile_opts* opts, int32_t* counters_out, ps_fault* fault_out);
 
+/* ---- T>C conversion and coverage track (tool `track`; no Java counterpart) ----------------------------------------
+ * Per position and strand: the coverage and the T>C events of the records the pileup keeps (ps_pileup_batch: unmapped
+ * records and those whose CIGAR holds (I or D) and N are skipped, duplicates counted; the same faults with the same
+ * ordinals, except that there is no 51-position limit -- PS_THROW_MASK51 is never raised).  Positions follow the CIGAR on
+ * the genome: M, =, X consume read and reference, D and N the reference only (no coverage), I and S the read only, H and
+ * P nothing.  BAM flag 0x10 puts a read on the minus track.  Every aligned base adds 1 to its strand's coverage, whatever
+ * the bases; a T>C event is ref T / read C on the plus strand and ref A / read G on the minus strand (T>C on the read's
+ * own strand), counted where the reference base is ACGTacgt and the read base is not listed in `exc`.
+ * A kept record whose start is smaller than the previous kept record's (contig order included:
+ * ps_reference_set_contig_order) gives PS_ERR_UNSORTED. */
+typedef struct ps_track_counters {
+  uint64_t num_reads_processed;
+  uint64_t unmapped;
+  uint64_t skipped_due_indel;
+  uint64_t reads_counted;        /* records on the track */
+  uint64_t aligned_bases[2];     /* [strand]: 0 plus, 1 minus; = sum over runs of (end0 - start0) * cov */
+  uint64_t t2c_events[2];        /* = sum of t2c over the strand's sites */
+  uint64_t n_runs[2];
+  uint64_t n_sites;
+  uint64_t fast_path_reads;      /* reads whose T>C bits were found bit-parallel (uniform length <= 64, one M/=/X op) */
+} ps_track_counters;
+typedef struct ps_track_run {    /* one bedGraph row: maximal run of equal non-zero coverage */
+  uint32_t contig;               /* FASTA index */
+  uint32_t start0;               /* 0-based, half-open */
+  uint32_t end0;
+  uint32_t cov;
+} ps_track_run;
+typedef struct ps_track_site {   /* one (position, strand) with at least one T>C event */
+  uint32_t contig;               /* FASTA index */
+  int32_t pos;                   /* 1-based */
+  uint32_t strand;               /* 0 plus, 1 minus */
+  uint32_t t2c;
+  uint32_t cov;                  /* coverage of that strand at pos */
+} ps_track_site;
+typedef struct ps_track ps_track;  /* opaque result handle (host memory) */
+/* One batch is the whole input.  Runs come by strand, contigs in the order the records visit them, then by position;
+ * sites likewise, plus before minus at one position.  The handle is returned with PS_OK and with a fault
+ * (PS_ERR_REFERENCE_WOULD_THROW, PS_ERR_UNSUPPORTED: ps_track_fault). */
+int ps_track_batch(ps_ctx* ctx, const ps_read_batch* host_batch, ps_track** out);
+int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* dev_batch, void* stream, ps_track** out);
+int ps_track_counters_get(const ps_track* h, ps_track_counters* out);
+/* copy up to `max` runs of `strand` (0 plus, 1 minus) / sites starting at `first`; returns the number copied */
+int64_t ps_track_runs(const ps_track* h, int strand, uint64_t first, ps_track_run* runs, uint64_t max);
+int64_t ps_track_sites(const ps_track* h, uint64_t first, ps_track_site* sites, uint64_t max);
+int ps_track_fault(const ps_track* h, ps_fault* out);
+void ps_track_close(ps_track* h);
+/* The tool from files: <out_prefix>.plus.bedGraph and <out_prefix>.minus.bedGraph (chrom, start0, end0, coverage; no
+ * header; one row per maximal run of equal non-zero coverage) and <out_prefix>.t2c.tsv (header
+ * chrom/pos/strand/t2c/coverage, one row per (position, strand) with t2c >= 1, pos 1-based).  Contigs come in the order the
+ * records visit them (the header's), rows by position.  The file is taken in windows of PARASUITE_B200_WINDOW_READS
+ * records; the files do not depend on the window size nor on the number of devices.  The reference must have been loaded
+ * with ps_reference_load_fasta / ps_multi_load_fasta (contig names).  counters_out / fault_out may be NULL. */
+int ps_track_bam(ps_ctx* ctx, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
+                 ps_fault* fault_out);
+
 /* ---- `comb` tool (host only): transcript hits lifted to genomic coordinates, merged with the genomic hits ---------------
  * Replaces CombineGenomeTranscript.combine / printReadsToBamFile (utils/postprocessing/CombineGenomeTranscript.java:36-666;
  * Main.java:438-486 `comb -g <genomic.bam> -t <transcript.bam> -o <combined.bam>`): the step that writes the `aMbNcM`
@@ -394,6 +451,9 @@ int ps_multi_pileup_bam(ps_multi* m, const char* bam_path, const ps_pileup_opts*
 int ps_multi_error_bam(ps_multi* m, const char* bam_path, const ps_profile_opts* opts, int32_t* counters_out, ps_fault* fault_out);
 int ps_multi_clust_bam(ps_multi* m, const char* bam_path, const char* out_path, const char* snp_vcf,
                        uint32_t min_read_coverage, ps_pileup_counters* counters_out, ps_fault* fault_out);
+/* windows round-robin over the devices; the files are byte-identical to ps_track_bam's */
+int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
+                       ps_fault* fault_out);
 
 /* ---- host batcher (usable without a GPU) --------------------------------------------------------
  * What htsjdk does for the two loops, as a library: FASTA(+.fai) -> packed reference; BGZF/BAM -> SoA batches in
@@ -490,7 +550,8 @@ void ps_clust_writer_close(ps_clust_writer* w);
 uint64_t ps_kernel_launches(const ps_ctx* ctx);
 /* device time (ms, CUDA events on the launching stream) of the last ps_*_batch_device call's dominant kernel */
 float ps_last_kernel_ms(const ps_ctx* ctx);
-/* device times (ms) of the dominant kernel of every ps_*_batch[_device] call since the last reset, in call
+/* device times (ms) of the dominant kernel of every ps_*_batch[_device] call since the last reset (a track call records
+ * five stages: key pass and scans, segment placement, accumulation, coverage scans, selection), in call
  * order (at most 512 are kept); returns how many were written.  reset(enabled=0) switches the event pairs off. */
 int ps_kernel_times(ps_ctx* ctx, float* ms, int max);
 void ps_kernel_times_reset(ps_ctx* ctx, int enabled);

@@ -325,6 +325,7 @@ void ps_destroy(ps_ctx* ctx) {
     s.tbo.release(); s.tqo.release(); s.tco.release(); s.teo.release(); s.exc.release(); s.flags8.release(); s.qual6.release(); s.start16.release(); s.tile_start.release();
   }
   for (auto& b : ctx->pl_scratch) b.release();
+  for (auto& b : ctx->tr_scratch) b.release();
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }

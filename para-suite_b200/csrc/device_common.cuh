@@ -34,6 +34,35 @@ __device__ __forceinline__ uint32_t contig_of(const DeviceRef& ref, uint64_t g) 
   return lo;
 }
 
+struct ContigCache {         // contig bounds of the last read looked up by this thread
+  uint64_t lo = 1, hi = 0;
+  uint32_t idx = 0;
+  uint32_t rank = 0;         // position of contig idx in the input's sort order (the pileup keys)
+};
+struct ContigCache32 {       // same in 32 bits (the global coordinate space is < 2^32 bases: set_contigs in ctx.cu)
+  uint32_t lo = 0, hi = 0;     // empty: hi - lo == 0, no offset passes the one-compare range test
+  uint32_t idx = 0;
+  uint32_t rank = 0;
+};
+__device__ __forceinline__ bool contig_lookup(const DeviceRef& ref, uint32_t g0, ContigCache32& c) {
+  if (g0 - c.lo < c.hi - c.lo) return true;       // lo <= g0 < hi in one unsigned compare
+  if (g0 >= ref.n_bases) return false;
+  c.idx = contig_of(ref, g0);
+  c.lo = (uint32_t)__ldg(ref.contig_off + c.idx);
+  c.hi = (uint32_t)__ldg(ref.contig_off + c.idx + 1);
+  c.rank = __ldg(ref.contig_rank + c.idx);
+  return true;
+}
+__device__ __forceinline__ bool contig_lookup(const DeviceRef& ref, uint64_t g0, ContigCache& c) {
+  if (g0 >= c.lo && g0 < c.hi) return true;
+  if (g0 >= ref.n_bases) return false;
+  c.idx = contig_of(ref, g0);
+  c.lo = __ldg(ref.contig_off + c.idx);
+  c.hi = __ldg(ref.contig_off + c.idx + 1);
+  c.rank = __ldg(ref.contig_rank + c.idx);
+  return true;
+}
+
 // per-read stream offsets (bytes of packed bases, bytes of qualities, cigar elements)
 struct ReadOffsets {
   uint64_t base, qual, cigar;

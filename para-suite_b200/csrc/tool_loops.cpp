@@ -14,6 +14,12 @@
 //                   summed dense coverage of the boundary cluster).
 //   clust files   : the merged closed clusters of every window go, with the window's records, through the flush
 //                   arithmetic and the native writers (flush.cpp, clust_writer.cpp).
+//   track         : windows round-robin over the contexts, each on a thread of its own while the next window decodes.
+//                   A window reports final runs and sites for the positions after the maximum end of the windows before
+//                   it and before its own last kept start; its head (up to that maximum end) and its tail (from its last
+//                   kept start on) come back as dense arrays, added on the host into one pending region -- in a sorted
+//                   file no later record reaches a position before the last kept start, so the region is bounded by the
+//                   longest reference span of a record.
 // No compute happens on the host: boundaries, masks, counts and sites all come from the kernels.
 #include <algorithm>
 #include <cstdio>
@@ -27,6 +33,7 @@
 #include <vector>
 
 #include "internal.h"
+#include "track.h"
 
 extern "C" int open_for_ctx(ps_ctx* ctx, const char* bam_path, uint64_t max_batch, ps_bam** B);
 int stage_batch(ps_ctx* ctx, const ps_read_batch* hb, bool with_qual, StagedBatch** out);
@@ -322,17 +329,11 @@ int pileup_windows_run(ps_multi* m, ps_bam* B, const ps_pileup_opts* opts, const
   return PS_OK;
 }
 
-// The windowed pileup over a file.  The records follow the contig order of the file's header, which need not be the
-// FASTA's: every context takes that order for the call (the window carry and the boundary keys follow it) and has the
-// caller's own order back afterwards, whatever the outcome.
-int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts, uint64_t window_reads, const WindowSink& sink,
-                   ps_pileup_counters* counters, OpenCluster* open_out, ps_fault* fault) {
-  if (m->ctx.empty()) return multi_fail(m, PS_ERR_STATE, "no context");
-  for (ps_ctx* c : m->ctx)
-    if (c->pl_pending) return multi_fail(m, PS_ERR_STATE, "a submitted pileup call of a context has not been waited for");
+// Opens a file for a windowed tool.  The records follow the contig order of the file's header, which need not be the
+// FASTA's: every context takes that order for the call (window carries and keys follow it) and has the caller's own order
+// back afterwards, whatever the outcome.
+int with_file_order(ps_multi* m, const char* bam_path, uint64_t window_reads, const std::function<int(ps_bam*)>& run) {
   ps_ctx* c0 = m->ctx[0];
-  if (opts && opts->carry_valid && opts->carry_contig >= c0->ref.n_contigs)
-    return multi_fail(m, PS_ERR_INVALID_ARG, "carry_contig is not a contig of the reference");
   ps_bam* B = nullptr;
   int st = open_for_ctx(c0, bam_path, window_reads, &B);
   if (st) return sync_fail(m, c0, st);
@@ -345,13 +346,254 @@ int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts
     st = set_contig_order(c, file_order.data(), (uint32_t)file_order.size());
     if (st != PS_OK) { sync_fail(m, c, st); break; }
   }
-  if (st == PS_OK) st = pileup_windows_run(m, B, opts, sink, counters, open_out, fault);
+  if (st == PS_OK) st = run(B);
   ps_bam_close(B);
   for (size_t i = 0; i < saved.size(); ++i) {
     const int rc = set_contig_order(m->ctx[i], saved[i].data(), (uint32_t)saved[i].size());
     if (rc != PS_OK && st == PS_OK) st = sync_fail(m, m->ctx[i], rc);
   }
   return st;
+}
+
+// The windowed pileup over a file.
+int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts, uint64_t window_reads, const WindowSink& sink,
+                   ps_pileup_counters* counters, OpenCluster* open_out, ps_fault* fault) {
+  if (m->ctx.empty()) return multi_fail(m, PS_ERR_STATE, "no context");
+  for (ps_ctx* c : m->ctx)
+    if (c->pl_pending) return multi_fail(m, PS_ERR_STATE, "a submitted pileup call of a context has not been waited for");
+  ps_ctx* c0 = m->ctx[0];
+  if (opts && opts->carry_valid && opts->carry_contig >= c0->ref.n_contigs)
+    return multi_fail(m, PS_ERR_INVALID_ARG, "carry_contig is not a contig of the reference");
+  return with_file_order(m, bam_path, window_reads, [&](ps_bam* B) {
+    return pileup_windows_run(m, B, opts, sink, counters, open_out, fault);
+  });
+}
+
+
+// ---- track files -------------------------------------------------------------------------------------------------------
+// The three files of the track tool.  Runs that touch with equal coverage are merged, so a run cut by a window boundary
+// is one row.
+struct TrackWriter {
+  FILE* f[3] = {nullptr, nullptr, nullptr};      // plus bedGraph, minus bedGraph, t2c tsv
+  std::vector<std::string> names;
+  ps_track_run last[2]{};
+  bool have[2] = {false, false};
+  uint64_t rows[3] = {0, 0, 0};
+  std::string buf[3];
+  int open(const std::string& prefix) {
+    const char* ext[3] = {".plus.bedGraph", ".minus.bedGraph", ".t2c.tsv"};
+    for (int k = 0; k < 3; ++k) {
+      f[k] = fopen((prefix + ext[k]).c_str(), "wb");
+      if (!f[k]) return PS_ERR_IO;
+    }
+    buf[2] = "chrom\tpos\tstrand\tt2c\tcoverage\n";
+    return PS_OK;
+  }
+  static void num(std::string& b, uint64_t v) {
+    char t[24];
+    int n = 0;
+    do { t[n++] = (char)('0' + v % 10); v /= 10; } while (v);
+    while (n) b.push_back(t[--n]);
+  }
+  int drain(int k, bool force) {
+    if (buf[k].size() < (1u << 20) && !force) return PS_OK;
+    if (!buf[k].empty() && fwrite(buf[k].data(), 1, buf[k].size(), f[k]) != buf[k].size()) return PS_ERR_IO;
+    buf[k].clear();
+    return PS_OK;
+  }
+  int flush_run(int s) {
+    if (!have[s]) return PS_OK;
+    std::string& b = buf[s];
+    b += names[last[s].contig]; b.push_back('\t');
+    num(b, last[s].start0); b.push_back('\t');
+    num(b, last[s].end0); b.push_back('\t');
+    num(b, last[s].cov); b.push_back('\n');
+    ++rows[s];
+    have[s] = false;
+    return drain(s, false);
+  }
+  int run(int s, const ps_track_run& r) {
+    if (have[s] && last[s].contig == r.contig && last[s].end0 == r.start0 && last[s].cov == r.cov) { last[s].end0 = r.end0; return PS_OK; }
+    const int rc = flush_run(s);
+    last[s] = r;
+    have[s] = true;
+    return rc;
+  }
+  int site(const ps_track_site& x) {
+    std::string& b = buf[2];
+    b += names[x.contig]; b.push_back('\t');
+    num(b, (uint32_t)x.pos); b.push_back('\t');
+    b.push_back(x.strand ? '-' : '+'); b.push_back('\t');
+    num(b, x.t2c); b.push_back('\t');
+    num(b, x.cov); b.push_back('\n');
+    ++rows[2];
+    return drain(2, false);
+  }
+  int finish() {
+    int rc = PS_OK;
+    for (int s = 0; s < 2; ++s) if (rc == PS_OK) rc = flush_run(s);
+    for (int k = 0; k < 3; ++k) if (rc == PS_OK) rc = drain(k, true);
+    return rc;
+  }
+  ~TrackWriter() { for (FILE* x : f) if (x) fclose(x); }
+};
+
+// what a window hands to the writer: final runs and sites, in file order
+struct TrackRows {
+  std::vector<ps_track_run> runs[2];
+  std::vector<ps_track_site> sites;
+};
+
+// positions not final yet: [key0, key0 + len) of one contig, cov+, cov-, t2c+, t2c-
+struct TrackPending {
+  unsigned long long key0 = 0;
+  std::vector<uint32_t> v[4];
+  size_t len() const { return v[0].size(); }
+  // rows of the positions before `upto` (keys), which leave the region
+  void emit_before(unsigned long long upto, const std::vector<uint32_t>& by_rank, TrackRows& out) {
+    const size_t n = len();
+    size_t k_end = 0;
+    if (upto > key0) k_end = (size_t)std::min<unsigned long long>(n, upto - key0);
+    if ((upto >> 32) != (key0 >> 32)) k_end = upto > key0 ? n : 0;
+    if (!k_end) return;
+    const uint32_t contig = by_rank[(uint32_t)(key0 >> 32) - 1];
+    const uint32_t p0 = (uint32_t)key0 - 1;         // 0-based position of entry 0
+    for (int s = 0; s < 2; ++s)
+      for (size_t k = 0; k < k_end; ++k) {
+        const uint32_t c = v[s][k];
+        if (!c) continue;
+        std::vector<ps_track_run>& r = out.runs[s];
+        if (!r.empty() && r.back().contig == contig && r.back().end0 == p0 + k && r.back().cov == c) r.back().end0++;
+        else r.push_back(ps_track_run{contig, p0 + (uint32_t)k, p0 + (uint32_t)k + 1, c});
+      }
+    for (size_t k = 0; k < k_end; ++k)
+      for (int s = 0; s < 2; ++s)
+        if (v[2 + s][k]) out.sites.push_back(ps_track_site{contig, (int32_t)(p0 + k + 1), (uint32_t)s, v[2 + s][k], v[s][k]});
+    for (auto& a : v) a.erase(a.begin(), a.begin() + (ptrdiff_t)k_end);
+    key0 += k_end;
+  }
+};
+
+struct TrackFlight {
+  ps_ctx* ctx = nullptr;
+  std::thread th;
+  TrackOut out;
+  int rc = PS_OK;
+  std::string err;
+  uint64_t offset = 0;
+  bool live = false;
+};
+
+// The windowed track over an open file (contexts keyed in the file's contig order)
+int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters* ctr, ps_fault* fault) {
+  ps_ctx* c0 = m->ctx[0];
+  const std::vector<uint64_t>& contig_off = c0->contig_off;
+  const std::vector<uint32_t>& by_rank = c0->contig_by_rank;
+  memset(ctr, 0, sizeof *ctr);
+  TrackPending P;
+  unsigned long long last_start = 0, max_end = 0;     // over the windows launched so far / completed so far
+  uint64_t offset = 0, window = 0;
+  TrackFlight fl[2];
+  std::thread sink_thread;
+  int sink_rc = PS_OK;
+  auto join_sink = [&]() -> int {
+    if (sink_thread.joinable()) sink_thread.join();
+    const int rc = sink_rc;
+    sink_rc = PS_OK;
+    return rc;
+  };
+  auto complete = [&](TrackFlight& f) -> int {
+    f.live = false;
+    f.th.join();
+    const TrackOut& o = f.out;
+    if (f.rc != PS_OK) {
+      if (o.fault.code && !fault->code) { *fault = o.fault; fault->read_ordinal += f.offset; }
+      return multi_fail(m, f.rc, f.err);
+    }
+    ctr->num_reads_processed += o.ctr.num_reads_processed;
+    ctr->unmapped += o.ctr.unmapped;
+    ctr->skipped_due_indel += o.ctr.skipped_due_indel;
+    ctr->reads_counted += o.ctr.reads_counted;
+    ctr->fast_path_reads += o.ctr.fast_path_reads;
+    for (int s = 0; s < 2; ++s) { ctr->aligned_bases[s] += o.ctr.aligned_bases[s]; ctr->t2c_events[s] += o.ctr.t2c_events[s]; }
+    if (!o.first_key) return PS_OK;                    // no kept record: nothing changes
+    if (o.first_key < last_start) return multi_fail(m, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
+    if (o.head.len) {
+      if (o.head.key0 < P.key0 || o.head.key0 + o.head.len > P.key0 + P.len())
+        return multi_fail(m, PS_ERR_STATE, "track: window head outside the pending region");
+      const size_t at = (size_t)(o.head.key0 - P.key0);
+      for (int j = 0; j < 4; ++j)
+        for (uint32_t k = 0; k < o.head.len; ++k) P.v[j][at + k] += o.head.v[(size_t)j * o.head.len + k];
+    }
+    auto rows = std::make_shared<TrackRows>();
+    P.emit_before(o.last_key, by_rank, *rows);
+    for (int s = 0; s < 2; ++s) rows->runs[s].insert(rows->runs[s].end(), o.runs[s].begin(), o.runs[s].end());
+    rows->sites.insert(rows->sites.end(), o.sites.begin(), o.sites.end());
+    if (o.tail.len) {
+      if (P.len() && P.key0 + P.len() != o.tail.key0) return multi_fail(m, PS_ERR_STATE, "track: window tail not next to the pending region");
+      if (!P.len()) P.key0 = o.tail.key0;
+      for (int j = 0; j < 4; ++j) P.v[j].insert(P.v[j].end(), o.tail.v.begin() + (ptrdiff_t)j * o.tail.len, o.tail.v.begin() + (ptrdiff_t)(j + 1) * o.tail.len);
+    }
+    last_start = o.last_key;
+    const int prev_rc = join_sink();
+    if (prev_rc != PS_OK) return prev_rc;
+    sink_thread = std::thread([&W, &sink_rc, rows] {
+      int rc = PS_OK;
+      for (int s = 0; s < 2 && rc == PS_OK; ++s)
+        for (const ps_track_run& r : rows->runs[s]) if ((rc = W.run(s, r)) != PS_OK) break;
+      for (const ps_track_site& x : rows->sites) if (rc != PS_OK || (rc = W.site(x)) != PS_OK) break;
+      sink_rc = rc;
+    });
+    return PS_OK;
+  };
+  int st = PS_OK;
+  for (;; ++window) {
+    TrackFlight& f = fl[window & 1];
+    if (f.live) { st = complete(f); if (st) break; }
+    ps_read_batch hb;
+    const int k = ps_bam_next(B, &hb);
+    if (k < 0) { st = multi_fail(m, k, ps_bam_error(B)); break; }
+    if (k == 0) break;
+    ps_ctx* c = m->ctx[window % m->ctx.size()];
+    TrackFlight& prev = fl[(window & 1) ^ 1];
+    if (prev.live && prev.ctx == c) { st = complete(prev); if (st) break; }
+    cudaSetDevice(c->device);
+    StagedBatch* sb = nullptr;
+    st = stage_batch(c, &hb, /*with_qual=*/false, &sb);     // the track reads no qualities
+    if (st != PS_OK) { sync_fail(m, c, st); break; }
+    f.ctx = c; f.offset = offset; f.rc = PS_OK; f.live = true;
+    const DeviceBatch view = sb->view;
+    const uint64_t prev_end = max_end;
+    f.th = std::thread([&f, c, view, prev_end] {
+      cudaSetDevice(c->device);
+      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out);
+      if (f.rc != PS_OK) f.err = c->err;
+    });
+    max_end = std::max<unsigned long long>(max_end, host_max_key(hb, contig_off, c0->contig_rank));
+    offset += hb.n_reads;
+  }
+  for (int i = 0; i < 2; ++i) {            // in file order; after an error only the threads are joined
+    TrackFlight& f = fl[(window + i) & 1];
+    if (!f.live) continue;
+    if (st == PS_OK) st = complete(f);
+    else { f.live = false; f.th.join(); }
+  }
+  {
+    const int rc = join_sink();
+    if (st == PS_OK) st = rc;
+  }
+  if (st != PS_OK) return st;
+  TrackRows rest;
+  P.emit_before(~0ull, by_rank, rest);
+  for (int s = 0; s < 2 && st == PS_OK; ++s)
+    for (const ps_track_run& r : rest.runs[s]) if ((st = W.run(s, r)) != PS_OK) break;
+  for (const ps_track_site& x : rest.sites) if (st != PS_OK || (st = W.site(x)) != PS_OK) break;
+  if (st == PS_OK) st = W.finish();
+  if (st != PS_OK) return multi_fail(m, st, "track: writing the output files failed");
+  ctr->n_runs[0] = W.rows[0];
+  ctr->n_runs[1] = W.rows[1];
+  ctr->n_sites = W.rows[2];
+  return PS_OK;
 }
 
 }  // namespace
@@ -617,6 +859,34 @@ int ps_clust_bam(ps_ctx* ctx, const char* bam_path, const char* out_path, const 
   ps_multi m;
   borrow(m, ctx);
   const int st = ps_multi_clust_bam(&m, bam_path, out_path, snp_vcf, min_read_coverage, counters_out, fault_out);
+  if (st != PS_OK && !m.err.empty()) set_error(ctx, st, m.err);
+  return st;
+}
+
+// The track tool from files: <out_prefix>.plus.bedGraph, .minus.bedGraph, .t2c.tsv
+int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
+                       ps_fault* fault_out) {
+  if (!m || !bam_path || !out_prefix) return PS_ERR_INVALID_ARG;
+  if (m->ctx.empty() || !m->ctx[0]->fasta) return multi_fail(m, PS_ERR_STATE, "load the reference first (ps_multi_load_fasta)");
+  ps_ctx* c0 = m->ctx[0];
+  TrackWriter W;
+  for (uint32_t i = 0; i < c0->ref.n_contigs; ++i) W.names.push_back(ps_fasta_contig_name(c0->fasta, i));
+  int st = W.open(out_prefix);
+  if (st != PS_OK) return multi_fail(m, st, std::string("cannot write ") + out_prefix + ".*");
+  ps_track_counters ctr{};
+  ps_fault fault{};
+  st = with_file_order(m, bam_path, window_reads_default(), [&](ps_bam* B) { return track_windows_run(m, B, W, &ctr, &fault); });
+  if (counters_out) *counters_out = ctr;
+  if (fault_out) *fault_out = fault;
+  return st;
+}
+
+int ps_track_bam(ps_ctx* ctx, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
+                 ps_fault* fault_out) {
+  if (!ctx || !bam_path || !out_prefix) return set_error(ctx, PS_ERR_INVALID_ARG, "NULL argument");
+  ps_multi m;
+  borrow(m, ctx);
+  const int st = ps_multi_track_bam(&m, bam_path, out_prefix, counters_out, fault_out);
   if (st != PS_OK && !m.err.empty()) set_error(ctx, st, m.err);
   return st;
 }

@@ -15,7 +15,7 @@ CSRC_DIR = os.path.join(ROOT_DIR, "csrc")
 REPO_DIR = os.path.dirname(ROOT_DIR)
 INCLUDE_DIR = os.path.join(REPO_DIR, "include")
 
-PS_ABI_VERSION = 3
+PS_ABI_VERSION = 4
 PS_OK = 0
 PS_ERR_INVALID_ARG = -1
 PS_ERR_NO_DEVICE = -2
@@ -124,6 +124,16 @@ class ps_pileup_opts(C.Structure):
                 ("t2c_masks_device", C.c_void_p)]
 
 
+class ps_track_counters(C.Structure):
+    _fields_ = [("num_reads_processed", C.c_uint64), ("unmapped", C.c_uint64), ("skipped_due_indel", C.c_uint64),
+                ("reads_counted", C.c_uint64), ("aligned_bases", C.c_uint64 * 2), ("t2c_events", C.c_uint64 * 2),
+                ("n_runs", C.c_uint64 * 2), ("n_sites", C.c_uint64), ("fast_path_reads", C.c_uint64)]
+
+    def as_dict(self) -> dict:
+        return {f: (list(getattr(self, f)) if hasattr(getattr(self, f), "__len__") else int(getattr(self, f)))
+                for f, _ in self._fields_}
+
+
 class ps_flush_totals(C.Structure):
     _fields_ = [("snp_hit", C.c_uint64), ("high_frequent_error", C.c_uint64), ("num_crosslinked_clusters", C.c_uint64),
                 ("num_allele_positions", C.c_uint64), ("allele_positions", C.c_uint64 * 51),
@@ -139,6 +149,9 @@ CLUSTER_DTYPE = [("first_read", "<u8"), ("running_id", "<u4"), ("contig", "<u4")
                  ("combined_strand", "u1"), ("reserved", "<u2"), ("mask51", "<u8"), ("site_begin", "<u8"),
                  ("site_end", "<u8")]
 SITE_DTYPE = [("pos", "<i4"), ("t2c", "<u4"), ("cov", "<u4"), ("reserved", "<u4"), ("order_key", "<u8")]
+# ps_track_run / ps_track_site
+TRACK_RUN_DTYPE = [("contig", "<u4"), ("start0", "<u4"), ("end0", "<u4"), ("cov", "<u4")]
+TRACK_SITE_DTYPE = [("contig", "<u4"), ("pos", "<i4"), ("strand", "<u4"), ("t2c", "<u4"), ("cov", "<u4")]
 
 # every symbol include/parasuite_b200.h declares: name -> (restype, argtypes)
 VP = C.c_void_p
@@ -223,6 +236,15 @@ EXPORTS = {
     "ps_flush_totals_get": (C.c_int, [VP, C.POINTER(ps_flush_totals), VP, C.c_uint64]),
     "ps_flush_error": (C.c_char_p, [VP]),
     "ps_flush_destroy": (None, [VP]),
+    "ps_track_batch": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(VP)]),
+    "ps_track_batch_device": (C.c_int, [VP, C.POINTER(ps_read_batch), VP, C.POINTER(VP)]),
+    "ps_track_counters_get": (C.c_int, [VP, C.POINTER(ps_track_counters)]),
+    "ps_track_runs": (C.c_int64, [VP, C.c_int, C.c_uint64, VP, C.c_uint64]),
+    "ps_track_sites": (C.c_int64, [VP, C.c_uint64, VP, C.c_uint64]),
+    "ps_track_fault": (C.c_int, [VP, C.POINTER(ps_fault)]),
+    "ps_track_close": (None, [VP]),
+    "ps_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),
+    "ps_multi_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),
     "ps_kernel_launches": (C.c_uint64, [VP]),
     "ps_last_kernel_ms": (C.c_float, [VP]),
     "ps_kernel_times": (C.c_int, [VP, VP, C.c_int]),

@@ -230,6 +230,14 @@ class Context:
         _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
         return np.array(list(ctr), dtype=np.int32)
 
+    def track_bam(self, bam_path: str, out_prefix: str) -> dict:
+        """The `track` tool from files: writes <out_prefix>.plus.bedGraph, <out_prefix>.minus.bedGraph and
+        <out_prefix>.t2c.tsv (per-position coverage and T>C events by strand); returns the run's counters."""
+        ctr, f = abi.ps_track_counters(), abi.ps_fault()
+        st = self.lib.ps_track_bam(self.h, bam_path.encode(), out_prefix.encode(), C.byref(ctr), C.byref(f))
+        _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
+        return ctr.as_dict()
+
     # ---- batches ---------------------------------------------------------------------------------
     def upload(self, batch) -> UploadedBatch:
         """One H2D copy of a host batch (ReadBatch / PinnedBatch); both tools can then run on the device view
@@ -403,6 +411,45 @@ class Context:
         """pileup_run + fetch of every record into host arrays."""
         with self.pileup_run(batch, first_running_id, carry, stream) as res:
             return res.fetch()
+
+    # ---- T>C conversion and coverage track ---------------------------------------------------------
+    def track(self, batch, stream: int = 0) -> dict:
+        """Per-position coverage and T>C events by strand of one whole input: {"runs_plus", "runs_minus", "sites",
+        "counters"}, runs and sites as numpy structured arrays (abi.TRACK_RUN_DTYPE / TRACK_SITE_DTYPE, contigs as FASTA
+        indices).  batch: host (ReadBatch / PinnedBatch) or device-resident (DeviceBatch / UploadedBatch)."""
+        h = C.c_void_p()
+        if isinstance(batch, (DeviceBatch, UploadedBatch)):
+            st = self.lib.ps_track_batch_device(self.h, C.byref(batch.struct), stream or None, C.byref(h))
+        else:
+            s = batch.struct if hasattr(batch, "struct") else batch.as_struct()
+            st = self.lib.ps_track_batch(self.h, C.byref(s), C.byref(h))
+        try:
+            if st != abi.PS_OK:
+                fault = None
+                if h:
+                    f = abi.ps_fault()
+                    self.lib.ps_track_fault(h, C.byref(f))
+                    fault = (f.code, f.read_ordinal)
+                msg = self.lib.ps_last_error(self.h).decode()
+                if st == abi.PS_ERR_REFERENCE_WOULD_THROW:
+                    raise abi.ReferenceWouldThrow(st, msg, fault)
+                raise abi.PsError(st, msg, fault)
+            ctr = abi.ps_track_counters()
+            self.lib.ps_track_counters_get(h, C.byref(ctr))
+            out = {"counters": ctr.as_dict()}
+            for s_, name in ((0, "runs_plus"), (1, "runs_minus")):
+                a = np.zeros(ctr.n_runs[s_], dtype=abi.TRACK_RUN_DTYPE)
+                if a.size:
+                    self.lib.ps_track_runs(h, s_, 0, a.ctypes.data, a.size)
+                out[name] = a
+            sites = np.zeros(ctr.n_sites, dtype=abi.TRACK_SITE_DTYPE)
+            if sites.size:
+                self.lib.ps_track_sites(h, 0, sites.ctypes.data, sites.size)
+            out["sites"] = sites
+            return out
+        finally:
+            if h:
+                self.lib.ps_track_close(h)
 
     def _pinned(self, key: str, nbytes: int) -> np.ndarray:
         """Reusable page-locked host buffer (grown on demand) viewed as uint8."""
@@ -585,6 +632,13 @@ class MultiContext:
                                          min_read_coverage, C.byref(ctr), C.byref(f))
         self._check(st, fault=(f.code, f.read_ordinal))
         return {k: getattr(ctr, k) for k, _ in abi.ps_pileup_counters._fields_}
+
+    def track_bam(self, bam_path: str, out_prefix: str) -> dict:
+        """Context.track_bam with windows round-robin over the devices; the files are byte-identical."""
+        ctr, f = abi.ps_track_counters(), abi.ps_fault()
+        st = self.lib.ps_multi_track_bam(self.h, bam_path.encode(), out_prefix.encode(), C.byref(ctr), C.byref(f))
+        self._check(st, fault=(f.code, f.read_ordinal))
+        return ctr.as_dict()
 
     def close(self):
         if getattr(self, "h", None):
