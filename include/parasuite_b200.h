@@ -105,7 +105,8 @@ typedef struct ps_read_batch {
   const uint64_t* tile_qual_off;  /* [n_tiles+1] byte offset of each tile in qual */
   const uint64_t* tile_cigar_off; /* [n_tiles+1] element offset of each tile in cigar */
   const uint32_t* tile_exc_off;   /* [n_tiles+1] element offset of each tile in exc */
-  const uint32_t* exc;            /* invalid read bases: (read_in_tile << 16) | position, sorted */
+  const uint32_t* exc;            /* invalid read bases: (read_in_tile << 16) | position, sorted.  Every tool reads a
+                                     listed base as N and ignores the code bases2 holds there (any value may be stored) */
   uint32_t uniform_len;           /* != 0: every read has this L (offsets are closed-form) */
   uint32_t uniform_ncigar;        /* != 0: every read has this many cigar ops */
   uint64_t bases_bytes;           /* total sizes of the streams (for copies) */

@@ -152,3 +152,17 @@ __device__ __forceinline__ bool read_pos_invalid(const DeviceBatch& b, ExcRange 
     if ((__ldg(b.exc + e) & 0xFFFFu) == p) return true;
   return false;
 }
+// the listed positions p < 64 of read r as a forward bit mask (bit p): the bit-parallel T>C paths clear them, whatever
+// code the producer stored there.  Call for reads with PS_RF_HAS_INVALID only.  One search for the read's first entry,
+// then a scan over its (few) entries.
+__device__ __forceinline__ unsigned long long read_exc_mask64(const DeviceBatch& b, uint64_t r) {
+  const uint64_t tile = r / PS_TILE_READS;
+  const uint32_t rit = (uint32_t)(r % PS_TILE_READS), hi = __ldg(b.tile_exc_off + tile + 1);
+  unsigned long long m = 0;
+  for (uint32_t e = exc_lower_bound(b.exc, __ldg(b.tile_exc_off + tile), hi, rit << 16); e < hi; ++e) {
+    const uint32_t v = __ldg(b.exc + e);
+    if ((v >> 16) != rit) break;
+    if ((v & 0xFFFFu) < 64u) m |= 1ull << (v & 0xFFFFu);
+  }
+  return m;
+}

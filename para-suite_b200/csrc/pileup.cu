@@ -619,7 +619,7 @@ __device__ __noinline__ void pl_decode_generic(const ClusterParams& P, uint64_t 
   x.mask = mask;
 }
 
-// PAR-CLIP shape: uniform length L <= 64, one M/=/X op of length L, no N call in the read.
+// PAR-CLIP shape: uniform length L <= 64, one M/=/X op of length L.
 __device__ __forceinline__ uint32_t compress_even(uint32_t c) {   // even bits of c -> low 16 bits
   c = (c | (c >> 1)) & 0x33333333u;
   c = (c | (c >> 2)) & 0x0F0F0F0Fu;
@@ -628,9 +628,11 @@ __device__ __forceinline__ uint32_t compress_even(uint32_t c) {   // even bits o
   return c;
 }
 
+// has_inv: read r has entries in `exc`; the positions they list are cleared like reference N
 template <int NW>
 __device__ __forceinline__ unsigned long long t2c_mask_fast(const DeviceRef& ref, uint32_t g0, uint32_t L, bool rev,
-                                                            const uint32_t (&bw)[NW + 1], uint32_t bshift) {
+                                                            const uint32_t (&bw)[NW + 1], uint32_t bshift,
+                                                            const DeviceBatch& b, uint64_t r, bool has_inv) {
   const uint32_t wi = g0 >> 4, sh = (g0 & 15u) * 2u;
   uint32_t w[NW + 1];
 #pragma unroll
@@ -650,6 +652,7 @@ __device__ __forceinline__ unsigned long long t2c_mask_fast(const DeviceRef& ref
                                  ((unsigned long long)(NW > 2 ? __funnelshift_r(i1, i2, s1) : 0u) << 32);
   m &= ~inv;
   m &= L >= 64 ? ~0ull : ((1ull << L) - 1ull);
+  if (has_inv && m) m &= ~read_exc_mask64(b, r);      // only a read with a candidate event needs its list
   if (rev) m = __brevll(m) >> (64u - L);      // i = alignedLength - 1 - j
   return m;
 }
@@ -720,15 +723,16 @@ __device__ __forceinline__ void pl_decode(const ClusterParams& P, uint64_t q, ui
       if (!in) return;
       const uint32_t L = P.b.uniform_len, bpr = (L + 3) >> 2;
       const uint32_t flags = PS_META_FLAGS(meta), g0 = raw.g0, cg = raw.cg;
-      // N calls are stored as code 0 (A): never read C (forward T>C) nor read G (reverse), so such reads need no
-      // look at the exception list; duplicates are not filtered by this tool and qualities are never read
+      // N calls are cleared from the mask by their `exc` entries (the code stored under them is arbitrary);
+      // duplicates are not filtered by this tool and qualities are never read
       constexpr uint32_t kHarmless = PS_RF_REVERSE | PS_RF_HAS_INVALID | PS_RF_DUPLICATE | PS_RF_QUAL_MISSING;
       bool fast = (flags & ~kHarmless) == 0 && op_is_match(cg & 15u) && (cg >> 4) == L && PS_META_LEN(meta) == L;
       fast = fast && contig_lookup(P.ref, g0, cc) && (uint64_t)g0 + L <= cc.hi;
       if (fast) {
         const bool rev = (flags & PS_RF_REVERSE) != 0;
         const uint64_t boff = r * (uint64_t)bpr;
-        unsigned long long m = t2c_mask_fast<NW>(P.ref, g0, L, rev, raw.bw, (uint32_t)(boff & 3u) * 8u);
+        unsigned long long m = t2c_mask_fast<NW>(P.ref, g0, L, rev, raw.bw, (uint32_t)(boff & 3u) * 8u, P.b, r,
+                                                 (flags & PS_RF_HAS_INVALID) != 0);
         const int32_t start = (int32_t)((uint64_t)g0 - cc.lo) + 1, end = start + (int32_t)L - 1;
         if (L > 51u && (m >> 51)) { raise_fault(&P.st->fault, r, PS_THROW_MASK51); return; }
         x.kept = true; x.mask = m; x.start = start; x.end = end; x.lo = start; x.hi = end; x.rev = rev; x.contig = cc.idx;

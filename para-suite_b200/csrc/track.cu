@@ -266,7 +266,7 @@ __device__ __noinline__ void tr_accum_generic(const TrParams& P, uint64_t r, uin
 }
 
 // NW > 0: the batch has uniform length L <= 64 and one cigar op per read; reads whose op is M/=/X of length L take the
-// bit-parallel path (read bases that are not ACGT are stored as A: never read C nor read G)
+// bit-parallel path (the positions listed in `exc` are cleared from its event mask: the code stored there is arbitrary)
 template <int NW>
 __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_constant__ TrParams P) {
   unsigned long long ev[2] = {0, 0}, fast = 0;
@@ -314,6 +314,7 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
                                        ((unsigned long long)(NW > 2 ? __funnelshift_r(i1, i2, s1) : 0u) << 32);
         m &= ~inv;
         m &= L >= 64 ? ~0ull : ((1ull << L) - 1ull);
+        if ((PS_META_FLAGS(meta) & PS_RF_HAS_INVALID) && m) m &= ~read_exc_mask64(P.b, r);   // only with a candidate event
         const int64_t c0 = (int64_t)g0 + to_compact;
         atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0, 1);
         atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0 + L, -1);
