@@ -89,7 +89,10 @@ struct PlState {                  // device-side run state (one per call)
   unsigned int first_slot1;       // first read of slot 1 (end of the head partial); n_reads if there is no slot 1
   unsigned int spec_failed;       // the speculative flag pass used a carry-in that pl_flag_scan_kernel found too small
   ps_cluster head, open;          // final records of slot 0 and of the last slot (written by pl_compact_kernel)
-  unsigned long long dbg[4];      // PARASUITE_B200_DEBUG: warp-routine calls, sweep give-ups, window passes, chunk decodes in windows
+  // PARASUITE_B200_DEBUG, counted by the warp routine over clusters with at least one T>C event: [0] clusters the
+  // ballot form could not take (the streaming sweep starts on them), [1] of those, the ones the sweep gave up on,
+  // [2] window passes the window loop made over them (one per PL_WINDOW positions from the first event to the last)
+  unsigned long long dbg[3];
 };
 
 struct PlRead {              // what the pileup needs from one read
@@ -1452,7 +1455,7 @@ __global__ void pl_init_state(PlState* st, unsigned int* tile_sites, uint32_t n_
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     st->fault = PS_FAULT_NONE; st->skipped = 0; st->dstr = 0; st->n_sites = 0; st->n_sites_final = 0; st->n_flags = 0;
     st->unsorted = 0; st->tile_ctr_flag = 0; st->tile_ctr_compact = 0; st->first_slot1 = 0xFFFFFFFFu; st->spec_failed = 0;
-    st->dbg[0] = st->dbg[1] = st->dbg[2] = st->dbg[3] = 0;
+    st->dbg[0] = st->dbg[1] = st->dbg[2] = 0;
   }
 }
 
