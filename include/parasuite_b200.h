@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define PS_ABI_VERSION 4
+#define PS_ABI_VERSION 5
 
 /* ---- status codes ------------------------------------------------------------------------ */
 #define PS_OK 0
@@ -54,6 +54,11 @@ extern "C" {
 /* not a reference exception: ps_fault.code of a record this SoA cannot hold (more than 255 CIGAR operations; htsjdk
  * takes any number, ErrorProfiling.java:206-207).  Reported with PS_ERR_UNSUPPORTED, never as a "would throw". */
 #define PS_FAULT_CIGAR_OPS 9
+/* not a reference exception: ps_fault.code of a mapped record that consumes no reference and whose POS lies past its
+ * contig's end (ps_read_batch.past_end).  Its POS has no offset on its contig, and a batch carries no contig per record,
+ * so the pileup, clust and track refuse it (PS_ERR_UNSUPPORTED) rather than place it on a contig.
+ * The profile keeps the JVM's own fault for it (PS_THROW_EMPTY_REF at POS = length + 1, PS_THROW_REF_RANGE beyond). */
+#define PS_FAULT_PAST_END 10
 
 /* ---- packed reference ---------------------------------------------------------------------
  * All contigs concatenated into one coordinate space ("global offset", 0-based, < 2^32).
@@ -130,6 +135,13 @@ typedef struct ps_read_batch {
   const uint8_t* qual6;
   const uint16_t* start16;
   const uint32_t* tile_start;
+  /* 1 + the ordinal of the first mapped record (POS != 0, at most 255 CIGAR operations) that consumes no reference and
+   * whose POS is past its contig's end; 0: the batch holds none.  Set by the producers, which know each record's contig
+   * (ps_bam_next, ReadBatch.from_records); the tools answer PS_FAULT_PAST_END for that record unless a record before it
+   * faults first.  The producers give every such record the offset of its contig's last base, so that a slice that
+   * leaves the first one out (and sets past_end relative to itself, 0 when the record lies outside it) keeps the rest
+   * on their own contigs. */
+  uint64_t past_end;
 } ps_read_batch;
 
 /* ---- error profile ------------------------------------------------------------------------ */

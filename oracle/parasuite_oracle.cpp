@@ -464,6 +464,9 @@ or_pileup_result* or_pileup_run(const ps_reference* ref, const ps_read_batch* b,
       hasI |= op == 1; hasD |= op == 2; hasN |= op == 3;
     }
     if ((hasI || hasD) && hasN) { R->counters.skipped_due_indel++; continue; }  // :152-157
+    if (b->past_end && ord == b->past_end - 1) {                          // no contig to put it on: refused
+      R->fault.code = PS_FAULT_PAST_END; R->fault.read_ordinal = ord; return R;
+    }
     // getAlignmentStart / getAlignmentEnd / getReferenceName
     int64_t contig, start, end;
     uint32_t refLen = cigar_ref_len(v.cigar, v.ncig);

@@ -42,6 +42,23 @@ class AIOOBE(Exception):
     pass
 
 
+PS_FAULT_PAST_END = 10
+
+
+class PastContigEnd(Exception):
+    """A mapped record that consumes no reference and starts past its contig's end: the SoA batch holds no contig per
+    record, so the library refuses it (ps_fault.code PS_FAULT_PAST_END) where the JVM would keep it."""
+
+    def __init__(self, ordinal: int):
+        super().__init__(f"record {ordinal}: no reference span, POS past its contig's end")
+        self.ordinal = ordinal
+        self.code = PS_FAULT_PAST_END
+
+
+def past_contig_end(r: "Rec", genome: "Genome") -> bool:
+    return r.ref_len() == 0 and r.rname in genome.contigs and r.pos > len(genome.contigs[r.rname])
+
+
 class JArray:
     """Java array: fixed length, zero filled, bounds checked (no negative indexing)."""
 
@@ -583,6 +600,8 @@ def pileup(records: List[Rec], genome: Genome, snps: SnpDb, min_cov: int) -> Pil
         if (("I" in cs) or ("D" in cs)) and ("N" in cs):          # :152-157
             st.skipped_due_indel += 1
             continue
+        if r.pos and past_contig_end(r, genome):
+            raise PastContigEnd(ordinal)
         if (t_end - r.pos) < 5 or r.rname != t_chr:               # :175-176
             if have_cluster:      # before the first read numReads==0 < minCov: nothing to flush
                 rec = snapshot(True)

@@ -134,6 +134,7 @@ or_track_result* or_track_run(const ps_reference* ref, const ps_read_batch* b) {
       hasI |= op == 1; hasD |= op == 2; hasN |= op == 3;
     }
     if ((hasI || hasD) && hasN) { R->ctr.skipped_due_indel++; continue; }
+    if (b->past_end && ord == b->past_end - 1) { fault(PS_FAULT_PAST_END, ord); break; }   // no contig to put it on
     if ((v.flags & PS_RF_POS_ZERO) || v.ref_start >= ref->n_bases) { fault(PS_THROW_REF_RANGE, ord); break; }
     const int64_t contig = contig_of(ref, v.ref_start);
     const uint64_t c_lo = ref->contig_off[contig], c_hi = ref->contig_off[contig + 1];
@@ -181,7 +182,7 @@ or_track_result* or_track_run(const ps_reference* ref, const ps_read_batch* b) {
     }
   }
   T.flush(R);
-  if (R->fault.code) R->status = R->fault.code == PS_FAULT_CIGAR_OPS ? PS_ERR_UNSUPPORTED : PS_ERR_REFERENCE_WOULD_THROW;
+  if (R->fault.code) R->status = (R->fault.code == PS_FAULT_CIGAR_OPS || R->fault.code == PS_FAULT_PAST_END) ? PS_ERR_UNSUPPORTED : PS_ERR_REFERENCE_WOULD_THROW;
   else if (unsorted) R->status = PS_ERR_UNSORTED;
   R->ctr.n_runs[0] = R->runs[0].size();
   R->ctr.n_runs[1] = R->runs[1].size();

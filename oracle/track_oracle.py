@@ -20,7 +20,7 @@ from typing import List, Optional
 
 import numpy as np
 
-from py_oracle import Genome, Rec
+from py_oracle import PS_FAULT_PAST_END, Genome, Rec, past_contig_end
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
@@ -35,7 +35,7 @@ _lib = None
 
 # ---- per-position T>C conversion and coverage track (tool `track`; no Java counterpart) --------------------------------
 class TrackFault(Exception):
-    """A record the pileup's loop would die on (or, code 9, one the SoA cannot hold): code as ps_fault.code."""
+    """A record the pileup's loop would die on (or, codes 9 and 10, one the SoA cannot hold): code as ps_fault.code."""
 
     def __init__(self, ordinal: int, code: int):
         super().__init__(f"record {ordinal}: fault {code}")
@@ -78,6 +78,8 @@ def track(records: List[Rec], genome: Genome, contig_order: Optional[List[str]] 
             continue
         if r.pos == 0 or r.rname not in genome.contigs:
             raise TrackFault(ordinal, 1)
+        if past_contig_end(r, genome):
+            raise TrackFault(ordinal, PS_FAULT_PAST_END)
         seq = genome.contigs[r.rname]
         for rd1, rf1, n in r.alignment_blocks():       # every block is fetched before a base is looked at
             if rd1 - 1 + n > len(r.seq):

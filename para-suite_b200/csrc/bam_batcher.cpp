@@ -801,6 +801,7 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
   const double t_p2 = now_s();
   static const int8_t kNib[16] = {-1, 0, 1, -1, 2, -1, -1, -1, 3, -1, -1, -1, -1, -1, -1, -1};   // "=ACMGRSVTWYHKDBN"
   const ps_packed_fasta* fa = B->fa;
+  std::atomic<uint64_t> past_end{UINT64_MAX};           // ordinal of the first record counted in ps_read_batch.past_end
   parallel_for(B->threads, n_tiles, [&](int, uint64_t lo, uint64_t hi) {
     for (uint64_t t = lo; t < hi; ++t) {
       uint64_t ob = tb[t], oq = tq[t], oc = tc[t];
@@ -847,7 +848,14 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
           else {
             const uint64_t clen = fa->off[c + 1] - fa->off[c];
             if ((uint64_t)pos + R > clen) fl |= PS_RF_REF_RANGE;  // stop > contig length: SAMException
-            const uint64_t g = fa->off[c] + (uint64_t)pos;
+            uint64_t g = fa->off[c] + (uint64_t)pos;
+            if (R == 0 && (uint64_t)pos >= clen && !(fl & PS_RF_CIGAR_OVERFLOW)) {
+              // no reference span and POS past the contig's end: its offset would name the next contig (the tools refuse
+              // the first such record by its ordinal); the contig's last base keeps every later one on its own contig
+              g = fa->off[c] + clen - 1;
+              uint64_t cur = past_end.load();
+              while (r < cur && !past_end.compare_exchange_weak(cur, r)) {}
+            }
             g32 = g > 0xFFFFFFFFull ? 0xFFFFFFFFu : (uint32_t)g;
           }
         }
@@ -882,6 +890,7 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
   out->qual6 = nullptr;
   out->start16 = nullptr;
   out->tile_start = nullptr;
+  out->past_end = past_end.load() == UINT64_MAX ? 0 : past_end.load() + 1;
   B->ordinal += n;
   return 1;
 }

@@ -33,6 +33,7 @@ static DeviceBatch view_of(const ps_read_batch* b) {
   v.uniform_ncigar = b->uniform_ncigar;
   v.cigar_count = b->cigar_count;
   v.max_len = b->max_len;
+  v.past_end = b->past_end;
   return v;
 }
 
@@ -171,6 +172,7 @@ int stage_batch(ps_ctx* ctx, const ps_read_batch* hb, bool with_qual, StagedBatc
   v.uniform_ncigar = hb->uniform_ncigar;
   v.cigar_count = compact_cigar ? n : hb->cigar_count;
   v.max_len = hb->max_len;
+  v.past_end = hb->past_end;
   *out = &s;
   return PS_OK;
 }

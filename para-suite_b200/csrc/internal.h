@@ -39,6 +39,7 @@ struct DeviceBatch {
   uint32_t uniform_ncigar;
   uint64_t cigar_count;    // total cigar elements (0: not known)
   uint32_t max_len;        // longest read (0: not known)
+  uint64_t past_end;       // ps_read_batch.past_end: the kernels never see it, the tools run on the reads before it
 };
 
 struct ProfileLayout {   // offsets (in int64 elements) inside the accumulator vector

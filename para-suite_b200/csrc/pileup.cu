@@ -1466,6 +1466,7 @@ struct ps_pileup {
   cudaStream_t stream = nullptr;
   DeviceBatch batch{};               // the records (device pointers): needed again only for the halo-merge coverage
   uint64_t stage_serial = 0;         // != 0: the batch lives in a staging slot of the context (valid for two uploads)
+  uint64_t past_end = 0;             // ps_read_batch.past_end of the call: `batch` holds the reads before that record
   int nw = 0;                        // kernel flavour the batch was run with
   // device results, owned by the handle (stream-ordered allocations)
   ps_cluster* d_cl = nullptr;        // slot 0 = head partial, 1..n_flags-1 closed, n_flags = open
@@ -1652,8 +1653,14 @@ static int pileup_finish(ps_ctx* ctx, ps_pileup* H) {
   H->pending = false;
   if (ctx->pl_pending == H) ctx->pl_pending = nullptr;
   auto done = [&](int rc) { H->rc = rc; return rc; };
+  auto past_end = [&]() {
+    H->fault.code = PS_FAULT_PAST_END;
+    H->fault.read_ordinal = H->past_end - 1;
+    return done(set_error(ctx, PS_ERR_UNSUPPORTED, "pileup: a record with no reference span starts past its contig's end"));
+  };
   cudaStream_t st = H->stream;
   const uint64_t n = H->n_reads;
+  if (n == 0) return past_end();        // only a call whose first record is past its contig's end waits here unlaunched
   PlState hs{};
   for (int attempt = 0;; ++attempt) {
     const PlState* hsp = ctx->h_pinned ? static_cast<const PlState*>(ctx->h_pinned) : &H->hs_fallback;
@@ -1688,6 +1695,7 @@ static int pileup_finish(ps_ctx* ctx, ps_pileup* H) {
       return done(set_error(ctx, PS_ERR_UNSUPPORTED, "pileup: a record of this batch has more than 255 CIGAR operations"));
     return done(set_error(ctx, PS_ERR_REFERENCE_WOULD_THROW, "pileup: the JVM would die on a record of this batch"));
   }
+  if (H->past_end) return past_end();
   if (hs.unsorted) return done(set_error(ctx, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED)));
 
   const uint64_t n_slots = (uint64_t)hs.n_flags + 1;
@@ -1728,12 +1736,24 @@ static int run_pileup(ps_ctx* ctx, const DeviceBatch& b, const ps_pileup_opts* o
   H->ctx = ctx;
   H->stream = st;
   H->batch = b;
+  if (b.past_end && b.past_end <= b.n_reads) {
+    // a record past its contig's end (pileup_finish answers PS_FAULT_PAST_END for it): the reads before it decide whether
+    // an earlier record faults first, and none of the kernels sees the record
+    H->past_end = b.past_end;
+    H->batch.n_reads = b.past_end - 1;
+  }
+  H->batch.past_end = 0;
   H->has_opts = opts != nullptr;
   if (opts) H->opts = *opts;
-  const uint64_t n = b.n_reads;
+  const uint64_t n = H->batch.n_reads;
   H->n_reads = n;
-  H->counters.num_reads_processed = n;
-  if (n == 0) return PS_OK;
+  H->counters.num_reads_processed = b.n_reads;
+  if (n == 0) {
+    if (!H->past_end) return PS_OK;
+    H->pending = true;
+    ctx->pl_pending = H;
+    return wait ? pileup_finish(ctx, H) : PS_OK;
+  }
   if (n >= 0xFFFFFFFFull) return set_error(ctx, PS_ERR_UNSUPPORTED, "pileup batch of >= 2^32 reads");
   H->nw = flavour_of(b);
   if (ctx->pl_cap_cl < 1024) ctx->pl_cap_cl = std::max<uint64_t>(1024, n / 8);
@@ -1751,6 +1771,7 @@ static DeviceBatch pl_view_of(const ps_read_batch* b) {
   v.cigar = b->cigar; v.tile_base_off = b->tile_base_off; v.tile_qual_off = b->tile_qual_off;
   v.tile_cigar_off = b->tile_cigar_off; v.tile_exc_off = b->tile_exc_off; v.exc = b->exc;
   v.uniform_len = b->uniform_len; v.uniform_ncigar = b->uniform_ncigar; v.cigar_count = b->cigar_count; v.max_len = b->max_len;
+  v.past_end = b->past_end;
   return v;
 }
 
@@ -1851,7 +1872,7 @@ int ps_pileup_batch_device(ps_ctx* ctx, const ps_read_batch* b, const ps_pileup_
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
   int rc = run_pileup(ctx, pl_view_of(b), opts, st, out);
-  if (rc != PS_OK && rc != PS_ERR_REFERENCE_WOULD_THROW) { free_handle(*out); *out = nullptr; }
+  if (rc != PS_OK && !(*out && (*out)->fault.code)) { free_handle(*out); *out = nullptr; }   // a fault stays readable
   return rc;
 }
 
@@ -1886,7 +1907,7 @@ int ps_pileup_batch(ps_ctx* ctx, const ps_read_batch* hb, const ps_pileup_opts* 
   o.t2c_masks_device = nullptr;      // mask words belong to a device-resident batch the caller ran the profile on
   rc = run_pileup(ctx, sb->view, opts ? &o : nullptr, ctx->stream, out);
   if (*out) (*out)->stage_serial = ctx->stage_serial;
-  if (rc != PS_OK && rc != PS_ERR_REFERENCE_WOULD_THROW) { free_handle(*out); *out = nullptr; }
+  if (rc != PS_OK && !(*out && (*out)->fault.code)) { free_handle(*out); *out = nullptr; }   // a fault stays readable
   return rc;
 }
 

@@ -379,6 +379,7 @@ struct TrackWriter {
   ps_track_run last[2]{};
   bool have[2] = {false, false};
   uint64_t rows[3] = {0, 0, 0};
+  uint64_t merged[2] = {0, 0};                  // runs joined to the one before
   std::string buf[3];
   int open(const std::string& prefix) {
     const char* ext[3] = {".plus.bedGraph", ".minus.bedGraph", ".t2c.tsv"};
@@ -413,7 +414,11 @@ struct TrackWriter {
     return drain(s, false);
   }
   int run(int s, const ps_track_run& r) {
-    if (have[s] && last[s].contig == r.contig && last[s].end0 == r.start0 && last[s].cov == r.cov) { last[s].end0 = r.end0; return PS_OK; }
+    if (have[s] && last[s].contig == r.contig && last[s].end0 == r.start0 && last[s].cov == r.cov) {
+      last[s].end0 = r.end0;
+      ++merged[s];
+      return PS_OK;
+    }
     const int rc = flush_run(s);
     last[s] = r;
     have[s] = true;
@@ -502,6 +507,13 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
     sink_rc = PS_OK;
     return rc;
   };
+  // PARASUITE_B200_DEBUG: per window, the kept records, the pending positions it made final and the pending length after it
+  const bool dbg = getenv("PARASUITE_B200_DEBUG") != nullptr;
+  auto print_window = [&](const TrackOut& o, size_t emitted) {
+    if (dbg)
+      fprintf(stderr, "[ps_track_window] kept %llu, emitted %zu, pending %zu\n", (unsigned long long)o.ctr.reads_counted,
+              emitted, P.len());
+  };
   auto complete = [&](TrackFlight& f) -> int {
     f.live = false;
     f.th.join();
@@ -516,7 +528,7 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
     ctr->reads_counted += o.ctr.reads_counted;
     ctr->fast_path_reads += o.ctr.fast_path_reads;
     for (int s = 0; s < 2; ++s) { ctr->aligned_bases[s] += o.ctr.aligned_bases[s]; ctr->t2c_events[s] += o.ctr.t2c_events[s]; }
-    if (!o.first_key) return PS_OK;                    // no kept record: nothing changes
+    if (!o.first_key) { print_window(o, 0); return PS_OK; }      // no kept record: nothing changes
     if (o.first_key < last_start) return multi_fail(m, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
     if (o.head.len) {
       if (o.head.key0 < P.key0 || o.head.key0 + o.head.len > P.key0 + P.len())
@@ -526,7 +538,9 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
         for (uint32_t k = 0; k < o.head.len; ++k) P.v[j][at + k] += o.head.v[(size_t)j * o.head.len + k];
     }
     auto rows = std::make_shared<TrackRows>();
+    const size_t pending_before = P.len();
     P.emit_before(o.last_key, by_rank, *rows);
+    const size_t emitted = pending_before - P.len();
     for (int s = 0; s < 2; ++s) rows->runs[s].insert(rows->runs[s].end(), o.runs[s].begin(), o.runs[s].end());
     rows->sites.insert(rows->sites.end(), o.sites.begin(), o.sites.end());
     if (o.tail.len) {
@@ -535,6 +549,7 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
       for (int j = 0; j < 4; ++j) P.v[j].insert(P.v[j].end(), o.tail.v.begin() + (ptrdiff_t)j * o.tail.len, o.tail.v.begin() + (ptrdiff_t)(j + 1) * o.tail.len);
     }
     last_start = o.last_key;
+    print_window(o, emitted);
     const int prev_rc = join_sink();
     if (prev_rc != PS_OK) return prev_rc;
     sink_thread = std::thread([&W, &sink_rc, rows] {
@@ -593,6 +608,10 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
   ctr->n_runs[0] = W.rows[0];
   ctr->n_runs[1] = W.rows[1];
   ctr->n_sites = W.rows[2];
+  if (dbg)
+    fprintf(stderr, "[ps_track_files] runs %llu %llu, merged %llu %llu, sites %llu\n", (unsigned long long)W.rows[0],
+            (unsigned long long)W.rows[1], (unsigned long long)W.merged[0], (unsigned long long)W.merged[1],
+            (unsigned long long)W.rows[2]);
   return PS_OK;
 }
 

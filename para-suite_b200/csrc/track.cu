@@ -466,6 +466,18 @@ uint32_t grid_for(uint64_t n, int threads = TR_THREADS) { return (uint32_t)std::
   } while (0)
 
 int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out) {
+  if (b.past_end && b.past_end <= b.n_reads) {
+    // a record past its contig's end: the reads before it decide whether an earlier record faults first
+    DeviceBatch head = b;
+    head.n_reads = b.past_end - 1;
+    head.past_end = 0;
+    const int rc = track_run(ctx, head, st, windowed, prev_end, out);
+    if (rc != PS_OK && rc != PS_ERR_UNSORTED) return rc;
+    out->ctr.num_reads_processed = b.n_reads;
+    out->fault.code = PS_FAULT_PAST_END;
+    out->fault.read_ordinal = b.past_end - 1;
+    return set_error(ctx, PS_ERR_UNSUPPORTED, "track: a record with no reference span starts past its contig's end");
+  }
   *out = TrackOut();
   const uint64_t n = b.n_reads;
   out->ctr.num_reads_processed = n;
@@ -508,7 +520,14 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   }
   if (hh.s.unsorted) return set_error(ctx, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
   const uint32_t n_segs = hh.n_segs;
-  if (n_segs == 0) return PS_OK;
+  // PARASUITE_B200_DEBUG: the shape of the call -- segments, compact size M, reported range [lo, hi), head and tail
+  const bool dbg = getenv("PARASUITE_B200_DEBUG") != nullptr;
+  auto print_shape = [&](uint64_t M, uint64_t reported) {
+    if (dbg)
+      fprintf(stderr, "[ps_track] segments %u, compact %llu, reported %llu, head %u, tail %u\n", n_segs,
+              (unsigned long long)M, (unsigned long long)reported, out->head.len, out->tail.len);
+  };
+  if (n_segs == 0) { print_shape(0, 0); return PS_OK; }
   out->first_key = hh.s.first_key;
   out->last_key = hh.total.y;
   out->max_end_key = hh.total.x;
@@ -644,6 +663,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   out->ctr.n_runs[0] = cnt[0];
   out->ctr.n_runs[1] = cnt[2];
   out->ctr.n_sites = cnt[4];
+  print_shape(M, nr);
   return PS_OK;
 }
 
@@ -657,6 +677,7 @@ static DeviceBatch tr_view_of(const ps_read_batch* b) {
   v.cigar = b->cigar; v.tile_base_off = b->tile_base_off; v.tile_qual_off = b->tile_qual_off;
   v.tile_cigar_off = b->tile_cigar_off; v.tile_exc_off = b->tile_exc_off; v.exc = b->exc;
   v.uniform_len = b->uniform_len; v.uniform_ncigar = b->uniform_ncigar; v.cigar_count = b->cigar_count; v.max_len = b->max_len;
+  v.past_end = b->past_end;
   return v;
 }
 

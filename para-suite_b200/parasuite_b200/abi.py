@@ -15,7 +15,7 @@ CSRC_DIR = os.path.join(ROOT_DIR, "csrc")
 REPO_DIR = os.path.dirname(ROOT_DIR)
 INCLUDE_DIR = os.path.join(REPO_DIR, "include")
 
-PS_ABI_VERSION = 4
+PS_ABI_VERSION = 5
 PS_OK = 0
 PS_ERR_INVALID_ARG = -1
 PS_ERR_NO_DEVICE = -2
@@ -38,6 +38,7 @@ PS_THROW_QUAL_RANGE = 6
 PS_THROW_MASK51 = 7
 PS_THROW_BLOCK_RANGE = 8
 PS_FAULT_CIGAR_OPS = 9
+PS_FAULT_PAST_END = 10
 
 PS_TILE_READS = 256
 PS_RF_UNMAPPED = 0x01
@@ -75,7 +76,7 @@ class ps_read_batch(C.Structure):
                 ("exc", C.c_void_p), ("uniform_len", C.c_uint32), ("uniform_ncigar", C.c_uint32),
                 ("bases_bytes", C.c_uint64), ("qual_bytes", C.c_uint64), ("cigar_count", C.c_uint64),
                 ("exc_count", C.c_uint64), ("max_len", C.c_uint32), ("uniform_cigar", C.c_uint32), ("flags8", C.c_void_p), ("qual6", C.c_void_p), ("start16", C.c_void_p),
-                ("tile_start", C.c_void_p)]
+                ("tile_start", C.c_void_p), ("past_end", C.c_uint64)]
 
 
 class ps_comb_stats(C.Structure):

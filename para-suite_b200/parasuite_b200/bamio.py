@@ -284,7 +284,7 @@ class BamBatcher:
             arr(s.tile_cigar_off, C.c_uint64, nt + 1), arr(s.tile_exc_off, C.c_uint32, nt + 1),
             arr(s.exc, C.c_uint32, s.exc_count + 16), uniform_len=int(s.uniform_len), uniform_ncigar=int(s.uniform_ncigar),
             bases_bytes=int(s.bases_bytes), qual_bytes=int(s.qual_bytes), cigar_count=int(s.cigar_count),
-            exc_count=int(s.exc_count))
+            exc_count=int(s.exc_count), past_end=int(s.past_end))
 
     def close(self):
         if getattr(self, "h", None):

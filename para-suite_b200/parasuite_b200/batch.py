@@ -115,8 +115,9 @@ class ReadBatch:
 
     def __init__(self, n_reads, meta, ref_start, bases2, qual, cigar, tile_base_off, tile_qual_off, tile_cigar_off,
                  tile_exc_off, exc, uniform_len=0, uniform_ncigar=0, bases_bytes=None, qual_bytes=None,
-                 cigar_count=None, exc_count=None):
+                 cigar_count=None, exc_count=None, past_end=0):
         self.n_reads = int(n_reads)
+        self.past_end = int(past_end)      # 1 + ordinal of the first record past its contig's end (ps_read_batch.past_end)
         self.meta = meta
         self.ref_start = ref_start
         self.bases2 = bases2
@@ -152,6 +153,7 @@ class ReadBatch:
         s.cigar_count = self.cigar_count
         s.exc_count = self.exc_count
         s.max_len = self.max_len
+        s.past_end = self.past_end
         return s
 
     def algorithmic_bytes(self, with_qual: bool = True) -> int:
@@ -178,6 +180,7 @@ class ReadBatch:
         n = len(records)
         T = abi.PS_TILE_READS
         n_tiles = (n + T - 1) // T
+        past_end = 0
         meta = np.zeros(n, dtype=np.uint32)
         ref_start = np.zeros(n, dtype=np.uint32)
         bases = bytearray()
@@ -233,6 +236,10 @@ class ReadBatch:
                     # htsjdk getSubsequenceAt(chr, pos, pos+R-1) throws iff stop > contig length
                     if rec.pos - 1 + R > ref.lengths[ci]:
                         fl |= abi.PS_RF_REF_RANGE
+                    if R == 0 and rec.pos > ref.lengths[ci] and not fl & abi.PS_RF_CIGAR_OVERFLOW:
+                        # no reference span, POS past the contig's end: as the native batcher (ps_read_batch.past_end)
+                        g = int(ref.contig_off[ci]) + ref.lengths[ci] - 1
+                        past_end = past_end or r + 1
                     ref_start[r] = min(g, 0xFFFFFFFF)
             meta[r] = (L & 0xFFFF) | ((len(ops) & 0xFF) << 16) | (fl << 24)
             lens.add(L)
@@ -246,4 +253,5 @@ class ReadBatch:
         ul = lens.pop() if len(lens) == 1 else 0
         uc = ncigs.pop() if len(ncigs) == 1 else 0
         return cls(n, meta, ref_start, bases2, qual, cigar, tb, tq, tc, te, exc_a, uniform_len=ul, uniform_ncigar=uc,
-                   bases_bytes=len(bases), qual_bytes=len(quals), cigar_count=len(cig), exc_count=len(exc))
+                   bases_bytes=len(bases), qual_bytes=len(quals), cigar_count=len(cig), exc_count=len(exc),
+                   past_end=past_end)

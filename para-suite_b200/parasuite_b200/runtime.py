@@ -21,7 +21,7 @@ def _check(lib, ctx, st, fault=None):
     msg = lib.ps_last_error(ctx).decode() if ctx else lib.ps_strerror(st).decode()
     if st == abi.PS_ERR_REFERENCE_WOULD_THROW:
         raise abi.ReferenceWouldThrow(st, msg, fault)
-    raise abi.PsError(st, msg or lib.ps_strerror(st).decode())
+    raise abi.PsError(st, msg or lib.ps_strerror(st).decode(), fault)
 
 
 class DeviceBatch:
@@ -201,7 +201,7 @@ class Context:
         st = self.lib.ps_pileup_bam(self.h, bam_path.encode(), C.byref(opts), C.byref(h))
         res = PileupResult(self, h, None)
         try:
-            if st == abi.PS_ERR_REFERENCE_WOULD_THROW and h:
+            if st in (abi.PS_ERR_REFERENCE_WOULD_THROW, abi.PS_ERR_UNSUPPORTED) and h:
                 f = abi.ps_fault()
                 self.lib.ps_pileup_fault(h, C.byref(f))
                 _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
@@ -375,7 +375,7 @@ class Context:
             st = self.lib.ps_pileup_batch(self.h, C.byref(s), C.byref(opts), C.byref(h))
         res = PileupResult(self, h, batch)
         try:
-            if st == abi.PS_ERR_REFERENCE_WOULD_THROW and h:
+            if st in (abi.PS_ERR_REFERENCE_WOULD_THROW, abi.PS_ERR_UNSUPPORTED) and h:
                 f = abi.ps_fault()
                 self.lib.ps_pileup_fault(h, C.byref(f))
                 _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
@@ -495,7 +495,7 @@ class PileupResult:
             return self
         self._pending = False
         st = self.ctx.lib.ps_pileup_wait(self.h)
-        if st == abi.PS_ERR_REFERENCE_WOULD_THROW:
+        if st in (abi.PS_ERR_REFERENCE_WOULD_THROW, abi.PS_ERR_UNSUPPORTED):
             f = abi.ps_fault()
             self.ctx.lib.ps_pileup_fault(self.h, C.byref(f))
             _check(self.ctx.lib, self.ctx.h, st, fault=(f.code, f.read_ordinal))

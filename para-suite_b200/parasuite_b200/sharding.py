@@ -65,7 +65,7 @@ def slice_batch(b: ReadBatch, lo: int, hi: int) -> ReadBatch:
         np.concatenate((b.cigar[c_lo:c_hi], pad32)), np.ascontiguousarray(boff), np.ascontiguousarray(qoff),
         np.ascontiguousarray(coff), teo, np.concatenate((exc, pad32)), uniform_len=b.uniform_len,
         uniform_ncigar=b.uniform_ncigar, bases_bytes=b_hi - b_lo, qual_bytes=q_hi - q_lo, cigar_count=c_hi - c_lo,
-        exc_count=len(exc))
+        exc_count=len(exc), past_end=b.past_end - lo if lo < b.past_end <= hi else 0)
 
 
 def take_uniform(b: ReadBatch, idx: np.ndarray) -> ReadBatch:
@@ -83,7 +83,8 @@ def take_uniform(b: ReadBatch, idx: np.ndarray) -> ReadBatch:
         n, np.ascontiguousarray(b.meta[idx]), np.ascontiguousarray(b.ref_start[idx]), np.concatenate((bases, pad8)),
         np.concatenate((qual, pad8)), np.concatenate((b.cigar[: b.n_reads][idx], pad32)), edges * np.uint64(bb),
         edges * np.uint64(L), edges.copy(), np.zeros(n_tiles + 1, dtype=np.uint32), pad32.copy(), uniform_len=L,
-        uniform_ncigar=1, bases_bytes=n * bb, qual_bytes=n * L, cigar_count=n, exc_count=0)
+        uniform_ncigar=1, bases_bytes=n * bb, qual_bytes=n * L, cigar_count=n, exc_count=0,
+        past_end=int(np.searchsorted(idx, b.past_end - 1)) + 1 if b.past_end and b.past_end - 1 in idx else 0)
 
 
 def shard_ranges(n_reads: int, world: int) -> List[Tuple[int, int]]:
