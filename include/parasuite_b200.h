@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define PS_ABI_VERSION 5
+#define PS_ABI_VERSION 6
 
 /* ---- status codes ------------------------------------------------------------------------ */
 #define PS_OK 0
@@ -419,6 +419,45 @@ int64_t ps_track_runs(const ps_track* h, int strand, uint64_t first, ps_track_ru
 int64_t ps_track_sites(const ps_track* h, uint64_t first, ps_track_site* sites, uint64_t max);
 int ps_track_fault(const ps_track* h, ps_fault* out);
 void ps_track_close(ps_track* h);
+/* Per-position base counts (opts->base_counts != 0), beside the runs and sites, which stay as they are:
+ * - Scope: the records, faults, ordinals, positions and strand rule of the track.  Every aligned base at a position whose
+ *   reference is ACGTacgt is counted by read base A, C, G, T or N; N is a base listed in `exc`, whatever bases2 holds.
+ *   Positions whose reference is not ACGT give no row and count toward no total (their coverage is in the runs as ever).
+ * - Orientation: bases on the read's strand.  On the minus strand reference and read base are complemented, so ref T /
+ *   column C is T>C on both strands: for a row with ref T, n[1] is the t2c of the site at (pos, strand), 0 without one.
+ * - A position gets a row on a strand when that strand's coverage is >= min_coverage and the selected substitutions
+ *   there number >= min_events.  substitutions: bit 4 * ref + read (A0 C1 G2 T3, strand orientation); diagonal bits are
+ *   ignored; 0 selects all twelve; bits above 15 give PS_ERR_INVALID_ARG.  N calls are never events; a threshold of 0
+ *   counts as 1.
+ * - Rows come in the sites' order: contigs in the order the records visit them, then by position, plus before minus.
+ * - totals.bases[strand][ref][read] counts every counted base, with or without a row: its cells sum to the aligned bases
+ *   at ACGT reference positions, and bases[s][3][1] == t2c_events[s].  ps_track_counters is the same with or without. */
+typedef struct ps_track_opts {
+  uint32_t base_counts;          /* 0: the plain track */
+  uint32_t min_coverage;
+  uint32_t min_events;
+  uint32_t substitutions;        /* 16-bit mask, 0 = all twelve */
+} ps_track_opts;
+typedef struct ps_track_base_row { /* 36 B */
+  uint32_t contig;               /* FASTA index */
+  int32_t pos;                   /* 1-based */
+  uint8_t strand;                /* 0 plus, 1 minus */
+  uint8_t ref;                   /* reference base in strand orientation, A0 C1 G2 T3 */
+  uint16_t reserved;
+  uint32_t cov;                  /* coverage of that strand at pos = n[0] + ... + n[4] */
+  uint32_t n[5];                 /* read bases A, C, G, T, N in strand orientation */
+} ps_track_base_row;
+typedef struct ps_track_base_totals {
+  uint64_t bases[2][4][5];       /* [strand][ref][read A C G T N] */
+  uint64_t n_rows;
+} ps_track_base_totals;
+/* opts == NULL: ps_track_batch / ps_track_batch_device */
+int ps_track_batch_ex(ps_ctx* ctx, const ps_read_batch* host_batch, const ps_track_opts* opts, ps_track** out);
+int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* dev_batch, const ps_track_opts* opts, void* stream,
+                             ps_track** out);
+/* PS_ERR_STATE on a handle made without base counts; rows: copy up to `max` from `first`, returns the number copied */
+int64_t ps_track_base_rows(const ps_track* h, uint64_t first, ps_track_base_row* rows, uint64_t max);
+int ps_track_base_totals_get(const ps_track* h, ps_track_base_totals* out);
 /* The tool from files: <out_prefix>.plus.bedGraph and <out_prefix>.minus.bedGraph (chrom, start0, end0, coverage; no
  * header; one row per maximal run of equal non-zero coverage) and <out_prefix>.t2c.tsv (header
  * chrom/pos/strand/t2c/coverage, one row per (position, strand) with t2c >= 1, pos 1-based).  Contigs come in the order the
@@ -427,6 +466,11 @@ void ps_track_close(ps_track* h);
  * with ps_reference_load_fasta / ps_multi_load_fasta (contig names).  counters_out / fault_out may be NULL. */
 int ps_track_bam(ps_ctx* ctx, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
                  ps_fault* fault_out);
+/* With opts->base_counts also <out_prefix>.bases.tsv (header chrom/pos/strand/ref/coverage/A/C/G/T/N, the rows of
+ * ps_track_base_rows, pos 1-based), independent of the window size and the number of devices; the other three files are
+ * byte-identical to ps_track_bam's.  opts == NULL: ps_track_bam.  totals_out may be NULL. */
+int ps_track_bam_ex(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                    ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out);
 
 /* ---- `comb` tool (host only): transcript hits lifted to genomic coordinates, merged with the genomic hits ---------------
  * Replaces CombineGenomeTranscript.combine / printReadsToBamFile (utils/postprocessing/CombineGenomeTranscript.java:36-666;
@@ -467,6 +511,8 @@ int ps_multi_clust_bam(ps_multi* m, const char* bam_path, const char* out_path, 
 /* windows round-robin over the devices; the files are byte-identical to ps_track_bam's */
 int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
                        ps_fault* fault_out);
+int ps_multi_track_bam_ex(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                          ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out);
 
 /* ---- host batcher (usable without a GPU) --------------------------------------------------------
  * What htsjdk does for the two loops, as a library: FASTA(+.fai) -> packed reference; BGZF/BAM -> SoA batches in

@@ -161,7 +161,7 @@ struct ps_ctx {
   bool pl_compact_lookback = false;   // PARASUITE_B200_COMPACT_LOOKBACK=1 at ps_create: always order the site runs with the look-back (tests)
   bool pl_exact_flags = false;   // a speculative flag pass failed on this context: keep to the exact look-back kernel
   // track scratch (track.cu): run state, keys, scans, segments, position arrays, selections, records, dense head / tail
-  DevBuf tr_scratch[12];
+  DevBuf tr_scratch[13];
 };
 
 // ---- pileup handles over host-resident records (pileup.cu; used by the windowed file loops in tool_loops.cpp) --------

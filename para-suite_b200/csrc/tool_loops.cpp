@@ -19,7 +19,8 @@
 //                   it and before its own last kept start; its head (up to that maximum end) and its tail (from its last
 //                   kept start on) come back as dense arrays, added on the host into one pending region -- in a sorted
 //                   file no later record reaches a position before the last kept start, so the region is bounded by the
-//                   longest reference span of a record.
+//                   longest reference span of a record.  With base counts the region also holds the ten event
+//                   counters, and its base rows take their reference base from the host packed FASTA.
 // No compute happens on the host: boundaries, masks, counts and sites all come from the kernels.
 #include <algorithm>
 #include <cstdio>
@@ -371,23 +372,26 @@ int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts
 
 
 // ---- track files -------------------------------------------------------------------------------------------------------
-// The three files of the track tool.  Runs that touch with equal coverage are merged, so a run cut by a window boundary
-// is one row.
+// The files of the track tool: three, and with base counts a fourth.  Runs that touch with equal coverage are merged, so
+// a run cut by a window boundary is one row.
 struct TrackWriter {
-  FILE* f[3] = {nullptr, nullptr, nullptr};      // plus bedGraph, minus bedGraph, t2c tsv
+  FILE* f[4] = {nullptr, nullptr, nullptr, nullptr};   // plus bedGraph, minus bedGraph, t2c tsv, bases tsv
+  int nf = 3;
   std::vector<std::string> names;
   ps_track_run last[2]{};
   bool have[2] = {false, false};
-  uint64_t rows[3] = {0, 0, 0};
+  uint64_t rows[4] = {0, 0, 0, 0};
   uint64_t merged[2] = {0, 0};                  // runs joined to the one before
-  std::string buf[3];
-  int open(const std::string& prefix) {
-    const char* ext[3] = {".plus.bedGraph", ".minus.bedGraph", ".t2c.tsv"};
-    for (int k = 0; k < 3; ++k) {
+  std::string buf[4];
+  int open(const std::string& prefix, bool bases) {
+    const char* ext[4] = {".plus.bedGraph", ".minus.bedGraph", ".t2c.tsv", ".bases.tsv"};
+    nf = bases ? 4 : 3;
+    for (int k = 0; k < nf; ++k) {
       f[k] = fopen((prefix + ext[k]).c_str(), "wb");
       if (!f[k]) return PS_ERR_IO;
     }
     buf[2] = "chrom\tpos\tstrand\tt2c\tcoverage\n";
+    if (bases) buf[3] = "chrom\tpos\tstrand\tref\tcoverage\tA\tC\tG\tT\tN\n";
     return PS_OK;
   }
   static void num(std::string& b, uint64_t v) {
@@ -434,25 +438,52 @@ struct TrackWriter {
     ++rows[2];
     return drain(2, false);
   }
+  int base_row(const ps_track_base_row& x) {
+    std::string& b = buf[3];
+    b += names[x.contig]; b.push_back('\t');
+    num(b, (uint32_t)x.pos); b.push_back('\t');
+    b.push_back(x.strand ? '-' : '+'); b.push_back('\t');
+    b.push_back("ACGT"[x.ref & 3]);
+    b.push_back('\t'); num(b, x.cov);
+    for (int k = 0; k < 5; ++k) { b.push_back('\t'); num(b, x.n[k]); }
+    b.push_back('\n');
+    ++rows[3];
+    return drain(3, false);
+  }
   int finish() {
     int rc = PS_OK;
     for (int s = 0; s < 2; ++s) if (rc == PS_OK) rc = flush_run(s);
-    for (int k = 0; k < 3; ++k) if (rc == PS_OK) rc = drain(k, true);
+    for (int k = 0; k < nf; ++k) if (rc == PS_OK) rc = drain(k, true);
     return rc;
   }
   ~TrackWriter() { for (FILE* x : f) if (x) fclose(x); }
+  // the rows of one window, in file order
+  int write(const std::vector<ps_track_run>* runs, const std::vector<ps_track_site>& sites,
+            const std::vector<ps_track_base_row>& base_rows) {
+    int rc = PS_OK;
+    for (int s = 0; s < 2 && rc == PS_OK; ++s)
+      for (const ps_track_run& r : runs[s]) if ((rc = run(s, r)) != PS_OK) break;
+    for (const ps_track_site& x : sites) if (rc != PS_OK || (rc = site(x)) != PS_OK) break;
+    for (const ps_track_base_row& x : base_rows) if (rc != PS_OK || (rc = base_row(x)) != PS_OK) break;
+    return rc;
+  }
 };
 
-// what a window hands to the writer: final runs and sites, in file order
+// what a window hands to the writer: final runs, sites and base rows, in file order
 struct TrackRows {
   std::vector<ps_track_run> runs[2];
   std::vector<ps_track_site> sites;
+  std::vector<ps_track_base_row> base_rows;
 };
 
-// positions not final yet: [key0, key0 + len) of one contig, cov+, cov-, t2c+, t2c-
+// positions not final yet: [key0, key0 + len) of one contig, cov+, cov-, t2c+, t2c-, and with base counts the ten
+// event counters (TrackDense)
 struct TrackPending {
   unsigned long long key0 = 0;
-  std::vector<uint32_t> v[4];
+  std::vector<uint32_t> v[14];
+  int nv = 4;
+  TrackBases bases;
+  const ps_reference* ref = nullptr;     // host packed FASTA: the reference base of a base row
   size_t len() const { return v[0].size(); }
   // rows of the positions before `upto` (keys), which leave the region
   void emit_before(unsigned long long upto, const std::vector<uint32_t>& by_rank, TrackRows& out) {
@@ -474,7 +505,22 @@ struct TrackPending {
     for (size_t k = 0; k < k_end; ++k)
       for (int s = 0; s < 2; ++s)
         if (v[2 + s][k]) out.sites.push_back(ps_track_site{contig, (int32_t)(p0 + k + 1), (uint32_t)s, v[2 + s][k], v[s][k]});
-    for (auto& a : v) a.erase(a.begin(), a.begin() + (ptrdiff_t)k_end);
+    if (bases.on)
+      for (size_t k = 0; k < k_end; ++k) {
+        const uint64_t g = ref->contig_off[contig] + p0 + k;
+        if ((ref->inv[g >> 5] >> (g & 31)) & 1u) continue;
+        const uint32_t c = (ref->seq2[g >> 4] >> (2 * (g & 15))) & 3u;
+        for (int s = 0; s < 2; ++s) {
+          uint32_t ev[5];
+          for (int b = 0; b < 5; ++b) ev[b] = v[4 + 5 * s + b][k];
+          ps_track_base_row x{};
+          const uint32_t a = c ^ (s ? 3u : 0u);
+          if (!track_base_row(bases, a, v[s][k], ev, x.n)) continue;
+          x.contig = contig; x.pos = (int32_t)(p0 + k + 1); x.strand = (uint8_t)s; x.ref = (uint8_t)a; x.cov = v[s][k];
+          out.base_rows.push_back(x);
+        }
+      }
+    for (int j = 0; j < nv; ++j) v[j].erase(v[j].begin(), v[j].begin() + (ptrdiff_t)k_end);
     key0 += k_end;
   }
 };
@@ -490,12 +536,17 @@ struct TrackFlight {
 };
 
 // The windowed track over an open file (contexts keyed in the file's contig order)
-int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters* ctr, ps_fault* fault) {
+int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWriter& W, ps_track_counters* ctr,
+                      ps_track_base_totals* totals, ps_fault* fault) {
   ps_ctx* c0 = m->ctx[0];
   const std::vector<uint64_t>& contig_off = c0->contig_off;
   const std::vector<uint32_t>& by_rank = c0->contig_by_rank;
   memset(ctr, 0, sizeof *ctr);
+  memset(totals, 0, sizeof *totals);
   TrackPending P;
+  P.bases = bases;
+  P.nv = bases.on ? 14 : 4;
+  P.ref = ps_fasta_reference(c0->fasta);
   unsigned long long last_start = 0, max_end = 0;     // over the windows launched so far / completed so far
   uint64_t offset = 0, window = 0;
   TrackFlight fl[2];
@@ -528,13 +579,16 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
     ctr->reads_counted += o.ctr.reads_counted;
     ctr->fast_path_reads += o.ctr.fast_path_reads;
     for (int s = 0; s < 2; ++s) { ctr->aligned_bases[s] += o.ctr.aligned_bases[s]; ctr->t2c_events[s] += o.ctr.t2c_events[s]; }
+    for (int s = 0; s < 2; ++s)
+      for (int a = 0; a < 4; ++a)
+        for (int c = 0; c < 5; ++c) totals->bases[s][a][c] += o.totals.bases[s][a][c];
     if (!o.first_key) { print_window(o, 0); return PS_OK; }      // no kept record: nothing changes
     if (o.first_key < last_start) return multi_fail(m, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
     if (o.head.len) {
       if (o.head.key0 < P.key0 || o.head.key0 + o.head.len > P.key0 + P.len())
         return multi_fail(m, PS_ERR_STATE, "track: window head outside the pending region");
       const size_t at = (size_t)(o.head.key0 - P.key0);
-      for (int j = 0; j < 4; ++j)
+      for (int j = 0; j < P.nv; ++j)
         for (uint32_t k = 0; k < o.head.len; ++k) P.v[j][at + k] += o.head.v[(size_t)j * o.head.len + k];
     }
     auto rows = std::make_shared<TrackRows>();
@@ -543,22 +597,17 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
     const size_t emitted = pending_before - P.len();
     for (int s = 0; s < 2; ++s) rows->runs[s].insert(rows->runs[s].end(), o.runs[s].begin(), o.runs[s].end());
     rows->sites.insert(rows->sites.end(), o.sites.begin(), o.sites.end());
+    rows->base_rows.insert(rows->base_rows.end(), o.base_rows.begin(), o.base_rows.end());
     if (o.tail.len) {
       if (P.len() && P.key0 + P.len() != o.tail.key0) return multi_fail(m, PS_ERR_STATE, "track: window tail not next to the pending region");
       if (!P.len()) P.key0 = o.tail.key0;
-      for (int j = 0; j < 4; ++j) P.v[j].insert(P.v[j].end(), o.tail.v.begin() + (ptrdiff_t)j * o.tail.len, o.tail.v.begin() + (ptrdiff_t)(j + 1) * o.tail.len);
+      for (int j = 0; j < P.nv; ++j) P.v[j].insert(P.v[j].end(), o.tail.v.begin() + (ptrdiff_t)j * o.tail.len, o.tail.v.begin() + (ptrdiff_t)(j + 1) * o.tail.len);
     }
     last_start = o.last_key;
     print_window(o, emitted);
     const int prev_rc = join_sink();
     if (prev_rc != PS_OK) return prev_rc;
-    sink_thread = std::thread([&W, &sink_rc, rows] {
-      int rc = PS_OK;
-      for (int s = 0; s < 2 && rc == PS_OK; ++s)
-        for (const ps_track_run& r : rows->runs[s]) if ((rc = W.run(s, r)) != PS_OK) break;
-      for (const ps_track_site& x : rows->sites) if (rc != PS_OK || (rc = W.site(x)) != PS_OK) break;
-      sink_rc = rc;
-    });
+    sink_thread = std::thread([&W, &sink_rc, rows] { sink_rc = W.write(rows->runs, rows->sites, rows->base_rows); });
     return PS_OK;
   };
   int st = PS_OK;
@@ -579,9 +628,9 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
     f.ctx = c; f.offset = offset; f.rc = PS_OK; f.live = true;
     const DeviceBatch view = sb->view;
     const uint64_t prev_end = max_end;
-    f.th = std::thread([&f, c, view, prev_end] {
+    f.th = std::thread([&f, c, view, prev_end, &bases] {
       cudaSetDevice(c->device);
-      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out);
+      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out, bases);
       if (f.rc != PS_OK) f.err = c->err;
     });
     max_end = std::max<unsigned long long>(max_end, host_max_key(hb, contig_off, c0->contig_rank));
@@ -600,14 +649,13 @@ int track_windows_run(ps_multi* m, ps_bam* B, TrackWriter& W, ps_track_counters*
   if (st != PS_OK) return st;
   TrackRows rest;
   P.emit_before(~0ull, by_rank, rest);
-  for (int s = 0; s < 2 && st == PS_OK; ++s)
-    for (const ps_track_run& r : rest.runs[s]) if ((st = W.run(s, r)) != PS_OK) break;
-  for (const ps_track_site& x : rest.sites) if (st != PS_OK || (st = W.site(x)) != PS_OK) break;
+  st = W.write(rest.runs, rest.sites, rest.base_rows);
   if (st == PS_OK) st = W.finish();
   if (st != PS_OK) return multi_fail(m, st, "track: writing the output files failed");
   ctr->n_runs[0] = W.rows[0];
   ctr->n_runs[1] = W.rows[1];
   ctr->n_sites = W.rows[2];
+  totals->n_rows = W.rows[3];
   if (dbg)
     fprintf(stderr, "[ps_track_files] runs %llu %llu, merged %llu %llu, sites %llu\n", (unsigned long long)W.rows[0],
             (unsigned long long)W.rows[1], (unsigned long long)W.merged[0], (unsigned long long)W.merged[1],
@@ -882,32 +930,48 @@ int ps_clust_bam(ps_ctx* ctx, const char* bam_path, const char* out_path, const 
   return st;
 }
 
-// The track tool from files: <out_prefix>.plus.bedGraph, .minus.bedGraph, .t2c.tsv
-int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
-                       ps_fault* fault_out) {
+// The track tool from files: <out_prefix>.plus.bedGraph, .minus.bedGraph, .t2c.tsv, and with base counts .bases.tsv
+int ps_multi_track_bam_ex(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                          ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out) {
   if (!m || !bam_path || !out_prefix) return PS_ERR_INVALID_ARG;
+  TrackBases bases;
+  if (track_bases_of(opts, &bases) != PS_OK) return multi_fail(m, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
   if (m->ctx.empty() || !m->ctx[0]->fasta) return multi_fail(m, PS_ERR_STATE, "load the reference first (ps_multi_load_fasta)");
   ps_ctx* c0 = m->ctx[0];
   TrackWriter W;
   for (uint32_t i = 0; i < c0->ref.n_contigs; ++i) W.names.push_back(ps_fasta_contig_name(c0->fasta, i));
-  int st = W.open(out_prefix);
+  int st = W.open(out_prefix, bases.on);
   if (st != PS_OK) return multi_fail(m, st, std::string("cannot write ") + out_prefix + ".*");
   ps_track_counters ctr{};
+  ps_track_base_totals totals{};
   ps_fault fault{};
-  st = with_file_order(m, bam_path, window_reads_default(), [&](ps_bam* B) { return track_windows_run(m, B, W, &ctr, &fault); });
+  st = with_file_order(m, bam_path, window_reads_default(), [&](ps_bam* B) {
+    return track_windows_run(m, B, bases, W, &ctr, &totals, &fault);
+  });
   if (counters_out) *counters_out = ctr;
+  if (totals_out) *totals_out = totals;
   if (fault_out) *fault_out = fault;
+  return st;
+}
+
+int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
+                       ps_fault* fault_out) {
+  return ps_multi_track_bam_ex(m, bam_path, out_prefix, nullptr, counters_out, nullptr, fault_out);
+}
+
+int ps_track_bam_ex(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                    ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out) {
+  if (!ctx || !bam_path || !out_prefix) return set_error(ctx, PS_ERR_INVALID_ARG, "NULL argument");
+  ps_multi m;
+  borrow(m, ctx);
+  const int st = ps_multi_track_bam_ex(&m, bam_path, out_prefix, opts, counters_out, totals_out, fault_out);
+  if (st != PS_OK && !m.err.empty()) set_error(ctx, st, m.err);
   return st;
 }
 
 int ps_track_bam(ps_ctx* ctx, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
                  ps_fault* fault_out) {
-  if (!ctx || !bam_path || !out_prefix) return set_error(ctx, PS_ERR_INVALID_ARG, "NULL argument");
-  ps_multi m;
-  borrow(m, ctx);
-  const int st = ps_multi_track_bam(&m, bam_path, out_prefix, counters_out, fault_out);
-  if (st != PS_OK && !m.err.empty()) set_error(ctx, st, m.err);
-  return st;
+  return ps_track_bam_ex(ctx, bam_path, out_prefix, nullptr, counters_out, nullptr, fault_out);
 }
 
 }  // extern "C"

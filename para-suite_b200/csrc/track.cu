@@ -17,11 +17,15 @@
 //   tr_seg_bounds_kernel first read and maximum end of every segment
 //   tr_seg_len_kernel    segment length + 1 slot for the -1 one past its end; (CUB) exclusive sum = compact base
 //   tr_seg_place_kernel  compact index range that is reported (windowed file tool: head and tail stay dense)
-//   tr_accum_kernel<NW>  per read: +1/-1 per alignment block into one int32 difference array per strand, +1 per T>C
-//                        event.  NW > 0: uniform length <= 64, one M/=/X op -- T>C bits found bit-parallel on the 2-bit
-//                        words of read and reference
+//   tr_accum_kernel<NW, BC>  per read: +1/-1 per alignment block into one int32 difference array per strand, +1 per
+//                        T>C event.  NW > 0: uniform length <= 64, one M/=/X op -- T>C bits found bit-parallel on the
+//                        2-bit words of read and reference.  BC (base counts): also +1 per event -- a read base other
+//                        than the reference base, or an N call -- into five uint32 counters (A C G T N, strand
+//                        orientation) per position and strand, and the genome-wide matrix in block-shared counters
 //   (CUB) sum scan       of each difference array = coverage (every segment's differences sum to zero)
-//   (CUB) select         run starts / ends per strand, T>C sites; tr_emit_*_kernel turn them into records
+//   (CUB) select         run starts / ends per strand, T>C sites; tr_emit_*_kernel turn them into records.  BC: a select
+//                        of the (position, strand) items with >= min_events non-N events, then tr_base_rows_kernel
+//                        (reference base, mask, min_coverage) and a select of the rows it kept
 // Compact space: M = sum over segments of (span + 1) <= sum over kept reads of (reference span + 1).
 #include <cub/cub.cuh>
 #include <thrust/iterator/counting_iterator.h>
@@ -51,6 +55,7 @@ struct TrState {
   unsigned long long first_key;      // min start key over the kept reads (~0: none)
   unsigned long long lo, hi;         // reported compact range [lo, hi)
   unsigned int unsorted;
+  unsigned long long bases[2][4][5]; // base counts: [strand][ref][read A C G T N], strand orientation
 };
 
 struct TrParams {
@@ -70,6 +75,7 @@ struct TrParams {
   uint64_t M;
   unsigned long long prev_end;       // windowed: max end key over the earlier windows (0: none)
   int windowed;
+  uint32_t* bc;                      // base counts: [2][5][M] events by read base A C G T N (strand orientation)
 };
 
 struct MaxPair {
@@ -265,11 +271,102 @@ __device__ __noinline__ void tr_accum_generic(const TrParams& P, uint64_t r, uin
   }
 }
 
+// base counts of one read, any CIGAR: an event per read base other than the reference base and per N call into P.bc,
+// every counted base into the block's matrix `tb` ([2][4][5], shared)
+__device__ __noinline__ void tr_bases_generic(const TrParams& P, uint64_t r, uint32_t meta, uint64_t off_base,
+                                              uint64_t off_cigar, int64_t to_compact, unsigned long long* tb) {
+  const uint32_t flags = PS_META_FLAGS(meta), ncig = PS_META_NCIGAR(meta);
+  const uint32_t* cig = P.b.cigar + off_cigar;
+  const bool rev = flags & PS_RF_REVERSE, has_inv = flags & PS_RF_HAS_INVALID;
+  const int s = rev ? 1 : 0;
+  const uint32_t flip = rev ? 3u : 0u;             // minus strand: complement (A0 <-> T3, C1 <-> G2)
+  uint32_t* bc = P.bc + (size_t)s * 5 * P.M;
+  tb += s * 20;
+  const uint8_t* rb = P.b.bases2 + off_base;
+  const uint64_t g0 = __ldg(P.b.ref_start + r);
+  ExcRange ex{0, 0};
+  if (has_inv) ex = read_exc_range(P.b, r / PS_TILE_READS, (uint32_t)(r % PS_TILE_READS));
+  int64_t rdp = 0, rfp = 0;
+  for (uint32_t e = 0; e < ncig; ++e) {
+    const uint32_t c = __ldg(cig + e), op = c & 15u;
+    const int64_t n = c >> 4;
+    if (op == 4u || op == 1u) rdp += n;
+    else if (op == 2u || op == 3u) rfp += n;
+    else if (op_is_match(op)) {
+      for (int64_t z = 0; z < n; ++z) {
+        const uint64_t g = g0 + (uint64_t)(rfp + z);
+        const uint32_t p = (uint32_t)(rdp + z);
+        if (ref_invalid_at(P.ref, g)) continue;
+        const uint32_t a = ref_code_at(P.ref, g) ^ flip;
+        const uint32_t bb = (has_inv && read_pos_invalid(P.b, ex, p)) ? 4u : (read_code_at(rb, p) ^ flip);
+        if (bb != a) atomicAdd(bc + (size_t)bb * P.M + (uint64_t)((int64_t)g + to_compact), 1u);
+        atomicAdd(tb + a * 5 + bb, 1ull);
+      }
+      rdp += n; rfp += n;
+    }
+  }
+}
+
+// base counts of one read on the bit-parallel path: mismatches are (ref ^ read) folded to one bit per base, N calls the
+// positions listed in `exc`; the matrix diagonal is one popcount per reference base minus its events and N calls
+template <int NW>
+__device__ __forceinline__ void tr_bases_fast(const TrParams& P, const uint32_t (&w)[NW + 1], const uint32_t (&bw)[NW + 1],
+                                              uint32_t sh, uint32_t bsh, unsigned long long inv, uint32_t L, uint32_t meta,
+                                              uint64_t r, int st, int64_t c0, unsigned long long* tb) {
+  const unsigned long long valid = ~inv & (L >= 64 ? ~0ull : ((1ull << L) - 1ull));
+  const unsigned long long nm = (PS_META_FLAGS(meta) & PS_RF_HAS_INVALID) ? (read_exc_mask64(P.b, r) & valid) : 0ull;
+  const uint32_t flip = st ? 3u : 0u;
+  uint32_t* bc = P.bc + (size_t)st * 5 * P.M + c0;
+  tb += st * 20;
+  unsigned long long lo = 0, hi = 0, mm = 0;
+#pragma unroll
+  for (int j = 0; j < NW; ++j) {
+    const uint32_t rf = __funnelshift_r(w[j], w[j + 1], sh), rd = __funnelshift_r(bw[j], bw[j + 1], bsh), x = rf ^ rd;
+    lo |= (unsigned long long)tr_even_bits(rf) << (16 * j);
+    hi |= (unsigned long long)tr_even_bits(rf >> 1) << (16 * j);
+    mm |= (unsigned long long)tr_even_bits(x | (x >> 1)) << (16 * j);
+  }
+  mm &= valid & ~nm;
+#pragma unroll
+  for (uint32_t c = 0; c < 4; ++c) {
+    const unsigned long long rc = ((c & 2u) ? hi : ~hi) & ((c & 1u) ? lo : ~lo) & valid;
+    const uint32_t all = (uint32_t)__popcll(rc), nn = (uint32_t)__popcll(rc & nm), ne = (uint32_t)__popcll(rc & mm);
+    const uint32_t a = c ^ flip;
+    if (all != nn + ne) atomicAdd(tb + a * 6, (unsigned long long)(all - nn - ne));      // [a][a]
+    if (nn) atomicAdd(tb + a * 5 + 4, (unsigned long long)nn);
+  }
+#pragma unroll
+  for (int j = 0; j < NW; ++j) {
+    uint32_t me = (uint32_t)(mm >> (16 * j)) & 0xFFFFu;
+    if (!me) continue;
+    const uint32_t rf = __funnelshift_r(w[j], w[j + 1], sh), rd = __funnelshift_r(bw[j], bw[j + 1], bsh);
+    while (me) {
+      const int k = __ffs((int)me) - 1;
+      me &= me - 1;
+      const uint32_t a = ((rf >> (2 * k)) & 3u) ^ flip, b = ((rd >> (2 * k)) & 3u) ^ flip;
+      atomicAdd(bc + (size_t)b * P.M + 16 * j + k, 1u);
+      atomicAdd(tb + a * 5 + b, 1ull);
+    }
+  }
+  for (unsigned long long q = nm; q;) {
+    const int k = __ffsll((long long)q) - 1;
+    q &= q - 1;
+    atomicAdd(bc + 4 * P.M + k, 1u);
+  }
+}
+
 // NW > 0: the batch has uniform length L <= 64 and one cigar op per read; reads whose op is M/=/X of length L take the
 // bit-parallel path (the positions listed in `exc` are cleared from its event mask: the code stored there is arbitrary)
-template <int NW>
+template <int NW, bool BC>
 __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_constant__ TrParams P) {
   unsigned long long ev[2] = {0, 0}, fast = 0;
+  unsigned long long* tb = nullptr;
+  if constexpr (BC) {
+    __shared__ unsigned long long sh_bases[40];
+    for (int k = threadIdx.x; k < 40; k += blockDim.x) sh_bases[k] = 0;
+    __syncthreads();
+    tb = sh_bases;
+  }
   const uint64_t n = P.b.n_reads;
   for (uint64_t q = ((uint64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31u)); q < n; q += (uint64_t)gridDim.x * blockDim.x) {
     const uint64_t r = q + (threadIdx.x & 31u);
@@ -325,17 +422,24 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
           m &= m - 1;
           atomicAdd(t2c + j, 1u);
         }
+        if constexpr (BC) tr_bases_fast<NW>(P, w, bw, sh, bsh, inv, L, meta, r, st, c0, tb);
         ++fast;
         continue;
       }
     }
     tr_accum_generic(P, r, meta, obase, ocig, to_compact, ev);
+    if constexpr (BC) tr_bases_generic(P, r, meta, obase, ocig, to_compact, tb);
   }
   ev[0] = warp_sum(ev[0]); ev[1] = warp_sum(ev[1]); fast = warp_sum(fast);
   if ((threadIdx.x & 31u) == 0) {
     if (ev[0]) atomicAdd(&P.st->t2c[0], ev[0]);
     if (ev[1]) atomicAdd(&P.st->t2c[1], ev[1]);
     if (fast) atomicAdd(&P.st->fast, fast);
+  }
+  if constexpr (BC) {
+    __syncthreads();
+    for (int k = threadIdx.x; k < 40; k += blockDim.x)
+      if (tb[k]) atomicAdd(&P.st->bases[0][0][0] + k, tb[k]);
   }
 }
 
@@ -359,6 +463,17 @@ struct SiteAt {          // item 2*i + strand
   __device__ __forceinline__ bool operator()(const unsigned long long& k) const {
     return t2c[(k & 1ull) * M + (k >> 1)] != 0u;
   }
+};
+
+struct BaseCandidate {   // item 2*i + strand: at least min_ev events other than N calls, whatever their type
+  const uint32_t* bc; uint64_t M; uint32_t min_ev;
+  __device__ __forceinline__ bool operator()(const unsigned long long& k) const {
+    const uint32_t* p = bc + (k & 1ull) * 5 * M + (k >> 1);
+    return p[0] + p[M] + p[2 * M] + p[3 * M] >= min_ev;
+  }
+};
+struct RowKept {
+  __device__ __forceinline__ bool operator()(const ps_track_base_row& x) const { return x.cov != 0u; }
 };
 
 // segment of compact index i (seg_base ascending)
@@ -405,7 +520,36 @@ __global__ void tr_emit_sites_kernel(const __grid_constant__ TrParams P, uint32_
   out[k] = x;
 }
 
-// dense copy of the positions [key0, key0 + len) (one contig) from the compact arrays: cov+, cov-, t2c+, t2c-
+// one base row per candidate (the reference base, the mask and min_coverage decide); cov = 0: no row
+__global__ void tr_base_rows_kernel(const __grid_constant__ TrParams P, uint32_t n_segs, const unsigned long long* cand,
+                                    uint64_t n, TrackBases sel, ps_track_base_row* out) {
+  const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const unsigned long long it = cand[k], i = it >> 1;
+  const uint32_t strand = (uint32_t)(it & 1ull);
+  const uint32_t s = seg_of(P, n_segs, i);
+  const uint64_t g = (uint64_t)P.seg_g[s] + (i - P.seg_base[s]);
+  ps_track_base_row x{};
+  if (!ref_invalid_at(P.ref, g)) {
+    const uint32_t a = ref_code_at(P.ref, g) ^ (strand ? 3u : 0u);
+    const uint32_t cov = (uint32_t)P.diff[(size_t)strand * (P.M + 1) + i];
+    uint32_t ev[5];
+#pragma unroll
+    for (int b = 0; b < 5; ++b) ev[b] = P.bc[((size_t)strand * 5 + b) * P.M + i];
+    if (track_base_row(sel, a, cov, ev, x.n)) {
+      x.contig = P.seg_contig[s];
+      x.pos = (int32_t)pos0_of(P, s, i) + 1;
+      x.strand = (uint8_t)strand;
+      x.ref = (uint8_t)a;
+      x.cov = cov;
+    }
+  }
+  out[k] = x;
+}
+
+// dense copy of the positions [key0, key0 + len) (one contig) from the compact arrays: cov+, cov-, t2c+, t2c-, and with
+// base counts (BC) the ten event counters
+template <bool BC>
 __global__ void tr_dense_kernel(const __grid_constant__ TrParams P, uint32_t n_segs, unsigned long long key0, uint32_t len,
                                 uint32_t* out) {
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -416,7 +560,8 @@ __global__ void tr_dense_kernel(const __grid_constant__ TrParams P, uint32_t n_s
     const uint32_t mid = (lo + hi) >> 1;
     if (P.seg_key[mid] <= key) lo = mid; else hi = mid;
   }
-  uint32_t v[4] = {0, 0, 0, 0};
+  constexpr int NV = BC ? 14 : 4;
+  uint32_t v[NV] = {};
   const unsigned long long k0 = P.seg_key[lo];
   if (key >= k0 && (key >> 32) == (k0 >> 32) && key - k0 < P.seg_end[lo]) {
     const unsigned long long i = P.seg_base[lo] + (key - k0);
@@ -424,9 +569,13 @@ __global__ void tr_dense_kernel(const __grid_constant__ TrParams P, uint32_t n_s
     v[1] = (uint32_t)P.diff[(P.M + 1) + i];
     v[2] = P.t2c[i];
     v[3] = P.t2c[P.M + i];
+    if constexpr (BC) {
+#pragma unroll
+      for (int j = 4; j < NV; ++j) v[j] = P.bc[(size_t)(j - 4) * P.M + i];
+    }
   }
 #pragma unroll
-  for (int j = 0; j < 4; ++j) out[(size_t)j * len + k] = v[j];
+  for (int j = 0; j < NV; ++j) out[(size_t)j * len + k] = v[j];
 }
 
 __global__ void tr_init_state(TrState* st) {
@@ -465,20 +614,35 @@ uint32_t grid_for(uint64_t n, int threads = TR_THREADS) { return (uint32_t)std::
     if (_e != cudaSuccess) return cuda_fail(ctx, _e, #expr); \
   } while (0)
 
-int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out) {
+int track_bases_of(const ps_track_opts* o, TrackBases* out) {
+  *out = TrackBases();
+  if (!o) return PS_OK;
+  if (o->substitutions >> 16) return PS_ERR_INVALID_ARG;
+  out->on = o->base_counts != 0;
+  out->min_cov = std::max<uint32_t>(1u, o->min_coverage);
+  out->min_ev = std::max<uint32_t>(1u, o->min_events);
+  out->mask = (o->substitutions ? o->substitutions : 0xFFFFu) & ~0x8421u;     // diagonal bits 4 * c + c cleared
+  return PS_OK;
+}
+
+int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out,
+              const TrackBases& bases) {
   if (b.past_end && b.past_end <= b.n_reads) {
     // a record past its contig's end: the reads before it decide whether an earlier record faults first
     DeviceBatch head = b;
     head.n_reads = b.past_end - 1;
     head.past_end = 0;
-    const int rc = track_run(ctx, head, st, windowed, prev_end, out);
+    const int rc = track_run(ctx, head, st, windowed, prev_end, out, bases);
     if (rc != PS_OK && rc != PS_ERR_UNSORTED) return rc;
+    out->base_rows.clear();                // a faulting call reports no base rows
+    out->totals = ps_track_base_totals{};
     out->ctr.num_reads_processed = b.n_reads;
     out->fault.code = PS_FAULT_PAST_END;
     out->fault.read_ordinal = b.past_end - 1;
     return set_error(ctx, PS_ERR_UNSUPPORTED, "track: a record with no reference span starts past its contig's end");
   }
   *out = TrackOut();
+  out->bases_on = bases.on;
   const uint64_t n = b.n_reads;
   out->ctr.num_reads_processed = n;
   if (n == 0) return PS_OK;
@@ -494,6 +658,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   const uint32_t grid_g = (uint32_t)std::min<uint64_t>(grid_for(n), (uint64_t)ctx->sm_count * 8);
   timer_begin(ctx, st);
   tr_init_state<<<1, 1, 0, st>>>(d_st);
+  if (bases.on) TR_CUDA(cudaMemsetAsync(d_st->bases, 0, sizeof d_st->bases, st));
   tr_read_kernel<<<grid_g, TR_THREADS, 0, st>>>(P);
   TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceScan::InclusiveScan(t, sz, P.keys, P.scan, MaxPair(), (int64_t)n, st); }));
   tr_segment_kernel<<<grid_for(n), TR_THREADS, 0, st>>>(P);
@@ -556,20 +721,32 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   if (M >= (1ull << 31)) return set_error(ctx, PS_ERR_UNSUPPORTED, "track: the reads of one batch span more than 2^31 positions");
   const uint64_t lo = std::min<uint64_t>(hp.lo, M), hi = std::max<uint64_t>(lo, std::min<uint64_t>(hp.hi, M));
   P.M = M;
-  P.diff = slot<int32_t>(ctx, 5, 4 * (M + 1), err);       // difference arrays / coverage, then the T>C counts
+  // difference arrays / coverage, the T>C counts, then (base counts) the event counters
+  P.diff = slot<int32_t>(ctx, 5, 4 * (M + 1) + (bases.on ? 10 * M : 0), err);
   TR_CUDA(err);
   P.t2c = reinterpret_cast<uint32_t*>(P.diff + 2 * (M + 1));
+  P.bc = bases.on ? P.t2c + 2 * M : nullptr;
   timer_begin(ctx, st);
   TR_CUDA(cudaMemsetAsync(P.diff, 0, 2 * (M + 1) * 4, st));
-  TR_CUDA(cudaMemsetAsync(P.t2c, 0, 2 * M * 4, st));
+  TR_CUDA(cudaMemsetAsync(P.t2c, 0, (bases.on ? 12 : 2) * M * 4, st));
   const uint32_t L = b.uniform_len;
   const int nw = (L >= 1 && L <= 64 && b.uniform_ncigar == 1 && (reinterpret_cast<uintptr_t>(b.bases2) & 3u) == 0) ? (int)((L + 15) / 16) : 0;
-  switch (nw) {
-    case 1: tr_accum_kernel<1><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-    case 2: tr_accum_kernel<2><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-    case 3: tr_accum_kernel<3><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-    case 4: tr_accum_kernel<4><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-    default: tr_accum_kernel<0><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+  if (!bases.on) {
+    switch (nw) {
+      case 1: tr_accum_kernel<1, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      case 2: tr_accum_kernel<2, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      case 3: tr_accum_kernel<3, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      case 4: tr_accum_kernel<4, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      default: tr_accum_kernel<0, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+    }
+  } else {
+    switch (nw) {
+      case 1: tr_accum_kernel<1, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      case 2: tr_accum_kernel<2, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      case 3: tr_accum_kernel<3, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      case 4: tr_accum_kernel<4, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+      default: tr_accum_kernel<0, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
+    }
   }
   timer_end(ctx, st);
   timer_begin(ctx, st);
@@ -584,6 +761,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   unsigned long long tot[3];
   TR_CUDA(cudaMemcpyAsync(tot, &d_st->fast, 8, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaMemcpyAsync(tot + 1, &d_st->t2c[0], 16, cudaMemcpyDeviceToHost, st));
+  if (bases.on) TR_CUDA(cudaMemcpyAsync(out->totals.bases, d_st->bases, sizeof out->totals.bases, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
   out->ctr.fast_path_reads = tot[0];
   out->ctr.t2c_events[0] = tot[1];
@@ -591,12 +769,19 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   const uint64_t nr = hi - lo;
   const uint64_t cap_r[2] = {std::min<uint64_t>(nr, 2 * hh.s.blocks[0] + 1), std::min<uint64_t>(nr, 2 * hh.s.blocks[1] + 1)};
   const uint64_t cap_s = std::min<uint64_t>(2 * nr, tot[1] + tot[2]);
+  // base-count candidates: at most one per min_ev events other than N calls
+  uint64_t events = 0;
+  if (bases.on)
+    for (int s = 0; s < 2; ++s)
+      for (int a = 0; a < 4; ++a)
+        for (int c = 0; c < 4; ++c) events += a == c ? 0 : out->totals.bases[s][a][c];
+  const uint64_t cap_c = std::min<uint64_t>(2 * nr, events / bases.min_ev);
   const uint64_t off_r[4] = {0, cap_r[0], 2 * cap_r[0], 2 * cap_r[0] + cap_r[1]}, off_s = 2 * (cap_r[0] + cap_r[1]);
-  unsigned long long* sel = slot<unsigned long long>(ctx, 6, off_s + cap_s + 8, err);
+  unsigned long long* sel = slot<unsigned long long>(ctx, 6, off_s + cap_s + cap_c + 8, err);
   TR_CUDA(err);
-  unsigned long long* d_cnt = sel + off_s + cap_s;
+  unsigned long long* d_cnt = sel + off_s + cap_s + cap_c;      // runs (4), sites, candidates, base rows
   timer_begin(ctx, st);
-  TR_CUDA(cudaMemsetAsync(d_cnt, 0, 5 * 8, st));
+  TR_CUDA(cudaMemsetAsync(d_cnt, 0, 7 * 8, st));
   thrust::counting_iterator<unsigned long long> it_pos(lo), it_site(2 * lo);
   for (int s = 0; s < 2 && nr; ++s) {
     const int32_t* cov = P.diff + (size_t)s * (M + 1);
@@ -605,10 +790,12 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   }
   unsigned long long* sites_sel = sel + off_s;
   if (nr && cap_s) TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, it_site, sites_sel, d_cnt + 4, (int64_t)(2 * nr), SiteAt{P.t2c, M}, st); }));
-  unsigned long long cnt[5] = {0, 0, 0, 0, 0};
-  TR_CUDA(cudaMemcpyAsync(cnt, d_cnt, sizeof cnt, cudaMemcpyDeviceToHost, st));
+  unsigned long long* cand = sel + off_s + cap_s;
+  if (nr && cap_c) TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, it_site, cand, d_cnt + 5, (int64_t)(2 * nr), BaseCandidate{P.bc, M, bases.min_ev}, st); }));
+  unsigned long long cnt[6] = {0, 0, 0, 0, 0, 0};
+  TR_CUDA(cudaMemcpyAsync(cnt, d_cnt, (bases.on ? 6 : 5) * 8, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
-  if (cnt[0] != cnt[1] || cnt[2] != cnt[3] || cnt[0] > cap_r[0] || cnt[2] > cap_r[1] || cnt[4] > cap_s)
+  if (cnt[0] != cnt[1] || cnt[2] != cnt[3] || cnt[0] > cap_r[0] || cnt[2] > cap_r[1] || cnt[4] > cap_s || cnt[5] > cap_c)
     return set_error(ctx, PS_ERR_CUDA, "track: run or site selection out of bounds");
   ps_track_run* d_runs = slot<ps_track_run>(ctx, 7, cnt[0] + cnt[2] + 1, err);
   ps_track_site* d_sites = slot<ps_track_site>(ctx, 8, cnt[4] + 1, err);
@@ -621,9 +808,18 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
     ctx->launches++;
   }
   if (cnt[4]) { tr_emit_sites_kernel<<<grid_for(cnt[4]), TR_THREADS, 0, st>>>(P, n_segs, sites_sel, cnt[4], d_sites); ctx->launches++; }
+  ps_track_base_row* d_rows = nullptr;             // [cnt[5]] one per candidate, then the kept ones
+  if (cnt[5]) {
+    d_rows = slot<ps_track_base_row>(ctx, 12, 2 * cnt[5], err);
+    TR_CUDA(err);
+    tr_base_rows_kernel<<<grid_for(cnt[5]), TR_THREADS, 0, st>>>(P, n_segs, cand, cnt[5], bases, d_rows);
+    ctx->launches++;
+    TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, d_rows, d_rows + cnt[5], d_cnt + 6, (int64_t)cnt[5], RowKept{}, st); }));
+  }
   timer_end(ctx, st);
   // windowed: positions up to prev_end (head) and from the split on (tail) stay dense for the host merge
   uint32_t* d_dense[2] = {nullptr, nullptr};
+  const uint32_t nv = bases.on ? 14 : 4;           // dense arrays a position hands over
   if (windowed) {
     const unsigned long long f = hh.s.first_key, E = hh.total.x;
     if (prev_end && (f >> 32) == (prev_end >> 32) && f <= prev_end) {
@@ -635,13 +831,14 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
       out->tail.key0 = t0;
       out->tail.len = (uint32_t)(E - t0 + 1);
     }
-    d_dense[0] = slot<uint32_t>(ctx, 10, 4ull * out->head.len, err);
-    d_dense[1] = slot<uint32_t>(ctx, 11, 4ull * out->tail.len, err);
+    d_dense[0] = slot<uint32_t>(ctx, 10, (uint64_t)nv * out->head.len, err);
+    d_dense[1] = slot<uint32_t>(ctx, 11, (uint64_t)nv * out->tail.len, err);
     TR_CUDA(err);
     TrackDense* dn[2] = {&out->head, &out->tail};
     for (int j = 0; j < 2; ++j) {
       if (!dn[j]->len) continue;
-      tr_dense_kernel<<<grid_for(dn[j]->len), TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+      if (bases.on) tr_dense_kernel<true><<<grid_for(dn[j]->len), TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+      else tr_dense_kernel<false><<<grid_for(dn[j]->len), TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
       ctx->launches++;
     }
   }
@@ -656,10 +853,19 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   TrackDense* dn[2] = {&out->head, &out->tail};
   for (int j = 0; j < 2; ++j) {
     if (!dn[j]->len) continue;
-    dn[j]->v.resize(4ull * dn[j]->len);
-    TR_CUDA(cudaMemcpyAsync(dn[j]->v.data(), d_dense[j], 16ull * dn[j]->len, cudaMemcpyDeviceToHost, st));
+    dn[j]->v.resize((uint64_t)nv * dn[j]->len);
+    TR_CUDA(cudaMemcpyAsync(dn[j]->v.data(), d_dense[j], 4ull * nv * dn[j]->len, cudaMemcpyDeviceToHost, st));
   }
+  unsigned long long n_rows = 0;
+  if (cnt[5]) TR_CUDA(cudaMemcpyAsync(&n_rows, d_cnt + 6, 8, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
+  if (n_rows > cnt[5]) return set_error(ctx, PS_ERR_CUDA, "track: base row selection out of bounds");
+  out->base_rows.resize(n_rows);
+  if (n_rows) {
+    TR_CUDA(cudaMemcpyAsync(out->base_rows.data(), d_rows + cnt[5], n_rows * sizeof(ps_track_base_row), cudaMemcpyDeviceToHost, st));
+    TR_CUDA(cudaStreamSynchronize(st));
+  }
+  out->totals.n_rows = n_rows;
   out->ctr.n_runs[0] = cnt[0];
   out->ctr.n_runs[1] = cnt[2];
   out->ctr.n_sites = cnt[4];
@@ -682,9 +888,9 @@ static DeviceBatch tr_view_of(const ps_read_batch* b) {
 }
 
 // a handle is returned with PS_OK and with a fault (PS_ERR_REFERENCE_WOULD_THROW, PS_ERR_UNSUPPORTED): ps_track_fault
-static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, ps_track** out) {
+static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const TrackBases& bases, ps_track** out) {
   ps_track* h = new ps_track();
-  const int rc = track_run(ctx, v, st, false, 0, &h->out);
+  const int rc = track_run(ctx, v, st, false, 0, &h->out, bases);
   if (rc == PS_OK || h->out.fault.code != 0) *out = h;
   else delete h;
   return rc;
@@ -692,9 +898,11 @@ static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, ps_tra
 
 extern "C" {
 
-int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream, ps_track** out) {
+int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts, void* stream, ps_track** out) {
   if (!ctx || !b || !out) return PS_ERR_INVALID_ARG;
   *out = nullptr;
+  TrackBases bases;
+  if (track_bases_of(opts, &bases) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
@@ -702,20 +910,33 @@ int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream, ps_
   for (int slot = 0; slot < 2; ++slot)
     if (st != ctx->stream && b->n_reads && b->meta == ctx->staged[slot].view.meta && ctx->staged_core[slot])
       cudaStreamWaitEvent(st, ctx->staged_core[slot], 0);
-  return track_call(ctx, tr_view_of(b), st, out);
+  return track_call(ctx, tr_view_of(b), st, bases, out);
 }
 
-int ps_track_batch(ps_ctx* ctx, const ps_read_batch* hb, ps_track** out) {
+int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream, ps_track** out) {
+  return ps_track_batch_device_ex(ctx, b, nullptr, stream, out);
+}
+
+int ps_track_batch_ex(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts, ps_track** out) {
   if (!ctx || !hb || !out) return PS_ERR_INVALID_ARG;
   *out = nullptr;
+  TrackBases bases;
+  if (track_bases_of(opts, &bases) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
-  if (hb->n_reads == 0) { *out = new ps_track(); (*out)->out.ctr.num_reads_processed = 0; return PS_OK; }
+  if (hb->n_reads == 0) {
+    *out = new ps_track();
+    (*out)->out.ctr.num_reads_processed = 0;
+    (*out)->out.bases_on = bases.on;
+    return PS_OK;
+  }
   StagedBatch* sb = nullptr;
   const int rc = stage_batch(ctx, hb, /*with_qual=*/false, &sb);
   if (rc) return rc;
-  return track_call(ctx, sb->view, ctx->stream, out);
+  return track_call(ctx, sb->view, ctx->stream, bases, out);
 }
+
+int ps_track_batch(ps_ctx* ctx, const ps_read_batch* hb, ps_track** out) { return ps_track_batch_ex(ctx, hb, nullptr, out); }
 
 int ps_track_counters_get(const ps_track* h, ps_track_counters* out) {
   if (!h || !out) return PS_ERR_INVALID_ARG;
@@ -739,6 +960,23 @@ int64_t ps_track_sites(const ps_track* h, uint64_t first, ps_track_site* sites, 
   const uint64_t k = std::min<uint64_t>(max, v.size() - first);
   if (k) std::memcpy(sites, v.data() + first, k * sizeof(ps_track_site));
   return (int64_t)k;
+}
+
+int64_t ps_track_base_rows(const ps_track* h, uint64_t first, ps_track_base_row* rows, uint64_t max) {
+  if (!h || (!rows && max)) return PS_ERR_INVALID_ARG;
+  if (!h->out.bases_on) return PS_ERR_STATE;
+  const std::vector<ps_track_base_row>& v = h->out.base_rows;
+  if (first >= v.size()) return 0;
+  const uint64_t k = std::min<uint64_t>(max, v.size() - first);
+  if (k) std::memcpy(rows, v.data() + first, k * sizeof(ps_track_base_row));
+  return (int64_t)k;
+}
+
+int ps_track_base_totals_get(const ps_track* h, ps_track_base_totals* out) {
+  if (!h || !out) return PS_ERR_INVALID_ARG;
+  if (!h->out.bases_on) return PS_ERR_STATE;
+  *out = h->out.totals;
+  return PS_OK;
 }
 
 int ps_track_fault(const ps_track* h, ps_fault* out) {

@@ -15,7 +15,7 @@ CSRC_DIR = os.path.join(ROOT_DIR, "csrc")
 REPO_DIR = os.path.dirname(ROOT_DIR)
 INCLUDE_DIR = os.path.join(REPO_DIR, "include")
 
-PS_ABI_VERSION = 5
+PS_ABI_VERSION = 6
 PS_OK = 0
 PS_ERR_INVALID_ARG = -1
 PS_ERR_NO_DEVICE = -2
@@ -135,6 +135,20 @@ class ps_track_counters(C.Structure):
                 for f, _ in self._fields_}
 
 
+class ps_track_opts(C.Structure):
+    _fields_ = [("base_counts", C.c_uint32), ("min_coverage", C.c_uint32), ("min_events", C.c_uint32),
+                ("substitutions", C.c_uint32)]
+
+
+class ps_track_base_row(C.Structure):
+    _fields_ = [("contig", C.c_uint32), ("pos", C.c_int32), ("strand", C.c_uint8), ("ref", C.c_uint8),
+                ("reserved", C.c_uint16), ("cov", C.c_uint32), ("n", C.c_uint32 * 5)]
+
+
+class ps_track_base_totals(C.Structure):
+    _fields_ = [("bases", ((C.c_uint64 * 5) * 4) * 2), ("n_rows", C.c_uint64)]
+
+
 class ps_flush_totals(C.Structure):
     _fields_ = [("snp_hit", C.c_uint64), ("high_frequent_error", C.c_uint64), ("num_crosslinked_clusters", C.c_uint64),
                 ("num_allele_positions", C.c_uint64), ("allele_positions", C.c_uint64 * 51),
@@ -153,6 +167,9 @@ SITE_DTYPE = [("pos", "<i4"), ("t2c", "<u4"), ("cov", "<u4"), ("reserved", "<u4"
 # ps_track_run / ps_track_site
 TRACK_RUN_DTYPE = [("contig", "<u4"), ("start0", "<u4"), ("end0", "<u4"), ("cov", "<u4")]
 TRACK_SITE_DTYPE = [("contig", "<u4"), ("pos", "<i4"), ("strand", "<u4"), ("t2c", "<u4"), ("cov", "<u4")]
+# ps_track_base_row: n holds the read bases A, C, G, T, N in strand orientation
+TRACK_BASE_ROW_DTYPE = [("contig", "<u4"), ("pos", "<i4"), ("strand", "u1"), ("ref", "u1"), ("reserved", "<u2"),
+                        ("cov", "<u4"), ("n", "<u4", (5,))]
 
 # every symbol include/parasuite_b200.h declares: name -> (restype, argtypes)
 VP = C.c_void_p
@@ -243,6 +260,15 @@ EXPORTS = {
     "ps_track_runs": (C.c_int64, [VP, C.c_int, C.c_uint64, VP, C.c_uint64]),
     "ps_track_sites": (C.c_int64, [VP, C.c_uint64, VP, C.c_uint64]),
     "ps_track_fault": (C.c_int, [VP, C.POINTER(ps_fault)]),
+    "ps_track_batch_ex": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_track_opts), C.POINTER(VP)]),
+    "ps_track_batch_device_ex": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_track_opts), VP, C.POINTER(VP)]),
+    "ps_track_base_rows": (C.c_int64, [VP, C.c_uint64, VP, C.c_uint64]),
+    "ps_track_base_totals_get": (C.c_int, [VP, C.POINTER(ps_track_base_totals)]),
+    "ps_track_bam_ex": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts), C.POINTER(ps_track_counters),
+                                  C.POINTER(ps_track_base_totals), C.POINTER(ps_fault)]),
+    "ps_multi_track_bam_ex": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts),
+                                        C.POINTER(ps_track_counters), C.POINTER(ps_track_base_totals),
+                                        C.POINTER(ps_fault)]),
     "ps_track_close": (None, [VP]),
     "ps_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),
     "ps_multi_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),

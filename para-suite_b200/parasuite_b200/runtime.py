@@ -24,6 +24,40 @@ def _check(lib, ctx, st, fault=None):
     raise abi.PsError(st, msg or lib.ps_strerror(st).decode(), fault)
 
 
+_BASE_CODE = {"A": 0, "C": 1, "G": 2, "T": 3}
+
+
+def substitution_mask(substitutions) -> int:
+    """ps_track_opts.substitutions of an iterable of "X>Y" strings (X != Y, both of ACGT, strand orientation); None: 0,
+    which selects all twelve."""
+    if substitutions is None:
+        return 0
+    if isinstance(substitutions, str):
+        substitutions = [substitutions]
+    mask = 0
+    for t in substitutions:
+        parts = str(t).strip().upper().split(">")
+        if len(parts) != 2 or parts[0] not in _BASE_CODE or parts[1] not in _BASE_CODE or parts[0] == parts[1]:
+            raise ValueError(f"not a substitution: {t!r} (expected X>Y with X != Y of A, C, G, T)")
+        mask |= 1 << (4 * _BASE_CODE[parts[0]] + _BASE_CODE[parts[1]])
+    if not mask:
+        raise ValueError("no substitution selected")
+    return mask
+
+
+def track_opts(base_counts: bool, min_coverage: int, min_events: int, substitutions) -> Optional[abi.ps_track_opts]:
+    """The ps_track_opts of the keywords of Context.track, or None for the plain track"""
+    if not base_counts:
+        return None
+    if min(int(min_coverage), int(min_events)) < 0:
+        raise ValueError("min_coverage and min_events must be >= 0")
+    return abi.ps_track_opts(1, int(min_coverage), int(min_events), substitution_mask(substitutions))
+
+
+def _base_totals_dict(tot) -> dict:
+    return {"base_totals": np.array(tot.bases, dtype=np.uint64).reshape(2, 4, 5), "n_base_rows": int(tot.n_rows)}
+
+
 class DeviceBatch:
     """A ReadBatch resident in HBM (torch tensors hold the memory; the kernels see raw pointers)."""
 
@@ -230,13 +264,21 @@ class Context:
         _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
         return np.array(list(ctr), dtype=np.int32)
 
-    def track_bam(self, bam_path: str, out_prefix: str) -> dict:
+    def track_bam(self, bam_path: str, out_prefix: str, *, base_counts: bool = False, min_coverage: int = 1,
+                  min_events: int = 1, substitutions=None) -> dict:
         """The `track` tool from files: writes <out_prefix>.plus.bedGraph, <out_prefix>.minus.bedGraph and
-        <out_prefix>.t2c.tsv (per-position coverage and T>C events by strand); returns the run's counters."""
-        ctr, f = abi.ps_track_counters(), abi.ps_fault()
-        st = self.lib.ps_track_bam(self.h, bam_path.encode(), out_prefix.encode(), C.byref(ctr), C.byref(f))
+        <out_prefix>.t2c.tsv (per-position coverage and T>C events by strand); returns the run's counters.
+        base_counts: also <out_prefix>.bases.tsv (keywords as Context.track), and the counters gain "base_totals"
+        ((2, 4, 5) uint64: strand, reference base, read base A C G T N) and "n_base_rows"."""
+        opts = track_opts(base_counts, min_coverage, min_events, substitutions)
+        ctr, f, tot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals()
+        st = self.lib.ps_track_bam_ex(self.h, bam_path.encode(), out_prefix.encode(), C.byref(opts) if opts else None,
+                                      C.byref(ctr), C.byref(tot), C.byref(f))
         _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
-        return ctr.as_dict()
+        out = ctr.as_dict()
+        if opts:
+            out.update(_base_totals_dict(tot))
+        return out
 
     # ---- batches ---------------------------------------------------------------------------------
     def upload(self, batch) -> UploadedBatch:
@@ -413,16 +455,23 @@ class Context:
             return res.fetch()
 
     # ---- T>C conversion and coverage track ---------------------------------------------------------
-    def track(self, batch, stream: int = 0) -> dict:
+    def track(self, batch, stream: int = 0, *, base_counts: bool = False, min_coverage: int = 1, min_events: int = 1,
+              substitutions=None) -> dict:
         """Per-position coverage and T>C events by strand of one whole input: {"runs_plus", "runs_minus", "sites",
         "counters"}, runs and sites as numpy structured arrays (abi.TRACK_RUN_DTYPE / TRACK_SITE_DTYPE, contigs as FASTA
-        indices).  batch: host (ReadBatch / PinnedBatch) or device-resident (DeviceBatch / UploadedBatch)."""
+        indices).  batch: host (ReadBatch / PinnedBatch) or device-resident (DeviceBatch / UploadedBatch).
+        base_counts: also "base_rows" (abi.TRACK_BASE_ROW_DTYPE: read bases A C G T N by position and strand, strand
+        orientation) for the positions with coverage >= min_coverage and >= min_events of the selected substitutions
+        (an iterable of "X>Y"; None: all twelve), and "base_totals" ((2, 4, 5) uint64: strand, reference base, read
+        base) over every counted base."""
+        opts = track_opts(base_counts, min_coverage, min_events, substitutions)
+        po = C.byref(opts) if opts else None
         h = C.c_void_p()
         if isinstance(batch, (DeviceBatch, UploadedBatch)):
-            st = self.lib.ps_track_batch_device(self.h, C.byref(batch.struct), stream or None, C.byref(h))
+            st = self.lib.ps_track_batch_device_ex(self.h, C.byref(batch.struct), po, stream or None, C.byref(h))
         else:
             s = batch.struct if hasattr(batch, "struct") else batch.as_struct()
-            st = self.lib.ps_track_batch(self.h, C.byref(s), C.byref(h))
+            st = self.lib.ps_track_batch_ex(self.h, C.byref(s), po, C.byref(h))
         try:
             if st != abi.PS_OK:
                 fault = None
@@ -446,6 +495,14 @@ class Context:
             if sites.size:
                 self.lib.ps_track_sites(h, 0, sites.ctypes.data, sites.size)
             out["sites"] = sites
+            if opts:
+                tot = abi.ps_track_base_totals()
+                _check(self.lib, self.h, self.lib.ps_track_base_totals_get(h, C.byref(tot)))
+                rows = np.zeros(tot.n_rows, dtype=abi.TRACK_BASE_ROW_DTYPE)
+                if rows.size:
+                    self.lib.ps_track_base_rows(h, 0, rows.ctypes.data, rows.size)
+                out["base_rows"] = rows
+                out["base_totals"] = _base_totals_dict(tot)["base_totals"]
             return out
         finally:
             if h:
@@ -633,12 +690,18 @@ class MultiContext:
         self._check(st, fault=(f.code, f.read_ordinal))
         return {k: getattr(ctr, k) for k, _ in abi.ps_pileup_counters._fields_}
 
-    def track_bam(self, bam_path: str, out_prefix: str) -> dict:
+    def track_bam(self, bam_path: str, out_prefix: str, *, base_counts: bool = False, min_coverage: int = 1,
+                  min_events: int = 1, substitutions=None) -> dict:
         """Context.track_bam with windows round-robin over the devices; the files are byte-identical."""
-        ctr, f = abi.ps_track_counters(), abi.ps_fault()
-        st = self.lib.ps_multi_track_bam(self.h, bam_path.encode(), out_prefix.encode(), C.byref(ctr), C.byref(f))
+        opts = track_opts(base_counts, min_coverage, min_events, substitutions)
+        ctr, f, tot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals()
+        st = self.lib.ps_multi_track_bam_ex(self.h, bam_path.encode(), out_prefix.encode(),
+                                            C.byref(opts) if opts else None, C.byref(ctr), C.byref(tot), C.byref(f))
         self._check(st, fault=(f.code, f.read_ordinal))
-        return ctr.as_dict()
+        out = ctr.as_dict()
+        if opts:
+            out.update(_base_totals_dict(tot))
+        return out
 
     def close(self):
         if getattr(self, "h", None):

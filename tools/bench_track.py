@@ -1,6 +1,7 @@
 """Measurement of the per-position T>C conversion and coverage track (tool `track`) on one GPU.
 
   python tools/bench_track.py [--steps 20] [--warmup 3] [--bam-reads 300000] [--bam-copies 40] [--out FILE]
+  python tools/bench_track.py --base-counts [--steps 20] [--warmup 3] [--out FILE]
 
 1. Config 2 as bench.py builds it (10 M x 36-nt reads through synth.py against a 100 Mb reference), resident in HBM:
    `--steps` timed passes of ps_track_batch_device after `--warmup` passes, with the five stage times of every pass from
@@ -11,6 +12,11 @@
    the file stays coordinate-sorted.  Reads/s over the whole call (decode, device, files).
 3. Parity: the timed batch against the C++ restatement (oracle/track_oracle.py).
 The card's name and power limit are recorded with the numbers.
+
+--base-counts measures the per-position base counts instead: on the same config-2 batch, the plain call and the call
+with base counts (all twelve substitutions, thresholds 1) alternate, `--steps` passes each after `--warmup` of each; the
+five stage times of both, the scratch the compact arrays take, the row counts, and the parity of the base-count call with
+the C++ restatement (tests/track_bases_oracle.py) go to profiles/track_bench_bases.json (or --out).
 """
 import argparse
 import json
@@ -34,6 +40,7 @@ ap.add_argument("--warmup", type=int, default=3)
 ap.add_argument("--bam-reads", type=int, default=300_000)
 ap.add_argument("--bam-copies", type=int, default=40)
 ap.add_argument("--out", default=None)
+ap.add_argument("--base-counts", action="store_true")
 args = ap.parse_args()
 
 import torch  # noqa: E402
@@ -85,6 +92,66 @@ def track_once():
     lib.ps_track_close(h)
     return ctr
 
+
+def base_counts_run():
+    """plain and base-count calls alternately on the config-2 batch"""
+    opts = abi.ps_track_opts(1, 1, 1, 0)
+
+    def once(with_bases):
+        h = C.c_void_p()
+        st = lib.ps_track_batch_device_ex(ctx.h, C.byref(db.struct), C.byref(opts) if with_bases else None, None,
+                                          C.byref(h))
+        assert st == abi.PS_OK, lib.ps_last_error(ctx.h)
+        ctr, tot = abi.ps_track_counters(), abi.ps_track_base_totals()
+        lib.ps_track_counters_get(h, C.byref(ctr))
+        if with_bases:
+            lib.ps_track_base_totals_get(h, C.byref(tot))
+        lib.ps_track_close(h)
+        return ctr, tot
+
+    for _ in range(args.warmup):
+        once(False)
+        once(True)
+    res = {False: {"walls": [], "stages": []}, True: {"walls": [], "stages": []}}
+    for _ in range(args.steps):
+        for wb in (False, True):
+            ctx.kernel_times_reset(True)
+            t0 = time.perf_counter()
+            ctr, tot = once(wb)
+            res[wb]["walls"].append(time.perf_counter() - t0)
+            res[wb]["stages"].append(ctx.kernel_times_ms().reshape(-1, len(STAGES))[-1])
+            res[wb]["ctr"], res[wb]["tot"] = ctr, tot
+    M = compact_positions(batch)
+    out["config2_base_counts"] = {"reads": batch.n_reads, "compact_positions": M, "steps": args.steps,
+                                  "warmup": args.warmup, "order": "plain and base-count calls alternate"}
+    for wb, name in ((False, "plain"), (True, "base_counts")):
+        st = np.array(res[wb]["stages"])
+        out["config2_base_counts"][name] = {
+            "wall_ms_median": 1e3 * float(np.median(res[wb]["walls"])),
+            "device_ms_median": float(np.median(st.sum(axis=1))),
+            "stage_ms_median": {k: float(np.median(st[:, i])) for i, k in enumerate(STAGES)},
+            "compact_scratch_bytes": 4 * (2 * (M + 1) + 2 * M) + (40 * M if wb else 0),
+            "runs": [int(res[wb]["ctr"].n_runs[0]), int(res[wb]["ctr"].n_runs[1])], "sites": int(res[wb]["ctr"].n_sites),
+        }
+    out["config2_base_counts"]["base_counts"]["base_rows"] = int(res[True]["tot"].n_rows)
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+    import track_bases_oracle  # noqa: E402
+    got = ctx.track(db, base_counts=True)
+    exp = track_bases_oracle.track_bases_cpp(ref, batch)
+    out["parity_with_restatement"] = bool(np.array_equal(got["base_rows"], exp["base_rows"]) and
+                                          np.array_equal(got["base_totals"], exp["base_totals"]) and
+                                          all(np.array_equal(got[k], exp[k]) for k in ("runs_plus", "runs_minus", "sites")))
+    print(json.dumps(out, indent=1))
+    path = args.out or os.path.join(REPO, "profiles", "track_bench_bases.json")
+    os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+    with open(path, "w") as f:
+        json.dump(out, f, indent=1)
+    ctx.close()
+
+
+if args.base_counts:
+    base_counts_run()
+    sys.exit(0)
 
 for _ in range(args.warmup):
     ctr = track_once()
