@@ -829,7 +829,7 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
         for (uint32_t e = 0; e < nc; ++e) {
           const uint32_t c = rd32(cg + 4 * e), op = c & 15u;
           cigar[oc + e] = c;
-          if ((0x18Du >> op) & 1u) R += c >> 4;                  // M, D, N, =, X consume the reference
+          if (op_consumes_ref(op)) R += c >> 4;
         }
         // bases: 2-bit codes, 4 per byte; everything that is not A, C, G, T goes to the exception list as code 0
         for (uint32_t k = 0; k < (l_seq + 3) / 4; ++k) bases2[ob + k] = 0;

@@ -27,6 +27,7 @@
 
 #include "parasuite_b200.h"
 #include "java_double.h"
+#include "record.h"
 
 namespace {
 
@@ -304,14 +305,8 @@ static void cw_walk_range(const ps_clust_writer* w, const ps_read_batch* hb, uin
     const uint32_t* cig = hb->cigar + coff;
     coff += ncig;
     const uint64_t ordinal = first_ordinal + r;
-    bool hasI = false, hasD = false, hasN = false;
-    int64_t R = 0;
-    for (uint32_t e = 0; e < ncig; ++e) {
-      const uint32_t op = cig[e] & 15u;
-      hasI |= op == 1u; hasD |= op == 2u; hasN |= op == 3u;
-      if ((0x18Du >> op) & 1u) R += cig[e] >> 4;
-    }
-    if ((flags & PS_RF_UNMAPPED) || ((hasI || hasD) && hasN)) {                // :146, :152-157
+    const CigarShape<int64_t> shape = cigar_shape<int64_t>(cig, ncig);
+    if ((flags & PS_RF_UNMAPPED) || shape.skip) {                              // :146, :152-157
       if (sc < n_starts && starts[sc] == ordinal) return stop(PS_ERR_STATE, kDisagree, ordinal);   // a cluster cannot begin here
       continue;
     }
@@ -323,7 +318,7 @@ static void cw_walk_range(const ps_clust_writer* w, const ps_read_batch* hb, uin
       while (hi - lo > 1) { const size_t mid = (lo + hi) / 2; if (w->fa.off[mid] <= g) lo = mid; else hi = mid; }
       ci = lo;
     }
-    const int64_t start = (int64_t)(g - w->fa.off[ci]) + 1, end = start + R - 1;
+    const int64_t start = (int64_t)(g - w->fa.off[ci]) + 1, end = start + shape.ref_span - 1;
     if (sc < n_starts && starts[sc] == ordinal) {
       ++sc;
       if (st.have) O.done.emplace_back(st.cluster_first, std::move(st.bytes));   // the previous cluster is flushed (:178)

@@ -16,27 +16,6 @@ int cuda_fail(ps_ctx* ctx, cudaError_t e, const char* what) {
   return set_error(ctx, e == cudaErrorMemoryAllocation ? PS_ERR_OOM : PS_ERR_CUDA, m);
 }
 
-static DeviceBatch view_of(const ps_read_batch* b) {
-  DeviceBatch v;
-  v.n_reads = b->n_reads;
-  v.meta = b->meta;
-  v.ref_start = b->ref_start;
-  v.bases2 = b->bases2;
-  v.qual = b->qual;
-  v.cigar = b->cigar;
-  v.tile_base_off = b->tile_base_off;
-  v.tile_qual_off = b->tile_qual_off;
-  v.tile_cigar_off = b->tile_cigar_off;
-  v.tile_exc_off = b->tile_exc_off;
-  v.exc = b->exc;
-  v.uniform_len = b->uniform_len;
-  v.uniform_ncigar = b->uniform_ncigar;
-  v.cigar_count = b->cigar_count;
-  v.max_len = b->max_len;
-  v.past_end = b->past_end;
-  return v;
-}
-
 static int check_batch(ps_ctx* ctx, const ps_read_batch* b, bool allow_compact = false) {
   if (!b) return set_error(ctx, PS_ERR_INVALID_ARG, "batch is NULL");
   if (b->n_reads == 0) return PS_OK;

@@ -1,4 +1,4 @@
-// Device helpers shared by the profile and pileup kernels (sm_100a).
+// Device helpers shared by the profile, pileup and track kernels (sm_100a).
 #pragma once
 #include <cstdint>
 
@@ -15,10 +15,6 @@ __device__ __forceinline__ bool ref_invalid_at(const DeviceRef& ref, uint64_t g)
 __device__ __forceinline__ uint32_t read_code_at(const uint8_t* b, uint32_t p) {
   return (__ldg(b + (p >> 2)) >> (2 * (p & 3))) & 3u;
 }
-
-// htsjdk Cigar.getReferenceLength: M, D, N, =, X consume the reference
-__device__ __forceinline__ bool op_consumes_ref(uint32_t op) { return (0x18Du >> op) & 1u; }   // bits 0,2,3,7,8
-__device__ __forceinline__ bool op_is_match(uint32_t op) { return (0x181u >> op) & 1u; }       // M, =, X
 
 __device__ __forceinline__ void raise_fault(unsigned long long* fault, uint64_t ordinal, uint32_t code) {
   atomicMin(fault, (unsigned long long)((ordinal << 8) | code));
@@ -165,4 +161,44 @@ __device__ __forceinline__ unsigned long long read_exc_mask64(const DeviceBatch&
     if ((v & 0xFFFFu) < 64u) m |= 1ull << (v & 0xFFFFu);
   }
   return m;
+}
+
+// even bits of c -> low 16 bits
+__device__ __forceinline__ uint32_t even_bits(uint32_t c) {
+  c &= 0x55555555u;
+  c = (c | (c >> 1)) & 0x33333333u;
+  c = (c | (c >> 2)) & 0x0F0F0F0Fu;
+  c = (c | (c >> 4)) & 0x00FF00FFu;
+  c = (c | (c >> 8)) & 0x0000FFFFu;
+  return c;
+}
+
+// Bit-parallel T>C events of a read of length L <= 64 whose one M/=/X op covers it, in genome orientation (bit j = read
+// position j): ref T (11) and read C (01) on the plus strand, ref A (00) and read G (10) on the minus strand.  w: the
+// reference words from g0 >> 4 on, bw: the read's words, bsh: the bit offset of its first base in bw[0].  The positions
+// over a reference N, from L on, and (has_exc: the read has entries in `exc`) of listed N calls are cleared: the codes
+// stored there are arbitrary.  ref_n: the reference-N window of the read, same orientation.
+struct T2cWord { unsigned long long t2c, ref_n; };
+template <int NW>
+__device__ __forceinline__ T2cWord t2c_word(const DeviceRef& ref, const DeviceBatch& b, uint64_t r, uint32_t g0, uint32_t L,
+                                            bool rev, bool has_exc, const uint32_t (&w)[NW + 1],
+                                            const uint32_t (&bw)[NW + 1], uint32_t bsh) {
+  const uint32_t sh = (g0 & 15u) * 2u, ii = g0 >> 5, s1 = g0 & 31u;
+  const uint32_t i0 = __ldg(ref.inv + ii), i1 = __ldg(ref.inv + ii + 1), i2 = NW > 2 ? __ldg(ref.inv + ii + 2) : 0u;
+  unsigned long long m = 0;
+#pragma unroll
+  for (int j = 0; j < NW; ++j) {
+    const uint32_t rf = __funnelshift_r(w[j], w[j + 1], sh);
+    const uint32_t rd = __funnelshift_r(bw[j], bw[j + 1], bsh);
+    const uint32_t h = rev ? (~(rf | (rf >> 1)) & (rd >> 1) & ~rd) : (rf & (rf >> 1) & rd & ~(rd >> 1));
+    m |= (unsigned long long)even_bits(h) << (16 * j);
+  }
+  T2cWord t;
+  t.ref_n = (unsigned long long)__funnelshift_r(i0, i1, s1) |
+            ((unsigned long long)(NW > 2 ? __funnelshift_r(i1, i2, s1) : 0u) << 32);
+  m &= ~t.ref_n;
+  m &= L >= 64 ? ~0ull : ((1ull << L) - 1ull);
+  if (has_exc && m) m &= ~read_exc_mask64(b, r);      // only a read with a candidate event needs its list
+  t.t2c = m;
+  return t;
 }

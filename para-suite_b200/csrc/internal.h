@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "parasuite_b200.h"
+#include "record.h"
 
 #define PS_BLOCK_THREADS 256   // == PS_TILE_READS: one read per thread, one tile per block iteration
 
@@ -41,6 +42,16 @@ struct DeviceBatch {
   uint32_t max_len;        // longest read (0: not known)
   uint64_t past_end;       // ps_read_batch.past_end: the kernels never see it, the tools run on the reads before it
 };
+
+inline DeviceBatch view_of(const ps_read_batch* b) {
+  DeviceBatch v;
+  v.n_reads = b->n_reads; v.meta = b->meta; v.ref_start = b->ref_start; v.bases2 = b->bases2; v.qual = b->qual;
+  v.cigar = b->cigar; v.tile_base_off = b->tile_base_off; v.tile_qual_off = b->tile_qual_off;
+  v.tile_cigar_off = b->tile_cigar_off; v.tile_exc_off = b->tile_exc_off; v.exc = b->exc;
+  v.uniform_len = b->uniform_len; v.uniform_ncigar = b->uniform_ncigar; v.cigar_count = b->cigar_count; v.max_len = b->max_len;
+  v.past_end = b->past_end;
+  return v;
+}
 
 struct ProfileLayout {   // offsets (in int64 elements) inside the accumulator vector
   uint32_t max_len;

@@ -133,17 +133,11 @@ struct FlagParams {
 template <bool COUNT = true>
 __device__ __forceinline__ unsigned long long pl_key(const FlagParams& P, uint64_t r, uint32_t meta, const uint32_t* cig,
                                                      uint32_t g0, ContigCache& cc, int32_t& start) {
-  const uint32_t flags = PS_META_FLAGS(meta), ncig = PS_META_NCIGAR(meta);
+  const uint32_t flags = PS_META_FLAGS(meta);
   start = 0;
   if (flags & PS_RF_UNMAPPED) return 0;                                      // :146
-  uint32_t R = 0;
-  bool hasI = false, hasD = false, hasN = false;
-  for (uint32_t e = 0; e < ncig; ++e) {
-    const uint32_t c = __ldg(cig + e), op = c & 15u;
-    hasI |= op == 1u; hasD |= op == 2u; hasN |= op == 3u;
-    if (op_consumes_ref(op)) R += c >> 4;
-  }
-  if ((hasI || hasD) && hasN) {                                              // :152-157
+  const CigarShape<> s = cigar_shape(cig, PS_META_NCIGAR(meta));
+  if (s.skip) {                                                              // :152-157
     if (COUNT) atomicAdd(&P.st->skipped, 1ull);
     return 0;
   }
@@ -151,7 +145,7 @@ __device__ __forceinline__ unsigned long long pl_key(const FlagParams& P, uint64
                                                                    // pl_cluster_kernel raises the fault
   if (!contig_lookup(P.ref, g0, cc)) return 0;    // likewise
   start = (int32_t)((uint64_t)g0 - cc.lo) + 1;
-  const int32_t end = start + (int32_t)R - 1;
+  const int32_t end = start + (int32_t)s.ref_span - 1;
   return ((unsigned long long)(cc.rank + 1) << 32) | (uint32_t)end;
 }
 
@@ -556,107 +550,63 @@ __device__ __noinline__ void pl_decode_generic(const ClusterParams& P, uint64_t 
   x.kept = false; x.mask = 0; x.start = 0; x.end = 0; x.lo = 1; x.hi = 0; x.rev = false; x.contig = 0;
   if (flags & PS_RF_UNMAPPED) return;                                        // :146
   if (flags & PS_RF_CIGAR_OVERFLOW) { raise_fault(&P.st->fault, r, PS_FAULT_CIGAR_OPS); return; }   // not representable
-  uint32_t R = 0, alen = 0;
-  bool hasI = false, hasD = false, hasN = false;
-  for (uint32_t e = 0; e < ncig; ++e) {
-    const uint32_t c = __ldg(cig + e), op = c & 15u;
-    hasI |= op == 1u; hasD |= op == 2u; hasN |= op == 3u;
-    if (op_consumes_ref(op)) R += c >> 4;
-    if (op_is_match(op)) alen += c >> 4;
-  }
-  if ((hasI || hasD) && hasN) return;                                        // :152-157 (counted by pl_flag_kernel)
+  const CigarShape<> sh = cigar_shape(cig, ncig);
+  const uint32_t alen = sh.aligned;
+  if (sh.skip) return;                                                       // :152-157 (counted by pl_flag_kernel)
   if (flags & PS_RF_POS_ZERO) { raise_fault(&P.st->fault, r, PS_THROW_REF_RANGE); return; }
   const uint64_t g0 = __ldg(P.b.ref_start + r);
   if (g0 >= P.ref.n_bases) { raise_fault(&P.st->fault, r, PS_THROW_REF_RANGE); return; }
   const uint32_t contig = contig_of(P.ref, g0);
   const uint64_t c_lo = __ldg(P.ref.contig_off + contig), c_hi = __ldg(P.ref.contig_off + contig + 1);
   const int32_t start = (int32_t)(g0 - c_lo) + 1;
-  const int32_t end = start + (int32_t)R - 1;
+  const int32_t end = start + (int32_t)sh.ref_span - 1;
   const bool rev = flags & PS_RF_REVERSE;
   const bool has_inv = flags & PS_RF_HAS_INVALID;
   const uint8_t* rb = P.b.bases2 + off_base;
   x.kept = true; x.start = start; x.end = end; x.rev = rev; x.contig = contig;
   if (rev) { x.hi = end; x.lo = end - (int32_t)alen + 1; }
   else { x.lo = start; x.hi = start + (int32_t)alen - 1; }
-  // alignment blocks (SAMUtils.getAlignmentBlocks): S,I advance the read; D,N the reference; H,P nothing.
-  // The reference slices every block (read bases, then FASTA) before it looks at a single base (:593-604).
-  int64_t rdp = 0, rfp = 0;
-  for (uint32_t e = 0; e < ncig; ++e) {
-    const uint32_t c = __ldg(cig + e), op = c & 15u;
-    const int64_t n = c >> 4;
-    if (op == 4u || op == 1u) rdp += n;
-    else if (op == 2u || op == 3u) rfp += n;
-    else if (op_is_match(op)) {
-      if (rdp + n > (int64_t)L) { raise_fault(&P.st->fault, r, PS_THROW_BLOCK_RANGE); return; }
-      if ((flags & PS_RF_REF_RANGE) || g0 + (uint64_t)(rfp + n) > c_hi) {
-        raise_fault(&P.st->fault, r, PS_THROW_REF_RANGE); return;
-      }
-      rdp += n; rfp += n;
-    }
-  }
-  rdp = 0; rfp = 0;
+  // the reference slices every block (read bases, then FASTA) before it looks at a single base (:593-604)
+  uint32_t code = 0;
+  for_each_block(cig, ncig, [&](int64_t rdp, int64_t rfp, int64_t n) {
+    if (rdp + n > (int64_t)L) code = PS_THROW_BLOCK_RANGE;
+    else if ((flags & PS_RF_REF_RANGE) || g0 + (uint64_t)(rfp + n) > c_hi) code = PS_THROW_REF_RANGE;
+    return code == 0;
+  });
+  if (code) { raise_fault(&P.st->fault, r, code); return; }
   uint32_t j = 0;             // index over the concatenated blocks (forward orientation)
   unsigned long long mask = 0;
-  for (uint32_t e = 0; e < ncig; ++e) {
-    const uint32_t c = __ldg(cig + e), op = c & 15u;
-    const int64_t n = c >> 4;
-    if (op == 4u || op == 1u) rdp += n;
-    else if (op == 2u || op == 3u) rfp += n;
-    else if (op_is_match(op)) {
-      for (int64_t z = 0; z < n; ++z, ++j) {
-        const uint64_t g = g0 + (uint64_t)(rfp + z);
-        const uint32_t p = (uint32_t)(rdp + z);
-        if (ref_invalid_at(P.ref, g)) continue;
-        const uint32_t a = ref_code_at(P.ref, g), bb = read_code_at(rb, p);
-        // minus strand: both arrays are reverse-complemented, so ref T & read C there is ref A & read G here
-        const bool hit = rev ? (a == 0u && bb == 2u) : (a == 3u && bb == 1u);
-        if (!hit) continue;
-        if (has_inv && read_pos_invalid(P.b, read_exc_range(P.b, r / PS_TILE_READS, (uint32_t)(r % PS_TILE_READS)), p)) continue;
-        const uint32_t i = rev ? alen - 1 - j : j;
-        if (i >= 51u) { raise_fault(&P.st->fault, r, PS_THROW_MASK51); return; }   // boolean[51] (:654)
-        mask |= 1ull << i;
-      }
-      rdp += n; rfp += n;
+  bool over = false;
+  for_each_block(cig, ncig, [&](int64_t rdp, int64_t rfp, int64_t n) {
+    for (int64_t z = 0; z < n; ++z, ++j) {
+      const uint64_t g = g0 + (uint64_t)(rfp + z);
+      const uint32_t p = (uint32_t)(rdp + z);
+      if (ref_invalid_at(P.ref, g)) continue;
+      const uint32_t a = ref_code_at(P.ref, g), bb = read_code_at(rb, p);
+      // minus strand: both arrays are reverse-complemented, so ref T & read C there is ref A & read G here
+      const bool hit = rev ? (a == 0u && bb == 2u) : (a == 3u && bb == 1u);
+      if (!hit) continue;
+      if (has_inv && read_pos_invalid(P.b, read_exc_range(P.b, r / PS_TILE_READS, (uint32_t)(r % PS_TILE_READS)), p)) continue;
+      const uint32_t i = rev ? alen - 1 - j : j;
+      if (i >= 51u) { raise_fault(&P.st->fault, r, PS_THROW_MASK51); over = true; return false; }   // boolean[51] (:654)
+      mask |= 1ull << i;
     }
-  }
-  x.mask = mask;
+    return true;
+  });
+  if (!over) x.mask = mask;
 }
 
-// PAR-CLIP shape: uniform length L <= 64, one M/=/X op of length L.
-__device__ __forceinline__ uint32_t compress_even(uint32_t c) {   // even bits of c -> low 16 bits
-  c = (c | (c >> 1)) & 0x33333333u;
-  c = (c | (c >> 2)) & 0x0F0F0F0Fu;
-  c = (c | (c >> 4)) & 0x00FF00FFu;
-  c = (c | (c >> 8)) & 0x0000FFFFu;
-  return c;
-}
-
-// has_inv: read r has entries in `exc`; the positions they list are cleared like reference N
+// PAR-CLIP shape: uniform length L <= 64, one M/=/X op of length L.  The T>C word in strand orientation
+// (i = alignedLength - 1 - j on the minus strand); bw: the read's words, loaded ahead (pl_load_raw)
 template <int NW>
 __device__ __forceinline__ unsigned long long t2c_mask_fast(const DeviceRef& ref, uint32_t g0, uint32_t L, bool rev,
                                                             const uint32_t (&bw)[NW + 1], uint32_t bshift,
                                                             const DeviceBatch& b, uint64_t r, bool has_inv) {
-  const uint32_t wi = g0 >> 4, sh = (g0 & 15u) * 2u;
   uint32_t w[NW + 1];
 #pragma unroll
-  for (int k = 0; k <= NW; ++k) w[k] = __ldg(ref.seq2 + wi + k);
-  const uint32_t ii = g0 >> 5, s1 = g0 & 31u;
-  const uint32_t i0 = __ldg(ref.inv + ii), i1 = __ldg(ref.inv + ii + 1), i2 = NW > 2 ? __ldg(ref.inv + ii + 2) : 0u;
-  unsigned long long m = 0;
-#pragma unroll
-  for (int k = 0; k < NW; ++k) {
-    const uint32_t rf = __funnelshift_r(w[k], w[k + 1], sh);
-    const uint32_t rd = __funnelshift_r(bw[k], bw[k + 1], bshift);
-    // forward: ref T (11) and read C (01);  reverse strand: ref A (00) and read G (10)
-    const uint32_t h = rev ? (~(rf | (rf >> 1)) & (rd >> 1) & ~rd) : (rf & (rf >> 1) & rd & ~(rd >> 1));
-    m |= (unsigned long long)compress_even(h & 0x55555555u) << (16 * k);
-  }
-  const unsigned long long inv = (unsigned long long)__funnelshift_r(i0, i1, s1) |
-                                 ((unsigned long long)(NW > 2 ? __funnelshift_r(i1, i2, s1) : 0u) << 32);
-  m &= ~inv;
-  m &= L >= 64 ? ~0ull : ((1ull << L) - 1ull);
-  if (has_inv && m) m &= ~read_exc_mask64(b, r);      // only a read with a candidate event needs its list
-  if (rev) m = __brevll(m) >> (64u - L);      // i = alignedLength - 1 - j
+  for (int k = 0; k <= NW; ++k) w[k] = __ldg(ref.seq2 + (g0 >> 4) + k);
+  unsigned long long m = t2c_word<NW>(ref, b, r, g0, L, rev, has_inv, w, bw, bshift).t2c;
+  if (rev) m = __brevll(m) >> (64u - L);
   return m;
 }
 
@@ -1765,16 +1715,6 @@ static int run_pileup(ps_ctx* ctx, const DeviceBatch& b, const ps_pileup_opts* o
   return wait ? pileup_finish(ctx, H) : PS_OK;
 }
 
-static DeviceBatch pl_view_of(const ps_read_batch* b) {
-  DeviceBatch v;
-  v.n_reads = b->n_reads; v.meta = b->meta; v.ref_start = b->ref_start; v.bases2 = b->bases2; v.qual = b->qual;
-  v.cigar = b->cigar; v.tile_base_off = b->tile_base_off; v.tile_qual_off = b->tile_qual_off;
-  v.tile_cigar_off = b->tile_cigar_off; v.tile_exc_off = b->tile_exc_off; v.exc = b->exc;
-  v.uniform_len = b->uniform_len; v.uniform_ncigar = b->uniform_ncigar; v.cigar_count = b->cigar_count; v.max_len = b->max_len;
-  v.past_end = b->past_end;
-  return v;
-}
-
 static void free_handle(ps_pileup* h) {
   if (!h) return;
   if (h->host_mode) { delete h; return; }
@@ -1871,7 +1811,7 @@ int ps_pileup_batch_device(ps_ctx* ctx, const ps_read_batch* b, const ps_pileup_
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-  int rc = run_pileup(ctx, pl_view_of(b), opts, st, out);
+  int rc = run_pileup(ctx, view_of(b), opts, st, out);
   if (rc != PS_OK && !(*out && (*out)->fault.code)) { free_handle(*out); *out = nullptr; }   // a fault stays readable
   return rc;
 }
@@ -1883,7 +1823,7 @@ int ps_pileup_submit_device(ps_ctx* ctx, const ps_read_batch* b, const ps_pileup
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-  int rc = run_pileup(ctx, pl_view_of(b), opts, st, out, /*wait=*/false);
+  int rc = run_pileup(ctx, view_of(b), opts, st, out, /*wait=*/false);
   if (rc != PS_OK) { free_handle(*out); *out = nullptr; }
   return rc;
 }
@@ -1928,7 +1868,7 @@ int ps_pileup_max_key_device(ps_ctx* ctx, const ps_read_batch* dev_batch, void* 
   PS_CUDA(ctx, cudaMemsetAsync(d_key, 0, 8, st));
   if (dev_batch->n_reads == 0) return PS_OK;
   FlagParams P{};
-  P.b = pl_view_of(dev_batch); P.ref = ctx->ref;
+  P.b = view_of(dev_batch); P.ref = ctx->ref;
   const uint32_t grid = (uint32_t)std::min<uint64_t>((dev_batch->n_reads + PL_THREADS - 1) / PL_THREADS, (uint64_t)ctx->sm_count * 8);
   pl_maxkey_kernel<<<grid, PL_THREADS, 0, st>>>(P, d_key);
   ctx->launches++;

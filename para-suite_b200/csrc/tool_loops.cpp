@@ -67,19 +67,13 @@ uint64_t host_max_key(const ps_read_batch& b, const std::vector<uint64_t>& conti
     const uint32_t* cig = b.cigar + coff;
     coff += ncig;
     if (flags & (PS_RF_UNMAPPED | PS_RF_POS_ZERO | PS_RF_CIGAR_OVERFLOW)) continue;
-    bool hasI = false, hasD = false, hasN = false;
-    uint64_t R = 0;
-    for (uint32_t e = 0; e < ncig; ++e) {
-      const uint32_t op = cig[e] & 15u;
-      hasI |= op == 1u; hasD |= op == 2u; hasN |= op == 3u;
-      if ((0x18Du >> op) & 1u) R += cig[e] >> 4;
-    }
-    if ((hasI || hasD) && hasN) continue;
+    const CigarShape<> s = cigar_shape(cig, ncig);
+    if (s.skip) continue;
     const uint64_t g = b.ref_start[r];
     if (g >= contig_off.back()) continue;
     if (!(g >= contig_off[ci] && g < contig_off[ci + 1]))
       ci = (size_t)(std::upper_bound(contig_off.begin(), contig_off.end(), g) - contig_off.begin()) - 1;
-    const uint64_t end = g - contig_off[ci] + R;          // start + R - 1 with start = g - off + 1
+    const uint64_t end = g - contig_off[ci] + s.ref_span;   // start + span - 1 with start = g - off + 1
     best = std::max(best, pileup_key(rank, (uint32_t)ci, (int32_t)(uint32_t)end));
   }
   return best;

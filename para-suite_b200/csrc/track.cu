@@ -19,9 +19,9 @@
 //   tr_seg_place_kernel  compact index range that is reported (windowed file tool: head and tail stay dense)
 //   tr_accum_kernel<NW, BC>  per read: +1/-1 per alignment block into one int32 difference array per strand, +1 per
 //                        T>C event.  NW > 0: uniform length <= 64, one M/=/X op -- T>C bits found bit-parallel on the
-//                        2-bit words of read and reference.  BC (base counts): also +1 per event -- a read base other
-//                        than the reference base, or an N call -- into five uint32 counters (A C G T N, strand
-//                        orientation) per position and strand, and the genome-wide matrix in block-shared counters
+//                        2-bit words of read and reference (t2c_word).  BC (base counts): also +1 per event -- a read
+//                        base other than the reference base, or an N call -- into five uint32 counters (A C G T N,
+//                        strand orientation) per position and strand, and the genome-wide matrix in block-shared counters
 //   (CUB) sum scan       of each difference array = coverage (every segment's differences sum to zero)
 //   (CUB) select         run starts / ends per strand, T>C sites; tr_emit_*_kernel turn them into records.  BC: a select
 //                        of the (position, strand) items with >= min_events non-N events, then tr_base_rows_kernel
@@ -90,7 +90,7 @@ __device__ __forceinline__ unsigned long long warp_sum(unsigned long long v) {
   return v;
 }
 
-// Filters and faults exactly as pl_decode_generic (and pl_key for skipped_due_indel), without the 51-position limit.
+// Filters and faults in pl_decode_generic's order (pl_key's for skipped_due_indel), without the 51-position limit.
 __global__ void __launch_bounds__(TR_THREADS) tr_read_kernel(const __grid_constant__ TrParams P) {
   ContigCache cc;
   unsigned long long n_unm = 0, n_skip = 0, n_cnt = 0, al[2] = {0, 0}, nb[2] = {0, 0}, first = ~0ull;
@@ -107,40 +107,24 @@ __global__ void __launch_bounds__(TR_THREADS) tr_read_kernel(const __grid_consta
     do {
       if (flags & PS_RF_UNMAPPED) { ++n_unm; break; }
       if (flags & PS_RF_CIGAR_OVERFLOW) { raise_fault(&P.st->fault, r, PS_FAULT_CIGAR_OPS); break; }
-      uint32_t R = 0, alen = 0, blk = 0;
-      bool hasI = false, hasD = false, hasN = false;
-      for (uint32_t e = 0; e < ncig; ++e) {
-        const uint32_t c = __ldg(cig + e), op = c & 15u;
-        hasI |= op == 1u; hasD |= op == 2u; hasN |= op == 3u;
-        if (op_consumes_ref(op)) R += c >> 4;
-        if (op_is_match(op)) { alen += c >> 4; ++blk; }
-      }
-      if ((hasI || hasD) && hasN) { ++n_skip; break; }
+      const CigarShape<> sh = cigar_shape(cig, ncig);
+      if (sh.skip) { ++n_skip; break; }
       if (flags & PS_RF_POS_ZERO) { raise_fault(&P.st->fault, r, PS_THROW_REF_RANGE); break; }
       const uint64_t g0 = __ldg(P.b.ref_start + r);
       if (!contig_lookup(P.ref, g0, cc)) { raise_fault(&P.st->fault, r, PS_THROW_REF_RANGE); break; }
-      bool bad = false;
-      int64_t rdp = 0, rfp = 0;
-      for (uint32_t e = 0; e < ncig && !bad; ++e) {
-        const uint32_t c = __ldg(cig + e), op = c & 15u;
-        const int64_t len = c >> 4;
-        if (op == 4u || op == 1u) rdp += len;
-        else if (op == 2u || op == 3u) rfp += len;
-        else if (op_is_match(op)) {
-          if (rdp + len > (int64_t)L) { raise_fault(&P.st->fault, r, PS_THROW_BLOCK_RANGE); bad = true; }
-          else if ((flags & PS_RF_REF_RANGE) || g0 + (uint64_t)(rfp + len) > cc.hi) {
-            raise_fault(&P.st->fault, r, PS_THROW_REF_RANGE); bad = true;
-          }
-          rdp += len; rfp += len;
-        }
-      }
-      if (bad) break;
-      const int32_t start = (int32_t)(g0 - cc.lo) + 1, end = start + (int32_t)R - 1;
+      uint32_t code = 0;
+      for_each_block(cig, ncig, [&](int64_t rdp, int64_t rfp, int64_t n) {
+        if (rdp + n > (int64_t)L) code = PS_THROW_BLOCK_RANGE;
+        else if ((flags & PS_RF_REF_RANGE) || g0 + (uint64_t)(rfp + n) > cc.hi) code = PS_THROW_REF_RANGE;
+        return code == 0;
+      });
+      if (code) { raise_fault(&P.st->fault, r, code); break; }
+      const int32_t start = (int32_t)(g0 - cc.lo) + 1, end = start + (int32_t)sh.ref_span - 1;
       const unsigned long long hi = (unsigned long long)(cc.rank + 1) << 32;
       key = make_ulonglong2(hi | (uint32_t)end, hi | (uint32_t)start);
       ++n_cnt;
-      al[(flags & PS_RF_REVERSE) ? 1 : 0] += alen;
-      nb[(flags & PS_RF_REVERSE) ? 1 : 0] += blk;
+      al[(flags & PS_RF_REVERSE) ? 1 : 0] += sh.aligned;
+      nb[(flags & PS_RF_REVERSE) ? 1 : 0] += sh.blocks;
       first = key.y < first ? key.y : first;
     } while (false);
     P.keys[r] = key;
@@ -222,16 +206,8 @@ __global__ void tr_seg_place_kernel(const __grid_constant__ TrParams P, uint32_t
   if (hi != ~0ull) atomicMin(&P.st->hi, hi);
 }
 
-__device__ __forceinline__ uint32_t tr_even_bits(uint32_t c) {   // even bits of c -> low 16 bits
-  c &= 0x55555555u;
-  c = (c | (c >> 1)) & 0x33333333u;
-  c = (c | (c >> 2)) & 0x0F0F0F0Fu;
-  c = (c | (c >> 4)) & 0x00FF00FFu;
-  c = (c | (c >> 8)) & 0x0000FFFFu;
-  return c;
-}
-
-// general path: one read, any CIGAR
+// general path: one read, any CIGAR.  It walks its blocks itself: through for_each_block every tr_accum_kernel
+// instantiation takes 2-4 more registers, and the BC ones spill (nvcc 12.9, sm_100a)
 __device__ __noinline__ void tr_accum_generic(const TrParams& P, uint64_t r, uint32_t meta, uint64_t off_base,
                                               uint64_t off_cigar, int64_t to_compact, unsigned long long* ev) {
   const uint32_t flags = PS_META_FLAGS(meta), ncig = PS_META_NCIGAR(meta);
@@ -286,25 +262,18 @@ __device__ __noinline__ void tr_bases_generic(const TrParams& P, uint64_t r, uin
   const uint64_t g0 = __ldg(P.b.ref_start + r);
   ExcRange ex{0, 0};
   if (has_inv) ex = read_exc_range(P.b, r / PS_TILE_READS, (uint32_t)(r % PS_TILE_READS));
-  int64_t rdp = 0, rfp = 0;
-  for (uint32_t e = 0; e < ncig; ++e) {
-    const uint32_t c = __ldg(cig + e), op = c & 15u;
-    const int64_t n = c >> 4;
-    if (op == 4u || op == 1u) rdp += n;
-    else if (op == 2u || op == 3u) rfp += n;
-    else if (op_is_match(op)) {
-      for (int64_t z = 0; z < n; ++z) {
-        const uint64_t g = g0 + (uint64_t)(rfp + z);
-        const uint32_t p = (uint32_t)(rdp + z);
-        if (ref_invalid_at(P.ref, g)) continue;
-        const uint32_t a = ref_code_at(P.ref, g) ^ flip;
-        const uint32_t bb = (has_inv && read_pos_invalid(P.b, ex, p)) ? 4u : (read_code_at(rb, p) ^ flip);
-        if (bb != a) atomicAdd(bc + (size_t)bb * P.M + (uint64_t)((int64_t)g + to_compact), 1u);
-        atomicAdd(tb + a * 5 + bb, 1ull);
-      }
-      rdp += n; rfp += n;
+  for_each_block(cig, ncig, [&](int64_t rdp, int64_t rfp, int64_t n) {
+    for (int64_t z = 0; z < n; ++z) {
+      const uint64_t g = g0 + (uint64_t)(rfp + z);
+      const uint32_t p = (uint32_t)(rdp + z);
+      if (ref_invalid_at(P.ref, g)) continue;
+      const uint32_t a = ref_code_at(P.ref, g) ^ flip;
+      const uint32_t bb = (has_inv && read_pos_invalid(P.b, ex, p)) ? 4u : (read_code_at(rb, p) ^ flip);
+      if (bb != a) atomicAdd(bc + (size_t)bb * P.M + (uint64_t)((int64_t)g + to_compact), 1u);
+      atomicAdd(tb + a * 5 + bb, 1ull);
     }
-  }
+    return true;
+  });
 }
 
 // base counts of one read on the bit-parallel path: mismatches are (ref ^ read) folded to one bit per base, N calls the
@@ -322,9 +291,9 @@ __device__ __forceinline__ void tr_bases_fast(const TrParams& P, const uint32_t 
 #pragma unroll
   for (int j = 0; j < NW; ++j) {
     const uint32_t rf = __funnelshift_r(w[j], w[j + 1], sh), rd = __funnelshift_r(bw[j], bw[j + 1], bsh), x = rf ^ rd;
-    lo |= (unsigned long long)tr_even_bits(rf) << (16 * j);
-    hi |= (unsigned long long)tr_even_bits(rf >> 1) << (16 * j);
-    mm |= (unsigned long long)tr_even_bits(x | (x >> 1)) << (16 * j);
+    lo |= (unsigned long long)even_bits(rf) << (16 * j);
+    hi |= (unsigned long long)even_bits(rf >> 1) << (16 * j);
+    mm |= (unsigned long long)even_bits(x | (x >> 1)) << (16 * j);
   }
   mm &= valid & ~nm;
 #pragma unroll
@@ -356,7 +325,7 @@ __device__ __forceinline__ void tr_bases_fast(const TrParams& P, const uint32_t 
 }
 
 // NW > 0: the batch has uniform length L <= 64 and one cigar op per read; reads whose op is M/=/X of length L take the
-// bit-parallel path (the positions listed in `exc` are cleared from its event mask: the code stored there is arbitrary)
+// bit-parallel path (t2c_word)
 template <int NW, bool BC>
 __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_constant__ TrParams P) {
   unsigned long long ev[2] = {0, 0}, fast = 0;
@@ -396,22 +365,8 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
         uint32_t bw[NW + 1], w[NW + 1];
 #pragma unroll
         for (int j = 0; j <= NW; ++j) { bw[j] = __ldg(src + j); w[j] = __ldg(P.ref.seq2 + (g0 >> 4) + j); }
-        const uint32_t sh = (g0 & 15u) * 2u, ii = g0 >> 5, s1 = g0 & 31u;
-        const uint32_t i0 = __ldg(P.ref.inv + ii), i1 = __ldg(P.ref.inv + ii + 1), i2 = NW > 2 ? __ldg(P.ref.inv + ii + 2) : 0u;
-        unsigned long long m = 0;
-#pragma unroll
-        for (int j = 0; j < NW; ++j) {
-          const uint32_t rf = __funnelshift_r(w[j], w[j + 1], sh);
-          const uint32_t rd = __funnelshift_r(bw[j], bw[j + 1], bsh);
-          // plus: ref T (11) and read C (01); minus: ref A (00) and read G (10)
-          const uint32_t h = rev ? (~(rf | (rf >> 1)) & (rd >> 1) & ~rd) : (rf & (rf >> 1) & rd & ~(rd >> 1));
-          m |= (unsigned long long)tr_even_bits(h) << (16 * j);
-        }
-        const unsigned long long inv = (unsigned long long)__funnelshift_r(i0, i1, s1) |
-                                       ((unsigned long long)(NW > 2 ? __funnelshift_r(i1, i2, s1) : 0u) << 32);
-        m &= ~inv;
-        m &= L >= 64 ? ~0ull : ((1ull << L) - 1ull);
-        if ((PS_META_FLAGS(meta) & PS_RF_HAS_INVALID) && m) m &= ~read_exc_mask64(P.b, r);   // only with a candidate event
+        const T2cWord tw = t2c_word<NW>(P.ref, P.b, r, g0, L, rev, (PS_META_FLAGS(meta) & PS_RF_HAS_INVALID) != 0, w, bw, bsh);
+        unsigned long long m = tw.t2c;
         const int64_t c0 = (int64_t)g0 + to_compact;
         atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0, 1);
         atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0 + L, -1);
@@ -422,7 +377,7 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
           m &= m - 1;
           atomicAdd(t2c + j, 1u);
         }
-        if constexpr (BC) tr_bases_fast<NW>(P, w, bw, sh, bsh, inv, L, meta, r, st, c0, tb);
+        if constexpr (BC) tr_bases_fast<NW>(P, w, bw, (g0 & 15u) * 2u, bsh, tw.ref_n, L, meta, r, st, c0, tb);
         ++fast;
         continue;
       }
@@ -877,16 +832,6 @@ struct ps_track {
   TrackOut out;
 };
 
-static DeviceBatch tr_view_of(const ps_read_batch* b) {
-  DeviceBatch v;
-  v.n_reads = b->n_reads; v.meta = b->meta; v.ref_start = b->ref_start; v.bases2 = b->bases2; v.qual = b->qual;
-  v.cigar = b->cigar; v.tile_base_off = b->tile_base_off; v.tile_qual_off = b->tile_qual_off;
-  v.tile_cigar_off = b->tile_cigar_off; v.tile_exc_off = b->tile_exc_off; v.exc = b->exc;
-  v.uniform_len = b->uniform_len; v.uniform_ncigar = b->uniform_ncigar; v.cigar_count = b->cigar_count; v.max_len = b->max_len;
-  v.past_end = b->past_end;
-  return v;
-}
-
 // a handle is returned with PS_OK and with a fault (PS_ERR_REFERENCE_WOULD_THROW, PS_ERR_UNSUPPORTED): ps_track_fault
 static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const TrackBases& bases, ps_track** out) {
   ps_track* h = new ps_track();
@@ -910,7 +855,7 @@ int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* b, const ps_track
   for (int slot = 0; slot < 2; ++slot)
     if (st != ctx->stream && b->n_reads && b->meta == ctx->staged[slot].view.meta && ctx->staged_core[slot])
       cudaStreamWaitEvent(st, ctx->staged_core[slot], 0);
-  return track_call(ctx, tr_view_of(b), st, bases, out);
+  return track_call(ctx, view_of(b), st, bases, out);
 }
 
 int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream, ps_track** out) {

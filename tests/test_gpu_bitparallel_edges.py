@@ -1,5 +1,5 @@
-"""GPU: the bit-parallel T>C decoders of the pileup (pl_decode<NW, false> -> t2c_mask_fast) and of the track
-(tr_accum_kernel<NW>) at their edges, bit for bit against the C++ restatements.
+"""GPU: the bit-parallel T>C word (t2c_word) in the pileup (pl_decode<NW, false> -> t2c_mask_fast) and in the track
+(tr_accum_kernel<NW>) at its edges, bit for bit against the C++ restatements.
 
 * every length arm: L = 1 .. 64 across the word edges 16 / 32 / 48, and 65, the first length on the generic paths;
   reads flush with both ends of every contig (the last one ends the genome), both strands, N calls, duplicates,
