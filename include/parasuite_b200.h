@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define PS_ABI_VERSION 6
+#define PS_ABI_VERSION 7
 
 /* ---- status codes ------------------------------------------------------------------------ */
 #define PS_OK 0
@@ -471,6 +471,67 @@ int ps_track_bam(ps_ctx* ctx, const char* bam_path, const char* out_prefix, ps_t
  * byte-identical to ps_track_bam's.  opts == NULL: ps_track_bam.  totals_out may be NULL. */
 int ps_track_bam_ex(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
                     ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out);
+/* Per-position deletion and insertion counts (indel_opts->indel_counts != 0), alone or beside base counts; the runs,
+ * sites and base rows stay as they are:
+ * - Scope: the records, faults, ordinals and strand rule of the track.  Records with (I or D) and N are skipped, so no
+ *   counted read has both an indel and a splice.
+ * - Deletions: every reference position inside a D op adds 1 to that position's deletion count on the read's strand.
+ *   This is not coverage (runs, sites and base rows do not change).  The reference base does not matter: a deletion over
+ *   a non-ACGT reference base is counted, and its row shows ref 4.
+ * - Insertions: every I op of non-zero length is one event, anchored at the last reference position the read consumed
+ *   before it, in genome orientation on both strands (as VCF and samtools place them).  An I with nothing before it but
+ *   S/H/P has no anchor: it counts in unanchored_insertions and gives no row.  3I2I is two events.
+ * - Zero-length ops (0D, 0I) count nothing.
+ * - Past the contig end: the track checks alignment blocks (and PS_RF_REF_RANGE, which ps_bam_next and the Python
+ *   batch producer set for a record whose span runs past its contig), so in a batch made otherwise a record such as
+ *   10M5D whose M block ends on the contig's last base spans past it.  Deleted positions past the contig's last base are
+ *   not counted (no row, not in deleted_bases; the op still counts in deletion_ops); an insertion anchored past it
+ *   counts as unanchored.
+ * - Rows: a (position, strand) gets one when del + ins >= min_events and cov + del >= min_depth (cov: that strand's
+ *   coverage there); a threshold of 0 counts as 1.  Rows come in the order of the sites and base rows: contigs in the
+ *   order the records visit them, then by position, plus before minus.  ref: the reference base in strand orientation,
+ *   A0 C1 G2 T3, 4 = not ACGT.
+ * - Totals per strand: sum over positions of del = deleted_bases, sum of ins = insertion_ops - unanchored_insertions;
+ *   with both thresholds at 1 the rows hold exactly those sums.  A faulting call reports no rows and zero totals. */
+typedef struct ps_track_indel_opts {
+  uint32_t indel_counts;         /* 0: off */
+  uint32_t min_depth;            /* cov + del at the position and strand */
+  uint32_t min_events;           /* del + ins */
+  uint32_t reserved;             /* must be 0: PS_ERR_INVALID_ARG otherwise */
+} ps_track_indel_opts;
+typedef struct ps_track_indel_row { /* 24 B */
+  uint32_t contig;               /* FASTA index */
+  int32_t pos;                   /* 1-based */
+  uint8_t strand;                /* 0 plus, 1 minus */
+  uint8_t ref;                   /* reference base in strand orientation, A0 C1 G2 T3, 4 = not ACGT */
+  uint16_t reserved;
+  uint32_t cov;                  /* coverage of that strand at pos */
+  uint32_t del;                  /* deletions over pos */
+  uint32_t ins;                  /* insertions anchored at pos */
+} ps_track_indel_row;
+typedef struct ps_track_indel_totals {
+  uint64_t deletion_ops[2];      /* [strand]: D ops of non-zero length */
+  uint64_t deleted_bases[2];     /* their positions on the contig */
+  uint64_t insertion_ops[2];     /* I ops of non-zero length */
+  uint64_t inserted_bases[2];
+  uint64_t unanchored_insertions[2];
+  uint64_t n_rows;
+} ps_track_indel_totals;
+/* indel_opts == NULL: ps_track_batch_ex / ps_track_batch_device_ex */
+int ps_track_batch_ex2(ps_ctx* ctx, const ps_read_batch* host_batch, const ps_track_opts* opts,
+                       const ps_track_indel_opts* indel_opts, ps_track** out);
+int ps_track_batch_device_ex2(ps_ctx* ctx, const ps_read_batch* dev_batch, const ps_track_opts* opts,
+                              const ps_track_indel_opts* indel_opts, void* stream, ps_track** out);
+/* PS_ERR_STATE on a handle made without indel counts; rows: copy up to `max` from `first`, returns the number copied */
+int64_t ps_track_indel_rows(const ps_track* h, uint64_t first, ps_track_indel_row* rows, uint64_t max);
+int ps_track_indel_totals_get(const ps_track* h, ps_track_indel_totals* out);
+/* With indel_opts->indel_counts also <out_prefix>.indels.tsv (header chrom/pos/strand/ref/coverage/deletions/insertions,
+ * the rows of ps_track_indel_rows, pos 1-based, ref a letter with N for 4), independent of the window size and the number
+ * of devices; the other files are byte-identical to ps_track_bam_ex's.  indel_opts == NULL: ps_track_bam_ex.
+ * indel_totals_out may be NULL. */
+int ps_track_bam_ex2(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                     const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
+                     ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out, ps_fault* fault_out);
 
 /* ---- `comb` tool (host only): transcript hits lifted to genomic coordinates, merged with the genomic hits ---------------
  * Replaces CombineGenomeTranscript.combine / printReadsToBamFile (utils/postprocessing/CombineGenomeTranscript.java:36-666;
@@ -513,6 +574,10 @@ int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix
                        ps_fault* fault_out);
 int ps_multi_track_bam_ex(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
                           ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out);
+int ps_multi_track_bam_ex2(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                           const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
+                           ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out,
+                           ps_fault* fault_out);
 
 /* ---- host batcher (usable without a GPU) --------------------------------------------------------
  * What htsjdk does for the two loops, as a library: FASTA(+.fai) -> packed reference; BGZF/BAM -> SoA batches in

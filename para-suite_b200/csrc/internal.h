@@ -171,8 +171,9 @@ struct ps_ctx {
   bool pl_flag_scan_kernel = false;   // PARASUITE_B200_FLAG_SCAN_KERNEL=1 at ps_create: always prefix the tile table with the one-block scan (tests)
   bool pl_compact_lookback = false;   // PARASUITE_B200_COMPACT_LOOKBACK=1 at ps_create: always order the site runs with the look-back (tests)
   bool pl_exact_flags = false;   // a speculative flag pass failed on this context: keep to the exact look-back kernel
-  // track scratch (track.cu): run state, keys, scans, segments, position arrays, selections, records, dense head / tail
-  DevBuf tr_scratch[13];
+  // track scratch (track.cu): run state, keys, scans, segments, position arrays, selections, records, dense head / tail,
+  // base rows, indel rows
+  DevBuf tr_scratch[14];
 };
 
 // ---- pileup handles over host-resident records (pileup.cu; used by the windowed file loops in tool_loops.cpp) --------

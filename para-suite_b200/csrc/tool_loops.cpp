@@ -366,26 +366,26 @@ int pileup_windows(ps_multi* m, const char* bam_path, const ps_pileup_opts* opts
 
 
 // ---- track files -------------------------------------------------------------------------------------------------------
-// The files of the track tool: three, and with base counts a fourth.  Runs that touch with equal coverage are merged, so
-// a run cut by a window boundary is one row.
+// The files of the track tool: three, with base counts a fourth and with indel counts a fifth.  Runs that touch with
+// equal coverage are merged, so a run cut by a window boundary is one row.
 struct TrackWriter {
-  FILE* f[4] = {nullptr, nullptr, nullptr, nullptr};   // plus bedGraph, minus bedGraph, t2c tsv, bases tsv
-  int nf = 3;
+  FILE* f[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // plus bedGraph, minus bedGraph, t2c, bases, indels
   std::vector<std::string> names;
   ps_track_run last[2]{};
   bool have[2] = {false, false};
-  uint64_t rows[4] = {0, 0, 0, 0};
+  uint64_t rows[5] = {0, 0, 0, 0, 0};
   uint64_t merged[2] = {0, 0};                  // runs joined to the one before
-  std::string buf[4];
-  int open(const std::string& prefix, bool bases) {
-    const char* ext[4] = {".plus.bedGraph", ".minus.bedGraph", ".t2c.tsv", ".bases.tsv"};
-    nf = bases ? 4 : 3;
-    for (int k = 0; k < nf; ++k) {
+  std::string buf[5];
+  int open(const std::string& prefix, bool bases, bool indels) {
+    const char* ext[5] = {".plus.bedGraph", ".minus.bedGraph", ".t2c.tsv", ".bases.tsv", ".indels.tsv"};
+    for (int k = 0; k < 5; ++k) {
+      if ((k == 3 && !bases) || (k == 4 && !indels)) continue;
       f[k] = fopen((prefix + ext[k]).c_str(), "wb");
       if (!f[k]) return PS_ERR_IO;
     }
     buf[2] = "chrom\tpos\tstrand\tt2c\tcoverage\n";
     if (bases) buf[3] = "chrom\tpos\tstrand\tref\tcoverage\tA\tC\tG\tT\tN\n";
+    if (indels) buf[4] = "chrom\tpos\tstrand\tref\tcoverage\tdeletions\tinsertions\n";
     return PS_OK;
   }
   static void num(std::string& b, uint64_t v) {
@@ -444,40 +444,56 @@ struct TrackWriter {
     ++rows[3];
     return drain(3, false);
   }
+  int indel_row(const ps_track_indel_row& x) {
+    std::string& b = buf[4];
+    b += names[x.contig]; b.push_back('\t');
+    num(b, (uint32_t)x.pos); b.push_back('\t');
+    b.push_back(x.strand ? '-' : '+'); b.push_back('\t');
+    b.push_back(x.ref < 4 ? "ACGT"[x.ref] : 'N');
+    b.push_back('\t'); num(b, x.cov);
+    b.push_back('\t'); num(b, x.del);
+    b.push_back('\t'); num(b, x.ins);
+    b.push_back('\n');
+    ++rows[4];
+    return drain(4, false);
+  }
   int finish() {
     int rc = PS_OK;
     for (int s = 0; s < 2; ++s) if (rc == PS_OK) rc = flush_run(s);
-    for (int k = 0; k < nf; ++k) if (rc == PS_OK) rc = drain(k, true);
+    for (int k = 0; k < 5; ++k) if (rc == PS_OK && f[k]) rc = drain(k, true);
     return rc;
   }
   ~TrackWriter() { for (FILE* x : f) if (x) fclose(x); }
   // the rows of one window, in file order
   int write(const std::vector<ps_track_run>* runs, const std::vector<ps_track_site>& sites,
-            const std::vector<ps_track_base_row>& base_rows) {
+            const std::vector<ps_track_base_row>& base_rows, const std::vector<ps_track_indel_row>& indel_rows) {
     int rc = PS_OK;
     for (int s = 0; s < 2 && rc == PS_OK; ++s)
       for (const ps_track_run& r : runs[s]) if ((rc = run(s, r)) != PS_OK) break;
     for (const ps_track_site& x : sites) if (rc != PS_OK || (rc = site(x)) != PS_OK) break;
     for (const ps_track_base_row& x : base_rows) if (rc != PS_OK || (rc = base_row(x)) != PS_OK) break;
+    for (const ps_track_indel_row& x : indel_rows) if (rc != PS_OK || (rc = indel_row(x)) != PS_OK) break;
     return rc;
   }
 };
 
-// what a window hands to the writer: final runs, sites and base rows, in file order
+// what a window hands to the writer: final runs, sites, base rows and indel rows, in file order
 struct TrackRows {
   std::vector<ps_track_run> runs[2];
   std::vector<ps_track_site> sites;
   std::vector<ps_track_base_row> base_rows;
+  std::vector<ps_track_indel_row> indel_rows;
 };
 
-// positions not final yet: [key0, key0 + len) of one contig, cov+, cov-, t2c+, t2c-, and with base counts the ten
-// event counters (TrackDense)
+// positions not final yet: [key0, key0 + len) of one contig, cov+, cov-, t2c+, t2c-, with base counts the ten event
+// counters, then with indel counts del+, del-, ins+, ins- (TrackDense)
 struct TrackPending {
   unsigned long long key0 = 0;
-  std::vector<uint32_t> v[14];
+  std::vector<uint32_t> v[18];
   int nv = 4;
   TrackBases bases;
-  const ps_reference* ref = nullptr;     // host packed FASTA: the reference base of a base row
+  TrackIndels indels;
+  const ps_reference* ref = nullptr;     // host packed FASTA: the reference base of a base or indel row
   size_t len() const { return v[0].size(); }
   // rows of the positions before `upto` (keys), which leave the region
   void emit_before(unsigned long long upto, const std::vector<uint32_t>& by_rank, TrackRows& out) {
@@ -514,6 +530,20 @@ struct TrackPending {
           out.base_rows.push_back(x);
         }
       }
+    if (indels.on) {
+      const int id = bases.on ? 14 : 4;              // del+, del-, ins+, ins-
+      for (size_t k = 0; k < k_end; ++k)
+        for (int s = 0; s < 2; ++s) {
+          const uint32_t del = v[id + s][k], ins = v[id + 2 + s][k];
+          if (!track_indel_row(indels, v[s][k], del, ins)) continue;
+          const uint64_t g = ref->contig_off[contig] + p0 + k;     // on the contig: nothing past its end is counted
+          ps_track_indel_row x{};
+          x.contig = contig; x.pos = (int32_t)(p0 + k + 1); x.strand = (uint8_t)s;
+          x.ref = ((ref->inv[g >> 5] >> (g & 31)) & 1u) ? 4 : (uint8_t)(((ref->seq2[g >> 4] >> (2 * (g & 15))) & 3u) ^ (s ? 3u : 0u));
+          x.cov = v[s][k]; x.del = del; x.ins = ins;
+          out.indel_rows.push_back(x);
+        }
+    }
     for (int j = 0; j < nv; ++j) v[j].erase(v[j].begin(), v[j].begin() + (ptrdiff_t)k_end);
     key0 += k_end;
   }
@@ -530,16 +560,19 @@ struct TrackFlight {
 };
 
 // The windowed track over an open file (contexts keyed in the file's contig order)
-int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWriter& W, ps_track_counters* ctr,
-                      ps_track_base_totals* totals, ps_fault* fault) {
+int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, const TrackIndels& indels, TrackWriter& W,
+                      ps_track_counters* ctr, ps_track_base_totals* totals, ps_track_indel_totals* indel_totals,
+                      ps_fault* fault) {
   ps_ctx* c0 = m->ctx[0];
   const std::vector<uint64_t>& contig_off = c0->contig_off;
   const std::vector<uint32_t>& by_rank = c0->contig_by_rank;
   memset(ctr, 0, sizeof *ctr);
   memset(totals, 0, sizeof *totals);
+  memset(indel_totals, 0, sizeof *indel_totals);
   TrackPending P;
   P.bases = bases;
-  P.nv = bases.on ? 14 : 4;
+  P.indels = indels;
+  P.nv = (bases.on ? 14 : 4) + (indels.on ? 4 : 0);
   P.ref = ps_fasta_reference(c0->fasta);
   unsigned long long last_start = 0, max_end = 0;     // over the windows launched so far / completed so far
   uint64_t offset = 0, window = 0;
@@ -576,6 +609,13 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWrit
     for (int s = 0; s < 2; ++s)
       for (int a = 0; a < 4; ++a)
         for (int c = 0; c < 5; ++c) totals->bases[s][a][c] += o.totals.bases[s][a][c];
+    for (int s = 0; s < 2; ++s) {
+      indel_totals->deletion_ops[s] += o.indel_totals.deletion_ops[s];
+      indel_totals->deleted_bases[s] += o.indel_totals.deleted_bases[s];
+      indel_totals->insertion_ops[s] += o.indel_totals.insertion_ops[s];
+      indel_totals->inserted_bases[s] += o.indel_totals.inserted_bases[s];
+      indel_totals->unanchored_insertions[s] += o.indel_totals.unanchored_insertions[s];
+    }
     if (!o.first_key) { print_window(o, 0); return PS_OK; }      // no kept record: nothing changes
     if (o.first_key < last_start) return multi_fail(m, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
     if (o.head.len) {
@@ -592,6 +632,7 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWrit
     for (int s = 0; s < 2; ++s) rows->runs[s].insert(rows->runs[s].end(), o.runs[s].begin(), o.runs[s].end());
     rows->sites.insert(rows->sites.end(), o.sites.begin(), o.sites.end());
     rows->base_rows.insert(rows->base_rows.end(), o.base_rows.begin(), o.base_rows.end());
+    rows->indel_rows.insert(rows->indel_rows.end(), o.indel_rows.begin(), o.indel_rows.end());
     if (o.tail.len) {
       if (P.len() && P.key0 + P.len() != o.tail.key0) return multi_fail(m, PS_ERR_STATE, "track: window tail not next to the pending region");
       if (!P.len()) P.key0 = o.tail.key0;
@@ -601,7 +642,7 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWrit
     print_window(o, emitted);
     const int prev_rc = join_sink();
     if (prev_rc != PS_OK) return prev_rc;
-    sink_thread = std::thread([&W, &sink_rc, rows] { sink_rc = W.write(rows->runs, rows->sites, rows->base_rows); });
+    sink_thread = std::thread([&W, &sink_rc, rows] { sink_rc = W.write(rows->runs, rows->sites, rows->base_rows, rows->indel_rows); });
     return PS_OK;
   };
   int st = PS_OK;
@@ -622,9 +663,9 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWrit
     f.ctx = c; f.offset = offset; f.rc = PS_OK; f.live = true;
     const DeviceBatch view = sb->view;
     const uint64_t prev_end = max_end;
-    f.th = std::thread([&f, c, view, prev_end, &bases] {
+    f.th = std::thread([&f, c, view, prev_end, &bases, &indels] {
       cudaSetDevice(c->device);
-      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out, bases);
+      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out, bases, indels);
       if (f.rc != PS_OK) f.err = c->err;
     });
     max_end = std::max<unsigned long long>(max_end, host_max_key(hb, contig_off, c0->contig_rank));
@@ -643,13 +684,14 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, TrackWrit
   if (st != PS_OK) return st;
   TrackRows rest;
   P.emit_before(~0ull, by_rank, rest);
-  st = W.write(rest.runs, rest.sites, rest.base_rows);
+  st = W.write(rest.runs, rest.sites, rest.base_rows, rest.indel_rows);
   if (st == PS_OK) st = W.finish();
   if (st != PS_OK) return multi_fail(m, st, "track: writing the output files failed");
   ctr->n_runs[0] = W.rows[0];
   ctr->n_runs[1] = W.rows[1];
   ctr->n_sites = W.rows[2];
   totals->n_rows = W.rows[3];
+  indel_totals->n_rows = W.rows[4];
   if (dbg)
     fprintf(stderr, "[ps_track_files] runs %llu %llu, merged %llu %llu, sites %llu\n", (unsigned long long)W.rows[0],
             (unsigned long long)W.rows[1], (unsigned long long)W.merged[0], (unsigned long long)W.merged[1],
@@ -924,28 +966,40 @@ int ps_clust_bam(ps_ctx* ctx, const char* bam_path, const char* out_path, const 
   return st;
 }
 
-// The track tool from files: <out_prefix>.plus.bedGraph, .minus.bedGraph, .t2c.tsv, and with base counts .bases.tsv
-int ps_multi_track_bam_ex(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
-                          ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out) {
+// The track tool from files: <out_prefix>.plus.bedGraph, .minus.bedGraph, .t2c.tsv, with base counts .bases.tsv and with
+// indel counts .indels.tsv
+int ps_multi_track_bam_ex2(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                           const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
+                           ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out,
+                           ps_fault* fault_out) {
   if (!m || !bam_path || !out_prefix) return PS_ERR_INVALID_ARG;
   TrackBases bases;
   if (track_bases_of(opts, &bases) != PS_OK) return multi_fail(m, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
+  TrackIndels indels;
+  if (track_indels_of(indel_opts, &indels) != PS_OK) return multi_fail(m, PS_ERR_INVALID_ARG, "track: indel option reserved field is not 0");
   if (m->ctx.empty() || !m->ctx[0]->fasta) return multi_fail(m, PS_ERR_STATE, "load the reference first (ps_multi_load_fasta)");
   ps_ctx* c0 = m->ctx[0];
   TrackWriter W;
   for (uint32_t i = 0; i < c0->ref.n_contigs; ++i) W.names.push_back(ps_fasta_contig_name(c0->fasta, i));
-  int st = W.open(out_prefix, bases.on);
+  int st = W.open(out_prefix, bases.on, indels.on);
   if (st != PS_OK) return multi_fail(m, st, std::string("cannot write ") + out_prefix + ".*");
   ps_track_counters ctr{};
   ps_track_base_totals totals{};
+  ps_track_indel_totals indel_totals{};
   ps_fault fault{};
   st = with_file_order(m, bam_path, window_reads_default(), [&](ps_bam* B) {
-    return track_windows_run(m, B, bases, W, &ctr, &totals, &fault);
+    return track_windows_run(m, B, bases, indels, W, &ctr, &totals, &indel_totals, &fault);
   });
   if (counters_out) *counters_out = ctr;
   if (totals_out) *totals_out = totals;
+  if (indel_totals_out) *indel_totals_out = indel_totals;
   if (fault_out) *fault_out = fault;
   return st;
+}
+
+int ps_multi_track_bam_ex(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                          ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out) {
+  return ps_multi_track_bam_ex2(m, bam_path, out_prefix, opts, nullptr, counters_out, totals_out, nullptr, fault_out);
 }
 
 int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,
@@ -953,14 +1007,21 @@ int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix
   return ps_multi_track_bam_ex(m, bam_path, out_prefix, nullptr, counters_out, nullptr, fault_out);
 }
 
-int ps_track_bam_ex(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
-                    ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out) {
+int ps_track_bam_ex2(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                     const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
+                     ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out, ps_fault* fault_out) {
   if (!ctx || !bam_path || !out_prefix) return set_error(ctx, PS_ERR_INVALID_ARG, "NULL argument");
   ps_multi m;
   borrow(m, ctx);
-  const int st = ps_multi_track_bam_ex(&m, bam_path, out_prefix, opts, counters_out, totals_out, fault_out);
+  const int st = ps_multi_track_bam_ex2(&m, bam_path, out_prefix, opts, indel_opts, counters_out, totals_out,
+                                        indel_totals_out, fault_out);
   if (st != PS_OK && !m.err.empty()) set_error(ctx, st, m.err);
   return st;
+}
+
+int ps_track_bam_ex(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                    ps_track_counters* counters_out, ps_track_base_totals* totals_out, ps_fault* fault_out) {
+  return ps_track_bam_ex2(ctx, bam_path, out_prefix, opts, nullptr, counters_out, totals_out, nullptr, fault_out);
 }
 
 int ps_track_bam(ps_ctx* ctx, const char* bam_path, const char* out_prefix, ps_track_counters* counters_out,

@@ -26,6 +26,10 @@
 //   (CUB) select         run starts / ends per strand, T>C sites; tr_emit_*_kernel turn them into records.  BC: a select
 //                        of the (position, strand) items with >= min_events non-N events, then tr_base_rows_kernel
 //                        (reference base, mask, min_coverage) and a select of the rows it kept
+//   tr_indel_kernel      (indel counts, in the accumulate stage) per read with a non-empty I or D: +1/-1 per D op into
+//                        one int32 difference array per strand, +1 per anchored I op; (CUB) sum scans beside the
+//                        coverage scans; a select of the (position, strand) items with >= min_events deletions and
+//                        insertions, tr_indel_rows_kernel (min_depth, reference base) and a select of the rows it kept
 // Compact space: M = sum over segments of (span + 1) <= sum over kept reads of (reference span + 1).
 #include <cub/cub.cuh>
 #include <thrust/iterator/counting_iterator.h>
@@ -56,6 +60,7 @@ struct TrState {
   unsigned long long lo, hi;         // reported compact range [lo, hi)
   unsigned int unsorted;
   unsigned long long bases[2][4][5]; // base counts: [strand][ref][read A C G T N], strand orientation
+  unsigned long long indel[10];      // indel counts: the ten per-strand totals of ps_track_indel_totals, in its order
 };
 
 struct TrParams {
@@ -76,6 +81,8 @@ struct TrParams {
   unsigned long long prev_end;       // windowed: max end key over the earlier windows (0: none)
   int windowed;
   uint32_t* bc;                      // base counts: [2][5][M] events by read base A C G T N (strand orientation)
+  int32_t* idel;                     // indel counts: [2][M + 1] deletion difference arrays, then (scan) deletions
+  uint32_t* ins;                     // indel counts: [2][M] insertions by anchor
 };
 
 struct MaxPair {
@@ -398,6 +405,92 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
   }
 }
 
+// indel counts, one read per thread, any CIGAR: a D op adds +1 / -1 to the deletion difference array of the read's strand
+// (one pair of atomics whatever its length), an I op +1 at its anchor, the last reference position consumed before it.
+// The anchor is on the left so that every counted position lies inside the read's span [start, end]: the segments, the
+// compact space and the window head / tail already cover that span and nothing else.  The blocks were checked against
+// the contig's end, the D ops were not: positions from the contig's end on are not counted (their global offsets would
+// read the next contig).  A read without a non-empty I or D leaves after its CIGAR words.
+__global__ void __launch_bounds__(TR_THREADS) tr_indel_kernel(const __grid_constant__ TrParams P) {
+  // TrState::indel per thread: the bases in 64 bits, the op counts in 32 (a read has at most 255 ops, and a batch fewer
+  // than 2^32 reads over at least 2048 threads)
+  unsigned long long td[2] = {0, 0}, ti[2] = {0, 0};   // deleted and inserted bases by strand
+  uint32_t t[6] = {0, 0, 0, 0, 0, 0};             // deletion ops, insertion ops, unanchored by strand
+  ContigCache cc;
+  const uint64_t n = P.b.n_reads;
+  for (uint64_t q = ((uint64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31u)); q < n; q += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t r = q + (threadIdx.x & 31u);
+    const bool in = r < n;
+    const uint32_t meta = in ? __ldg(P.b.meta + r) : 0u;
+    const ReadOffsets off = warp_read_offsets(P.b, q, r, in, meta);    // warp-collective
+    if (!in) continue;
+    const uint32_t ncig = PS_META_NCIGAR(meta);
+    const uint32_t* cig = P.b.cigar + off.cigar;
+    bool any = false;
+    for (uint32_t e = 0; e < ncig; ++e) {
+      const uint32_t c = __ldg(cig + e), op = c & 15u;
+      any |= (op == 1u || op == 2u) && (c >> 4);
+    }
+    if (!any) continue;
+    const ulonglong2 k = P.keys[r];
+    if (!k.x) continue;
+    const uint32_t s = P.flag[r] - 1;
+    const int64_t to_compact = (int64_t)P.seg_base[s] - (int64_t)P.seg_g[s];
+    const uint64_t g0 = __ldg(P.b.ref_start + r);
+    contig_lookup(P.ref, g0, cc);
+    const int st = (PS_META_FLAGS(meta) & PS_RF_REVERSE) ? 1 : 0;
+    int32_t* del = P.idel + (size_t)st * (P.M + 1);
+    uint32_t* ins = P.ins + (size_t)st * P.M;
+    uint32_t c3[3] = {0, 0, 0};                    // this read's totals: the strand index stays static
+    unsigned long long cd = 0, ci = 0;
+    uint64_t g = g0;                               // the next reference position
+    for (uint32_t e = 0; e < ncig; ++e) {
+      const uint32_t c = __ldg(cig + e), op = c & 15u, len = c >> 4;
+      if (op == 2u && len) {
+        ++c3[0];
+        if (g < cc.hi) {
+          const uint64_t m = min((uint64_t)len, cc.hi - g);
+          const int64_t i0 = (int64_t)g + to_compact;
+          atomicAdd(del + i0, 1);
+          atomicAdd(del + i0 + (int64_t)m, -1);
+          cd += m;
+        }
+      } else if (op == 1u && len) {
+        ++c3[1];
+        ci += len;
+        if (g > g0 && g - 1 < cc.hi) atomicAdd(ins + ((int64_t)g - 1 + to_compact), 1u);
+        else ++c3[2];
+      }
+      if (op_consumes_ref(op)) g += len;
+    }
+    td[0] += st ? 0ull : cd;
+    td[1] += st ? cd : 0ull;
+    ti[0] += st ? 0ull : ci;
+    ti[1] += st ? ci : 0ull;
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+      t[2 * j] += st ? 0u : c3[j];
+      t[2 * j + 1] += st ? c3[j] : 0u;
+    }
+  }
+  // warp sums in 64 bits, one atomic per warp and counter: deletion_ops, deleted_bases, insertion_ops, inserted_bases,
+  // unanchored_insertions (ps_track_indel_totals order)
+  unsigned long long w[10];
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    w[s] = warp_sum(t[s]);
+    w[2 + s] = warp_sum(td[s]);
+    w[4 + s] = warp_sum(t[2 + s]);
+    w[6 + s] = warp_sum(ti[s]);
+    w[8 + s] = warp_sum(t[4 + s]);
+  }
+  if ((threadIdx.x & 31u) == 0) {
+#pragma unroll
+    for (int j = 0; j < 10; ++j)
+      if (w[j]) atomicAdd(&P.st->indel[j], w[j]);
+  }
+}
+
 // ---- selection predicates over compact indices -------------------------------------------------------------------
 struct RunStart {
   const int32_t* cov; unsigned long long lo;
@@ -429,6 +522,16 @@ struct BaseCandidate {   // item 2*i + strand: at least min_ev events other than
 };
 struct RowKept {
   __device__ __forceinline__ bool operator()(const ps_track_base_row& x) const { return x.cov != 0u; }
+};
+struct IndelCandidate {  // item 2*i + strand: at least min_ev deletions and insertions
+  const int32_t* del; const uint32_t* ins; uint64_t M; uint32_t min_ev;
+  __device__ __forceinline__ bool operator()(const unsigned long long& k) const {
+    const uint64_t s = k & 1ull, i = k >> 1;
+    return (uint64_t)(uint32_t)del[s * (M + 1) + i] + ins[s * M + i] >= min_ev;
+  }
+};
+struct IndelRowKept {
+  __device__ __forceinline__ bool operator()(const ps_track_indel_row& x) const { return x.del != 0u || x.ins != 0u; }
 };
 
 // segment of compact index i (seg_base ascending)
@@ -502,9 +605,33 @@ __global__ void tr_base_rows_kernel(const __grid_constant__ TrParams P, uint32_t
   out[k] = x;
 }
 
-// dense copy of the positions [key0, key0 + len) (one contig) from the compact arrays: cov+, cov-, t2c+, t2c-, and with
-// base counts (BC) the ten event counters
-template <bool BC>
+// one indel row per candidate (min_depth decides, track_indel_row); del = ins = 0: no row
+__global__ void tr_indel_rows_kernel(const __grid_constant__ TrParams P, uint32_t n_segs, const unsigned long long* cand,
+                                     uint64_t n, TrackIndels sel, ps_track_indel_row* out) {
+  const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const unsigned long long it = cand[k], i = it >> 1;
+  const uint32_t strand = (uint32_t)(it & 1ull);
+  const uint32_t s = seg_of(P, n_segs, i);
+  const uint32_t cov = (uint32_t)P.diff[(size_t)strand * (P.M + 1) + i];
+  const uint32_t del = (uint32_t)P.idel[(size_t)strand * (P.M + 1) + i], ins = P.ins[(size_t)strand * P.M + i];
+  ps_track_indel_row x{};
+  if (track_indel_row(sel, cov, del, ins)) {
+    const uint64_t g = (uint64_t)P.seg_g[s] + (i - P.seg_base[s]);   // on the contig: nothing past its end is counted
+    x.contig = P.seg_contig[s];
+    x.pos = (int32_t)pos0_of(P, s, i) + 1;
+    x.strand = (uint8_t)strand;
+    x.ref = (uint8_t)(ref_invalid_at(P.ref, g) ? 4u : ref_code_at(P.ref, g) ^ (strand ? 3u : 0u));
+    x.cov = cov;
+    x.del = del;
+    x.ins = ins;
+  }
+  out[k] = x;
+}
+
+// dense copy of the positions [key0, key0 + len) (one contig) from the compact arrays: cov+, cov-, t2c+, t2c-, with
+// base counts (BC) the ten event counters, then with indel counts (ID) del+, del-, ins+, ins-
+template <bool BC, bool ID>
 __global__ void tr_dense_kernel(const __grid_constant__ TrParams P, uint32_t n_segs, unsigned long long key0, uint32_t len,
                                 uint32_t* out) {
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -515,7 +642,7 @@ __global__ void tr_dense_kernel(const __grid_constant__ TrParams P, uint32_t n_s
     const uint32_t mid = (lo + hi) >> 1;
     if (P.seg_key[mid] <= key) lo = mid; else hi = mid;
   }
-  constexpr int NV = BC ? 14 : 4;
+  constexpr int NB = BC ? 14 : 4, NV = NB + (ID ? 4 : 0);
   uint32_t v[NV] = {};
   const unsigned long long k0 = P.seg_key[lo];
   if (key >= k0 && (key >> 32) == (k0 >> 32) && key - k0 < P.seg_end[lo]) {
@@ -526,7 +653,13 @@ __global__ void tr_dense_kernel(const __grid_constant__ TrParams P, uint32_t n_s
     v[3] = P.t2c[P.M + i];
     if constexpr (BC) {
 #pragma unroll
-      for (int j = 4; j < NV; ++j) v[j] = P.bc[(size_t)(j - 4) * P.M + i];
+      for (int j = 4; j < NB; ++j) v[j] = P.bc[(size_t)(j - 4) * P.M + i];
+    }
+    if constexpr (ID) {
+      v[NB] = (uint32_t)P.idel[i];
+      v[NB + 1] = (uint32_t)P.idel[(P.M + 1) + i];
+      v[NB + 2] = P.ins[i];
+      v[NB + 3] = P.ins[P.M + i];
     }
   }
 #pragma unroll
@@ -580,17 +713,29 @@ int track_bases_of(const ps_track_opts* o, TrackBases* out) {
   return PS_OK;
 }
 
+int track_indels_of(const ps_track_indel_opts* o, TrackIndels* out) {
+  *out = TrackIndels();
+  if (!o) return PS_OK;
+  if (o->reserved) return PS_ERR_INVALID_ARG;
+  out->on = o->indel_counts != 0;
+  out->min_depth = std::max<uint32_t>(1u, o->min_depth);
+  out->min_ev = std::max<uint32_t>(1u, o->min_events);
+  return PS_OK;
+}
+
 int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out,
-              const TrackBases& bases) {
+              const TrackBases& bases, const TrackIndels& indels) {
   if (b.past_end && b.past_end <= b.n_reads) {
     // a record past its contig's end: the reads before it decide whether an earlier record faults first
     DeviceBatch head = b;
     head.n_reads = b.past_end - 1;
     head.past_end = 0;
-    const int rc = track_run(ctx, head, st, windowed, prev_end, out, bases);
+    const int rc = track_run(ctx, head, st, windowed, prev_end, out, bases, indels);
     if (rc != PS_OK && rc != PS_ERR_UNSORTED) return rc;
-    out->base_rows.clear();                // a faulting call reports no base rows
+    out->base_rows.clear();                // a faulting call reports no base or indel rows
     out->totals = ps_track_base_totals{};
+    out->indel_rows.clear();
+    out->indel_totals = ps_track_indel_totals{};
     out->ctr.num_reads_processed = b.n_reads;
     out->fault.code = PS_FAULT_PAST_END;
     out->fault.read_ordinal = b.past_end - 1;
@@ -598,6 +743,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   }
   *out = TrackOut();
   out->bases_on = bases.on;
+  out->indels_on = indels.on;
   const uint64_t n = b.n_reads;
   out->ctr.num_reads_processed = n;
   if (n == 0) return PS_OK;
@@ -614,6 +760,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   timer_begin(ctx, st);
   tr_init_state<<<1, 1, 0, st>>>(d_st);
   if (bases.on) TR_CUDA(cudaMemsetAsync(d_st->bases, 0, sizeof d_st->bases, st));
+  if (indels.on) TR_CUDA(cudaMemsetAsync(d_st->indel, 0, sizeof d_st->indel, st));
   tr_read_kernel<<<grid_g, TR_THREADS, 0, st>>>(P);
   TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceScan::InclusiveScan(t, sz, P.keys, P.scan, MaxPair(), (int64_t)n, st); }));
   tr_segment_kernel<<<grid_for(n), TR_THREADS, 0, st>>>(P);
@@ -676,14 +823,18 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   if (M >= (1ull << 31)) return set_error(ctx, PS_ERR_UNSUPPORTED, "track: the reads of one batch span more than 2^31 positions");
   const uint64_t lo = std::min<uint64_t>(hp.lo, M), hi = std::max<uint64_t>(lo, std::min<uint64_t>(hp.hi, M));
   P.M = M;
-  // difference arrays / coverage, the T>C counts, then (base counts) the event counters
-  P.diff = slot<int32_t>(ctx, 5, 4 * (M + 1) + (bases.on ? 10 * M : 0), err);
+  // difference arrays / coverage, the T>C counts, (base counts) the event counters, then (indel counts) the deletion
+  // difference arrays / deletions and the insertions: 16 B more per position
+  P.diff = slot<int32_t>(ctx, 5, 4 * (M + 1) + (bases.on ? 10 * M : 0) + (indels.on ? 4 * (M + 1) : 0), err);
   TR_CUDA(err);
   P.t2c = reinterpret_cast<uint32_t*>(P.diff + 2 * (M + 1));
   P.bc = bases.on ? P.t2c + 2 * M : nullptr;
+  P.idel = indels.on ? reinterpret_cast<int32_t*>(P.t2c + (bases.on ? 12 : 2) * M) : nullptr;
+  P.ins = indels.on ? reinterpret_cast<uint32_t*>(P.idel + 2 * (M + 1)) : nullptr;
   timer_begin(ctx, st);
   TR_CUDA(cudaMemsetAsync(P.diff, 0, 2 * (M + 1) * 4, st));
   TR_CUDA(cudaMemsetAsync(P.t2c, 0, (bases.on ? 12 : 2) * M * 4, st));
+  if (indels.on) TR_CUDA(cudaMemsetAsync(P.idel, 0, (4 * M + 2) * 4, st));
   const uint32_t L = b.uniform_len;
   const int nw = (L >= 1 && L <= 64 && b.uniform_ncigar == 1 && (reinterpret_cast<uintptr_t>(b.bases2) & 3u) == 0) ? (int)((L + 15) / 16) : 0;
   if (!bases.on) {
@@ -703,20 +854,26 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
       default: tr_accum_kernel<0, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
     }
   }
+  if (indels.on) tr_indel_kernel<<<grid_g, TR_THREADS, 0, st>>>(P);
   timer_end(ctx, st);
   timer_begin(ctx, st);
   for (int s = 0; s < 2; ++s) {
     int32_t* d = P.diff + (size_t)s * (M + 1);
     TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceScan::InclusiveSum(t, sz, d, d, (int64_t)M, st); }));
   }
+  for (int s = 0; s < 2 && indels.on; ++s) {
+    int32_t* d = P.idel + (size_t)s * (M + 1);
+    TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceScan::InclusiveSum(t, sz, d, d, (int64_t)M, st); }));
+  }
   timer_end(ctx, st);
-  ctx->launches += 3;
+  ctx->launches += indels.on ? 6 : 3;
 
   // selection of the reported range [lo, hi): at most 2 * blocks + 1 runs a strand (edges), at most one site a T>C event
   unsigned long long tot[3];
   TR_CUDA(cudaMemcpyAsync(tot, &d_st->fast, 8, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaMemcpyAsync(tot + 1, &d_st->t2c[0], 16, cudaMemcpyDeviceToHost, st));
   if (bases.on) TR_CUDA(cudaMemcpyAsync(out->totals.bases, d_st->bases, sizeof out->totals.bases, cudaMemcpyDeviceToHost, st));
+  if (indels.on) TR_CUDA(cudaMemcpyAsync(&out->indel_totals, d_st->indel, sizeof d_st->indel, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
   out->ctr.fast_path_reads = tot[0];
   out->ctr.t2c_events[0] = tot[1];
@@ -731,12 +888,18 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
       for (int a = 0; a < 4; ++a)
         for (int c = 0; c < 4; ++c) events += a == c ? 0 : out->totals.bases[s][a][c];
   const uint64_t cap_c = std::min<uint64_t>(2 * nr, events / bases.min_ev);
+  // indel candidates: at most one per min_ev deletions and anchored insertions
+  const ps_track_indel_totals& it = out->indel_totals;
+  uint64_t indel_events = 0;
+  for (int s = 0; s < 2; ++s) indel_events += it.deleted_bases[s] + it.insertion_ops[s] - it.unanchored_insertions[s];
+  const uint64_t cap_i = indels.on ? std::min<uint64_t>(2 * nr, indel_events / indels.min_ev) : 0;
   const uint64_t off_r[4] = {0, cap_r[0], 2 * cap_r[0], 2 * cap_r[0] + cap_r[1]}, off_s = 2 * (cap_r[0] + cap_r[1]);
-  unsigned long long* sel = slot<unsigned long long>(ctx, 6, off_s + cap_s + cap_c + 8, err);
+  unsigned long long* sel = slot<unsigned long long>(ctx, 6, off_s + cap_s + cap_c + cap_i + (indels.on ? 10 : 8), err);
   TR_CUDA(err);
-  unsigned long long* d_cnt = sel + off_s + cap_s + cap_c;      // runs (4), sites, candidates, base rows
+  // runs (4), sites, candidates, base rows, then (indel counts) indel candidates, indel rows
+  unsigned long long* d_cnt = sel + off_s + cap_s + cap_c + cap_i;
   timer_begin(ctx, st);
-  TR_CUDA(cudaMemsetAsync(d_cnt, 0, 7 * 8, st));
+  TR_CUDA(cudaMemsetAsync(d_cnt, 0, (indels.on ? 9 : 7) * 8, st));
   thrust::counting_iterator<unsigned long long> it_pos(lo), it_site(2 * lo);
   for (int s = 0; s < 2 && nr; ++s) {
     const int32_t* cov = P.diff + (size_t)s * (M + 1);
@@ -747,10 +910,13 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   if (nr && cap_s) TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, it_site, sites_sel, d_cnt + 4, (int64_t)(2 * nr), SiteAt{P.t2c, M}, st); }));
   unsigned long long* cand = sel + off_s + cap_s;
   if (nr && cap_c) TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, it_site, cand, d_cnt + 5, (int64_t)(2 * nr), BaseCandidate{P.bc, M, bases.min_ev}, st); }));
-  unsigned long long cnt[6] = {0, 0, 0, 0, 0, 0};
-  TR_CUDA(cudaMemcpyAsync(cnt, d_cnt, (bases.on ? 6 : 5) * 8, cudaMemcpyDeviceToHost, st));
+  unsigned long long* icand = sel + off_s + cap_s + cap_c;
+  if (nr && cap_i) TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, it_site, icand, d_cnt + 7, (int64_t)(2 * nr), IndelCandidate{P.idel, P.ins, M, indels.min_ev}, st); }));
+  unsigned long long cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  TR_CUDA(cudaMemcpyAsync(cnt, d_cnt, (indels.on ? 8 : bases.on ? 6 : 5) * 8, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
-  if (cnt[0] != cnt[1] || cnt[2] != cnt[3] || cnt[0] > cap_r[0] || cnt[2] > cap_r[1] || cnt[4] > cap_s || cnt[5] > cap_c)
+  if (cnt[0] != cnt[1] || cnt[2] != cnt[3] || cnt[0] > cap_r[0] || cnt[2] > cap_r[1] || cnt[4] > cap_s || cnt[5] > cap_c ||
+      cnt[7] > cap_i)
     return set_error(ctx, PS_ERR_CUDA, "track: run or site selection out of bounds");
   ps_track_run* d_runs = slot<ps_track_run>(ctx, 7, cnt[0] + cnt[2] + 1, err);
   ps_track_site* d_sites = slot<ps_track_site>(ctx, 8, cnt[4] + 1, err);
@@ -771,10 +937,18 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
     ctx->launches++;
     TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, d_rows, d_rows + cnt[5], d_cnt + 6, (int64_t)cnt[5], RowKept{}, st); }));
   }
+  ps_track_indel_row* d_irows = nullptr;           // [cnt[7]] one per indel candidate, then the kept ones
+  if (cnt[7]) {
+    d_irows = slot<ps_track_indel_row>(ctx, 13, 2 * cnt[7], err);
+    TR_CUDA(err);
+    tr_indel_rows_kernel<<<grid_for(cnt[7]), TR_THREADS, 0, st>>>(P, n_segs, icand, cnt[7], indels, d_irows);
+    ctx->launches++;
+    TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceSelect::If(t, sz, d_irows, d_irows + cnt[7], d_cnt + 8, (int64_t)cnt[7], IndelRowKept{}, st); }));
+  }
   timer_end(ctx, st);
   // windowed: positions up to prev_end (head) and from the split on (tail) stay dense for the host merge
   uint32_t* d_dense[2] = {nullptr, nullptr};
-  const uint32_t nv = bases.on ? 14 : 4;           // dense arrays a position hands over
+  const uint32_t nv = (bases.on ? 14 : 4) + (indels.on ? 4 : 0);   // dense arrays a position hands over
   if (windowed) {
     const unsigned long long f = hh.s.first_key, E = hh.total.x;
     if (prev_end && (f >> 32) == (prev_end >> 32) && f <= prev_end) {
@@ -792,8 +966,14 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
     TrackDense* dn[2] = {&out->head, &out->tail};
     for (int j = 0; j < 2; ++j) {
       if (!dn[j]->len) continue;
-      if (bases.on) tr_dense_kernel<true><<<grid_for(dn[j]->len), TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
-      else tr_dense_kernel<false><<<grid_for(dn[j]->len), TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+      const uint32_t g = grid_for(dn[j]->len);
+      if (indels.on) {
+        if (bases.on) tr_dense_kernel<true, true><<<g, TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+        else tr_dense_kernel<false, true><<<g, TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+      } else {
+        if (bases.on) tr_dense_kernel<true, false><<<g, TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+        else tr_dense_kernel<false, false><<<g, TR_THREADS, 0, st>>>(P, n_segs, dn[j]->key0, dn[j]->len, d_dense[j]);
+      }
       ctx->launches++;
     }
   }
@@ -811,16 +991,19 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
     dn[j]->v.resize((uint64_t)nv * dn[j]->len);
     TR_CUDA(cudaMemcpyAsync(dn[j]->v.data(), d_dense[j], 4ull * nv * dn[j]->len, cudaMemcpyDeviceToHost, st));
   }
-  unsigned long long n_rows = 0;
+  unsigned long long n_rows = 0, n_irows = 0;
   if (cnt[5]) TR_CUDA(cudaMemcpyAsync(&n_rows, d_cnt + 6, 8, cudaMemcpyDeviceToHost, st));
+  if (cnt[7]) TR_CUDA(cudaMemcpyAsync(&n_irows, d_cnt + 8, 8, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
   if (n_rows > cnt[5]) return set_error(ctx, PS_ERR_CUDA, "track: base row selection out of bounds");
+  if (n_irows > cnt[7]) return set_error(ctx, PS_ERR_CUDA, "track: indel row selection out of bounds");
   out->base_rows.resize(n_rows);
-  if (n_rows) {
-    TR_CUDA(cudaMemcpyAsync(out->base_rows.data(), d_rows + cnt[5], n_rows * sizeof(ps_track_base_row), cudaMemcpyDeviceToHost, st));
-    TR_CUDA(cudaStreamSynchronize(st));
-  }
+  out->indel_rows.resize(n_irows);
+  if (n_rows) TR_CUDA(cudaMemcpyAsync(out->base_rows.data(), d_rows + cnt[5], n_rows * sizeof(ps_track_base_row), cudaMemcpyDeviceToHost, st));
+  if (n_irows) TR_CUDA(cudaMemcpyAsync(out->indel_rows.data(), d_irows + cnt[7], n_irows * sizeof(ps_track_indel_row), cudaMemcpyDeviceToHost, st));
+  if (n_rows || n_irows) TR_CUDA(cudaStreamSynchronize(st));
   out->totals.n_rows = n_rows;
+  out->indel_totals.n_rows = n_irows;
   out->ctr.n_runs[0] = cnt[0];
   out->ctr.n_runs[1] = cnt[2];
   out->ctr.n_sites = cnt[4];
@@ -833,9 +1016,10 @@ struct ps_track {
 };
 
 // a handle is returned with PS_OK and with a fault (PS_ERR_REFERENCE_WOULD_THROW, PS_ERR_UNSUPPORTED): ps_track_fault
-static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const TrackBases& bases, ps_track** out) {
+static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const TrackBases& bases,
+                      const TrackIndels& indels, ps_track** out) {
   ps_track* h = new ps_track();
-  const int rc = track_run(ctx, v, st, false, 0, &h->out, bases);
+  const int rc = track_run(ctx, v, st, false, 0, &h->out, bases, indels);
   if (rc == PS_OK || h->out.fault.code != 0) *out = h;
   else delete h;
   return rc;
@@ -843,11 +1027,14 @@ static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const 
 
 extern "C" {
 
-int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts, void* stream, ps_track** out) {
+int ps_track_batch_device_ex2(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts,
+                              const ps_track_indel_opts* indel_opts, void* stream, ps_track** out) {
   if (!ctx || !b || !out) return PS_ERR_INVALID_ARG;
   *out = nullptr;
   TrackBases bases;
   if (track_bases_of(opts, &bases) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
+  TrackIndels indels;
+  if (track_indels_of(indel_opts, &indels) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: indel option reserved field is not 0");
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
@@ -855,30 +1042,42 @@ int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* b, const ps_track
   for (int slot = 0; slot < 2; ++slot)
     if (st != ctx->stream && b->n_reads && b->meta == ctx->staged[slot].view.meta && ctx->staged_core[slot])
       cudaStreamWaitEvent(st, ctx->staged_core[slot], 0);
-  return track_call(ctx, view_of(b), st, bases, out);
+  return track_call(ctx, view_of(b), st, bases, indels, out);
+}
+
+int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts, void* stream, ps_track** out) {
+  return ps_track_batch_device_ex2(ctx, b, opts, nullptr, stream, out);
 }
 
 int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream, ps_track** out) {
   return ps_track_batch_device_ex(ctx, b, nullptr, stream, out);
 }
 
-int ps_track_batch_ex(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts, ps_track** out) {
+int ps_track_batch_ex2(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts,
+                       const ps_track_indel_opts* indel_opts, ps_track** out) {
   if (!ctx || !hb || !out) return PS_ERR_INVALID_ARG;
   *out = nullptr;
   TrackBases bases;
   if (track_bases_of(opts, &bases) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
+  TrackIndels indels;
+  if (track_indels_of(indel_opts, &indels) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: indel option reserved field is not 0");
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   if (hb->n_reads == 0) {
     *out = new ps_track();
     (*out)->out.ctr.num_reads_processed = 0;
     (*out)->out.bases_on = bases.on;
+    (*out)->out.indels_on = indels.on;
     return PS_OK;
   }
   StagedBatch* sb = nullptr;
   const int rc = stage_batch(ctx, hb, /*with_qual=*/false, &sb);
   if (rc) return rc;
-  return track_call(ctx, sb->view, ctx->stream, bases, out);
+  return track_call(ctx, sb->view, ctx->stream, bases, indels, out);
+}
+
+int ps_track_batch_ex(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts, ps_track** out) {
+  return ps_track_batch_ex2(ctx, hb, opts, nullptr, out);
 }
 
 int ps_track_batch(ps_ctx* ctx, const ps_read_batch* hb, ps_track** out) { return ps_track_batch_ex(ctx, hb, nullptr, out); }
@@ -921,6 +1120,23 @@ int ps_track_base_totals_get(const ps_track* h, ps_track_base_totals* out) {
   if (!h || !out) return PS_ERR_INVALID_ARG;
   if (!h->out.bases_on) return PS_ERR_STATE;
   *out = h->out.totals;
+  return PS_OK;
+}
+
+int64_t ps_track_indel_rows(const ps_track* h, uint64_t first, ps_track_indel_row* rows, uint64_t max) {
+  if (!h || (!rows && max)) return PS_ERR_INVALID_ARG;
+  if (!h->out.indels_on) return PS_ERR_STATE;
+  const std::vector<ps_track_indel_row>& v = h->out.indel_rows;
+  if (first >= v.size()) return 0;
+  const uint64_t k = std::min<uint64_t>(max, v.size() - first);
+  if (k) std::memcpy(rows, v.data() + first, k * sizeof(ps_track_indel_row));
+  return (int64_t)k;
+}
+
+int ps_track_indel_totals_get(const ps_track* h, ps_track_indel_totals* out) {
+  if (!h || !out) return PS_ERR_INVALID_ARG;
+  if (!h->out.indels_on) return PS_ERR_STATE;
+  *out = h->out.indel_totals;
   return PS_OK;
 }
 

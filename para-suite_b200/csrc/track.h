@@ -6,7 +6,7 @@
 
 // Positions [key0, key0 + len) of one contig, keys (rank + 1) << 32 | 1-based position (ps_ctx::contig_rank);
 // v = cov+, cov-, t2c+, t2c-, len entries each; with base counts ten more: the event counters A, C, G, T, N of the plus
-// strand, then of the minus strand (TrackBases).
+// strand, then of the minus strand (TrackBases); with indel counts four more at the end: del+, del-, ins+, ins-.
 struct TrackDense {
   unsigned long long key0 = 0;
   uint32_t len = 0;
@@ -37,6 +37,20 @@ __host__ __device__ inline bool track_base_row(const TrackBases& sel, uint32_t a
   return true;
 }
 
+// The indel option of a call (ps_track_indel_opts), thresholds normalised: on == false counts no indels.  With it on,
+// TrackDense::v gains four arrays after the others: del+, del-, ins+, ins-.
+struct TrackIndels {
+  bool on = false;
+  uint32_t min_depth = 1, min_ev = 1;
+};
+// ps_track_indel_opts -> TrackIndels; PS_ERR_INVALID_ARG for reserved != 0
+int track_indels_of(const ps_track_indel_opts* o, TrackIndels* out);
+// The indel row rule of one position and strand (device selection and host pending region alike): cov is that strand's
+// coverage, del / ins its deletions and anchored insertions.
+__host__ __device__ inline bool track_indel_row(const TrackIndels& sel, uint32_t cov, uint32_t del, uint32_t ins) {
+  return (uint64_t)del + ins >= sel.min_ev && (uint64_t)cov + del >= sel.min_depth;
+}
+
 // One track call.  Runs and sites are final for the positions reported; keys as in TrackDense.
 struct TrackOut {
   std::vector<ps_track_run> runs[2];
@@ -48,12 +62,15 @@ struct TrackOut {
   bool bases_on = false;
   std::vector<ps_track_base_row> base_rows;
   ps_track_base_totals totals{};
+  bool indels_on = false;
+  std::vector<ps_track_indel_row> indel_rows;
+  ps_track_indel_totals indel_totals{};
 };
 
 // windowed == false: the batch is the whole input, every position is reported.
 // windowed == true (one window of a sorted file): positions up to prev_end (the maximum end key of the windows before,
 // 0 if none) come back dense in `head`, positions from the last kept start on dense in `tail`; the runs and sites cover
 // the positions in between.  Waits for the device.
-// `bases`: the base-count option (rows for the reported positions, totals over every kept read).
+// `bases`, `indels`: the base-count and indel options (rows for the reported positions, totals over every kept read).
 int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out,
-              const TrackBases& bases = TrackBases());
+              const TrackBases& bases = TrackBases(), const TrackIndels& indels = TrackIndels());

@@ -15,7 +15,7 @@ CSRC_DIR = os.path.join(ROOT_DIR, "csrc")
 REPO_DIR = os.path.dirname(ROOT_DIR)
 INCLUDE_DIR = os.path.join(REPO_DIR, "include")
 
-PS_ABI_VERSION = 6
+PS_ABI_VERSION = 7
 PS_OK = 0
 PS_ERR_INVALID_ARG = -1
 PS_ERR_NO_DEVICE = -2
@@ -149,6 +149,24 @@ class ps_track_base_totals(C.Structure):
     _fields_ = [("bases", ((C.c_uint64 * 5) * 4) * 2), ("n_rows", C.c_uint64)]
 
 
+class ps_track_indel_opts(C.Structure):
+    _fields_ = [("indel_counts", C.c_uint32), ("min_depth", C.c_uint32), ("min_events", C.c_uint32),
+                ("reserved", C.c_uint32)]
+
+
+class ps_track_indel_row(C.Structure):
+    _fields_ = [("contig", C.c_uint32), ("pos", C.c_int32), ("strand", C.c_uint8), ("ref", C.c_uint8),
+                ("reserved", C.c_uint16), ("cov", C.c_uint32), ("del", C.c_uint32), ("ins", C.c_uint32)]
+
+
+class ps_track_indel_totals(C.Structure):
+    _fields_ = [("deletion_ops", C.c_uint64 * 2), ("deleted_bases", C.c_uint64 * 2), ("insertion_ops", C.c_uint64 * 2),
+                ("inserted_bases", C.c_uint64 * 2), ("unanchored_insertions", C.c_uint64 * 2), ("n_rows", C.c_uint64)]
+
+    def as_dict(self):
+        return {f: (list(getattr(self, f)) if f != "n_rows" else int(self.n_rows)) for f, _ in self._fields_}
+
+
 class ps_flush_totals(C.Structure):
     _fields_ = [("snp_hit", C.c_uint64), ("high_frequent_error", C.c_uint64), ("num_crosslinked_clusters", C.c_uint64),
                 ("num_allele_positions", C.c_uint64), ("allele_positions", C.c_uint64 * 51),
@@ -170,6 +188,9 @@ TRACK_SITE_DTYPE = [("contig", "<u4"), ("pos", "<i4"), ("strand", "<u4"), ("t2c"
 # ps_track_base_row: n holds the read bases A, C, G, T, N in strand orientation
 TRACK_BASE_ROW_DTYPE = [("contig", "<u4"), ("pos", "<i4"), ("strand", "u1"), ("ref", "u1"), ("reserved", "<u2"),
                         ("cov", "<u4"), ("n", "<u4", (5,))]
+# ps_track_indel_row: ref in strand orientation, 4 = not ACGT; del / ins: deletions over and insertions anchored at pos
+TRACK_INDEL_ROW_DTYPE = [("contig", "<u4"), ("pos", "<i4"), ("strand", "u1"), ("ref", "u1"), ("reserved", "<u2"),
+                         ("cov", "<u4"), ("del", "<u4"), ("ins", "<u4")]
 
 # every symbol include/parasuite_b200.h declares: name -> (restype, argtypes)
 VP = C.c_void_p
@@ -269,6 +290,19 @@ EXPORTS = {
     "ps_multi_track_bam_ex": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts),
                                         C.POINTER(ps_track_counters), C.POINTER(ps_track_base_totals),
                                         C.POINTER(ps_fault)]),
+    "ps_track_batch_ex2": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_track_opts),
+                                     C.POINTER(ps_track_indel_opts), C.POINTER(VP)]),
+    "ps_track_batch_device_ex2": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_track_opts),
+                                            C.POINTER(ps_track_indel_opts), VP, C.POINTER(VP)]),
+    "ps_track_indel_rows": (C.c_int64, [VP, C.c_uint64, VP, C.c_uint64]),
+    "ps_track_indel_totals_get": (C.c_int, [VP, C.POINTER(ps_track_indel_totals)]),
+    "ps_track_bam_ex2": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts), C.POINTER(ps_track_indel_opts),
+                                   C.POINTER(ps_track_counters), C.POINTER(ps_track_base_totals),
+                                   C.POINTER(ps_track_indel_totals), C.POINTER(ps_fault)]),
+    "ps_multi_track_bam_ex2": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts),
+                                         C.POINTER(ps_track_indel_opts), C.POINTER(ps_track_counters),
+                                         C.POINTER(ps_track_base_totals), C.POINTER(ps_track_indel_totals),
+                                         C.POINTER(ps_fault)]),
     "ps_track_close": (None, [VP]),
     "ps_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),
     "ps_multi_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),

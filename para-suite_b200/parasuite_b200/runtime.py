@@ -54,6 +54,15 @@ def track_opts(base_counts: bool, min_coverage: int, min_events: int, substituti
     return abi.ps_track_opts(1, int(min_coverage), int(min_events), substitution_mask(substitutions))
 
 
+def track_indel_opts(indel_counts: bool, min_indel_depth: int, min_indel_events: int) -> Optional[abi.ps_track_indel_opts]:
+    """The ps_track_indel_opts of the indel keywords of Context.track, or None without indel counts"""
+    if not indel_counts:
+        return None
+    if min(int(min_indel_depth), int(min_indel_events)) < 0:
+        raise ValueError("min_indel_depth and min_indel_events must be >= 0")
+    return abi.ps_track_indel_opts(1, int(min_indel_depth), int(min_indel_events), 0)
+
+
 def _base_totals_dict(tot) -> dict:
     return {"base_totals": np.array(tot.bases, dtype=np.uint64).reshape(2, 4, 5), "n_base_rows": int(tot.n_rows)}
 
@@ -265,19 +274,25 @@ class Context:
         return np.array(list(ctr), dtype=np.int32)
 
     def track_bam(self, bam_path: str, out_prefix: str, *, base_counts: bool = False, min_coverage: int = 1,
-                  min_events: int = 1, substitutions=None) -> dict:
+                  min_events: int = 1, substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1,
+                  min_indel_events: int = 1) -> dict:
         """The `track` tool from files: writes <out_prefix>.plus.bedGraph, <out_prefix>.minus.bedGraph and
         <out_prefix>.t2c.tsv (per-position coverage and T>C events by strand); returns the run's counters.
         base_counts: also <out_prefix>.bases.tsv (keywords as Context.track), and the counters gain "base_totals"
-        ((2, 4, 5) uint64: strand, reference base, read base A C G T N) and "n_base_rows"."""
+        ((2, 4, 5) uint64: strand, reference base, read base A C G T N) and "n_base_rows".
+        indel_counts: also <out_prefix>.indels.tsv (keywords as Context.track), and the counters gain "indel_totals"."""
         opts = track_opts(base_counts, min_coverage, min_events, substitutions)
-        ctr, f, tot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals()
-        st = self.lib.ps_track_bam_ex(self.h, bam_path.encode(), out_prefix.encode(), C.byref(opts) if opts else None,
-                                      C.byref(ctr), C.byref(tot), C.byref(f))
+        iopts = track_indel_opts(indel_counts, min_indel_depth, min_indel_events)
+        ctr, f, tot, itot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals(), abi.ps_track_indel_totals()
+        st = self.lib.ps_track_bam_ex2(self.h, bam_path.encode(), out_prefix.encode(), C.byref(opts) if opts else None,
+                                       C.byref(iopts) if iopts else None, C.byref(ctr), C.byref(tot), C.byref(itot),
+                                       C.byref(f))
         _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
         out = ctr.as_dict()
         if opts:
             out.update(_base_totals_dict(tot))
+        if iopts:
+            out["indel_totals"] = itot.as_dict()
         return out
 
     # ---- batches ---------------------------------------------------------------------------------
@@ -456,22 +471,27 @@ class Context:
 
     # ---- T>C conversion and coverage track ---------------------------------------------------------
     def track(self, batch, stream: int = 0, *, base_counts: bool = False, min_coverage: int = 1, min_events: int = 1,
-              substitutions=None) -> dict:
+              substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1, min_indel_events: int = 1) -> dict:
         """Per-position coverage and T>C events by strand of one whole input: {"runs_plus", "runs_minus", "sites",
         "counters"}, runs and sites as numpy structured arrays (abi.TRACK_RUN_DTYPE / TRACK_SITE_DTYPE, contigs as FASTA
         indices).  batch: host (ReadBatch / PinnedBatch) or device-resident (DeviceBatch / UploadedBatch).
         base_counts: also "base_rows" (abi.TRACK_BASE_ROW_DTYPE: read bases A C G T N by position and strand, strand
         orientation) for the positions with coverage >= min_coverage and >= min_events of the selected substitutions
         (an iterable of "X>Y"; None: all twelve), and "base_totals" ((2, 4, 5) uint64: strand, reference base, read
-        base) over every counted base."""
+        base) over every counted base.
+        indel_counts: also "indel_rows" (abi.TRACK_INDEL_ROW_DTYPE: deletions over and insertions anchored at each
+        position by strand) for the positions with deletions + insertions >= min_indel_events and coverage + deletions
+        >= min_indel_depth, and "indel_totals" (abi.ps_track_indel_totals as a dict of [plus, minus] lists and
+        "n_rows")."""
         opts = track_opts(base_counts, min_coverage, min_events, substitutions)
-        po = C.byref(opts) if opts else None
+        iopts = track_indel_opts(indel_counts, min_indel_depth, min_indel_events)
+        po, pi = C.byref(opts) if opts else None, C.byref(iopts) if iopts else None
         h = C.c_void_p()
         if isinstance(batch, (DeviceBatch, UploadedBatch)):
-            st = self.lib.ps_track_batch_device_ex(self.h, C.byref(batch.struct), po, stream or None, C.byref(h))
+            st = self.lib.ps_track_batch_device_ex2(self.h, C.byref(batch.struct), po, pi, stream or None, C.byref(h))
         else:
             s = batch.struct if hasattr(batch, "struct") else batch.as_struct()
-            st = self.lib.ps_track_batch_ex(self.h, C.byref(s), po, C.byref(h))
+            st = self.lib.ps_track_batch_ex2(self.h, C.byref(s), po, pi, C.byref(h))
         try:
             if st != abi.PS_OK:
                 fault = None
@@ -503,6 +523,14 @@ class Context:
                     self.lib.ps_track_base_rows(h, 0, rows.ctypes.data, rows.size)
                 out["base_rows"] = rows
                 out["base_totals"] = _base_totals_dict(tot)["base_totals"]
+            if iopts:
+                itot = abi.ps_track_indel_totals()
+                _check(self.lib, self.h, self.lib.ps_track_indel_totals_get(h, C.byref(itot)))
+                rows = np.zeros(itot.n_rows, dtype=abi.TRACK_INDEL_ROW_DTYPE)
+                if rows.size:
+                    self.lib.ps_track_indel_rows(h, 0, rows.ctypes.data, rows.size)
+                out["indel_rows"] = rows
+                out["indel_totals"] = itot.as_dict()
             return out
         finally:
             if h:
@@ -691,16 +719,21 @@ class MultiContext:
         return {k: getattr(ctr, k) for k, _ in abi.ps_pileup_counters._fields_}
 
     def track_bam(self, bam_path: str, out_prefix: str, *, base_counts: bool = False, min_coverage: int = 1,
-                  min_events: int = 1, substitutions=None) -> dict:
+                  min_events: int = 1, substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1,
+                  min_indel_events: int = 1) -> dict:
         """Context.track_bam with windows round-robin over the devices; the files are byte-identical."""
         opts = track_opts(base_counts, min_coverage, min_events, substitutions)
-        ctr, f, tot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals()
-        st = self.lib.ps_multi_track_bam_ex(self.h, bam_path.encode(), out_prefix.encode(),
-                                            C.byref(opts) if opts else None, C.byref(ctr), C.byref(tot), C.byref(f))
+        iopts = track_indel_opts(indel_counts, min_indel_depth, min_indel_events)
+        ctr, f, tot, itot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals(), abi.ps_track_indel_totals()
+        st = self.lib.ps_multi_track_bam_ex2(self.h, bam_path.encode(), out_prefix.encode(),
+                                             C.byref(opts) if opts else None, C.byref(iopts) if iopts else None,
+                                             C.byref(ctr), C.byref(tot), C.byref(itot), C.byref(f))
         self._check(st, fault=(f.code, f.read_ordinal))
         out = ctr.as_dict()
         if opts:
             out.update(_base_totals_dict(tot))
+        if iopts:
+            out["indel_totals"] = itot.as_dict()
         return out
 
     def close(self):

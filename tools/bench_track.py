@@ -2,6 +2,7 @@
 
   python tools/bench_track.py [--steps 20] [--warmup 3] [--bam-reads 300000] [--bam-copies 40] [--out FILE]
   python tools/bench_track.py --base-counts [--steps 20] [--warmup 3] [--out FILE]
+  python tools/bench_track.py --indels [--steps 20] [--warmup 3] [--indel-reads 4000000] [--parent-lib SO] [--out FILE]
 
 1. Config 2 as bench.py builds it (10 M x 36-nt reads through synth.py against a 100 Mb reference), resident in HBM:
    `--steps` timed passes of ps_track_batch_device after `--warmup` passes, with the five stage times of every pass from
@@ -17,6 +18,14 @@ The card's name and power limit are recorded with the numbers.
 with base counts (all twelve substitutions, thresholds 1) alternate, `--steps` passes each after `--warmup` of each; the
 five stage times of both, the scratch the compact arrays take, the row counts, and the parity of the base-count call with
 the C++ restatement (tests/track_bases_oracle.py) go to profiles/track_bench_bases.json (or --out).
+
+--indels measures the per-position deletion and insertion counts: on config 5 (--indel-reads x 150-nt reads with indels
+and soft clips, synth mode 1, resident in HBM) and on config 2 (10 M x 36-nt reads, no indel), against the same 100 Mb
+reference, the plain call and the call with indel counts (thresholds 1) alternate, `--steps` passes each after `--warmup`
+of each.  --parent-lib: a build of the library from before the option (ABI 6); its plain call joins the alternation on
+the same device-resident batch, so the plain call of both builds is timed in one run.  The five stage times of every
+call, the scratch the compact arrays take, the row counts and the parity of the indel call with the C++ restatement
+(tests/track_indels_oracle.py) go to profiles/track_bench_indels.json (or --out).
 """
 import argparse
 import json
@@ -41,6 +50,9 @@ ap.add_argument("--bam-reads", type=int, default=300_000)
 ap.add_argument("--bam-copies", type=int, default=40)
 ap.add_argument("--out", default=None)
 ap.add_argument("--base-counts", action="store_true")
+ap.add_argument("--indels", action="store_true")
+ap.add_argument("--indel-reads", type=int, default=4_000_000)
+ap.add_argument("--parent-lib", default=None)
 args = ap.parse_args()
 
 import torch  # noqa: E402
@@ -64,8 +76,28 @@ def compact_positions(batch):
     n = batch.n_reads
     s = np.asarray(batch.ref_start[:n]).astype(np.int64)
     e = s + batch.uniform_len - 1
+    return _segments(s, e)
+
+
+def compact_positions_cigar(batch):
+    """compact_positions for any CIGAR: the reference span of every kept read (mapped, no I or D together with N)"""
+    n = batch.n_reads
+    meta = np.asarray(batch.meta[:n]).astype(np.int64)
+    ncig = (meta >> 16) & 0xFF
+    off = np.concatenate([[0], np.cumsum(ncig)])
+    cig = np.asarray(batch.cigar[:off[-1]]).astype(np.int64)
+    op, ln = cig & 15, cig >> 4
+    rid = np.repeat(np.arange(n), ncig)
+    span = np.bincount(rid, weights=ln * np.isin(op, [0, 2, 3, 7, 8]), minlength=n).astype(np.int64)
+    has = {k: np.bincount(rid, weights=(op == k), minlength=n) > 0 for k in (1, 2, 3)}
+    kept = (((meta >> 24) & abi.PS_RF_UNMAPPED) == 0) & ~((has[1] | has[2]) & has[3])
+    s = np.asarray(batch.ref_start[:n]).astype(np.int64)[kept]
+    return _segments(s, s + span[kept] - 1)
+
+
+def _segments(s, e):
     pm = np.maximum.accumulate(e)
-    new = np.ones(n, dtype=bool)
+    new = np.ones(s.size, dtype=bool)
     new[1:] = s[1:] > pm[:-1] + 1
     seg = np.cumsum(new) - 1
     seg_s = s[new]
@@ -149,8 +181,130 @@ def base_counts_run():
     ctx.close()
 
 
+class ParentTrack:
+    """The plain track call of another build of the library, on a context of its own (same device, same process)."""
+
+    def __init__(self, path):
+        self.lib = C.CDLL(os.path.abspath(path))
+        for name in ("ps_create", "ps_destroy", "ps_last_error", "ps_reference_upload", "ps_track_batch_device",
+                     "ps_track_counters_get", "ps_track_close", "ps_kernel_times", "ps_kernel_times_reset"):
+            f = getattr(self.lib, name)
+            f.restype, f.argtypes = abi.EXPORTS[name]
+        self.version = int(self.lib.ps_abi_version())
+        self.h = C.c_void_p()
+        assert self.lib.ps_create(C.byref(self.h), 0) == abi.PS_OK
+        s = ref.as_struct()
+        assert self.lib.ps_reference_upload(self.h, C.byref(s)) == abi.PS_OK
+
+    def once(self, dbatch):
+        h = C.c_void_p()
+        st = self.lib.ps_track_batch_device(self.h, C.byref(dbatch.struct), None, C.byref(h))
+        assert st == abi.PS_OK, self.lib.ps_last_error(self.h)
+        ctr = abi.ps_track_counters()
+        self.lib.ps_track_counters_get(h, C.byref(ctr))
+        self.lib.ps_track_close(h)
+        return ctr
+
+    def stages(self):
+        buf = np.zeros(512, dtype=np.float32)
+        n = self.lib.ps_kernel_times(self.h, buf.ctypes.data, buf.size)
+        return buf[:max(n, 0)].reshape(-1, len(STAGES))[-1]
+
+    def close(self):
+        self.lib.ps_destroy(self.h)
+
+
+def indels_run():
+    """plain and indel calls alternately on config 5 and config 2 (and the parent build's plain call)"""
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+    import track_indels_oracle  # noqa: E402
+    iopts = abi.ps_track_indel_opts(1, 1, 1, 0)
+    parent = ParentTrack(args.parent_lib) if args.parent_lib else None
+    if parent:
+        out["parent_lib_abi_version"] = parent.version
+
+    def once(with_indels, dbatch):
+        h = C.c_void_p()
+        st = lib.ps_track_batch_device_ex2(ctx.h, C.byref(dbatch.struct), None, C.byref(iopts) if with_indels else None,
+                                           None, C.byref(h))
+        assert st == abi.PS_OK, lib.ps_last_error(ctx.h)
+        ctr, tot = abi.ps_track_counters(), abi.ps_track_indel_totals()
+        lib.ps_track_counters_get(h, C.byref(ctr))
+        if with_indels:
+            lib.ps_track_indel_totals_get(h, C.byref(tot))
+        lib.ps_track_close(h)
+        return ctr, tot
+
+    shapes = (("config5", args.indel_reads, 150, 1), ("config2", 10_000_000, 36, 0))
+    parity = True
+    for name, n, L, mode in shapes:
+        b = synth.synth_reads(ref, n, L, seed=0x5EED0002, mode=mode)
+        d = DeviceBatch(b, "cuda:0")
+        arms = {"plain": lambda: once(False, d), "indels": lambda: once(True, d)}
+        if parent:
+            arms["parent_plain"] = lambda: (parent.once(d), None)
+        for _ in range(args.warmup):
+            for f in arms.values():
+                f()
+        res = {k: {"walls": [], "stages": []} for k in arms}
+        for _ in range(args.steps):
+            for k, f in arms.items():
+                tctx = parent if k == "parent_plain" else ctx
+                if k == "parent_plain":
+                    parent.lib.ps_kernel_times_reset(parent.h, 1)
+                else:
+                    ctx.kernel_times_reset(True)
+                t0 = time.perf_counter()
+                ctr, tot = f()
+                res[k]["walls"].append(time.perf_counter() - t0)
+                res[k]["stages"].append(parent.stages() if tctx is parent else
+                                        ctx.kernel_times_ms().reshape(-1, len(STAGES))[-1])
+                res[k]["ctr"], res[k]["tot"] = ctr, tot
+        M = compact_positions_cigar(b)
+        o = {"reads": b.n_reads, "read_len": L, "synth_mode": mode, "steps": args.steps, "warmup": args.warmup,
+             "order": " / ".join(arms) + " calls alternate"}
+        for k in arms:
+            st = np.array(res[k]["stages"])
+            c = res[k]["ctr"]
+            o[k] = {"wall_ms_median": 1e3 * float(np.median(res[k]["walls"])),
+                    "device_ms_median": float(np.median(st.sum(axis=1))),
+                    "stage_ms_median": {s: float(np.median(st[:, i])) for i, s in enumerate(STAGES)},
+                    "stage_ms_min": {s: float(np.min(st[:, i])) for i, s in enumerate(STAGES)},
+                    "runs": [int(c.n_runs[0]), int(c.n_runs[1])], "sites": int(c.n_sites),
+                    "reads_counted": int(c.reads_counted), "skipped_due_indel": int(c.skipped_due_indel)}
+        o["indels"]["indel_totals"] = res["indels"]["tot"].as_dict()
+        o["indels"]["indel_rows"] = int(res["indels"]["tot"].n_rows)
+        o["compact_positions"] = M
+        o["plain"]["compact_scratch_bytes"] = 4 * (2 * (M + 1) + 2 * M)
+        o["indels"]["compact_scratch_bytes"] = 4 * (2 * (M + 1) + 2 * M) + 4 * (2 * (M + 1) + 2 * M)
+        got = ctx.track(d, indel_counts=True)
+        exp = track_indels_oracle.track_indels_cpp(ref, b)
+        same = bool(np.array_equal(got["indel_rows"], exp["indel_rows"]) and got["indel_totals"] == exp["indel_totals"]
+                    and all(np.array_equal(got[k], exp[k]) for k in ("runs_plus", "runs_minus", "sites")))
+        o["parity_with_restatement"] = same
+        if parent:
+            o["parent_plain_same_counters"] = res["parent_plain"]["ctr"].as_dict() == res["plain"]["ctr"].as_dict()
+            same = same and o["parent_plain_same_counters"]
+        parity = parity and same
+        out[name + "_indels"] = o
+        print(json.dumps(o, indent=1), flush=True)
+        del d, got, exp
+    out["parity_with_restatement"] = parity
+    print(json.dumps(out, indent=1))
+    path = args.out or os.path.join(REPO, "profiles", "track_bench_indels.json")
+    os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+    with open(path, "w") as f:
+        json.dump(out, f, indent=1)
+    if parent:
+        parent.close()
+    ctx.close()
+
+
 if args.base_counts:
     base_counts_run()
+    sys.exit(0)
+if args.indels:
+    indels_run()
     sys.exit(0)
 
 for _ in range(args.warmup):
