@@ -1,8 +1,10 @@
 // C ABI of libparasuite_b200.so: context, reference residency, error-profile entry points.
 // (include/parasuite_b200.h documents which reference lines each call replaces.)
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 
 #include "internal.h"
 
@@ -157,13 +159,64 @@ int stage_batch(ps_ctx* ctx, const ps_read_batch* hb, bool with_qual, StagedBatc
 }
 
 void timer_begin(ps_ctx* ctx, cudaStream_t st) {
+  ctx->cur_ts = nullptr;
   if (!ctx->timers_on || ctx->ev_count >= PS_TIMER_RING) return;
+  ctx->ev_stamped[ctx->ev_count] = false;
   cudaEventRecord(ctx->ev_start[ctx->ev_count], st);
 }
-void timer_end(ps_ctx* ctx, cudaStream_t st) {
+// a timed section of chained kernels: no event record in front of them, the kernels stamp the slot's pair (ctx->cur_ts)
+void timer_begin_chained(ps_ctx* ctx, cudaStream_t st) {
+  if (!ctx->pdl || !ctx->ts_ring.p) return timer_begin(ctx, st);
+  ctx->cur_ts = nullptr;
   if (!ctx->timers_on || ctx->ev_count >= PS_TIMER_RING) return;
-  cudaEventRecord(ctx->ev_stop[ctx->ev_count], st);
+  ctx->ev_stamped[ctx->ev_count] = true;
+  ctx->cur_ts = static_cast<unsigned long long*>(ctx->ts_ring.p) + 2 * ctx->ev_count;
+}
+void timer_end(ps_ctx* ctx, cudaStream_t st) {
+  ctx->cur_ts = nullptr;
+  if (!ctx->timers_on || ctx->ev_count >= PS_TIMER_RING) return;
+  if (!ctx->ev_stamped[ctx->ev_count]) cudaEventRecord(ctx->ev_stop[ctx->ev_count], st);
   ctx->ev_count++;
+}
+// milliseconds between a stamp pair (device_common.cuh); NaN when a kernel of the section did not stamp
+static float stamp_ms(unsigned long long start_word, unsigned long long end) {
+  const unsigned long long start = ~start_word;
+  if (start_word == 0 || end == 0 || end < start) return __builtin_nanf("");
+  return (float)((double)(end - start) * 1e-6);
+}
+static int clear_stamps(ps_ctx* ctx) {
+  if (!ctx->ts_ring.p) return PS_OK;
+  PS_CUDA(ctx, cudaDeviceSynchronize());      // no kernel of an earlier section may still stamp a slot
+  PS_CUDA(ctx, cudaMemset(ctx->ts_ring.p, 0, ctx->ts_ring.cap));
+  return PS_OK;
+}
+// The dynamic shared memory a kernel may use is state of the (device, kernel) pair, shared by every context of the
+// process on that device: one record per pair, which only ever raises the attribute, so that no launch of another
+// context finds it lowered below what that launch needs.
+static cudaError_t allow_dynamic_smem(int device, const void* fn, size_t smem) {
+  struct Allowed { int device; const void* fn; size_t smem; };
+  static std::mutex mu;
+  static std::vector<Allowed> allowed;
+  std::lock_guard<std::mutex> lock(mu);
+  for (auto& a : allowed) {
+    if (a.device != device || a.fn != fn) continue;
+    if (a.smem >= smem) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) a.smem = smem;
+    return e;
+  }
+  const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e == cudaSuccess) allowed.push_back({device, fn, smem});
+  return e;
+}
+
+cudaError_t fn_blocks_per_sm(ps_ctx* ctx, const void* fn, int threads, size_t smem, int* per_sm) {
+  for (const auto& a : ctx->fn_attr)
+    if (a.fn == fn && a.smem == smem) { *per_sm = a.per_sm; return cudaSuccess; }
+  cudaError_t e = allow_dynamic_smem(ctx->device, fn, smem);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, fn, threads, smem);
+  if (e == cudaSuccess) ctx->fn_attr.push_back({fn, smem, *per_sm});
+  return e;
 }
 
 // ---- reference: contig table and contig order -----------------------------------------------------
@@ -255,6 +308,12 @@ int ps_create(ps_ctx** out, int device) {
   ctx->sm_count = prop.multiProcessorCount;
   if (const char* e = getenv("PARASUITE_B200_COMPACT_LOOKBACK")) ctx->pl_compact_lookback = e[0] == '1';
   if (const char* e = getenv("PARASUITE_B200_FLAG_SCAN_KERNEL")) ctx->pl_flag_scan_kernel = e[0] == '1';
+  if (const char* e = getenv("PARASUITE_B200_PDL")) ctx->pdl = e[0] != '0';
+  if (ctx->pdl && (ctx->ts_ring.reserve(2 * PS_TIMER_RING * sizeof(unsigned long long)) != cudaSuccess ||
+                   cudaMemset(ctx->ts_ring.p, 0, ctx->ts_ring.cap) != cudaSuccess)) {
+    cudaGetLastError();
+    ctx->ts_ring.release();      // the timers fall back to events
+  }
   if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) { delete ctx; return PS_ERR_CUDA; }
   if (cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking) != cudaSuccess) { cudaGetLastError(); ctx->stream2 = nullptr; }
   if (cudaStreamCreateWithFlags(&ctx->stream_rb, cudaStreamNonBlocking) != cudaSuccess) { cudaGetLastError(); ctx->stream_rb = nullptr; }
@@ -299,6 +358,7 @@ void ps_destroy(ps_ctx* ctx) {
   if (ctx->stream_rb) cudaStreamDestroy(ctx->stream_rb);
   if (ctx->prof_done_ev) cudaEventDestroy(ctx->prof_done_ev);
   ctx->ref_seq2.release(); ctx->ref_inv.release(); ctx->ref_contig.release(); ctx->ref_rank.release();
+  ctx->ts_ring.release();
   ctx->acc.release(); ctx->fault.release(); ctx->deferred.release(); ctx->t2c_mask.release();
   ctx->rg_okmap.release(); ctx->rg_off.release(); ctx->rg_bases.release(); ctx->rg_qual.release(); ctx->rg_op0.release();
   for (auto& s : ctx->staged) {
@@ -439,9 +499,7 @@ int ps_profile_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream) {
     masks = static_cast<unsigned long long*>(ctx->t2c_mask.p);
   }
   bool written = false;
-  timer_begin(ctx, s);
   PS_CUDA(ctx, launch_profile(ctx, view_of(b), ctx->reads_seen, s, masks, &written));
-  timer_end(ctx, s);
   if (written) ctx->t2c_mask_n = b->n_reads;
   ctx->reads_seen += b->n_reads;
   early_readback(ctx, s);
@@ -460,9 +518,7 @@ int ps_profile_batch(ps_ctx* ctx, const ps_read_batch* hb) {
   if (st) return st;
   PS_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->reset_ev, 0));
   ctx->profile_stream = ctx->stream;
-  timer_begin(ctx, ctx->stream);
   PS_CUDA(ctx, launch_profile(ctx, sb->view, ctx->reads_seen, ctx->stream));
-  timer_end(ctx, ctx->stream);
   ctx->reads_seen += hb->n_reads;
   early_readback(ctx, ctx->stream);
   return PS_OK;
@@ -588,15 +644,37 @@ uint64_t ps_kernel_launches(const ps_ctx* ctx) { return ctx ? ctx->launches : 0;
 float ps_last_kernel_ms(const ps_ctx* ctx) {
   if (!ctx || ctx->ev_count == 0) return -1.f;
   float ms = -1.f;
-  cudaEventSynchronize(ctx->ev_stop[ctx->ev_count - 1]);
-  cudaEventElapsedTime(&ms, ctx->ev_start[ctx->ev_count - 1], ctx->ev_stop[ctx->ev_count - 1]);
+  const uint32_t i = ctx->ev_count - 1;
+  cudaSetDevice(ctx->device);
+  if (ctx->ev_stamped[i]) {
+    unsigned long long w[2];
+    if (cudaDeviceSynchronize() != cudaSuccess ||
+        cudaMemcpy(w, static_cast<const unsigned long long*>(ctx->ts_ring.p) + 2 * i, sizeof w, cudaMemcpyDeviceToHost) != cudaSuccess) {
+      cudaGetLastError();
+      return -1.f;
+    }
+    return stamp_ms(w[0], w[1]);
+  }
+  cudaEventSynchronize(ctx->ev_stop[i]);
+  cudaEventElapsedTime(&ms, ctx->ev_start[i], ctx->ev_stop[i]);
   return ms;
 }
 
 int ps_kernel_times(ps_ctx* ctx, float* ms, int max) {
   if (!ctx || !ms) return PS_ERR_INVALID_ARG;
+  cudaSetDevice(ctx->device);
   int n = (int)ctx->ev_count < max ? (int)ctx->ev_count : max;
+  std::vector<unsigned long long> w;
   for (int i = 0; i < n; ++i) {
+    if (ctx->ev_stamped[i]) {
+      if (w.empty()) {
+        w.resize(2 * (size_t)n);
+        PS_CUDA(ctx, cudaDeviceSynchronize());
+        PS_CUDA(ctx, cudaMemcpy(w.data(), ctx->ts_ring.p, w.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+      }
+      ms[i] = stamp_ms(w[2 * i], w[2 * i + 1]);
+      continue;
+    }
     cudaEventSynchronize(ctx->ev_stop[i]);
     cudaEventElapsedTime(&ms[i], ctx->ev_start[i], ctx->ev_stop[i]);
   }
@@ -605,6 +683,10 @@ int ps_kernel_times(ps_ctx* ctx, float* ms, int max) {
 
 int ps_pileup_stage_times(ps_ctx* ctx, float* ms3) {
   if (!ctx || !ms3) return PS_ERR_INVALID_ARG;
+  if (ctx->pl_ts_valid) {      // stamps of the last call (PlState::ts): flag, cluster and compaction kernels' starts, end
+    for (int i = 0; i < 3; ++i) ms3[i] = stamp_ms(ctx->pl_ts[i], i < 2 ? ~ctx->pl_ts[i + 1] : ctx->pl_ts[3]);
+    return PS_OK;
+  }
   if (!ctx->pl_ev_valid) return PS_ERR_STATE;
   cudaEventSynchronize(ctx->pl_ev[3]);
   for (int i = 0; i < 3; ++i) cudaEventElapsedTime(&ms3[i], ctx->pl_ev[i], ctx->pl_ev[i + 1]);
@@ -615,8 +697,11 @@ int ps_pileup_flag_mode(const ps_ctx* ctx) { return ctx && ctx->pl_exact_flags ?
 
 void ps_kernel_times_reset(ps_ctx* ctx, int enabled) {
   if (!ctx) return;
+  cudaSetDevice(ctx->device);
   ctx->ev_count = 0;
   ctx->timers_on = enabled != 0;
+  ctx->cur_ts = nullptr;
+  if (clear_stamps(ctx) != PS_OK) ctx->ts_ring.release();   // the timers fall back to events
 }
 
 }  // extern "C"

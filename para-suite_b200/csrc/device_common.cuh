@@ -4,6 +4,24 @@
 
 #include "internal.h"
 
+// ---- chained launches (launch_chained, internal.h) ---------------------------------------------------------------
+// Both are no-ops in a grid launched without programmatic stream serialization.  pdl_wait returns once the preceding
+// grid of the stream has completed and its writes are visible; every chained kernel calls it before its first access to
+// anything an earlier kernel writes or reads, and on every path before it exits (the next grid's wait covers only this
+// one).  pdl_launch_dependents lets the next grid become resident; that grid still waits for this one to complete.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// Timer stamps of the chained kernels (no event may sit between them): %globaltimer in ns.  A pair of words that start
+// at 0 holds [0] = ~(earliest start), [1] = latest end, both kept with atomicMax.
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+__device__ __forceinline__ void stamp_start(unsigned long long* w) { atomicMax(w, ~globaltimer_ns()); }
+__device__ __forceinline__ void stamp_end(unsigned long long* w) { atomicMax(w, globaltimer_ns()); }
+
 // 2-bit reference code at global offset g (undefined where the invalid bit is set)
 __device__ __forceinline__ uint32_t ref_code_at(const DeviceRef& ref, uint64_t g) {
   return (__ldg(ref.seq2 + (g >> 4)) >> (2 * (g & 15))) & 3u;

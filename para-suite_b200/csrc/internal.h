@@ -4,6 +4,7 @@
 
 #include <cstdint>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "parasuite_b200.h"
@@ -149,6 +150,19 @@ struct ps_ctx {
   uint32_t ev_count = 0;   // pairs recorded since reset
   bool timers_on = true;
   cudaEvent_t pl_ev[4] = {nullptr, nullptr, nullptr, nullptr};   // around the three pileup kernels of the last call
+  // chained launches (launch_chained): the kernels of the resident step carry programmatic stream serialization unless
+  // PARASUITE_B200_PDL=0 at ps_create.  No event may sit between chained kernels, so their timers are %globaltimer
+  // stamps: ts_ring holds one stamp pair per timer slot (device_common.cuh: stamp_start / stamp_end), ev_stamped tells
+  // which slots took stamps instead of events, cur_ts is the pair of the open slot (null: events or timers off)
+  bool pdl = true;
+  DevBuf ts_ring;
+  bool ev_stamped[PS_TIMER_RING] = {};
+  unsigned long long* cur_ts = nullptr;
+  unsigned long long pl_ts[4] = {0, 0, 0, 0};   // stage stamps of the last pileup call (PlState::ts)
+  bool pl_ts_valid = false;
+  // occupancy, once per (kernel, dynamic shared memory) on this context's device (fn_blocks_per_sm)
+  struct FnAttr { const void* fn; size_t smem; int per_sm; };
+  std::vector<FnAttr> fn_attr;
   cudaEvent_t reset_ev = nullptr;   // accumulators of the current profile run have been cleared
   bool pl_ev_valid = false;
   void* h_pinned = nullptr;   // 4 KB of page-locked host memory for small read-backs
@@ -203,6 +217,34 @@ inline void pileup_key_decode(const std::vector<uint32_t>& by_rank, uint64_t key
 // t2c_mask (optional): n_reads words; *mask_written tells whether the batch took the fast kernel, which fills them
 cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0, cudaStream_t stream,
                            unsigned long long* t2c_mask = nullptr, bool* mask_written = nullptr);
+
+// Blocks of `threads` threads of kernel `fn` with `smem` bytes of dynamic shared memory that fit one SM, cached per
+// context; the kernel's dynamic shared memory attribute is raised to at least `smem` on the context's device (one
+// process-wide record per device and kernel: it is never lowered), so the launch path makes no such call again.
+cudaError_t fn_blocks_per_sm(ps_ctx* ctx, const void* fn, int threads, size_t smem, int* per_sm);
+
+// Launch of a kernel of the resident step (profile kernels, pileup kernels): with ctx->pdl it carries programmatic
+// stream serialization, so the grid becomes resident while its predecessor drains (device_common.cuh: pdl_wait).
+template <typename... KArgs, typename... Args>
+cudaError_t launch_chained(const ps_ctx* ctx, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                           Args&&... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = ctx->pdl ? 1 : 0;
+  return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+}
+
+// timed sections (ctx.cu): a pair of events, or for chained kernels the stamp pair ctx->cur_ts
+void timer_begin(ps_ctx* ctx, cudaStream_t st);
+void timer_begin_chained(ps_ctx* ctx, cudaStream_t st);
+void timer_end(ps_ctx* ctx, cudaStream_t st);
 
 int set_error(ps_ctx* ctx, int status, const std::string& msg);
 int cuda_fail(ps_ctx* ctx, cudaError_t e, const char* what);

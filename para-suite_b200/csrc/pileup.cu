@@ -93,6 +93,9 @@ struct PlState {                  // device-side run state (one per call)
   // ballot form could not take (the streaming sweep starts on them), [1] of those, the ones the sweep gave up on,
   // [2] window passes the window loop made over them (one per PL_WINDOW positions from the first event to the last)
   unsigned long long dbg[3];
+  // timer stamps of the chained kernels (device_common.cuh), cleared by pl_init_state: ~start of the flag, cluster and
+  // compaction stages (earliest block past its pdl_wait), end of the compaction
+  unsigned long long ts[4];
 };
 
 struct PlRead {              // what the pileup needs from one read
@@ -125,6 +128,7 @@ struct FlagParams {
   uint32_t* tile_cnt;             // [n_tiles] boundary flags per tile, then (scan kernel) their exclusive prefix
   uint32_t* flag_words;           // one word per thread (bit j = read j of the thread)
   uint32_t scan_in_expand;        // no pl_flag_scan_kernel: the expand kernel sums the tile counts itself
+  uint32_t stamp;                 // stamp PlState::ts
 };
 
 // (rank of the contig + 1) << 32 | end of a kept record, 0 otherwise (PileupClusters.java:146-158).  The rank is the
@@ -232,6 +236,9 @@ __global__ void __launch_bounds__(FLAG_THREADS, FLAG_BLOCKS_PER_SM) pl_flag_kern
   __shared__ unsigned long long s_halo[FLAG_WARPS];
   __shared__ unsigned int s_tile;
   __shared__ unsigned long long s_pre;
+  pdl_wait();
+  pdl_launch_dependents();
+  if (P.stamp && threadIdx.x == 0) stamp_start(&P.st->ts[0]);
 
   if constexpr (!SPEC) {      // the look-backs need forward progress: tile numbers in the order the blocks start
     if (threadIdx.x == 0) s_tile = atomicAdd(&P.st->tile_ctr_flag, 1u);
@@ -410,6 +417,8 @@ constexpr int SCAN_THREADS = 1024;
 constexpr int SCAN_ITEMS = 8;        // consecutive tiles per thread and round
 __global__ void __launch_bounds__(SCAN_THREADS) pl_flag_scan_kernel(const __grid_constant__ FlagParams P) {
   __shared__ unsigned long long s_wtot[SCAN_THREADS / 32];
+  pdl_wait();
+  pdl_launch_dependents();
   unsigned long long carry = P.carry_key;
   for (uint32_t k = 0; k < P.carry_keys_n; ++k) {
     const unsigned long long ck = __ldg(P.carry_keys + k);
@@ -465,6 +474,8 @@ template <int ITEMS>
 __global__ void __launch_bounds__(FLAG_THREADS) pl_flag_expand_kernel(const __grid_constant__ FlagParams P) {
   __shared__ unsigned long long s_wtot[FLAG_WARPS];
   __shared__ unsigned long long s_base;
+  pdl_wait();
+  pdl_launch_dependents();
   const uint32_t tile = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t fl = P.flag_words[(size_t)tile * FLAG_THREADS + threadIdx.x];
   unsigned long long part = 0;
@@ -534,6 +545,7 @@ struct ClusterParams {
   unsigned int* tile_sites;   // [slots / COMPACT_TILE] sites per tile of pl_compact_kernel (zeroed by the host), or nullptr
   const unsigned long long* t2c_mask;   // optional: one T>C mask word per read, left by profile_fast_kernel for THIS batch
                                         // (bit 63 valid, bit 62 minus strand, bits 0..61 mask by strand-oriented index)
+  uint32_t stamp;                       // pl_cluster_kernel: stamp PlState::ts
 };
 #ifndef COMPACT_ITEMS_
 #define COMPACT_ITEMS_ 2
@@ -1036,6 +1048,9 @@ __global__ void __launch_bounds__(CB_THREADS, CB_BLOCKS_PER_SM) pl_cluster_kerne
   __shared__ unsigned long long s_wtot[CB_WARPS];
   __shared__ unsigned long long s_base;
   __shared__ uint32_t s_nfb;
+  pdl_wait();      // before any path, the early returns included: the mask words are four launches back
+  pdl_launch_dependents();
+  if (P.stamp && threadIdx.x == 0) stamp_start(&P.st->ts[1]);
   ClusterSmem S;
   S.mask = reinterpret_cast<unsigned long long*>(smem_raw);
   S.lo = reinterpret_cast<int32_t*>(S.mask + CB_CHUNK);
@@ -1286,9 +1301,11 @@ struct CompactParams {
   uint64_t cap_cl, cap_sites;
   const unsigned int* tile_sites;   // sites per tile, summed up by pl_cluster_kernel: every tile adds up the entries in
                                     // front of it (no chain between the tiles); nullptr = decoupled look-back
+  uint32_t stamp;                   // stamp PlState::ts
+  unsigned long long* sec_ts;       // optional: stamp pair of the timed section, whose end this kernel is
 };
 
-__global__ void __launch_bounds__(PL_THREADS) pl_compact_kernel(const __grid_constant__ CompactParams P) {
+__device__ __forceinline__ void pl_compact_body(const CompactParams& P) {
   constexpr int ITEMS = COMPACT_ITEMS;
   __shared__ unsigned long long s_wtot[PL_WARPS];
   __shared__ unsigned long long s_pre;
@@ -1387,6 +1404,20 @@ __global__ void __launch_bounds__(PL_THREADS) pl_compact_kernel(const __grid_con
   }
 }
 
+__global__ void __launch_bounds__(PL_THREADS) pl_compact_kernel(const __grid_constant__ CompactParams P) {
+  pdl_wait();
+  pdl_launch_dependents();
+  if (P.stamp && threadIdx.x == 0) stamp_start(&P.st->ts[2]);
+  pl_compact_body(P);
+  if (P.stamp) {      // every thread is back from the body's returns
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      stamp_end(&P.st->ts[3]);
+      if (P.sec_ts) stamp_end(P.sec_ts + 1);
+    }
+  }
+}
+
 // checkPosition interval of reads [r0, r1) (halo merge: dense coverage of a boundary cluster)
 template <int NW>
 __global__ void pl_interval_kernel(const __grid_constant__ ClusterParams P, uint32_t r0, uint32_t r1, int2* out) {
@@ -1400,12 +1431,16 @@ __global__ void pl_interval_kernel(const __grid_constant__ ClusterParams P, uint
 }
 
 // run state of a call, and the per-tile site totals of the compaction (one launch instead of a kernel and a memset)
-__global__ void pl_init_state(PlState* st, unsigned int* tile_sites, uint32_t n_tile_sites) {
+__global__ void pl_init_state(PlState* st, unsigned int* tile_sites, uint32_t n_tile_sites, unsigned long long* sec_ts) {
+  pdl_wait();
+  pdl_launch_dependents();
+  if (sec_ts && threadIdx.x == 0) stamp_start(sec_ts);
   for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n_tile_sites; k += gridDim.x * blockDim.x) tile_sites[k] = 0;
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     st->fault = PS_FAULT_NONE; st->skipped = 0; st->dstr = 0; st->n_sites = 0; st->n_sites_final = 0; st->n_flags = 0;
     st->unsorted = 0; st->tile_ctr_flag = 0; st->tile_ctr_compact = 0; st->first_slot1 = 0xFFFFFFFFu; st->spec_failed = 0;
     st->dbg[0] = st->dbg[1] = st->dbg[2] = 0;
+    st->ts[0] = st->ts[1] = st->ts[2] = st->ts[3] = 0;
   }
 }
 
@@ -1437,6 +1472,7 @@ struct ps_pileup {
   ps_pileup_opts opts{};
   bool spec = false;                 // the attempt in flight used the speculative flag pass
   uint64_t cap_cl = 0, cap_sites = 0;   // capacities of the attempt in flight
+  bool stamped = false;              // the attempt in flight stamps PlState::ts instead of recording pl_ev
   PlState hs_fallback{};             // landing place of the run state when the context has no page-locked scratch
   // host mode (windowed ps_pileup_bam / ps_multi_pileup_bam, tool_loops.cpp): the merged records of all windows live in
   // host vectors; nothing is resident on a device
@@ -1477,27 +1513,29 @@ static int flavour_of(const DeviceBatch& b) {   // 0 = generic decode, 1..4 = PA
 }
 
 template <int NW, bool MK>
-static void launch_cluster_nw(uint32_t grid, cudaStream_t st, const ClusterParams& Q) {
-  // per launch: the attribute belongs to the (device, kernel) pair and a process may hold contexts on several GPUs
-  cudaFuncSetAttribute(pl_cluster_kernel<NW, MK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemBytes);
-  pl_cluster_kernel<NW, MK><<<grid, CB_THREADS, kClusterSmemBytes, st>>>(Q);
+static cudaError_t launch_cluster_nw(ps_ctx* ctx, uint32_t grid, cudaStream_t st, const ClusterParams& Q) {
+  auto kern = pl_cluster_kernel<NW, MK>;
+  int per_sm = 0;
+  cudaError_t e = fn_blocks_per_sm(ctx, reinterpret_cast<const void*>(kern), CB_THREADS, kClusterSmemBytes, &per_sm);
+  if (e != cudaSuccess) return e;
+  return launch_chained(ctx, kern, grid, CB_THREADS, kClusterSmemBytes, st, Q);
 }
-static void launch_cluster(int nw, uint32_t grid, cudaStream_t st, const ClusterParams& Q) {
+static cudaError_t launch_cluster(ps_ctx* ctx, int nw, uint32_t grid, cudaStream_t st, const ClusterParams& Q) {
   if (Q.t2c_mask != nullptr) {
     switch (nw) {
-      case 1: launch_cluster_nw<1, true>(grid, st, Q); return;
-      case 2: launch_cluster_nw<2, true>(grid, st, Q); return;
-      case 3: launch_cluster_nw<3, true>(grid, st, Q); return;
-      case 4: launch_cluster_nw<4, true>(grid, st, Q); return;
+      case 1: return launch_cluster_nw<1, true>(ctx, grid, st, Q);
+      case 2: return launch_cluster_nw<2, true>(ctx, grid, st, Q);
+      case 3: return launch_cluster_nw<3, true>(ctx, grid, st, Q);
+      case 4: return launch_cluster_nw<4, true>(ctx, grid, st, Q);
       default: break;      // no mask words exist for other shapes
     }
   }
   switch (nw) {
-    case 1: launch_cluster_nw<1, false>(grid, st, Q); break;
-    case 2: launch_cluster_nw<2, false>(grid, st, Q); break;
-    case 3: launch_cluster_nw<3, false>(grid, st, Q); break;
-    case 4: launch_cluster_nw<4, false>(grid, st, Q); break;
-    default: launch_cluster_nw<0, false>(grid, st, Q); break;
+    case 1: return launch_cluster_nw<1, false>(ctx, grid, st, Q);
+    case 2: return launch_cluster_nw<2, false>(ctx, grid, st, Q);
+    case 3: return launch_cluster_nw<3, false>(ctx, grid, st, Q);
+    case 4: return launch_cluster_nw<4, false>(ctx, grid, st, Q);
+    default: return launch_cluster_nw<0, false>(ctx, grid, st, Q);
   }
 }
 
@@ -1551,14 +1589,22 @@ static int pileup_launch(ps_ctx* ctx, ps_pileup* H) {
     tile_sites = scratch<unsigned int>(ctx, 11, n_ctiles, err);
     if (err != cudaSuccess) return cuda_fail(ctx, err, "pileup scratch");
   }
-  timer_begin(ctx, st);        // the timer pair is complete when the launch returns (a submitted call may be waited for
-                               // after other timed calls of the context)
-  pl_init_state<<<tile_sites ? (uint32_t)((n_ctiles + 255) / 256) : 1u, 256, 0, st>>>(d_state, tile_sites, tile_sites ? (uint32_t)n_ctiles : 0u);
-  const bool ev = ctx->timers_on;
+  // the kernels are chained (launch_chained): with that on, no event sits between them and the timers are stamps
+  const bool stamp = ctx->pdl && ctx->timers_on;
+  const bool ev = ctx->timers_on && !stamp;
+  H->stamped = stamp;
+  ctx->pl_ts_valid = false;
+  const unsigned int compact_epoch = next_epoch(ctx, st);   // its occasional memset goes in front of the kernels
+  timer_begin_chained(ctx, st);   // the timer pair is complete when the launch returns (a submitted call may be waited
+                                  // for after other timed calls of the context)
+  unsigned long long* sec_ts = ctx->cur_ts;
+  PS_CUDA(ctx, launch_chained(ctx, pl_init_state, tile_sites ? (uint32_t)((n_ctiles + 255) / 256) : 1u, 256, 0, st, d_state,
+                              tile_sites, tile_sites ? (uint32_t)n_ctiles : 0u, sec_ts));
   if (ev) cudaEventRecord(ctx->pl_ev[0], st);
   const bool spec = vec && !ctx->pl_exact_flags;
   H->spec = spec;
   P.tile_ein = nullptr; P.tile_agg = nullptr; P.tile_cnt = nullptr; P.flag_words = nullptr; P.scan_in_expand = 0;
+  P.stamp = stamp ? 1u : 0u;
   if (spec) {
     P.tile_ein = scratch<unsigned long long>(ctx, 1, n_tiles, err);
     P.tile_agg = scratch<unsigned long long>(ctx, 7, n_tiles, err);
@@ -1568,12 +1614,15 @@ static int pileup_launch(ps_ctx* ctx, ps_pileup* H) {
     // up to kFlagSumTiles tiles (16.7 M reads) the expand kernel takes the prefix over the tile table itself (every
     // block sums the counts in front of it: quadratic, but a few thousand entries); beyond that the one-block scan
     P.scan_in_expand = (n_tiles <= kFlagSumTiles && !ctx->pl_flag_scan_kernel) ? 1u : 0u;
-    pl_flag_kernel<PL_FLAG_ITEMS, true><<<n_tiles, FLAG_THREADS, 0, st>>>(P);
-    if (!P.scan_in_expand) { pl_flag_scan_kernel<<<1, SCAN_THREADS, 0, st>>>(P); ctx->launches += 1; }
-    pl_flag_expand_kernel<PL_FLAG_ITEMS><<<n_tiles, FLAG_THREADS, 0, st>>>(P);
+    PS_CUDA(ctx, launch_chained(ctx, pl_flag_kernel<PL_FLAG_ITEMS, true>, n_tiles, FLAG_THREADS, 0, st, P));
+    if (!P.scan_in_expand) {
+      PS_CUDA(ctx, launch_chained(ctx, pl_flag_scan_kernel, 1, SCAN_THREADS, 0, st, P));
+      ctx->launches += 1;
+    }
+    PS_CUDA(ctx, launch_chained(ctx, pl_flag_expand_kernel<PL_FLAG_ITEMS>, n_tiles, FLAG_THREADS, 0, st, P));
     ctx->launches += 1;
-  } else if (vec) pl_flag_kernel<PL_FLAG_ITEMS, false><<<n_tiles, FLAG_THREADS, 0, st>>>(P);
-  else pl_flag_kernel<1, false><<<n_tiles, FLAG_THREADS, 0, st>>>(P);
+  } else if (vec) PS_CUDA(ctx, launch_chained(ctx, pl_flag_kernel<PL_FLAG_ITEMS, false>, n_tiles, FLAG_THREADS, 0, st, P));
+  else PS_CUDA(ctx, launch_chained(ctx, pl_flag_kernel<1, false>, n_tiles, FLAG_THREADS, 0, st, P));
   if (ev) cudaEventRecord(ctx->pl_ev[1], st);
   ClusterParams Q;
   Q.b = b; Q.ref = ctx->ref; Q.st = d_state;
@@ -1581,15 +1630,17 @@ static int pileup_launch(ps_ctx* ctx, ps_pileup* H) {
   Q.cap_cl = cap_cl; Q.cap_sites = cap_sites;
   Q.tile_sites = tile_sites;
   Q.t2c_mask = (nw > 0 && opts) ? reinterpret_cast<const unsigned long long*>(opts->t2c_masks_device) : nullptr;
-  launch_cluster(nw, c_tiles, st, Q);
+  Q.stamp = P.stamp;
+  PS_CUDA(ctx, launch_cluster(ctx, nw, c_tiles, st, Q));
   if (ev) cudaEventRecord(ctx->pl_ev[2], st);
   CompactParams R;
-  R.st = d_state; R.d_cnt = d_sc; R.epoch = next_epoch(ctx, st); R.cl = H->d_cl; R.src = d_tmp; R.dst = H->d_sites;
+  R.st = d_state; R.d_cnt = d_sc; R.epoch = compact_epoch; R.cl = H->d_cl; R.src = d_tmp; R.dst = H->d_sites;
   R.cap_cl = cap_cl; R.cap_sites = cap_sites; R.tile_sites = Q.tile_sites;
-  pl_compact_kernel<<<(uint32_t)n_ctiles, PL_THREADS, 0, st>>>(R);
+  R.stamp = P.stamp; R.sec_ts = sec_ts;
+  PS_CUDA(ctx, launch_chained(ctx, pl_compact_kernel, (uint32_t)n_ctiles, PL_THREADS, 0, st, R));
   if (ev) { cudaEventRecord(ctx->pl_ev[3], st); ctx->pl_ev_valid = true; }
+  if (stamp) ctx->pl_ev_valid = false;
   ctx->launches += 4;
-  PS_CUDA(ctx, cudaGetLastError());
   PlState* hsp = ctx->h_pinned ? static_cast<PlState*>(ctx->h_pinned) : &H->hs_fallback;
   PS_CUDA(ctx, cudaMemcpyAsync(hsp, d_state, sizeof(PlState), cudaMemcpyDeviceToHost, st));
   timer_end(ctx, st);
@@ -1636,6 +1687,10 @@ static int pileup_finish(ps_ctx* ctx, ps_pileup* H) {
     if (!again) break;
     const int rc = pileup_launch(ctx, H);
     if (rc != PS_OK) return done(rc);
+  }
+  if (H->stamped) {
+    for (int i = 0; i < 4; ++i) ctx->pl_ts[i] = hs.ts[i];
+    ctx->pl_ts_valid = true;
   }
   H->counters.skipped_due_indel = hs.skipped;
   if (hs.fault != PS_FAULT_NONE) {

@@ -42,6 +42,7 @@ struct ProfileParams {
   uint32_t* okmap;                     // fast kernel, optional (-q): bit r%32 of word r/32 = read r took the fast path
   const uint32_t* off3;                // deferred kernel on a re-laid ragged batch: [3][n_reads] in-tile offsets of every read
                                        // (bytes of bases, bytes of qualities, cigar elements), written by the repack kernel
+  unsigned long long* ts;              // fast and deferred kernels, optional: stamp pair of the timed section
 };
 
 // shared-memory histograms of the generic path
@@ -578,6 +579,9 @@ __global__ void __launch_bounds__(PS_BLOCK_THREADS) profile_deferred_kernel(cons
   S.s_indel = S.s_conv + P.lay.max_len * 16;
   for (uint32_t k = threadIdx.x; k < P.lay.max_len * 18; k += blockDim.x) S.s_conv[k] = 0;
   if (threadIdx.x < 48) S.s_q[threadIdx.x] = 0;
+  pdl_wait();      // the list and its count come from the fast kernel
+  pdl_launch_dependents();
+  if (P.ts && threadIdx.x == 0) stamp_start(P.ts);
   __syncthreads();
   const unsigned int n = *P.deferred_count;
   if (blockIdx.x == 0 && threadIdx.x == 0) *P.deferred_count_next = 0;
@@ -600,6 +604,7 @@ __global__ void __launch_bounds__(PS_BLOCK_THREADS) profile_deferred_kernel(cons
   }
   __syncthreads();
   flush_generic(P, S);
+  if (P.ts && threadIdx.x == 0) stamp_end(P.ts + 1);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -707,11 +712,8 @@ static cudaError_t launch_generic(ps_ctx* ctx, ProfileParams P, uint64_t first_r
   size_t smem = 48 * 8 + ((size_t)(ctx->layout.max_len | 1u) * 16 + 2 * (size_t)ctx->layout.max_len) * 4 +
                 (PS_BLOCK_THREADS / 32) * 32 * 4 +     // + the warps' 32-bit mismatch-quality cells
                 (PS_BLOCK_THREADS / 32) * 32 * 48 + 16; // + the warps' lane-per-read state (48 bytes per read, 16-byte aligned)
-  // per launch: the attribute belongs to the (device, kernel) pair and a process may hold contexts on several GPUs
-  cudaError_t e = cudaFuncSetAttribute(profile_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
   int per_sm = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, profile_generic_kernel, PS_BLOCK_THREADS, smem);
+  cudaError_t e = fn_blocks_per_sm(ctx, reinterpret_cast<const void*>(profile_generic_kernel), PS_BLOCK_THREADS, smem, &per_sm);
   if (e != cudaSuccess) return e;
   if (per_sm < 1) per_sm = 1;
   uint32_t grid = (uint32_t)ctx->sm_count * (uint32_t)per_sm;
@@ -726,11 +728,12 @@ static cudaError_t launch_generic(ps_ctx* ctx, ProfileParams P, uint64_t first_r
 
 static cudaError_t launch_deferred(ps_ctx* ctx, const ProfileParams& P, cudaStream_t stream) {
   size_t smem = 48 * 8 + (size_t)ctx->layout.max_len * 18 * 4;
-  cudaError_t e = cudaFuncSetAttribute(profile_deferred_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  int per_sm = 0;
+  cudaError_t e = fn_blocks_per_sm(ctx, reinterpret_cast<const void*>(profile_deferred_kernel), PS_BLOCK_THREADS, smem, &per_sm);
   if (e != cudaSuccess) return e;
-  profile_deferred_kernel<<<(uint32_t)ctx->sm_count, PS_BLOCK_THREADS, smem, stream>>>(P);
+  e = launch_chained(ctx, profile_deferred_kernel, (uint32_t)ctx->sm_count, PS_BLOCK_THREADS, smem, stream, P);
   ctx->launches++;
-  return cudaGetLastError();
+  return e;
 }
 
 // `-q` on the fast path: baseQualitiesPerPos[i].add(readQualities[i]) for every i < L (ErrorProfiling.java:402-407) of the
@@ -776,10 +779,8 @@ static cudaError_t launch_qhist(ps_ctx* ctx, const uint8_t* qual, const uint32_t
                                 uint32_t stride, uint32_t uniform_L, unsigned long long* acc, cudaStream_t stream) {
   const uint32_t max_len = ctx->layout.max_len;
   const size_t smem = (size_t)max_len * 257 * 4;
-  cudaError_t e = cudaFuncSetAttribute(profile_qhist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
   int per_sm = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, profile_qhist_kernel, 256, smem);
+  cudaError_t e = fn_blocks_per_sm(ctx, reinterpret_cast<const void*>(profile_qhist_kernel), 256, smem, &per_sm);
   if (e != cudaSuccess) return e;
   if (per_sm < 1) return cudaErrorInvalidConfiguration;
   const uint64_t need = (n_reads + 255) / 256;
@@ -797,7 +798,11 @@ static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0, cudaStream_t stream,
                            unsigned long long* t2c_mask, bool* mask_written) {
   if (mask_written) *mask_written = false;
-  if (b.n_reads == 0) return cudaSuccess;
+  if (b.n_reads == 0) {
+    timer_begin(ctx, stream);
+    timer_end(ctx, stream);
+    return cudaSuccess;
+  }
   ProfileParams P;
   P.b = b;
   P.ref = ctx->ref;
@@ -811,6 +816,7 @@ cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0,
   P.t2c_mask = nullptr;
   P.off3 = nullptr;
   P.okmap = nullptr;
+  P.ts = nullptr;
   // both counters are zero at the start of a run (ps_profile_begin clears the words behind the fault word)
   P.deferred_count = reinterpret_cast<unsigned int*>(P.fault + 2) + (ctx->profile_batches & 1u);
   P.deferred_count_next = reinterpret_cast<unsigned int*>(P.fault + 2) + ((ctx->profile_batches + 1u) & 1u);
@@ -833,6 +839,9 @@ cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0,
       P.okmap = static_cast<uint32_t*>(ctx->rg_okmap.p);
     }
     ctx->profile_batches++;
+    // the fast and the deferred kernel are chained (launch_chained): their section's time comes from their stamps
+    timer_begin_chained(ctx, stream);
+    P.ts = ctx->cur_ts;
     const uint32_t n_wt = (uint32_t)((b.n_reads + WT_READS - 1) / WT_READS);   // the fast kernel takes every read
     const uint32_t nw = (L + 15) / 16;
     cudaError_t e;
@@ -849,7 +858,9 @@ cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0,
     else e = launch_fast<4, 5, 0>(ctx, P, n_wt, stream);
     if (e != cudaSuccess) return e;
     if (P.okmap && (e = launch_qhist(ctx, b.qual, b.meta, P.okmap, b.n_reads, L, L, P.acc, stream)) != cudaSuccess) return e;
-    return launch_deferred(ctx, P, stream);
+    e = launch_deferred(ctx, P, stream);
+    timer_end(ctx, stream);
+    return e;
   }
   // Ragged batches of short reads (adapter-trimmed PAR-CLIP reads as an aligner leaves them): re-lay them as rows of
   // S = 16 * ceil(max_read_length / 16) positions and run the fast kernel with per-read lengths.  Reads of another
@@ -883,6 +894,7 @@ cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0,
       P.okmap = static_cast<uint32_t*>(ctx->rg_okmap.p);
     }
     ctx->profile_batches++;
+    timer_begin(ctx, stream);
     for (uint64_t c0 = 0; c0 < b.n_reads; c0 += chunk) {
       const uint64_t cn = std::min<uint64_t>(chunk, b.n_reads - c0);
       RepackParams R;
@@ -917,7 +929,12 @@ cudaError_t launch_profile(ps_ctx* ctx, const DeviceBatch& b, uint64_t ordinal0,
       if (e != cudaSuccess) return e;
       if (P.okmap && (e = launch_qhist(ctx, Q.b.qual, Q.b.meta, P.okmap, cn, S, 0, P.acc, stream)) != cudaSuccess) return e;
     }
-    return launch_deferred(ctx, P, stream);
+    e = launch_deferred(ctx, P, stream);
+    timer_end(ctx, stream);
+    return e;
   }
-  return launch_generic(ctx, P, done, stream);
+  timer_begin(ctx, stream);
+  const cudaError_t e = launch_generic(ctx, P, done, stream);
+  timer_end(ctx, stream);
+  return e;
 }

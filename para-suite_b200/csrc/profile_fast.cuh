@@ -299,6 +299,10 @@ __global__ void __launch_bounds__(FAST_THREADS, RG ? (NW <= 3 ? 4 : 3) : FAST_BL
     bulk_g2s(dst + lay.bases, P.b.bases2 + r0 * bpr, bb, bar);
     bulk_g2s(dst + lay.qual, P.b.qual + r0 * L, qb, bar);
   };
+  // before the first load of the batch: a ragged batch's rows come from the repack kernel in front of this one
+  pdl_wait();
+  pdl_launch_dependents();
+  if (P.ts && threadIdx.x == 0) stamp_start(P.ts);
   if (elect_one()) {
 #pragma unroll
     for (int s = 0; s < FAST_STAGES; ++s) {
@@ -755,6 +759,7 @@ __global__ void __launch_bounds__(FAST_THREADS, RG ? (NW <= 3 ? 4 : 3) : FAST_BL
     atomicAdd(P.acc + P.lay.ctr + PS_PC_NUM_READS_PROCESSED, s_misc[8]);
     atomicAdd(P.fault + 1, s_misc[8]);   // debug word: reads that took the fast path
   }
+  if (P.ts && threadIdx.x == 0) stamp_end(P.ts + 1);
 }
 
 // a block may add this many reads before the 32-bit shared mismatch-quality cells could overflow
@@ -765,10 +770,8 @@ template <int NW, int NPL, int LT, bool RG = false>
 cudaError_t launch_fast(ps_ctx* ctx, const ProfileParams& P, uint32_t n_wt, cudaStream_t stream) {
   const size_t smem = fast_layout(P.lay.max_len, P.b.uniform_len, NW).total + 128;
   auto kern = profile_fast_kernel<NW, NPL, LT, RG>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
   int per_sm = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, FAST_THREADS, smem);
+  cudaError_t e = fn_blocks_per_sm(ctx, reinterpret_cast<const void*>(kern), FAST_THREADS, smem, &per_sm);
   if (e != cudaSuccess) return e;
   if (per_sm < 1) return cudaErrorInvalidConfiguration;
   uint32_t grid = (uint32_t)ctx->sm_count * (uint32_t)per_sm;
@@ -795,9 +798,8 @@ cudaError_t launch_fast(ps_ctx* ctx, const ProfileParams& P, uint32_t n_wt, cuda
     Q.first_read = P.first_read + r0;    // offset added to deferred read indices
     if (Q.t2c_mask) Q.t2c_mask += r0;
     if (Q.okmap) Q.okmap += r0 / 32;
-    kern<<<grid, FAST_THREADS, smem, stream>>>(Q);
+    e = launch_chained(ctx, kern, grid, FAST_THREADS, smem, stream, Q);
     ctx->launches++;
-    e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }
   return cudaSuccess;
