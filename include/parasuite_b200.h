@@ -532,6 +532,60 @@ int ps_track_indel_totals_get(const ps_track* h, ps_track_indel_totals* out);
 int ps_track_bam_ex2(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
                      const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
                      ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out, ps_fault* fault_out);
+/* Read and base filters (filter != NULL), as samtools view -q / -f / -F and mpileup -Q; all four are off at 0, and
+ * options of all zeros give what the _ex2 calls give:
+ * - Record filter: a record is filtered when (flag & exclude_flags) != 0, (flag & require_flags) != require_flags or
+ *   mapq < min_mapq; flag and mapq are the BAM FLAG and MAPQ fields, read from ps_read_aux.  The test comes first,
+ *   before the unmapped check, the (I or D)-with-N skip and every fault: a filtered record is treated as absent.  It
+ *   raises no fault, takes no part in the sortedness check, opens no segment and adds to no maximum end; it counts in
+ *   num_reads_processed and in filtered_flags when it fails a flag test, else in filtered_mapq.  So with
+ *   exclude_flags = 0x4 an unmapped record counts in filtered_flags, not in unmapped.  One exception: the batch-level
+ *   PS_FAULT_PAST_END (ps_read_batch.past_end) is raised for its record even when the filter drops it, because the
+ *   producers mark only the first such record and dropping it could hide a later one that is not filtered.
+ * - Base filter: min_base_quality = q > 0 applies to every aligned (M, =, X) base of a kept record.  A base whose quality
+ *   byte is < q counts nowhere -- not in coverage (runs, and the cov of sites, base rows and indel rows), not as a T>C
+ *   event, not in base counts, not in aligned_bases -- only in low_quality_bases[strand].  A record with
+ *   PS_RF_QUAL_MISSING has no qualities: all its bases pass.  Deletions and insertions are not filtered by base quality
+ *   (as in samtools); the indel row rule cov + del >= min_depth uses the filtered coverage.  Segments are still cut on
+ *   read spans: a low-quality stretch is a stretch of zero coverage inside one.  The invariants of the counters, base
+ *   totals and indel totals hold as without the filter.
+ * - Counters of a call without a fault: num_reads_processed = filtered_flags + filtered_mapq + unmapped +
+ *   skipped_due_indel + reads_counted.
+ * - PS_ERR_INVALID_ARG: a reserved field that is not 0, min_mapq or min_base_quality above 255, flag masks above 16
+ *   bits, or a flag (MAPQ) filter when aux->sam_flags (aux->mapq) is NULL. */
+typedef struct ps_read_aux {     /* per record, in batch order: host arrays with a host batch, device arrays with a device
+                                    batch; either may be NULL */
+  const uint16_t* sam_flags;     /* BAM FLAG */
+  const uint8_t* mapq;           /* BAM MAPQ */
+} ps_read_aux;
+typedef struct ps_track_filter_opts { /* 32 B */
+  uint32_t min_mapq;             /* 0..255 */
+  uint32_t require_flags;        /* samtools -f */
+  uint32_t exclude_flags;        /* samtools -F */
+  uint32_t min_base_quality;     /* 0..255, samtools mpileup -Q */
+  uint32_t reserved[4];          /* must be 0 */
+} ps_track_filter_opts;
+typedef struct ps_track_filter_counters { /* 32 B */
+  uint64_t filtered_flags;       /* records dropped by a flag test */
+  uint64_t filtered_mapq;        /* records that passed the flag tests and were dropped for their MAPQ */
+  uint64_t low_quality_bases[2]; /* [strand]: aligned bases of kept records below min_base_quality */
+} ps_track_filter_counters;
+/* aux == NULL and filter == NULL: ps_track_batch_ex2 / ps_track_batch_device_ex2 */
+int ps_track_batch_ex3(ps_ctx* ctx, const ps_read_batch* host_batch, const ps_track_opts* opts,
+                       const ps_track_indel_opts* indel_opts, const ps_read_aux* aux,
+                       const ps_track_filter_opts* filter, ps_track** out);
+int ps_track_batch_device_ex3(ps_ctx* ctx, const ps_read_batch* dev_batch, const ps_track_opts* opts,
+                              const ps_track_indel_opts* indel_opts, const ps_read_aux* aux,
+                              const ps_track_filter_opts* filter, void* stream, ps_track** out);
+/* PS_ERR_STATE on a handle made without filter options */
+int ps_track_filter_counters_get(const ps_track* h, ps_track_filter_counters* out);
+/* The file tool with filters (the aux arrays come from the batcher); the files do not depend on the window size nor on
+ * the number of devices.  filter == NULL: ps_track_bam_ex2.  filter_counters_out may be NULL. */
+int ps_track_bam_ex3(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                     const ps_track_indel_opts* indel_opts, const ps_track_filter_opts* filter,
+                     ps_track_counters* counters_out, ps_track_base_totals* totals_out,
+                     ps_track_indel_totals* indel_totals_out, ps_track_filter_counters* filter_counters_out,
+                     ps_fault* fault_out);
 
 /* ---- `comb` tool (host only): transcript hits lifted to genomic coordinates, merged with the genomic hits ---------------
  * Replaces CombineGenomeTranscript.combine / printReadsToBamFile (utils/postprocessing/CombineGenomeTranscript.java:36-666;
@@ -578,6 +632,11 @@ int ps_multi_track_bam_ex2(ps_multi* m, const char* bam_path, const char* out_pr
                            const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
                            ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out,
                            ps_fault* fault_out);
+int ps_multi_track_bam_ex3(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                           const ps_track_indel_opts* indel_opts, const ps_track_filter_opts* filter,
+                           ps_track_counters* counters_out, ps_track_base_totals* totals_out,
+                           ps_track_indel_totals* indel_totals_out, ps_track_filter_counters* filter_counters_out,
+                           ps_fault* fault_out);
 
 /* ---- host batcher (usable without a GPU) --------------------------------------------------------
  * What htsjdk does for the two loops, as a library: FASTA(+.fai) -> packed reference; BGZF/BAM -> SoA batches in
@@ -609,6 +668,9 @@ int ps_bam_open_ex(ps_bam** out, const char* bam_path, const ps_packed_fasta* re
 int64_t ps_bam_contig_order(const ps_bam* b, uint32_t* order, uint64_t max);
 /* 1: *batch filled (host pointers, valid until the third-next call); 0: end of file; < 0: status */
 int ps_bam_next(ps_bam* b, ps_read_batch* batch);
+/* The aux arrays (ps_read_aux) of the batch the last ps_bam_next returned: BAM FLAG and MAPQ fields, SAM columns 2 and
+ * 5.  Host pointers into that batch's allocation, valid as long as the batch. */
+int ps_bam_aux(ps_bam* b, ps_read_aux* out);
 const char* ps_bam_error(const ps_bam* b);
 void ps_bam_close(ps_bam* b);
 

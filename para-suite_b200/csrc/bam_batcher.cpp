@@ -5,6 +5,7 @@
 // loops then see SAMRecord objects in file order).  The record view presented to the kernels is the one SURVEY.md 8(b)
 // lists: POS+1 (0 when POS = -1), flags 0x4 / 0x10 / 0x400, cigar ops 0..8 = MIDNSHP=X, bases from 4-bit nibbles via
 // "=ACMGRSVTWYHKDBN" (only A, C, G, T are countable), raw phred bytes (first byte 0xFF = missing), header sort order.
+// Beside the batch, the whole 16-bit FLAG and the MAPQ of every record (ps_bam_aux: the track's read filters).
 //
 // BGZF blocks are independent deflate streams: the block table is scanned once (sequential, 18 bytes per block), the
 // blocks of a window are inflated by a pool of threads straight into their place of one contiguous buffer, records are
@@ -264,6 +265,7 @@ struct ps_bam {
   uint64_t ordinal = 0;
   std::string err;
   std::vector<uint64_t> rec_off;   // scratch: offsets of the records of the batch being built
+  ps_read_aux aux{};               // FLAG and MAPQ of the last batch (ps_bam_aux), in its slab
   // SAM text input (htsjdk opens SAM and BAM through one factory, ErrorProfiling.java:104-107): the text is turned into
   // the byte stream an inflated BAM would give -- header, then records in BAM encoding -- so everything behind
   // bam_fill is shared
@@ -416,6 +418,7 @@ static int sam_fill(ps_bam* B, size_t want) {
     put32(B->buf, at + 4, (uint32_t)ref_id);
     put32(B->buf, at + 8, (uint32_t)pos);
     d[12] = 2;                                                                   // l_read_name ("r\0": names are never read)
+    d[13] = (uint8_t)strtoul(std::string(f[4], fl[4]).c_str(), nullptr, 10);   // MAPQ
     const uint16_t ncg = (uint16_t)cig.size(), fl16 = (uint16_t)flag;
     memcpy(d + 16, &ncg, 2);
     memcpy(d + 18, &fl16, 2);
@@ -778,7 +781,8 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
   size_t off_qual = up(off_bases + bases_bytes + 64), off_cigar = up(off_qual + qual_bytes + 64);
   size_t off_exc = up(off_cigar + (cigar_count + 16) * 4), off_tb = up(off_exc + (exc_count + 16) * 4);
   size_t off_tq = up(off_tb + (n_tiles + 1) * 8), off_tc = up(off_tq + (n_tiles + 1) * 8), off_te = up(off_tc + (n_tiles + 1) * 8);
-  const size_t total = up(off_te + (n_tiles + 1) * 4);
+  const size_t off_sflag = up(off_te + (n_tiles + 1) * 4), off_mapq = up(off_sflag + n * 2);
+  const size_t total = up(off_mapq + n);
   Slab& S = B->slab[B->cur];
   B->cur = (B->cur + 1) % 3;
   if (!S.reserve(total)) return bam_fail(B, PS_ERR_OOM, "out of host memory for the batch");
@@ -788,6 +792,8 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
   uint8_t* qual = S.p + off_qual;
   uint32_t* cigar = (uint32_t*)(S.p + off_cigar);
   uint32_t* exc = (uint32_t*)(S.p + off_exc);
+  uint16_t* sam_flags = (uint16_t*)(S.p + off_sflag);
+  uint8_t* mapq = S.p + off_mapq;
   memcpy(S.p + off_tb, tb.data(), (n_tiles + 1) * 8);
   memcpy(S.p + off_tq, tq.data(), (n_tiles + 1) * 8);
   memcpy(S.p + off_tc, tc.data(), (n_tiles + 1) * 8);
@@ -861,6 +867,8 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
         }
         ref_start[r] = g32;
         meta[r] = PS_MAKE_META(l_seq, nc, fl);
+        sam_flags[r] = (uint16_t)flag;
+        mapq[r] = p[9];
         ob += (l_seq + 3) / 4; oq += l_seq; oc += nc;
       }
     }
@@ -891,8 +899,17 @@ int ps_bam_next(ps_bam* B, ps_read_batch* out) {
   out->start16 = nullptr;
   out->tile_start = nullptr;
   out->past_end = past_end.load() == UINT64_MAX ? 0 : past_end.load() + 1;
+  B->aux.sam_flags = sam_flags;
+  B->aux.mapq = mapq;
   B->ordinal += n;
   return 1;
+}
+
+int ps_bam_aux(ps_bam* B, ps_read_aux* out) {
+  if (!B || !out) return PS_ERR_INVALID_ARG;
+  if (!B->aux.sam_flags) return bam_fail(B, PS_ERR_STATE, "no batch returned yet");
+  *out = B->aux;
+  return PS_OK;
 }
 
 // ---- whole-tool entry points -------------------------------------------------------------------------------------

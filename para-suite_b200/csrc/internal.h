@@ -97,6 +97,7 @@ struct DevBuf {
 
 struct StagedBatch {   // device copy of a host batch
   DevBuf meta, ref_start, bases2, qual, cigar, tbo, tqo, tco, teo, exc, flags8, qual6, start16, tile_start;
+  DevBuf sam_flags, mapq;   // the track's read filters (track_stage_aux)
   DeviceBatch view{};
 };
 

@@ -58,14 +58,17 @@ static int multi_fail(ps_multi* m, int st, const std::string& msg) {
 namespace {
 
 // max over the kept records of a host batch of their pileup keys (what pl_maxkey_kernel computes); rank: the context's
-// contig order (ps_ctx::contig_rank)
-uint64_t host_max_key(const ps_read_batch& b, const std::vector<uint64_t>& contig_off, const std::vector<uint32_t>& rank) {
+// contig order (ps_ctx::contig_rank).  filter (the track's): records its record filter drops are not kept.
+uint64_t host_max_key(const ps_read_batch& b, const std::vector<uint64_t>& contig_off, const std::vector<uint32_t>& rank,
+                      const TrackFilter* filter = nullptr, const ps_read_aux* aux = nullptr) {
   uint64_t best = 0, coff = (!b.uniform_ncigar && b.tile_cigar_off) ? b.tile_cigar_off[0] : 0;
   size_t ci = 0;
   for (uint64_t r = 0; r < b.n_reads; ++r) {
     const uint32_t meta = b.meta[r], flags = PS_META_FLAGS(meta), ncig = PS_META_NCIGAR(meta);
     const uint32_t* cig = b.cigar + coff;
     coff += ncig;
+    if (filter && filter->records && track_filtered(*filter, aux->sam_flags ? aux->sam_flags[r] : 0u, aux->mapq ? aux->mapq[r] : 255u))
+      continue;
     if (flags & (PS_RF_UNMAPPED | PS_RF_POS_ZERO | PS_RF_CIGAR_OVERFLOW)) continue;
     const CigarShape<> s = cigar_shape(cig, ncig);
     if (s.skip) continue;
@@ -560,15 +563,16 @@ struct TrackFlight {
 };
 
 // The windowed track over an open file (contexts keyed in the file's contig order)
-int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, const TrackIndels& indels, TrackWriter& W,
-                      ps_track_counters* ctr, ps_track_base_totals* totals, ps_track_indel_totals* indel_totals,
-                      ps_fault* fault) {
+int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, const TrackIndels& indels,
+                      const TrackFilter& filter, TrackWriter& W, ps_track_counters* ctr, ps_track_base_totals* totals,
+                      ps_track_indel_totals* indel_totals, ps_track_filter_counters* fctr, ps_fault* fault) {
   ps_ctx* c0 = m->ctx[0];
   const std::vector<uint64_t>& contig_off = c0->contig_off;
   const std::vector<uint32_t>& by_rank = c0->contig_by_rank;
   memset(ctr, 0, sizeof *ctr);
   memset(totals, 0, sizeof *totals);
   memset(indel_totals, 0, sizeof *indel_totals);
+  memset(fctr, 0, sizeof *fctr);
   TrackPending P;
   P.bases = bases;
   P.indels = indels;
@@ -616,6 +620,9 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, const Tra
       indel_totals->inserted_bases[s] += o.indel_totals.inserted_bases[s];
       indel_totals->unanchored_insertions[s] += o.indel_totals.unanchored_insertions[s];
     }
+    fctr->filtered_flags += o.fctr.filtered_flags;
+    fctr->filtered_mapq += o.fctr.filtered_mapq;
+    for (int s = 0; s < 2; ++s) fctr->low_quality_bases[s] += o.fctr.low_quality_bases[s];
     if (!o.first_key) { print_window(o, 0); return PS_OK; }      // no kept record: nothing changes
     if (o.first_key < last_start) return multi_fail(m, PS_ERR_UNSORTED, ps_strerror(PS_ERR_UNSORTED));
     if (o.head.len) {
@@ -657,18 +664,22 @@ int track_windows_run(ps_multi* m, ps_bam* B, const TrackBases& bases, const Tra
     TrackFlight& prev = fl[(window & 1) ^ 1];
     if (prev.live && prev.ctx == c) { st = complete(prev); if (st) break; }
     cudaSetDevice(c->device);
+    ps_read_aux aux{}, dev{};
+    if (filter.records && (st = ps_bam_aux(B, &aux)) != PS_OK) { st = multi_fail(m, st, ps_bam_error(B)); break; }
     StagedBatch* sb = nullptr;
-    st = stage_batch(c, &hb, /*with_qual=*/false, &sb);     // the track reads no qualities
+    st = stage_batch(c, &hb, /*with_qual=*/filter.min_bq > 0, &sb);     // qualities only for the base filter
+    if (st == PS_OK) st = track_stage_aux(c, sb, hb.n_reads, &aux, filter, &dev);
     if (st != PS_OK) { sync_fail(m, c, st); break; }
     f.ctx = c; f.offset = offset; f.rc = PS_OK; f.live = true;
     const DeviceBatch view = sb->view;
     const uint64_t prev_end = max_end;
-    f.th = std::thread([&f, c, view, prev_end, &bases, &indels] {
+    f.th = std::thread([&f, c, view, prev_end, &bases, &indels, &filter, dev] {
       cudaSetDevice(c->device);
-      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out, bases, indels);
+      f.rc = track_run(c, view, c->stream, true, prev_end, &f.out, bases, indels, filter, dev);
       if (f.rc != PS_OK) f.err = c->err;
     });
-    max_end = std::max<unsigned long long>(max_end, host_max_key(hb, contig_off, c0->contig_rank));
+    // a record the filter drops reaches no window: it must not move the next window's prev_end either
+    max_end = std::max<unsigned long long>(max_end, host_max_key(hb, contig_off, c0->contig_rank, &filter, &aux));
     offset += hb.n_reads;
   }
   for (int i = 0; i < 2; ++i) {            // in file order; after an error only the threads are joined
@@ -968,15 +979,21 @@ int ps_clust_bam(ps_ctx* ctx, const char* bam_path, const char* out_path, const 
 
 // The track tool from files: <out_prefix>.plus.bedGraph, .minus.bedGraph, .t2c.tsv, with base counts .bases.tsv and with
 // indel counts .indels.tsv
-int ps_multi_track_bam_ex2(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
-                           const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
-                           ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out,
+int ps_multi_track_bam_ex3(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                           const ps_track_indel_opts* indel_opts, const ps_track_filter_opts* filter_opts,
+                           ps_track_counters* counters_out, ps_track_base_totals* totals_out,
+                           ps_track_indel_totals* indel_totals_out, ps_track_filter_counters* filter_counters_out,
                            ps_fault* fault_out) {
   if (!m || !bam_path || !out_prefix) return PS_ERR_INVALID_ARG;
   TrackBases bases;
   if (track_bases_of(opts, &bases) != PS_OK) return multi_fail(m, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
   TrackIndels indels;
   if (track_indels_of(indel_opts, &indels) != PS_OK) return multi_fail(m, PS_ERR_INVALID_ARG, "track: indel option reserved field is not 0");
+  TrackFilter filter;
+  const uint16_t any_flags = 0;
+  const uint8_t any_mapq = 0;
+  const ps_read_aux from_batcher{&any_flags, &any_mapq};   // the batcher always fills both
+  if (track_filter_of(filter_opts, &from_batcher, &filter) != PS_OK) return multi_fail(m, PS_ERR_INVALID_ARG, "track: invalid filter options");
   if (m->ctx.empty() || !m->ctx[0]->fasta) return multi_fail(m, PS_ERR_STATE, "load the reference first (ps_multi_load_fasta)");
   ps_ctx* c0 = m->ctx[0];
   TrackWriter W;
@@ -986,15 +1003,25 @@ int ps_multi_track_bam_ex2(ps_multi* m, const char* bam_path, const char* out_pr
   ps_track_counters ctr{};
   ps_track_base_totals totals{};
   ps_track_indel_totals indel_totals{};
+  ps_track_filter_counters fctr{};
   ps_fault fault{};
   st = with_file_order(m, bam_path, window_reads_default(), [&](ps_bam* B) {
-    return track_windows_run(m, B, bases, indels, W, &ctr, &totals, &indel_totals, &fault);
+    return track_windows_run(m, B, bases, indels, filter, W, &ctr, &totals, &indel_totals, &fctr, &fault);
   });
   if (counters_out) *counters_out = ctr;
   if (totals_out) *totals_out = totals;
   if (indel_totals_out) *indel_totals_out = indel_totals;
+  if (filter_counters_out) *filter_counters_out = fctr;
   if (fault_out) *fault_out = fault;
   return st;
+}
+
+int ps_multi_track_bam_ex2(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                           const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
+                           ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out,
+                           ps_fault* fault_out) {
+  return ps_multi_track_bam_ex3(m, bam_path, out_prefix, opts, indel_opts, nullptr, counters_out, totals_out,
+                                indel_totals_out, nullptr, fault_out);
 }
 
 int ps_multi_track_bam_ex(ps_multi* m, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
@@ -1007,16 +1034,25 @@ int ps_multi_track_bam(ps_multi* m, const char* bam_path, const char* out_prefix
   return ps_multi_track_bam_ex(m, bam_path, out_prefix, nullptr, counters_out, nullptr, fault_out);
 }
 
-int ps_track_bam_ex2(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
-                     const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
-                     ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out, ps_fault* fault_out) {
+int ps_track_bam_ex3(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                     const ps_track_indel_opts* indel_opts, const ps_track_filter_opts* filter,
+                     ps_track_counters* counters_out, ps_track_base_totals* totals_out,
+                     ps_track_indel_totals* indel_totals_out, ps_track_filter_counters* filter_counters_out,
+                     ps_fault* fault_out) {
   if (!ctx || !bam_path || !out_prefix) return set_error(ctx, PS_ERR_INVALID_ARG, "NULL argument");
   ps_multi m;
   borrow(m, ctx);
-  const int st = ps_multi_track_bam_ex2(&m, bam_path, out_prefix, opts, indel_opts, counters_out, totals_out,
-                                        indel_totals_out, fault_out);
+  const int st = ps_multi_track_bam_ex3(&m, bam_path, out_prefix, opts, indel_opts, filter, counters_out, totals_out,
+                                        indel_totals_out, filter_counters_out, fault_out);
   if (st != PS_OK && !m.err.empty()) set_error(ctx, st, m.err);
   return st;
+}
+
+int ps_track_bam_ex2(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,
+                     const ps_track_indel_opts* indel_opts, ps_track_counters* counters_out,
+                     ps_track_base_totals* totals_out, ps_track_indel_totals* indel_totals_out, ps_fault* fault_out) {
+  return ps_track_bam_ex3(ctx, bam_path, out_prefix, opts, indel_opts, nullptr, counters_out, totals_out,
+                          indel_totals_out, nullptr, fault_out);
 }
 
 int ps_track_bam_ex(ps_ctx* ctx, const char* bam_path, const char* out_prefix, const ps_track_opts* opts,

@@ -61,6 +61,8 @@ struct TrState {
   unsigned int unsorted;
   unsigned long long bases[2][4][5]; // base counts: [strand][ref][read A C G T N], strand orientation
   unsigned long long indel[10];      // indel counts: the ten per-strand totals of ps_track_indel_totals, in its order
+  unsigned long long filtered[2];    // filters: records dropped by a flag test, for their MAPQ
+  unsigned long long lowq[2];        // filters: aligned bases below min_base_quality by strand
 };
 
 struct TrParams {
@@ -83,6 +85,8 @@ struct TrParams {
   uint32_t* bc;                      // base counts: [2][5][M] events by read base A C G T N (strand orientation)
   int32_t* idel;                     // indel counts: [2][M + 1] deletion difference arrays, then (scan) deletions
   uint32_t* ins;                     // indel counts: [2][M] insertions by anchor
+  TrackFilter flt;                   // read and base filters
+  ps_read_aux aux;                   // device arrays of the record filter
 };
 
 struct MaxPair {
@@ -98,9 +102,12 @@ __device__ __forceinline__ unsigned long long warp_sum(unsigned long long v) {
 }
 
 // Filters and faults in pl_decode_generic's order (pl_key's for skipped_due_indel), without the 51-position limit.
+// RF: the record filter (track_filtered) comes before all of them; a filtered record keeps key 0.
+template <bool RF>
 __global__ void __launch_bounds__(TR_THREADS) tr_read_kernel(const __grid_constant__ TrParams P) {
   ContigCache cc;
   unsigned long long n_unm = 0, n_skip = 0, n_cnt = 0, al[2] = {0, 0}, nb[2] = {0, 0}, first = ~0ull;
+  unsigned long long n_flt[2] = {0, 0};
   const uint64_t n = P.b.n_reads;
   for (uint64_t q = ((uint64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31u)); q < n; q += (uint64_t)gridDim.x * blockDim.x) {
     const uint64_t r = q + (threadIdx.x & 31u);
@@ -112,6 +119,12 @@ __global__ void __launch_bounds__(TR_THREADS) tr_read_kernel(const __grid_consta
     const uint32_t flags = PS_META_FLAGS(meta), L = PS_META_LEN(meta), ncig = PS_META_NCIGAR(meta);
     const uint32_t* cig = P.b.cigar + off.cigar;
     do {
+      if constexpr (RF) {
+        const uint32_t sf = (P.flt.require | P.flt.exclude) ? __ldg(P.aux.sam_flags + r) : 0u;
+        const uint32_t mq = P.flt.min_mapq ? __ldg(P.aux.mapq + r) : 255u;
+        const int why = track_filtered(P.flt, sf, mq);
+        if (why) { ++n_flt[why - 1]; break; }
+      }
       if (flags & PS_RF_UNMAPPED) { ++n_unm; break; }
       if (flags & PS_RF_CIGAR_OVERFLOW) { raise_fault(&P.st->fault, r, PS_FAULT_CIGAR_OPS); break; }
       const CigarShape<> sh = cigar_shape(cig, ncig);
@@ -149,6 +162,13 @@ __global__ void __launch_bounds__(TR_THREADS) tr_read_kernel(const __grid_consta
     if (nb[0]) atomicAdd(&P.st->blocks[0], nb[0]);
     if (nb[1]) atomicAdd(&P.st->blocks[1], nb[1]);
     if (first != ~0ull) atomicMin(&P.st->first_key, first);
+  }
+  if constexpr (RF) {
+    n_flt[0] = warp_sum(n_flt[0]); n_flt[1] = warp_sum(n_flt[1]);
+    if ((threadIdx.x & 31u) == 0) {
+      if (n_flt[0]) atomicAdd(&P.st->filtered[0], n_flt[0]);
+      if (n_flt[1]) atomicAdd(&P.st->filtered[1], n_flt[1]);
+    }
   }
 }
 
@@ -214,9 +234,12 @@ __global__ void tr_seg_place_kernel(const __grid_constant__ TrParams P, uint32_t
 }
 
 // general path: one read, any CIGAR.  It walks its blocks itself: through for_each_block every tr_accum_kernel
-// instantiation takes 2-4 more registers, and the BC ones spill (nvcc 12.9, sm_100a)
+// instantiation takes 2-4 more registers, and the BC ones spill (nvcc 12.9, sm_100a).
+// BQ (base filter): `oq` is the read's quality offset; a base below min_base_quality counts in ev[2 + strand] only, and
+// each maximal run of them is a -1 / +1 hole in the block's coverage.  BQ = false takes no `oq`, so its call is as before.
+template <bool BQ, typename... Q>
 __device__ __noinline__ void tr_accum_generic(const TrParams& P, uint64_t r, uint32_t meta, uint64_t off_base,
-                                              uint64_t off_cigar, int64_t to_compact, unsigned long long* ev) {
+                                              uint64_t off_cigar, int64_t to_compact, unsigned long long* ev, Q... oq) {
   const uint32_t flags = PS_META_FLAGS(meta), ncig = PS_META_NCIGAR(meta);
   const uint32_t* cig = P.b.cigar + off_cigar;
   const bool rev = flags & PS_RF_REVERSE, has_inv = flags & PS_RF_HAS_INVALID;
@@ -239,15 +262,36 @@ __device__ __noinline__ void tr_accum_generic(const TrParams& P, uint64_t r, uin
         atomicAdd(diff + i0, 1);
         atomicAdd(diff + i0 + n, -1);
       }
-      for (int64_t z = 0; z < n; ++z) {
-        const uint64_t g = g0 + (uint64_t)(rfp + z);
-        const uint32_t p = (uint32_t)(rdp + z);
-        if (ref_invalid_at(P.ref, g)) continue;
-        const uint32_t a = ref_code_at(P.ref, g), bb = read_code_at(rb, p);
-        if (!(rev ? (a == 0u && bb == 2u) : (a == 3u && bb == 1u))) continue;
-        if (has_inv && read_pos_invalid(P.b, ex, p)) continue;
-        atomicAdd(t2c + ((int64_t)g + to_compact), 1u);
-        ++ev[s];
+      if constexpr (BQ) {
+        const uint8_t* qp = P.b.qual + (0 + ... + oq) + rdp;
+        const bool qmiss = flags & PS_RF_QUAL_MISSING;
+        const int64_t i0 = (int64_t)(g0 + (uint64_t)rfp) + to_compact;
+        int64_t lo = -1;                           // first base of the open low-quality run
+        for (int64_t z = 0; z <= n; ++z) {
+          const bool low = z < n && !qmiss && __ldg(qp + z) < P.flt.min_bq;
+          if (low) { if (lo < 0) lo = z; ++ev[2 + s]; continue; }
+          if (lo >= 0) { atomicAdd(diff + i0 + lo, -1); atomicAdd(diff + i0 + z, 1); lo = -1; }
+          if (z == n) break;
+          const uint64_t g = g0 + (uint64_t)(rfp + z);
+          const uint32_t p = (uint32_t)(rdp + z);
+          if (ref_invalid_at(P.ref, g)) continue;
+          const uint32_t a = ref_code_at(P.ref, g), bb = read_code_at(rb, p);
+          if (!(rev ? (a == 0u && bb == 2u) : (a == 3u && bb == 1u))) continue;
+          if (has_inv && read_pos_invalid(P.b, ex, p)) continue;
+          atomicAdd(t2c + ((int64_t)g + to_compact), 1u);
+          ++ev[s];
+        }
+      } else {
+        for (int64_t z = 0; z < n; ++z) {
+          const uint64_t g = g0 + (uint64_t)(rfp + z);
+          const uint32_t p = (uint32_t)(rdp + z);
+          if (ref_invalid_at(P.ref, g)) continue;
+          const uint32_t a = ref_code_at(P.ref, g), bb = read_code_at(rb, p);
+          if (!(rev ? (a == 0u && bb == 2u) : (a == 3u && bb == 1u))) continue;
+          if (has_inv && read_pos_invalid(P.b, ex, p)) continue;
+          atomicAdd(t2c + ((int64_t)g + to_compact), 1u);
+          ++ev[s];
+        }
       }
       rdp += n; rfp += n;
     }
@@ -255,9 +299,11 @@ __device__ __noinline__ void tr_accum_generic(const TrParams& P, uint64_t r, uin
 }
 
 // base counts of one read, any CIGAR: an event per read base other than the reference base and per N call into P.bc,
-// every counted base into the block's matrix `tb` ([2][4][5], shared)
+// every counted base into the block's matrix `tb` ([2][4][5], shared).  BQ: bases below min_base_quality are skipped
+// (`oq` as tr_accum_generic's)
+template <bool BQ, typename... Q>
 __device__ __noinline__ void tr_bases_generic(const TrParams& P, uint64_t r, uint32_t meta, uint64_t off_base,
-                                              uint64_t off_cigar, int64_t to_compact, unsigned long long* tb) {
+                                              uint64_t off_cigar, int64_t to_compact, unsigned long long* tb, Q... oq) {
   const uint32_t flags = PS_META_FLAGS(meta), ncig = PS_META_NCIGAR(meta);
   const uint32_t* cig = P.b.cigar + off_cigar;
   const bool rev = flags & PS_RF_REVERSE, has_inv = flags & PS_RF_HAS_INVALID;
@@ -273,6 +319,9 @@ __device__ __noinline__ void tr_bases_generic(const TrParams& P, uint64_t r, uin
     for (int64_t z = 0; z < n; ++z) {
       const uint64_t g = g0 + (uint64_t)(rfp + z);
       const uint32_t p = (uint32_t)(rdp + z);
+      if constexpr (BQ) {
+        if (!(flags & PS_RF_QUAL_MISSING) && __ldg(P.b.qual + (0 + ... + oq) + p) < P.flt.min_bq) continue;
+      }
       if (ref_invalid_at(P.ref, g)) continue;
       const uint32_t a = ref_code_at(P.ref, g) ^ flip;
       const uint32_t bb = (has_inv && read_pos_invalid(P.b, ex, p)) ? 4u : (read_code_at(rb, p) ^ flip);
@@ -331,11 +380,32 @@ __device__ __forceinline__ void tr_bases_fast(const TrParams& P, const uint32_t 
   }
 }
 
+// bits k < L of the qualities q[0..L) below min_bq: four bytes at a time (__vcmpltu4), each lane's top bit folded to one
+// bit per base; q need not be word-aligned (funnel shifts, as for the bases)
+template <int NW>
+__device__ __forceinline__ unsigned long long tr_low_quality(const uint8_t* q, uint32_t L, uint32_t min_bq) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(q);
+  const uint32_t* src = reinterpret_cast<const uint32_t*>(a & ~(uintptr_t)3);
+  const uint32_t sh = (uint32_t)(a & 3u) * 8u, qq = min_bq * 0x01010101u;
+  unsigned long long lq = 0;
+  uint32_t lo = __ldg(src);
+#pragma unroll
+  for (int j = 0; j < 4 * NW; ++j) {
+    const uint32_t hi = __ldg(src + j + 1), lt = __vcmpltu4(__funnelshift_r(lo, hi, sh), qq);
+    lq |= (unsigned long long)(((lt & 0x80808080u) * 0x00204081u) >> 28) << (4 * j);   // bits 7, 15, 23, 31 -> 28..31
+    lo = hi;
+  }
+  return lq & (L >= 64 ? ~0ull : ((1ull << L) - 1ull));
+}
+
 // NW > 0: the batch has uniform length L <= 64 and one cigar op per read; reads whose op is M/=/X of length L take the
-// bit-parallel path (t2c_word)
-template <int NW, bool BC>
-__global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_constant__ TrParams P) {
-  unsigned long long ev[2] = {0, 0}, fast = 0;
+// bit-parallel path (t2c_word).  BQ (base filter): the low-quality bases of a read leave its coverage (one -1 / +1 pair
+// per maximal run of them), its T>C events and its base counts, and count in ev[2 + strand].  BC with BQ asks for three
+// blocks an SM, which lets ptxas use 72-76 registers: at its own choice of 64, <2, true, true> spilled (nvcc 12.9); the
+// other instantiations carry no minimum, as before
+template <int NW, bool BC, bool BQ>
+__global__ void __launch_bounds__(TR_THREADS, (BC && BQ) ? 3 : 0) tr_accum_kernel(const __grid_constant__ TrParams P) {
+  unsigned long long ev[BQ ? 4 : 2] = {}, fast = 0;
   unsigned long long* tb = nullptr;
   if constexpr (BC) {
     __shared__ unsigned long long sh_bases[40];
@@ -348,13 +418,15 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
     const uint64_t r = q + (threadIdx.x & 31u);
     const bool in = r < n;
     const uint32_t meta = in ? __ldg(P.b.meta + r) : 0u;
-    uint64_t obase = 0, ocig = 0;
+    uint64_t obase = 0, ocig = 0, oqual = 0;
     if constexpr (NW == 0) {
       const ReadOffsets off = warp_read_offsets(P.b, q, r, in, meta);   // warp-collective
       obase = off.base; ocig = off.cigar;
+      if constexpr (BQ) oqual = off.qual;
     } else {
       obase = r * (uint64_t)((P.b.uniform_len + 3) >> 2);
       ocig = r;
+      if constexpr (BQ) oqual = r * (uint64_t)P.b.uniform_len;
     }
     if (!in) continue;
     const ulonglong2 k = P.keys[r];
@@ -367,6 +439,10 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
         const bool rev = PS_META_FLAGS(meta) & PS_RF_REVERSE;
         const int st = rev ? 1 : 0;
         const uint32_t g0 = __ldg(P.b.ref_start + r);
+        unsigned long long lq = 0;                   // BQ: low-quality bases, found before the base words are live
+        if constexpr (BQ) {
+          if (!(PS_META_FLAGS(meta) & PS_RF_QUAL_MISSING)) lq = tr_low_quality<NW>(P.b.qual + oqual, L, P.flt.min_bq);
+        }
         const uint32_t* src = reinterpret_cast<const uint32_t*>(P.b.bases2 + (obase & ~3ull));
         const uint32_t bsh = (uint32_t)(obase & 3u) * 8u;
         uint32_t bw[NW + 1], w[NW + 1];
@@ -377,6 +453,14 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
         const int64_t c0 = (int64_t)g0 + to_compact;
         atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0, 1);
         atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0 + L, -1);
+        if constexpr (BQ) {
+          for (unsigned long long a = lq & ~(lq << 1), e = lq & ~(lq >> 1); a; a &= a - 1, e &= e - 1) {
+            atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0 + (__ffsll((long long)a) - 1), -1);
+            atomicAdd(P.diff + (size_t)st * (P.M + 1) + c0 + __ffsll((long long)e), 1);
+          }
+          m &= ~lq;
+          ev[2 + st] += (unsigned long long)__popcll(lq);
+        }
         uint32_t* t2c = P.t2c + (size_t)st * P.M + c0;
         ev[st] += (unsigned long long)__popcll(m);
         while (m) {
@@ -384,19 +468,31 @@ __global__ void __launch_bounds__(TR_THREADS) tr_accum_kernel(const __grid_const
           m &= m - 1;
           atomicAdd(t2c + j, 1u);
         }
-        if constexpr (BC) tr_bases_fast<NW>(P, w, bw, (g0 & 15u) * 2u, bsh, tw.ref_n, L, meta, r, st, c0, tb);
+        if constexpr (BC) tr_bases_fast<NW>(P, w, bw, (g0 & 15u) * 2u, bsh, tw.ref_n | lq, L, meta, r, st, c0, tb);
         ++fast;
         continue;
       }
     }
-    tr_accum_generic(P, r, meta, obase, ocig, to_compact, ev);
-    if constexpr (BC) tr_bases_generic(P, r, meta, obase, ocig, to_compact, tb);
+    if constexpr (BQ) {
+      tr_accum_generic<true>(P, r, meta, obase, ocig, to_compact, ev, oqual);
+      if constexpr (BC) tr_bases_generic<true>(P, r, meta, obase, ocig, to_compact, tb, oqual);
+    } else {
+      tr_accum_generic<false>(P, r, meta, obase, ocig, to_compact, ev);
+      if constexpr (BC) tr_bases_generic<false>(P, r, meta, obase, ocig, to_compact, tb);
+    }
   }
   ev[0] = warp_sum(ev[0]); ev[1] = warp_sum(ev[1]); fast = warp_sum(fast);
   if ((threadIdx.x & 31u) == 0) {
     if (ev[0]) atomicAdd(&P.st->t2c[0], ev[0]);
     if (ev[1]) atomicAdd(&P.st->t2c[1], ev[1]);
     if (fast) atomicAdd(&P.st->fast, fast);
+  }
+  if constexpr (BQ) {
+    ev[2] = warp_sum(ev[2]); ev[3] = warp_sum(ev[3]);
+    if ((threadIdx.x & 31u) == 0) {
+      if (ev[2]) atomicAdd(&P.st->lowq[0], ev[2]);
+      if (ev[3]) atomicAdd(&P.st->lowq[1], ev[3]);
+    }
   }
   if constexpr (BC) {
     __syncthreads();
@@ -723,14 +819,60 @@ int track_indels_of(const ps_track_indel_opts* o, TrackIndels* out) {
   return PS_OK;
 }
 
+int track_filter_of(const ps_track_filter_opts* o, const ps_read_aux* aux, TrackFilter* out) {
+  *out = TrackFilter();
+  if (!o) return PS_OK;
+  for (uint32_t v : o->reserved)
+    if (v) return PS_ERR_INVALID_ARG;
+  if (o->min_mapq > 255 || o->min_base_quality > 255 || (o->require_flags | o->exclude_flags) >> 16) return PS_ERR_INVALID_ARG;
+  if ((o->require_flags | o->exclude_flags) && !(aux && aux->sam_flags)) return PS_ERR_INVALID_ARG;
+  if (o->min_mapq && !(aux && aux->mapq)) return PS_ERR_INVALID_ARG;
+  out->on = true;
+  out->records = o->min_mapq || o->require_flags || o->exclude_flags;
+  out->min_mapq = o->min_mapq;
+  out->require = o->require_flags;
+  out->exclude = o->exclude_flags;
+  out->min_bq = o->min_base_quality;
+  return PS_OK;
+}
+
+int track_stage_aux(ps_ctx* ctx, StagedBatch* sb, uint64_t n, const ps_read_aux* aux, const TrackFilter& filter,
+                    ps_read_aux* dev) {
+  *dev = ps_read_aux{};
+  if (!filter.records) return PS_OK;
+  if (filter.require | filter.exclude) {
+    PS_CUDA(ctx, sb->sam_flags.reserve(n * 2 + 64));
+    PS_CUDA(ctx, cudaMemcpyAsync(sb->sam_flags.p, aux->sam_flags, n * 2, cudaMemcpyHostToDevice, ctx->stream));
+    dev->sam_flags = static_cast<const uint16_t*>(sb->sam_flags.p);
+  }
+  if (filter.min_mapq) {
+    PS_CUDA(ctx, sb->mapq.reserve(n + 64));
+    PS_CUDA(ctx, cudaMemcpyAsync(sb->mapq.p, aux->mapq, n, cudaMemcpyHostToDevice, ctx->stream));
+    dev->mapq = static_cast<const uint8_t*>(sb->mapq.p);
+  }
+  return PS_OK;
+}
+
+// the accumulate kernel of a call: base counts (BC), base filter (BQ), bit-parallel words (nw, 0: general path)
+template <bool BC, bool BQ>
+void launch_accum(int nw, uint32_t grid, cudaStream_t st, const TrParams& P) {
+  switch (nw) {
+    case 1: tr_accum_kernel<1, BC, BQ><<<grid, TR_THREADS, 0, st>>>(P); break;
+    case 2: tr_accum_kernel<2, BC, BQ><<<grid, TR_THREADS, 0, st>>>(P); break;
+    case 3: tr_accum_kernel<3, BC, BQ><<<grid, TR_THREADS, 0, st>>>(P); break;
+    case 4: tr_accum_kernel<4, BC, BQ><<<grid, TR_THREADS, 0, st>>>(P); break;
+    default: tr_accum_kernel<0, BC, BQ><<<grid, TR_THREADS, 0, st>>>(P); break;
+  }
+}
+
 int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out,
-              const TrackBases& bases, const TrackIndels& indels) {
+              const TrackBases& bases, const TrackIndels& indels, const TrackFilter& filter, const ps_read_aux& aux) {
   if (b.past_end && b.past_end <= b.n_reads) {
     // a record past its contig's end: the reads before it decide whether an earlier record faults first
     DeviceBatch head = b;
     head.n_reads = b.past_end - 1;
     head.past_end = 0;
-    const int rc = track_run(ctx, head, st, windowed, prev_end, out, bases, indels);
+    const int rc = track_run(ctx, head, st, windowed, prev_end, out, bases, indels, filter, aux);
     if (rc != PS_OK && rc != PS_ERR_UNSORTED) return rc;
     out->base_rows.clear();                // a faulting call reports no base or indel rows
     out->totals = ps_track_base_totals{};
@@ -744,6 +886,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   *out = TrackOut();
   out->bases_on = bases.on;
   out->indels_on = indels.on;
+  out->filter_on = filter.on;
   const uint64_t n = b.n_reads;
   out->ctr.num_reads_processed = n;
   if (n == 0) return PS_OK;
@@ -752,6 +895,7 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   TrState* d_st = slot<TrState>(ctx, 0, 1, err);
   TrParams P{};
   P.b = b; P.ref = ctx->ref; P.st = d_st; P.prev_end = windowed ? prev_end : 0; P.windowed = windowed;
+  P.flt = filter; P.aux = aux;
   P.keys = slot<ulonglong2>(ctx, 1, n, err);
   P.scan = slot<ulonglong2>(ctx, 2, n, err);
   P.flag = slot<uint32_t>(ctx, 3, n, err);
@@ -761,7 +905,9 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   tr_init_state<<<1, 1, 0, st>>>(d_st);
   if (bases.on) TR_CUDA(cudaMemsetAsync(d_st->bases, 0, sizeof d_st->bases, st));
   if (indels.on) TR_CUDA(cudaMemsetAsync(d_st->indel, 0, sizeof d_st->indel, st));
-  tr_read_kernel<<<grid_g, TR_THREADS, 0, st>>>(P);
+  if (filter.on) TR_CUDA(cudaMemsetAsync(d_st->filtered, 0, sizeof d_st->filtered + sizeof d_st->lowq, st));
+  if (filter.records) tr_read_kernel<true><<<grid_g, TR_THREADS, 0, st>>>(P);
+  else tr_read_kernel<false><<<grid_g, TR_THREADS, 0, st>>>(P);
   TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceScan::InclusiveScan(t, sz, P.keys, P.scan, MaxPair(), (int64_t)n, st); }));
   tr_segment_kernel<<<grid_for(n), TR_THREADS, 0, st>>>(P);
   TR_CUDA(cub_call(ctx, [&](void* t, size_t& sz) { return cub::DeviceScan::InclusiveSum(t, sz, P.flag, P.flag, (int64_t)n, st); }));
@@ -778,6 +924,8 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   out->ctr.reads_counted = hh.s.counted;
   out->ctr.aligned_bases[0] = hh.s.aligned[0];
   out->ctr.aligned_bases[1] = hh.s.aligned[1];
+  out->fctr.filtered_flags = hh.s.filtered[0];
+  out->fctr.filtered_mapq = hh.s.filtered[1];
   if (hh.s.fault != PS_FAULT_NONE) {
     out->fault.code = (int32_t)(hh.s.fault & 0xFF);
     out->fault.read_ordinal = hh.s.fault >> 8;
@@ -837,22 +985,12 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   if (indels.on) TR_CUDA(cudaMemsetAsync(P.idel, 0, (4 * M + 2) * 4, st));
   const uint32_t L = b.uniform_len;
   const int nw = (L >= 1 && L <= 64 && b.uniform_ncigar == 1 && (reinterpret_cast<uintptr_t>(b.bases2) & 3u) == 0) ? (int)((L + 15) / 16) : 0;
-  if (!bases.on) {
-    switch (nw) {
-      case 1: tr_accum_kernel<1, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      case 2: tr_accum_kernel<2, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      case 3: tr_accum_kernel<3, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      case 4: tr_accum_kernel<4, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      default: tr_accum_kernel<0, false><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-    }
+  if (filter.min_bq) {
+    if (bases.on) launch_accum<true, true>(nw, grid_g, st, P);
+    else launch_accum<false, true>(nw, grid_g, st, P);
   } else {
-    switch (nw) {
-      case 1: tr_accum_kernel<1, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      case 2: tr_accum_kernel<2, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      case 3: tr_accum_kernel<3, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      case 4: tr_accum_kernel<4, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-      default: tr_accum_kernel<0, true><<<grid_g, TR_THREADS, 0, st>>>(P); break;
-    }
+    if (bases.on) launch_accum<true, false>(nw, grid_g, st, P);
+    else launch_accum<false, false>(nw, grid_g, st, P);
   }
   if (indels.on) tr_indel_kernel<<<grid_g, TR_THREADS, 0, st>>>(P);
   timer_end(ctx, st);
@@ -874,12 +1012,16 @@ int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed,
   TR_CUDA(cudaMemcpyAsync(tot + 1, &d_st->t2c[0], 16, cudaMemcpyDeviceToHost, st));
   if (bases.on) TR_CUDA(cudaMemcpyAsync(out->totals.bases, d_st->bases, sizeof out->totals.bases, cudaMemcpyDeviceToHost, st));
   if (indels.on) TR_CUDA(cudaMemcpyAsync(&out->indel_totals, d_st->indel, sizeof d_st->indel, cudaMemcpyDeviceToHost, st));
+  if (filter.min_bq) TR_CUDA(cudaMemcpyAsync(out->fctr.low_quality_bases, d_st->lowq, sizeof d_st->lowq, cudaMemcpyDeviceToHost, st));
   TR_CUDA(cudaStreamSynchronize(st));
   out->ctr.fast_path_reads = tot[0];
   out->ctr.t2c_events[0] = tot[1];
   out->ctr.t2c_events[1] = tot[2];
+  for (int s = 0; s < 2; ++s) out->ctr.aligned_bases[s] -= out->fctr.low_quality_bases[s];
   const uint64_t nr = hi - lo;
-  const uint64_t cap_r[2] = {std::min<uint64_t>(nr, 2 * hh.s.blocks[0] + 1), std::min<uint64_t>(nr, 2 * hh.s.blocks[1] + 1)};
+  // base filter: every low-quality run adds two edges inside a block, so the blocks bound nothing
+  const uint64_t cap_r[2] = {std::min<uint64_t>(nr, filter.min_bq ? nr : 2 * hh.s.blocks[0] + 1),
+                             std::min<uint64_t>(nr, filter.min_bq ? nr : 2 * hh.s.blocks[1] + 1)};
   const uint64_t cap_s = std::min<uint64_t>(2 * nr, tot[1] + tot[2]);
   // base-count candidates: at most one per min_ev events other than N calls
   uint64_t events = 0;
@@ -1017,9 +1159,9 @@ struct ps_track {
 
 // a handle is returned with PS_OK and with a fault (PS_ERR_REFERENCE_WOULD_THROW, PS_ERR_UNSUPPORTED): ps_track_fault
 static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const TrackBases& bases,
-                      const TrackIndels& indels, ps_track** out) {
+                      const TrackIndels& indels, const TrackFilter& filter, const ps_read_aux& aux, ps_track** out) {
   ps_track* h = new ps_track();
-  const int rc = track_run(ctx, v, st, false, 0, &h->out, bases, indels);
+  const int rc = track_run(ctx, v, st, false, 0, &h->out, bases, indels, filter, aux);
   if (rc == PS_OK || h->out.fault.code != 0) *out = h;
   else delete h;
   return rc;
@@ -1027,22 +1169,32 @@ static int track_call(ps_ctx* ctx, const DeviceBatch& v, cudaStream_t st, const 
 
 extern "C" {
 
-int ps_track_batch_device_ex2(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts,
-                              const ps_track_indel_opts* indel_opts, void* stream, ps_track** out) {
+int ps_track_batch_device_ex3(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts,
+                              const ps_track_indel_opts* indel_opts, const ps_read_aux* aux,
+                              const ps_track_filter_opts* filter_opts, void* stream, ps_track** out) {
   if (!ctx || !b || !out) return PS_ERR_INVALID_ARG;
   *out = nullptr;
   TrackBases bases;
   if (track_bases_of(opts, &bases) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
   TrackIndels indels;
   if (track_indels_of(indel_opts, &indels) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: indel option reserved field is not 0");
+  TrackFilter filter;
+  if (track_filter_of(filter_opts, aux, &filter) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: invalid filter options");
+  if (filter.min_bq && b->n_reads && !b->qual) return set_error(ctx, PS_ERR_INVALID_ARG, "track: the base filter needs the batch's qualities");
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-  // a batch in a staging slot of this context: the track reads no qualities, so the core of the upload suffices
+  // a batch in a staging slot of this context: without the base filter the track reads no qualities, so the core of
+  // the upload suffices
   for (int slot = 0; slot < 2; ++slot)
     if (st != ctx->stream && b->n_reads && b->meta == ctx->staged[slot].view.meta && ctx->staged_core[slot])
-      cudaStreamWaitEvent(st, ctx->staged_core[slot], 0);
-  return track_call(ctx, view_of(b), st, bases, indels, out);
+      cudaStreamWaitEvent(st, filter.min_bq ? ctx->staged_done[slot] : ctx->staged_core[slot], 0);
+  return track_call(ctx, view_of(b), st, bases, indels, filter, filter.records ? *aux : ps_read_aux{}, out);
+}
+
+int ps_track_batch_device_ex2(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts,
+                              const ps_track_indel_opts* indel_opts, void* stream, ps_track** out) {
+  return ps_track_batch_device_ex3(ctx, b, opts, indel_opts, nullptr, nullptr, stream, out);
 }
 
 int ps_track_batch_device_ex(ps_ctx* ctx, const ps_read_batch* b, const ps_track_opts* opts, void* stream, ps_track** out) {
@@ -1053,14 +1205,17 @@ int ps_track_batch_device(ps_ctx* ctx, const ps_read_batch* b, void* stream, ps_
   return ps_track_batch_device_ex(ctx, b, nullptr, stream, out);
 }
 
-int ps_track_batch_ex2(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts,
-                       const ps_track_indel_opts* indel_opts, ps_track** out) {
+int ps_track_batch_ex3(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts,
+                       const ps_track_indel_opts* indel_opts, const ps_read_aux* aux,
+                       const ps_track_filter_opts* filter_opts, ps_track** out) {
   if (!ctx || !hb || !out) return PS_ERR_INVALID_ARG;
   *out = nullptr;
   TrackBases bases;
   if (track_bases_of(opts, &bases) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: substitutions has bits above 15");
   TrackIndels indels;
   if (track_indels_of(indel_opts, &indels) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: indel option reserved field is not 0");
+  TrackFilter filter;
+  if (track_filter_of(filter_opts, aux, &filter) != PS_OK) return set_error(ctx, PS_ERR_INVALID_ARG, "track: invalid filter options");
   if (!ctx->ref_loaded) return set_error(ctx, PS_ERR_STATE, "no reference loaded");
   cudaSetDevice(ctx->device);
   if (hb->n_reads == 0) {
@@ -1068,12 +1223,21 @@ int ps_track_batch_ex2(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts
     (*out)->out.ctr.num_reads_processed = 0;
     (*out)->out.bases_on = bases.on;
     (*out)->out.indels_on = indels.on;
+    (*out)->out.filter_on = filter.on;
     return PS_OK;
   }
   StagedBatch* sb = nullptr;
-  const int rc = stage_batch(ctx, hb, /*with_qual=*/false, &sb);
+  int rc = stage_batch(ctx, hb, /*with_qual=*/filter.min_bq > 0, &sb);     // qualities only for the base filter
   if (rc) return rc;
-  return track_call(ctx, sb->view, ctx->stream, bases, indels, out);
+  ps_read_aux dev{};
+  rc = track_stage_aux(ctx, sb, hb->n_reads, aux, filter, &dev);
+  if (rc) return rc;
+  return track_call(ctx, sb->view, ctx->stream, bases, indels, filter, dev, out);
+}
+
+int ps_track_batch_ex2(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts,
+                       const ps_track_indel_opts* indel_opts, ps_track** out) {
+  return ps_track_batch_ex3(ctx, hb, opts, indel_opts, nullptr, nullptr, out);
 }
 
 int ps_track_batch_ex(ps_ctx* ctx, const ps_read_batch* hb, const ps_track_opts* opts, ps_track** out) {
@@ -1137,6 +1301,13 @@ int ps_track_indel_totals_get(const ps_track* h, ps_track_indel_totals* out) {
   if (!h || !out) return PS_ERR_INVALID_ARG;
   if (!h->out.indels_on) return PS_ERR_STATE;
   *out = h->out.indel_totals;
+  return PS_OK;
+}
+
+int ps_track_filter_counters_get(const ps_track* h, ps_track_filter_counters* out) {
+  if (!h || !out) return PS_ERR_INVALID_ARG;
+  if (!h->out.filter_on) return PS_ERR_STATE;
+  *out = h->out.fctr;
   return PS_OK;
 }
 

@@ -51,6 +51,20 @@ __host__ __device__ inline bool track_indel_row(const TrackIndels& sel, uint32_t
   return (uint64_t)del + ins >= sel.min_ev && (uint64_t)cov + del >= sel.min_depth;
 }
 
+// The read and base filters of a call (ps_track_filter_opts), validated: on == false is the unfiltered track.
+// records: a flag or MAPQ test is set (tr_read_kernel<true>); min_bq > 0: the base filter (tr_accum_kernel<.., true>).
+struct TrackFilter {
+  bool on = false, records = false;
+  uint32_t min_mapq = 0, require = 0, exclude = 0, min_bq = 0;
+};
+// ps_track_filter_opts -> TrackFilter; PS_ERR_INVALID_ARG as the header says (aux may be NULL)
+int track_filter_of(const ps_track_filter_opts* o, const ps_read_aux* aux, TrackFilter* out);
+// The record filter (device and host alike): 0 kept, 1 dropped by a flag test, 2 dropped for its MAPQ
+__host__ __device__ inline int track_filtered(const TrackFilter& f, uint32_t sam_flags, uint32_t mapq) {
+  if ((sam_flags & f.exclude) || (sam_flags & f.require) != f.require) return 1;
+  return mapq < f.min_mapq ? 2 : 0;
+}
+
 // One track call.  Runs and sites are final for the positions reported; keys as in TrackDense.
 struct TrackOut {
   std::vector<ps_track_run> runs[2];
@@ -65,6 +79,8 @@ struct TrackOut {
   bool indels_on = false;
   std::vector<ps_track_indel_row> indel_rows;
   ps_track_indel_totals indel_totals{};
+  bool filter_on = false;
+  ps_track_filter_counters fctr{};
 };
 
 // windowed == false: the batch is the whole input, every position is reported.
@@ -72,5 +88,10 @@ struct TrackOut {
 // 0 if none) come back dense in `head`, positions from the last kept start on dense in `tail`; the runs and sites cover
 // the positions in between.  Waits for the device.
 // `bases`, `indels`: the base-count and indel options (rows for the reported positions, totals over every kept read).
+// `filter`, `aux`: the read and base filters and the device aux arrays they read (b.qual for the base filter).
 int track_run(ps_ctx* ctx, const DeviceBatch& b, cudaStream_t st, bool windowed, uint64_t prev_end, TrackOut* out,
-              const TrackBases& bases = TrackBases(), const TrackIndels& indels = TrackIndels());
+              const TrackBases& bases = TrackBases(), const TrackIndels& indels = TrackIndels(),
+              const TrackFilter& filter = TrackFilter(), const ps_read_aux& aux = ps_read_aux{});
+// Copies the host aux arrays the filter reads into the staging slot `sb` (ctx->stream); *dev: their device pointers
+int track_stage_aux(ps_ctx* ctx, StagedBatch* sb, uint64_t n, const ps_read_aux* aux, const TrackFilter& filter,
+                    ps_read_aux* dev);

@@ -167,6 +167,23 @@ class ps_track_indel_totals(C.Structure):
         return {f: (list(getattr(self, f)) if f != "n_rows" else int(self.n_rows)) for f, _ in self._fields_}
 
 
+class ps_read_aux(C.Structure):
+    _fields_ = [("sam_flags", C.c_void_p), ("mapq", C.c_void_p)]
+
+
+class ps_track_filter_opts(C.Structure):
+    _fields_ = [("min_mapq", C.c_uint32), ("require_flags", C.c_uint32), ("exclude_flags", C.c_uint32),
+                ("min_base_quality", C.c_uint32), ("reserved", C.c_uint32 * 4)]
+
+
+class ps_track_filter_counters(C.Structure):
+    _fields_ = [("filtered_flags", C.c_uint64), ("filtered_mapq", C.c_uint64), ("low_quality_bases", C.c_uint64 * 2)]
+
+    def as_dict(self) -> dict:
+        return {"filtered_flags": int(self.filtered_flags), "filtered_mapq": int(self.filtered_mapq),
+                "low_quality_bases": list(self.low_quality_bases)}
+
+
 class ps_flush_totals(C.Structure):
     _fields_ = [("snp_hit", C.c_uint64), ("high_frequent_error", C.c_uint64), ("num_crosslinked_clusters", C.c_uint64),
                 ("num_allele_positions", C.c_uint64), ("allele_positions", C.c_uint64 * 51),
@@ -265,6 +282,7 @@ EXPORTS = {
     "ps_bam_open": (C.c_int, [C.POINTER(VP), C.c_char_p, VP, C.c_uint64, C.c_int]),
     "ps_bam_open_ex": (C.c_int, [C.POINTER(VP), C.c_char_p, VP, C.c_uint64, C.c_int, C.c_uint32]),
     "ps_bam_next": (C.c_int, [VP, C.POINTER(ps_read_batch)]),
+    "ps_bam_aux": (C.c_int, [VP, C.POINTER(ps_read_aux)]),
     "ps_bam_error": (C.c_char_p, [VP]),
     "ps_bam_contig_order": (C.c_int64, [VP, VP, C.c_uint64]),
     "ps_bam_close": (None, [VP]),
@@ -302,6 +320,22 @@ EXPORTS = {
     "ps_multi_track_bam_ex2": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts),
                                          C.POINTER(ps_track_indel_opts), C.POINTER(ps_track_counters),
                                          C.POINTER(ps_track_base_totals), C.POINTER(ps_track_indel_totals),
+                                         C.POINTER(ps_fault)]),
+    "ps_track_batch_ex3": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_track_opts),
+                                     C.POINTER(ps_track_indel_opts), C.POINTER(ps_read_aux),
+                                     C.POINTER(ps_track_filter_opts), C.POINTER(VP)]),
+    "ps_track_batch_device_ex3": (C.c_int, [VP, C.POINTER(ps_read_batch), C.POINTER(ps_track_opts),
+                                            C.POINTER(ps_track_indel_opts), C.POINTER(ps_read_aux),
+                                            C.POINTER(ps_track_filter_opts), VP, C.POINTER(VP)]),
+    "ps_track_filter_counters_get": (C.c_int, [VP, C.POINTER(ps_track_filter_counters)]),
+    "ps_track_bam_ex3": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts), C.POINTER(ps_track_indel_opts),
+                                   C.POINTER(ps_track_filter_opts), C.POINTER(ps_track_counters),
+                                   C.POINTER(ps_track_base_totals), C.POINTER(ps_track_indel_totals),
+                                   C.POINTER(ps_track_filter_counters), C.POINTER(ps_fault)]),
+    "ps_multi_track_bam_ex3": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_opts),
+                                         C.POINTER(ps_track_indel_opts), C.POINTER(ps_track_filter_opts),
+                                         C.POINTER(ps_track_counters), C.POINTER(ps_track_base_totals),
+                                         C.POINTER(ps_track_indel_totals), C.POINTER(ps_track_filter_counters),
                                          C.POINTER(ps_fault)]),
     "ps_track_close": (None, [VP]),
     "ps_track_bam": (C.c_int, [VP, C.c_char_p, C.c_char_p, C.POINTER(ps_track_counters), C.POINTER(ps_fault)]),

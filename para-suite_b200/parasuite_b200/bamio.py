@@ -64,6 +64,7 @@ def encode_bam_record(rec: Record, ref_ids: dict, name: bytes = b"r", mapq: int 
         nib = _NIB.get(chr(ch).upper(), 15)
         seq[k >> 1] |= nib << (4 if k % 2 == 0 else 0)
     qual = bytes(rec.qual) if len(rec.qual) == L else b"\xff" * L
+    mapq = mapq if rec.mapq is None else rec.mapq
     body = struct.pack("<iiBBHHHIiii", ref_id, pos, len(name) + 1, mapq, bin_, len(ops), rec.flag & 0xFFFF, L, -1, -1, 0)
     body += name + b"\0" + b"".join(struct.pack("<I", (n << 4) | op) for op, n in ops) + bytes(seq) + qual
     return struct.pack("<I", len(body)) + body
@@ -148,7 +149,8 @@ def write_sam(path: str, contigs: Sequence[Tuple[str, int]], records: Iterable[R
             missing = len(q) == 0 or q[0] == 0xFF
             qual = "*" if missing else "".join(chr(33 + (b & 0xFF)) if (b & 0xFF) + 33 < 127 else "~" for b in q)
             seq = r.seq.decode() if len(r.seq) else "*"
-            f.write("\t".join([f"r{k}", str(r.flag), r.rname, str(r.pos), "30", r.cigar if r.cigar else "*", "*", "0", "0", seq,
+            mapq = "30" if r.mapq is None else str(r.mapq)
+            f.write("\t".join([f"r{k}", str(r.flag), r.rname, str(r.pos), mapq, r.cigar if r.cigar else "*", "*", "0", "0", seq,
                                qual]) + "\n")
 
 
@@ -277,6 +279,10 @@ class BamBatcher:
         def arr(ptr, ctype, count):
             return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(ctype)), shape=(count,)).copy()
 
+        aux = abi.ps_read_aux()
+        st = self.lib.ps_bam_aux(self.h, C.byref(aux))
+        if st != abi.PS_OK:
+            raise abi.PsError(st, self.lib.ps_bam_error(self.h).decode())
         return ReadBatch(
             n, arr(s.meta, C.c_uint32, n), arr(s.ref_start, C.c_uint32, n), arr(s.bases2, C.c_uint8, s.bases_bytes + 64),
             arr(s.qual, C.c_uint8, s.qual_bytes + 64), arr(s.cigar, C.c_uint32, s.cigar_count + 16),
@@ -284,7 +290,8 @@ class BamBatcher:
             arr(s.tile_cigar_off, C.c_uint64, nt + 1), arr(s.tile_exc_off, C.c_uint32, nt + 1),
             arr(s.exc, C.c_uint32, s.exc_count + 16), uniform_len=int(s.uniform_len), uniform_ncigar=int(s.uniform_ncigar),
             bases_bytes=int(s.bases_bytes), qual_bytes=int(s.qual_bytes), cigar_count=int(s.cigar_count),
-            exc_count=int(s.exc_count), past_end=int(s.past_end))
+            exc_count=int(s.exc_count), past_end=int(s.past_end), sam_flags=arr(aux.sam_flags, C.c_uint16, n),
+            mapq=arr(aux.mapq, C.c_uint8, n))
 
     def close(self):
         if getattr(self, "h", None):

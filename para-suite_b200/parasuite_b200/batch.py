@@ -92,6 +92,7 @@ class Record:
     cigar: str          # SAM text, "*" when none
     seq: bytes          # ASCII
     qual: bytes         # raw phred bytes; b"" or first byte 0xFF = missing
+    mapq: Optional[int] = None   # MAPQ; None = 255 (unavailable), as the BAM writer stores it
 
 
 def parse_cigar(text: str) -> List[Tuple[int, int]]:
@@ -115,8 +116,11 @@ class ReadBatch:
 
     def __init__(self, n_reads, meta, ref_start, bases2, qual, cigar, tile_base_off, tile_qual_off, tile_cigar_off,
                  tile_exc_off, exc, uniform_len=0, uniform_ncigar=0, bases_bytes=None, qual_bytes=None,
-                 cigar_count=None, exc_count=None, past_end=0):
+                 cigar_count=None, exc_count=None, past_end=0, sam_flags=None, mapq=None):
         self.n_reads = int(n_reads)
+        # per record, for the track's read filters (ps_read_aux): the 16-bit FLAG (uint16) and MAPQ (uint8), or None
+        self.sam_flags = sam_flags
+        self.mapq = mapq
         self.past_end = int(past_end)      # 1 + ordinal of the first record past its contig's end (ps_read_batch.past_end)
         self.meta = meta
         self.ref_start = ref_start
@@ -156,6 +160,10 @@ class ReadBatch:
         s.past_end = self.past_end
         return s
 
+    def aux_struct(self) -> abi.ps_read_aux:
+        """ps_read_aux of the host arrays (NULL where absent)"""
+        return abi.ps_read_aux(_ptr(self.sam_flags), _ptr(self.mapq))
+
     def algorithmic_bytes(self, with_qual: bool = True) -> int:
         """SURVEY 8(d): ceil(L/4) + L + 4*n_cigar + 4 + 4 + ceil(R/4) summed over reads."""
         L = (self.meta & 0xFFFF).astype(np.int64)
@@ -183,6 +191,8 @@ class ReadBatch:
         past_end = 0
         meta = np.zeros(n, dtype=np.uint32)
         ref_start = np.zeros(n, dtype=np.uint32)
+        sam_flags = np.array([rec.flag & 0xFFFF for rec in records], dtype=np.uint16)
+        mapq = np.array([255 if rec.mapq is None else rec.mapq for rec in records], dtype=np.uint8)
         bases = bytearray()
         quals = bytearray()
         cig: List[int] = []
@@ -254,4 +264,4 @@ class ReadBatch:
         uc = ncigs.pop() if len(ncigs) == 1 else 0
         return cls(n, meta, ref_start, bases2, qual, cigar, tb, tq, tc, te, exc_a, uniform_len=ul, uniform_ncigar=uc,
                    bases_bytes=len(bases), qual_bytes=len(quals), cigar_count=len(cig), exc_count=len(exc),
-                   past_end=past_end)
+                   past_end=past_end, sam_flags=sam_flags, mapq=mapq)

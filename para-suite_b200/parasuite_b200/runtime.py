@@ -63,6 +63,21 @@ def track_indel_opts(indel_counts: bool, min_indel_depth: int, min_indel_events:
     return abi.ps_track_indel_opts(1, int(min_indel_depth), int(min_indel_events), 0)
 
 
+def track_filter_opts(min_mapq: int, require_flags: int, exclude_flags: int,
+                      min_base_quality: int) -> Optional[abi.ps_track_filter_opts]:
+    """The ps_track_filter_opts of the filter keywords of Context.track, or None when all four are 0 (no filter)"""
+    vals = (int(min_mapq), int(require_flags), int(exclude_flags), int(min_base_quality))
+    if not any(vals):
+        return None
+    if not 0 <= vals[0] <= 255:
+        raise ValueError("min_mapq must be in 0..255")
+    if not 0 <= vals[3] <= 255:
+        raise ValueError("min_base_quality must be in 0..255")
+    if not (0 <= vals[1] <= 0xFFFF and 0 <= vals[2] <= 0xFFFF):
+        raise ValueError("require_flags and exclude_flags must be 16-bit flag masks")
+    return abi.ps_track_filter_opts(*vals)
+
+
 def _base_totals_dict(tot) -> dict:
     return {"base_totals": np.array(tot.bases, dtype=np.uint64).reshape(2, 4, 5), "n_base_rows": int(tot.n_rows)}
 
@@ -87,6 +102,13 @@ class DeviceBatch:
             setattr(s, f, None if self._t[f] is None else self._t[f].data_ptr())
         self.struct = s
         self.nbytes = sum(t.numel() for t in self._t.values() if t is not None)
+        # the aux arrays of the track's read filters, when the host batch has them
+        aux = {}
+        for f in ("sam_flags", "mapq"):
+            a = getattr(host, f, None)
+            aux[f] = None if a is None else torch.from_numpy(np.ascontiguousarray(a).view(np.uint8)).to(device)
+        self._aux = aux
+        self.aux = abi.ps_read_aux(*(None if aux[f] is None else aux[f].data_ptr() for f in ("sam_flags", "mapq")))
 
 
 class UploadedBatch:
@@ -108,6 +130,7 @@ class PinnedBatch:
         less); the upload expands all three on the device."""
         import torch
         self.n_reads = host.n_reads
+        self.host = host             # the aux arrays of the track's read filters stay on the host
         self._t = {}
         s = host.as_struct()
         n = host.n_reads
@@ -275,24 +298,36 @@ class Context:
 
     def track_bam(self, bam_path: str, out_prefix: str, *, base_counts: bool = False, min_coverage: int = 1,
                   min_events: int = 1, substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1,
-                  min_indel_events: int = 1) -> dict:
+                  min_indel_events: int = 1, min_mapq: int = 0, require_flags: int = 0, exclude_flags: int = 0,
+                  min_base_quality: int = 0) -> dict:
         """The `track` tool from files: writes <out_prefix>.plus.bedGraph, <out_prefix>.minus.bedGraph and
         <out_prefix>.t2c.tsv (per-position coverage and T>C events by strand); returns the run's counters.
         base_counts: also <out_prefix>.bases.tsv (keywords as Context.track), and the counters gain "base_totals"
         ((2, 4, 5) uint64: strand, reference base, read base A C G T N) and "n_base_rows".
-        indel_counts: also <out_prefix>.indels.tsv (keywords as Context.track), and the counters gain "indel_totals"."""
+        indel_counts: also <out_prefix>.indels.tsv (keywords as Context.track), and the counters gain "indel_totals".
+        min_mapq, require_flags, exclude_flags, min_base_quality: the read and base filters of Context.track; with any
+        of them set the counters gain "filter_counters"."""
         opts = track_opts(base_counts, min_coverage, min_events, substitutions)
         iopts = track_indel_opts(indel_counts, min_indel_depth, min_indel_events)
+        fopts = track_filter_opts(min_mapq, require_flags, exclude_flags, min_base_quality)
         ctr, f, tot, itot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals(), abi.ps_track_indel_totals()
-        st = self.lib.ps_track_bam_ex2(self.h, bam_path.encode(), out_prefix.encode(), C.byref(opts) if opts else None,
-                                       C.byref(iopts) if iopts else None, C.byref(ctr), C.byref(tot), C.byref(itot),
-                                       C.byref(f))
+        fctr = abi.ps_track_filter_counters()
+        if fopts is None:
+            st = self.lib.ps_track_bam_ex2(self.h, bam_path.encode(), out_prefix.encode(), C.byref(opts) if opts else None,
+                                           C.byref(iopts) if iopts else None, C.byref(ctr), C.byref(tot), C.byref(itot),
+                                           C.byref(f))
+        else:
+            st = self.lib.ps_track_bam_ex3(self.h, bam_path.encode(), out_prefix.encode(), C.byref(opts) if opts else None,
+                                           C.byref(iopts) if iopts else None, C.byref(fopts), C.byref(ctr), C.byref(tot),
+                                           C.byref(itot), C.byref(fctr), C.byref(f))
         _check(self.lib, self.h, st, fault=(f.code, f.read_ordinal))
         out = ctr.as_dict()
         if opts:
             out.update(_base_totals_dict(tot))
         if iopts:
             out["indel_totals"] = itot.as_dict()
+        if fopts is not None:
+            out["filter_counters"] = fctr.as_dict()
         return out
 
     # ---- batches ---------------------------------------------------------------------------------
@@ -471,7 +506,8 @@ class Context:
 
     # ---- T>C conversion and coverage track ---------------------------------------------------------
     def track(self, batch, stream: int = 0, *, base_counts: bool = False, min_coverage: int = 1, min_events: int = 1,
-              substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1, min_indel_events: int = 1) -> dict:
+              substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1, min_indel_events: int = 1,
+              min_mapq: int = 0, require_flags: int = 0, exclude_flags: int = 0, min_base_quality: int = 0) -> dict:
         """Per-position coverage and T>C events by strand of one whole input: {"runs_plus", "runs_minus", "sites",
         "counters"}, runs and sites as numpy structured arrays (abi.TRACK_RUN_DTYPE / TRACK_SITE_DTYPE, contigs as FASTA
         indices).  batch: host (ReadBatch / PinnedBatch) or device-resident (DeviceBatch / UploadedBatch).
@@ -482,16 +518,43 @@ class Context:
         indel_counts: also "indel_rows" (abi.TRACK_INDEL_ROW_DTYPE: deletions over and insertions anchored at each
         position by strand) for the positions with deletions + insertions >= min_indel_events and coverage + deletions
         >= min_indel_depth, and "indel_totals" (abi.ps_track_indel_totals as a dict of [plus, minus] lists and
-        "n_rows")."""
+        "n_rows").
+        Read and base filters (all off at 0; samtools view -q / -f / -F, mpileup -Q): records with MAPQ < min_mapq, or
+        whose FLAG lacks a bit of require_flags or has one of exclude_flags, are left out; aligned bases with quality
+        < min_base_quality count nowhere but in "filter_counters" ("filtered_flags", "filtered_mapq",
+        "low_quality_bases" [plus, minus]), which the result gains when any filter is set.  The record filter reads
+        the batch's FLAG and MAPQ arrays (ReadBatch.sam_flags / mapq: from_records fills them, DeviceBatch uploads
+        them; PinnedBatch and UploadedBatch take them from the host batch they came from)."""
         opts = track_opts(base_counts, min_coverage, min_events, substitutions)
         iopts = track_indel_opts(indel_counts, min_indel_depth, min_indel_events)
+        fopts = track_filter_opts(min_mapq, require_flags, exclude_flags, min_base_quality)
         po, pi = C.byref(opts) if opts else None, C.byref(iopts) if iopts else None
         h = C.c_void_p()
-        if isinstance(batch, (DeviceBatch, UploadedBatch)):
-            st = self.lib.ps_track_batch_device_ex2(self.h, C.byref(batch.struct), po, pi, stream or None, C.byref(h))
+        if fopts is None:
+            if isinstance(batch, (DeviceBatch, UploadedBatch)):
+                st = self.lib.ps_track_batch_device_ex2(self.h, C.byref(batch.struct), po, pi, stream or None, C.byref(h))
+            else:
+                s = batch.struct if hasattr(batch, "struct") else batch.as_struct()
+                st = self.lib.ps_track_batch_ex2(self.h, C.byref(s), po, pi, C.byref(h))
+        elif isinstance(batch, DeviceBatch):
+            st = self.lib.ps_track_batch_device_ex3(self.h, C.byref(batch.struct), po, pi, C.byref(batch.aux),
+                                                    C.byref(fopts), stream or None, C.byref(h))
+        elif isinstance(batch, UploadedBatch):
+            # the upload holds no aux arrays: device copies of the host batch's, kept alive for the call
+            import torch
+            src = getattr(batch._source, "host", batch._source)
+            keep = [None if getattr(src, f, None) is None else
+                    torch.from_numpy(np.ascontiguousarray(getattr(src, f)).view(np.uint8)).to(f"cuda:{self.device}")
+                    for f in ("sam_flags", "mapq")]
+            aux = abi.ps_read_aux(*(None if t is None else t.data_ptr() for t in keep))
+            torch.cuda.synchronize(self.device)
+            st = self.lib.ps_track_batch_device_ex3(self.h, C.byref(batch.struct), po, pi, C.byref(aux), C.byref(fopts),
+                                                    stream or None, C.byref(h))
         else:
             s = batch.struct if hasattr(batch, "struct") else batch.as_struct()
-            st = self.lib.ps_track_batch_ex2(self.h, C.byref(s), po, pi, C.byref(h))
+            host = getattr(batch, "host", batch)
+            aux = host.aux_struct() if hasattr(host, "aux_struct") else abi.ps_read_aux()
+            st = self.lib.ps_track_batch_ex3(self.h, C.byref(s), po, pi, C.byref(aux), C.byref(fopts), C.byref(h))
         try:
             if st != abi.PS_OK:
                 fault = None
@@ -531,6 +594,10 @@ class Context:
                     self.lib.ps_track_indel_rows(h, 0, rows.ctypes.data, rows.size)
                 out["indel_rows"] = rows
                 out["indel_totals"] = itot.as_dict()
+            if fopts is not None:
+                fctr = abi.ps_track_filter_counters()
+                _check(self.lib, self.h, self.lib.ps_track_filter_counters_get(h, C.byref(fctr)))
+                out["filter_counters"] = fctr.as_dict()
             return out
         finally:
             if h:
@@ -720,20 +787,31 @@ class MultiContext:
 
     def track_bam(self, bam_path: str, out_prefix: str, *, base_counts: bool = False, min_coverage: int = 1,
                   min_events: int = 1, substitutions=None, indel_counts: bool = False, min_indel_depth: int = 1,
-                  min_indel_events: int = 1) -> dict:
+                  min_indel_events: int = 1, min_mapq: int = 0, require_flags: int = 0, exclude_flags: int = 0,
+                  min_base_quality: int = 0) -> dict:
         """Context.track_bam with windows round-robin over the devices; the files are byte-identical."""
         opts = track_opts(base_counts, min_coverage, min_events, substitutions)
         iopts = track_indel_opts(indel_counts, min_indel_depth, min_indel_events)
+        fopts = track_filter_opts(min_mapq, require_flags, exclude_flags, min_base_quality)
         ctr, f, tot, itot = abi.ps_track_counters(), abi.ps_fault(), abi.ps_track_base_totals(), abi.ps_track_indel_totals()
-        st = self.lib.ps_multi_track_bam_ex2(self.h, bam_path.encode(), out_prefix.encode(),
-                                             C.byref(opts) if opts else None, C.byref(iopts) if iopts else None,
-                                             C.byref(ctr), C.byref(tot), C.byref(itot), C.byref(f))
+        fctr = abi.ps_track_filter_counters()
+        if fopts is None:
+            st = self.lib.ps_multi_track_bam_ex2(self.h, bam_path.encode(), out_prefix.encode(),
+                                                 C.byref(opts) if opts else None, C.byref(iopts) if iopts else None,
+                                                 C.byref(ctr), C.byref(tot), C.byref(itot), C.byref(f))
+        else:
+            st = self.lib.ps_multi_track_bam_ex3(self.h, bam_path.encode(), out_prefix.encode(),
+                                                 C.byref(opts) if opts else None, C.byref(iopts) if iopts else None,
+                                                 C.byref(fopts), C.byref(ctr), C.byref(tot), C.byref(itot),
+                                                 C.byref(fctr), C.byref(f))
         self._check(st, fault=(f.code, f.read_ordinal))
         out = ctr.as_dict()
         if opts:
             out.update(_base_totals_dict(tot))
         if iopts:
             out["indel_totals"] = itot.as_dict()
+        if fopts is not None:
+            out["filter_counters"] = fctr.as_dict()
         return out
 
     def close(self):

@@ -3,6 +3,7 @@
   python tools/bench_track.py [--steps 20] [--warmup 3] [--bam-reads 300000] [--bam-copies 40] [--out FILE]
   python tools/bench_track.py --base-counts [--steps 20] [--warmup 3] [--out FILE]
   python tools/bench_track.py --indels [--steps 20] [--warmup 3] [--indel-reads 4000000] [--parent-lib SO] [--out FILE]
+  python tools/bench_track.py --filters [--steps 20] [--warmup 3] [--filter-reads 4000000] [--parent-lib SO] [--out FILE]
 
 1. Config 2 as bench.py builds it (10 M x 36-nt reads through synth.py against a 100 Mb reference), resident in HBM:
    `--steps` timed passes of ps_track_batch_device after `--warmup` passes, with the five stage times of every pass from
@@ -26,6 +27,12 @@ of each.  --parent-lib: a build of the library from before the option (ABI 6); i
 the same device-resident batch, so the plain call of both builds is timed in one run.  The five stage times of every
 call, the scratch the compact arrays take, the row counts and the parity of the indel call with the C++ restatement
 (tests/track_indels_oracle.py) go to profiles/track_bench_indels.json (or --out).
+
+--filters measures the read and base filters: on config 2 (10 M x 36-nt reads, the bit-parallel path) and config 5
+(--filter-reads x 150-nt reads with indels, the per-base path), resident in HBM with numpy-drawn FLAG, MAPQ and
+qualities, the plain call and the filtered call (MAPQ >= 10, -F 0x904, Q >= 20) alternate, with the parent build's plain
+call (--parent-lib) in the same alternation.  Per-stage medians, the filter counters and the parity of the filtered call
+with the C++ restatement (tests/track_filters_oracle.py) go to profiles/track_bench_filters.json (or --out).
 """
 import argparse
 import json
@@ -53,6 +60,8 @@ ap.add_argument("--base-counts", action="store_true")
 ap.add_argument("--indels", action="store_true")
 ap.add_argument("--indel-reads", type=int, default=4_000_000)
 ap.add_argument("--parent-lib", default=None)
+ap.add_argument("--filters", action="store_true")
+ap.add_argument("--filter-reads", type=int, default=4_000_000)
 args = ap.parse_args()
 
 import torch  # noqa: E402
@@ -185,7 +194,9 @@ class ParentTrack:
     """The plain track call of another build of the library, on a context of its own (same device, same process)."""
 
     def __init__(self, path):
-        self.lib = C.CDLL(os.path.abspath(path))
+        # RTLD_DEEPBIND: the build's calls between its own functions (track_run, timer_begin, ...) bind to its own
+        # definitions, not to those of the library loaded before it with RTLD_GLOBAL, whose ps_ctx layout may differ
+        self.lib = C.CDLL(os.path.abspath(path), mode=os.RTLD_LOCAL | os.RTLD_DEEPBIND)
         for name in ("ps_create", "ps_destroy", "ps_last_error", "ps_reference_upload", "ps_track_batch_device",
                      "ps_track_counters_get", "ps_track_close", "ps_kernel_times", "ps_kernel_times_reset"):
             f = getattr(self.lib, name)
@@ -300,8 +311,105 @@ def indels_run():
     ctx.close()
 
 
+def filters_run():
+    """plain and filtered calls alternately on config 2 and config 5 (and the parent build's plain call)"""
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+    import track_filters_oracle  # noqa: E402
+    fo = abi.ps_track_filter_opts(10, 0, 0x904, 20)
+    parent = ParentTrack(args.parent_lib) if args.parent_lib else None
+    if parent:
+        out["parent_lib_abi_version"] = parent.version
+    out["filter"] = {"min_mapq": 10, "exclude_flags": 0x904, "min_base_quality": 20}
+
+    def once(filtered, dbatch):
+        h = C.c_void_p()
+        if filtered:
+            st = lib.ps_track_batch_device_ex3(ctx.h, C.byref(dbatch.struct), None, None, C.byref(dbatch.aux),
+                                               C.byref(fo), None, C.byref(h))
+        else:
+            st = lib.ps_track_batch_device_ex2(ctx.h, C.byref(dbatch.struct), None, None, None, C.byref(h))
+        assert st == abi.PS_OK, lib.ps_last_error(ctx.h)
+        ctr, fc = abi.ps_track_counters(), abi.ps_track_filter_counters()
+        lib.ps_track_counters_get(h, C.byref(ctr))
+        if filtered:
+            lib.ps_track_filter_counters_get(h, C.byref(fc))
+        lib.ps_track_close(h)
+        return ctr, fc
+
+    rng = np.random.default_rng(0x5EED0004)
+    parity = True
+    for name, n, L, mode in (("config2", 10_000_000, 36, 0), ("config5", args.filter_reads, 150, 1)):
+        b = synth.synth_reads(ref, n, L, seed=0x5EED0002, mode=mode)
+        # FLAG: 10 % secondary, 2 % supplementary, 1 % QC-fail, 5 % duplicate besides the strand; MAPQ: 8 % below 10;
+        # qualities uniform in 2..40 (about half of them below 20)
+        rev = ((np.asarray(b.meta[:n]) >> np.uint32(24)) & abi.PS_RF_REVERSE) != 0
+        extra = rng.choice(np.array([0x100, 0x800, 0x200, 0x400, 0], dtype=np.uint16), size=n,
+                           p=[0.10, 0.02, 0.01, 0.05, 0.82])
+        b.sam_flags = (np.where(rev, 0x10, 0) | extra).astype(np.uint16)
+        b.mapq = rng.choice(np.array([0, 3, 30, 60], dtype=np.uint8), size=n, p=[0.05, 0.03, 0.22, 0.70])
+        b.qual = np.asarray(b.qual).copy()
+        b.qual[:b.qual_bytes] = rng.integers(2, 41, size=b.qual_bytes, dtype=np.uint8)
+        d = DeviceBatch(b, "cuda:0")
+        arms = {"plain": lambda: once(False, d), "filtered": lambda: once(True, d)}
+        if parent:
+            arms["parent_plain"] = lambda: (parent.once(d), None)
+        for _ in range(args.warmup):
+            for f in arms.values():
+                f()
+        res = {k: {"walls": [], "stages": []} for k in arms}
+        for _ in range(args.steps):
+            for k, f in arms.items():
+                if k == "parent_plain":
+                    parent.lib.ps_kernel_times_reset(parent.h, 1)
+                else:
+                    ctx.kernel_times_reset(True)
+                t0 = time.perf_counter()
+                ctr, fc = f()
+                res[k]["walls"].append(time.perf_counter() - t0)
+                res[k]["stages"].append(parent.stages() if k == "parent_plain" else
+                                        ctx.kernel_times_ms().reshape(-1, len(STAGES))[-1])
+                res[k]["ctr"], res[k]["fc"] = ctr, fc
+        o = {"reads": b.n_reads, "read_len": L, "synth_mode": mode, "steps": args.steps, "warmup": args.warmup,
+             "order": " / ".join(arms) + " calls alternate"}
+        for k in arms:
+            st = np.array(res[k]["stages"])
+            c = res[k]["ctr"]
+            o[k] = {"wall_ms_median": 1e3 * float(np.median(res[k]["walls"])),
+                    "device_ms_median": float(np.median(st.sum(axis=1))),
+                    "stage_ms_median": {s: float(np.median(st[:, i])) for i, s in enumerate(STAGES)},
+                    "stage_ms_min": {s: float(np.min(st[:, i])) for i, s in enumerate(STAGES)},
+                    "runs": [int(c.n_runs[0]), int(c.n_runs[1])], "sites": int(c.n_sites),
+                    "reads_counted": int(c.reads_counted), "fast_path_reads": int(c.fast_path_reads)}
+        o["filtered"]["filter_counters"] = res["filtered"]["fc"].as_dict()
+        got = ctx.track(d, **out["filter"])
+        exp = track_filters_oracle.track_cpp(ref, b, **out["filter"])
+        same = bool(got["filter_counters"] == exp["filter_counters"] and got["counters"]["aligned_bases"] ==
+                    exp["counters"]["aligned_bases"] and all(np.array_equal(got[k], exp[k])
+                                                             for k in ("runs_plus", "runs_minus", "sites")))
+        o["parity_with_restatement"] = same
+        if parent:
+            o["parent_plain_same_counters"] = res["parent_plain"]["ctr"].as_dict() == res["plain"]["ctr"].as_dict()
+            same = same and o["parent_plain_same_counters"]
+        parity = parity and same
+        out[name + "_filters"] = o
+        print(json.dumps(o, indent=1), flush=True)
+        del d, got, exp
+    out["parity_with_restatement"] = parity
+    print(json.dumps(out, indent=1))
+    path = args.out or os.path.join(REPO, "profiles", "track_bench_filters.json")
+    os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+    with open(path, "w") as f:
+        json.dump(out, f, indent=1)
+    if parent:
+        parent.close()
+    ctx.close()
+
+
 if args.base_counts:
     base_counts_run()
+    sys.exit(0)
+if args.filters:
+    filters_run()
     sys.exit(0)
 if args.indels:
     indels_run()
